@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the MENT-Flow hot path on B200 (see DESIGN.md "Measurement").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 One *step* = one pass of the hot path over one batch of particles on every rank:
@@ -12,6 +12,10 @@ config C3: 6D, K=100 random 1-D projections, 64 bins, `--particles` (default 1e6
 Prints ONE JSON line (rank 0).  `value` = particles/s over all ranks with the base-noise z
 already resident in HBM, timed with CUDA events (max over ranks); `e2e` = the same through the
 public API with z arriving from pinned host memory and the loss read back every step.
+
+`--dump-outputs DIR` writes what the last step of `value`'s timed loop returned -- loss.npy,
+entropy.npy and discrepancies.npy (one per projection) -- so that two builds run with the same
+arguments (hence the same seeded weights, measurements and base noise) can be compared.
 """
 import argparse
 import json
@@ -21,6 +25,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -47,7 +52,14 @@ def parse():
     ap.add_argument("--host-chunks", type=int, default=3, help="pieces the pinned-host input is copied in (e2e leg)")
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel eagerly instead of replaying a CUDA graph")
     ap.add_argument("--no-extra", action="store_true", help="skip the secondary configurations (C1, C3/25, C4, training steps)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss, entropy and discrepancies of the last timed step as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs records the CUDA path (--impl b200)")
+    return args
 
 
 def peaks():
@@ -530,7 +542,7 @@ def main():
             L, H, D = model.loss_from_particles(x, logq)
             if timers:
                 timers[2].record()
-        return L
+        return L, H, D
 
     params = list(model.parameters())
 
@@ -561,8 +573,9 @@ def main():
         graphed = GraphedLoss(model, n, warmup=2, host_chunks=args.host_chunks)
 
     def run_step(z):
+        """(L, H, [D_k]) of one step"""
         if graphed is not None:
-            return graphed(z)[0]
+            return graphed(z)
         if z is None:
             z = gen.sample_base(n)
         return step(z)
@@ -599,12 +612,20 @@ def main():
         flush.zero_()                      # evict L2 between timed iterations (outside the [e0, e1] bracket)
         e0, e1 = ev(), ev()
         e0.record()
-        L = run_step(None)                 # the base noise is drawn on the device inside the step (Philox)
+        L, H, D = run_step(None)           # the base noise is drawn on the device inside the step (Philox)
         e1.record()
         marks.append((e0, e1))
         losses.append(L.clone())
     barrier()
     total_ms = sum(a.elapsed_time(b) for a, b in marks)
+    if args.dump_outputs and rank == 0:
+        # a graph replay returns its static output tensors: save them before the next leg replays the graph
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        outputs = {"loss": L, "entropy": torch.as_tensor(H), "discrepancies": torch.stack(D)}
+        for name, t in outputs.items():
+            t = t.detach().cpu()
+            np.save(os.path.join(args.dump_outputs, name + ".npy"),
+                    t.numpy().astype(np.float64 if t.dtype == torch.float64 else np.float32))
     # ---- end to end through the public API: model.loss(batch_size) as GraphedLoss(model, n)() -------
     # The step's only host-side inputs are the batch size (a constant of the captured graph) and the state
     # of torch's random generator.  Every step re-seeds the generator the way a reproducible training loop
@@ -615,7 +636,7 @@ def main():
         if graphed is not None:
             L = graphed(None)[0]
         else:
-            L = step(gen.sample_base(n))
+            L = step(gen.sample_base(n))[0]
         return float(L.item())
 
     e2e_s = 0.0
@@ -636,10 +657,10 @@ def main():
         torch.cuda.synchronize()
         t0 = time.perf_counter()
         if graphed is not None:
-            L = run_step(z_host)           # pinned host -> device copy, then the replay
+            L = run_step(z_host)[0]        # pinned host -> device copy, then the replay
         else:
             z_in.copy_(z_host, non_blocking=True)
-            L = step(z_in)
+            L = step(z_in)[0]
         lval = float(L.item())
         if it < 0:
             continue
