@@ -356,6 +356,10 @@ int mfb_selftest_umma_ts(const float* a, const float* b, int n, float* d, int* e
  * of a 64-wide SWIZZLE_128B tile (the layouts the flow kernel mixes).  n = 64 or 128.        */
 int mfb_selftest_umma_sw32(const float* a, const float* b, int n, int mode, int kstep, float* d, int* err,
                            void* stream);
+/* The 2-SM MMA of a CTA pair (cluster of 2, cta_group::2): d[256][64] = a[256][K] * b[64][K]^T (values rounded to
+ * fp16), each CTA holding 128 rows of a and 32 rows of b.  mode 0: K = 16, SWIZZLE_32B tiles; mode 1: K = 64,
+ * SWIZZLE_128B tiles.  err: 1 / 2 = the completion / request mbarrier timed out.                            */
+int mfb_selftest_umma_pair(const float* a, const float* b, int mode, float* d, int* err, void* stream);
 
 #ifdef __cplusplus
 }

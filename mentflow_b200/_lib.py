@@ -76,6 +76,7 @@ SIGNATURES = {
     "mfb_selftest_umma": (c_int, [P, P, c_int, P, P, P]),
     "mfb_selftest_umma_ts": (c_int, [P, P, c_int, P, P, P]),
     "mfb_selftest_umma_sw32": (c_int, [P, P, c_int, c_int, c_int, P, P, P]),
+    "mfb_selftest_umma_pair": (c_int, [P, P, c_int, P, P, P]),
     "mfb_nsf_pack_params": (c_int, [P, P, P, P, P, P, P, P, P, c_int, c_int, c_int, c_int, c_int, P, P, P]),
     "mfb_nsf_unpack_grads": (c_int, [P, P, P, P, c_int, c_int, c_int, c_int, c_int, P, P, P, P, P, P, P]),
     "mfb_moments_workspace_bytes": (c_int64, [c_int64, c_int]),

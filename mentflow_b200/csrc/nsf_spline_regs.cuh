@@ -145,16 +145,26 @@ MFB_HD void two_sum(float a, float b, float& s, float& err) {
 // 1e-4 of float64: 1.0-1.2x torch-fp32's, was 4x).  MFB_SPLINE_COMP additionally carries the group
 // prefixes as (hi, lo) pairs (0.3-0.9x torch-fp32's).
 // Multiplies jac by dy/dv (1 outside [-B, B]) and returns y.
-template <int NB>
-MFB_HD float rq_spline_regs(const float (&a)[64], float v, float& jac) {
+//
+// The raw parameters come in two pieces through load(col, float (&dst)[N]) = columns [col, col + N): the NB
+// widths first, then the NB heights and NB - 1 derivatives (plus one padding column) once the widths are reduced
+// to the few values the search keeps.  The flow kernel reads them from tensor memory that way, so that at most
+// 2 NB of the 64 accumulator columns are live in registers; the loader sees the second piece last and may
+// release the accumulator after it.
+template <int NB, class Load>
+MFB_HD float rq_spline_regs_ld(Load&& load, float v, float& jac) {
   static_assert(NB % 4 == 0 && NB >= 8, "bins are searched in groups of four");
   constexpr int G = NB / 4;
   constexpr float cW = kClipW / kLog2e, cD = kClipD / kLog2e;
   // ---- widths: e_j, sums of the groups of four and their prefixes P_g (short dependency chains)
   float e[NB], pre[G + 1], plo[G + 1];
+  {
+    float aw[NB];
+    load(0, aw);
 #pragma unroll
-  for (int j = 0; j < NB; j += 4) {
-    clip_exp2_quad(a[j], a[j + 1], a[j + 2], a[j + 3], cW, e[j], e[j + 1], e[j + 2], e[j + 3]);
+    for (int j = 0; j < NB; j += 4) {
+      clip_exp2_quad(aw[j], aw[j + 1], aw[j + 2], aw[j + 3], cW, e[j], e[j + 1], e[j + 2], e[j + 3]);
+    }
   }
   pre[0] = 0.f;
   plo[0] = 0.f;
@@ -197,12 +207,14 @@ MFB_HD float rq_spline_regs(const float (&a)[64], float v, float& jac) {
   const bool r0 = q0 < rem, r1 = i1 < rem, r2 = i2 < rem;
   const float numer = rem - (r2 ? i2 : (r1 ? i1 : (r0 ? q0 : 0.f)));
   const float ek = r2 ? q3 : (r1 ? q2 : (r0 ? q1 : q0));
+  float a[2 * NB];   // a[j] = raw parameter NB + j: heights, then derivatives
+  load(NB, a);
   // ---- heights, one group at a time
   float run = 0.f, runl = 0.f, yg = 0.f, ygl = 0.f, h0s = 0.f, h1s = 0.f, h2s = 0.f, h3s = 0.f;
 #pragma unroll
   for (int g = 0; g < G; ++g) {
     float h0, h1, h2, h3;
-    clip_exp2_quad(a[NB + 4 * g], a[NB + 4 * g + 1], a[NB + 4 * g + 2], a[NB + 4 * g + 3], cW, h0, h1, h2, h3);
+    clip_exp2_quad(a[4 * g], a[4 * g + 1], a[4 * g + 2], a[4 * g + 3], cW, h0, h1, h2, h3);
     const bool take = g == 0 ? true : pg[g > 0 ? g - 1 : 0];
     h0s = take ? h0 : h0s;
     h1s = take ? h1 : h1s;
@@ -231,8 +243,8 @@ MFB_HD float rq_spline_regs(const float (&a)[64], float v, float& jac) {
   float um = 0.f, u0 = 0.f, u1 = 0.f, u2 = 0.f, u3 = 0.f, prev = 0.f;
 #pragma unroll
   for (int g = 0; g < G; ++g) {
-    const float t0 = a[2 * NB + 4 * g], t1 = a[2 * NB + 4 * g + 1], t2 = a[2 * NB + 4 * g + 2];
-    const float t3 = (4 * g + 3 < NB - 1) ? a[2 * NB + 4 * g + 3] : 0.f;
+    const float t0 = a[NB + 4 * g], t1 = a[NB + 4 * g + 1], t2 = a[NB + 4 * g + 2];
+    const float t3 = (4 * g + 3 < NB - 1) ? a[NB + 4 * g + 3] : 0.f;
     const bool take = g == 0 ? true : pg[g > 0 ? g - 1 : 0];
     um = take ? prev : um;
     u0 = take ? t0 : u0;
@@ -260,6 +272,15 @@ MFB_HD float rq_spline_regs(const float (&a)[64], float v, float& jac) {
   const bool inside = (v > -kBound) && (v <= kBound);
   jac *= inside ? j1 : 1.0f;
   return inside ? y : v;
+}
+// ... from all raw parameters at once
+template <int NB>
+MFB_HD float rq_spline_regs(const float (&a)[64], float v, float& jac) {
+  return rq_spline_regs_ld<NB>(
+      [&](int col, auto& dst) {
+        for (int j = 0; j < (int)(sizeof(dst) / sizeof(dst[0])); ++j) dst[j] = a[col + j];
+      },
+      v, jac);
 }
 
 // soft clip + exp of four parameters like clip_exp2_quad; additionally returns 1 / (1 + c |t_j|) in place

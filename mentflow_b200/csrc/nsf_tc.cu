@@ -307,21 +307,27 @@ __device__ __forceinline__ void store_hidden(const float (&acc)[64], unsigned ch
 #ifndef MFB_TC_TS
 #define MFB_TC_TS 1
 #endif
-__device__ __forceinline__ void store_hidden_ts(const float (&acc)[64], uint32_t tmem_a_hi, unsigned char* a_lo, int row) {
+// The forward variant converts its accumulator in two pieces of 32 columns (chunks 4 piece .. 4 piece + 3 of the
+// row), so that only half of it is live in registers; kTS: the hi half goes to tensor memory (the caller waits for
+// the tcgen05.st after the last piece).
+template <bool kTS>
+__device__ __forceinline__ void store_hidden_piece(const float (&acc)[32], int piece, uint32_t tmem_a_hi,
+                                                   unsigned char* a_hi, unsigned char* a_lo, int row) {
 #pragma unroll
-  for (int c2 = 0; c2 < 4; ++c2) {   // two 16-byte chunks = eight packed columns at a time: few registers in flight
+  for (int c2 = 0; c2 < 2; ++c2) {   // two 16-byte chunks = eight packed columns at a time: few registers in flight
     uint32_t hi[8];
 #pragma unroll
     for (int h = 0; h < 2; ++h) {
-      const int c = 2 * c2 + h;
+      const int cl = 2 * c2 + h, c = 4 * piece + cl;
       uint32_t lo[4];
 #pragma unroll
-      for (int e = 0; e < 4; ++e) split_relu_pair(acc[8 * c + 2 * e], acc[8 * c + 2 * e + 1], hi[4 * h + e], lo[e]);
+      for (int e = 0; e < 4; ++e) split_relu_pair(acc[8 * cl + 2 * e], acc[8 * cl + 2 * e + 1], hi[4 * h + e], lo[e]);
       *reinterpret_cast<uint4*>(a_lo + umma::sw128_offset(row, c)) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+      if constexpr (!kTS)
+        *reinterpret_cast<uint4*>(a_hi + umma::sw128_offset(row, c)) = make_uint4(hi[4 * h], hi[4 * h + 1], hi[4 * h + 2], hi[4 * h + 3]);
     }
-    umma::tmem_st8(tmem_a_hi + 8 * c2, hi);
+    if constexpr (kTS) umma::tmem_st8(tmem_a_hi + 8 * (2 * piece + c2), hi);
   }
-  umma::tmem_wait_st();
 }
 
 // Backward variant: the rows a warp has just written to the A tile (32 rows x 128 B = 4 KB of the hi plane and 4 KB
@@ -599,12 +605,21 @@ nsf_tc_layer_kernel(const float* __restrict__ v, int64_t n, const unsigned char*
   // GEMM (l < L-1) or the first two output-layer tiles (l == L-1)
   auto hidden_step = [&](int l) {
     wait_buf(kHB);
-    float acc[64];
-    tmem_ld64(col0 + (uint32_t)(kHB * 64) + lane_sel, acc);
-    if constexpr (kBwd) mirror_wait();
     // biases are already in the accumulator (bias MMA)
-    if constexpr (kTS) store_hidden_ts(acc, ta_hi + lane_sel, a_lo, t);
-    else store_hidden(acc, a_hi, a_lo, t);
+    float acc[kBwd ? 64 : 1];
+    if constexpr (kBwd) {
+      tmem_ld64(col0 + (uint32_t)(kHB * 64) + lane_sel, acc);
+      mirror_wait();
+      store_hidden(acc, a_hi, a_lo, t);
+    } else {
+#pragma unroll
+      for (int piece = 0; piece < 2; ++piece) {
+        float part[32];
+        tmem_ld_cols(col0 + (uint32_t)(kHB * 64 + 32 * piece) + lane_sel, part);
+        store_hidden_piece<kTS>(part, piece, ta_hi + lane_sel, a_hi, a_lo, t);
+      }
+      if constexpr (kTS) umma::tmem_wait_st();
+    }
     fence_proxy_async();
     umma::fence_before_sync();
     request_arrive(req_chain);
@@ -674,7 +689,7 @@ nsf_tc_layer_kernel(const float* __restrict__ v, int64_t n, const unsigned char*
     float lq_in = 0.f;       // loaded a tile's worth of work before it is needed
     if (!kBwd && cur && valid && logq_out && !first_layer) lq_in = logq_in[p];
     // backward variant: upstream gradients of this particle, running maximum of |dL/dphi|
-    float gyr[D], glq = 0.f, amax = 0.f;
+    float gyr[D] = {}, glq = 0.f, amax = 0.f;
     if constexpr (kBwd) {
 #pragma unroll
       for (int i = 0; i < D; ++i) gyr[i] = valid ? bio.gy[p * D + i] : 0.f;
@@ -711,26 +726,8 @@ nsf_tc_layer_kernel(const float* __restrict__ v, int64_t n, const unsigned char*
 #pragma unroll 1
     for (int s = kBwd ? -1 : 0; s < S; ++s) {
       const int b = s & 1;
-      float acc[64];
-      if (kBwd && s < 0) {
-        if (cur) {
-          const float4* cb = reinterpret_cast<const float4*>(ctab + kConstRows * kCT);
-#pragma unroll
-          for (int i = 0; i < 16; ++i) {
-            const float4 q4 = cb[i];
-            acc[4 * i] = q4.x; acc[4 * i + 1] = q4.y; acc[4 * i + 2] = q4.z; acc[4 * i + 3] = q4.w;
-          }
-        }
-      } else if (cur) {
-        if (!(S >= 2 && s == S - 1)) wait_buf(b);   // the last slot was already waited for at kFork
-        tmem_ld64(col0 + (uint32_t)(b * 64) + lane_sel, acc);
-        umma::fence_before_sync();
-        if (s + 2 < S) request_arrive(req_chain + 1 + b);
-        // slot 0 is complete => every warp is past its last read of the other staging buffer
-        if (s == 0 && t == 0 && has_next) prefetch(tile + tstride, nbuf);
-        TRACE(10 + s);
-      }
-      if (s == kFork) {
+      // after slot kFork's accumulator has been read: the chain of the next tile may start (it runs in that buffer)
+      auto fork = [&]() {
         if (cur && S >= 2) wait_buf((S - 1) & 1);   // every output-layer MMA of this tile is done: A is free
         if (has_next) {
           if (nbuf == 0) {
@@ -741,17 +738,55 @@ nsf_tc_layer_kernel(const float* __restrict__ v, int64_t n, const unsigned char*
             sph1 ^= 1;
           }
         }
-      }
-      if (cur) {
-        const int f = (kBwd && s < 0) ? meta.const_feature : meta.slot_feature[s < 0 ? 0 : s];
-        if constexpr (kBwd) {
-          feature_bwd(acc, f);
-        } else {
-          const float vf = sc[f];
-          ss = fmaf(vf, vf, ss);
-          sc[f] = rq_spline_regs<NB>(acc, vf, jac);
+      };
+      // the last slot was already waited for at kFork; slot 0 is complete => every warp is past its last read of
+      // the other staging buffer
+      auto slot_ready = [&]() {
+        if (!(S >= 2 && s == S - 1)) wait_buf(b);
+        if (s == 0 && t == 0 && has_next) prefetch(tile + tstride, nbuf);
+      };
+      if constexpr (kBwd) {
+        float acc[64];
+        if (s < 0) {
+          if (cur) {
+            const float4* cb = reinterpret_cast<const float4*>(ctab + kConstRows * kCT);
+#pragma unroll
+            for (int i = 0; i < 16; ++i) {
+              const float4 q4 = cb[i];
+              acc[4 * i] = q4.x; acc[4 * i + 1] = q4.y; acc[4 * i + 2] = q4.z; acc[4 * i + 3] = q4.w;
+            }
+          }
+        } else if (cur) {
+          slot_ready();
+          tmem_ld64(col0 + (uint32_t)(b * 64) + lane_sel, acc);
+          umma::fence_before_sync();
+          if (s + 2 < S) request_arrive(req_chain + 1 + b);
+          TRACE(10 + s);
         }
+        if (s == kFork) fork();
+        if (cur) {
+          feature_bwd(acc, s < 0 ? meta.const_feature : meta.slot_feature[s < 0 ? 0 : s]);
+          TRACE(20 + s);
+        }
+      } else if (cur) {
+        // the spline reads the accumulator in two pieces; after the second the buffer is released
+        slot_ready();
+        const int f = meta.slot_feature[s];
+        const float vf = sc[f];
+        ss = fmaf(vf, vf, ss);
+        sc[f] = rq_spline_regs_ld<NB>(
+            [&](int col, auto& dst) {
+              tmem_ld_cols(col0 + (uint32_t)(b * 64 + col) + lane_sel, dst);
+              if (col == 0) return;
+              umma::fence_before_sync();
+              if (s + 2 < S) request_arrive(req_chain + 1 + b);
+              TRACE(10 + s);
+              if (s == kFork) fork();
+            },
+            vf, jac);
         TRACE(20 + s);
+      } else if (s == kFork) {
+        fork();
       }
       if (has_next) {
         if (s == kFork) hidden_step(0);

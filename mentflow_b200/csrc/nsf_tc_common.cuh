@@ -116,6 +116,57 @@ __device__ __forceinline__ void tmem_ld64(uint32_t taddr, float (&v)[64]) {
   for (int i = 0; i < 64; ++i) v[i] = __uint_as_float(r[i]);
 }
 
+// N (a multiple of 4) consecutive columns of this thread's TMEM lane with ONE wait: the spline and the hidden
+// steps read their accumulator in pieces, so that no more of it is live in registers than the step works on.
+template <int W>
+__device__ __forceinline__ void tmem_ld_issue(uint32_t taddr, uint32_t* r) {
+  static_assert(W == 4 || W == 8 || W == 16 || W == 32, "tcgen05.ld widths used here");
+  if constexpr (W == 4) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];"
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
+                 : "r"(taddr)
+                 : "memory");
+  } else if constexpr (W == 8) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
+                 : "r"(taddr)
+                 : "memory");
+  } else if constexpr (W == 16) {
+    asm volatile(
+        "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
+        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
+        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
+          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+        : "r"(taddr)
+        : "memory");
+  } else {
+    asm volatile(
+        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
+        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
+        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
+        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
+          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
+          "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
+          "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
+        : "r"(taddr)
+        : "memory");
+  }
+}
+template <int N>
+__device__ __forceinline__ void tmem_ld_cols(uint32_t taddr, float (&v)[N]) {
+  static_assert(N % 4 == 0 && N <= 64, "pieces of 4 to 64 columns");
+  uint32_t r[N];
+  int c = 0;
+#pragma unroll
+  for (; c + 32 <= N; c += 32) tmem_ld_issue<32>(taddr + c, r + c);
+  if constexpr ((N & 16) != 0) { tmem_ld_issue<16>(taddr + c, r + c); c += 16; }
+  if constexpr ((N & 8) != 0) { tmem_ld_issue<8>(taddr + c, r + c); c += 8; }
+  if constexpr ((N & 4) != 0) { tmem_ld_issue<4>(taddr + c, r + c); }
+  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+  for (int i = 0; i < N; ++i) v[i] = __uint_as_float(r[i]);
+}
+
 // Split MMAs of one K step.  The cross terms (hi*lo + lo*hi, 2^-11 of the result) of ALL K steps
 // are accumulated first, the hi*hi terms last: the tensor core rounds the fp32 accumulator once per
 // MMA, so only the last few MMAs round at the full magnitude of the result.

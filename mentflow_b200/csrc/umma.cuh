@@ -115,6 +115,72 @@ __device__ __forceinline__ void tmem_dealloc(uint32_t addr, uint32_t cols) {
   asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(addr), "r"(cols) : "memory");
 }
 
+// ---- CTA pairs (cta_group::2): one MMA of M = 256 over the tensor cores of two SMs of a cluster.  Each CTA of the
+// pair holds its 128 rows of A and HALF of B (rows [N/2 r, N/2 r + N/2) for cluster rank r) at the same shared-memory
+// offsets; D row 128 r + m lands in TMEM lane m of CTA r.  As in CUTLASS's 2-SM kernels, the even CTA issues the MMAs
+// and commits, one warp of EACH CTA (the same warp index) allocates and frees the columns, and both CTAs stay
+// resident until the last MMA of the pair has completed.
+__device__ __forceinline__ uint32_t cluster_rank() {
+  uint32_t r;
+  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+  return r;
+}
+// all threads of both CTAs; orders the shared-memory writes (mbarrier init included) before it cluster-wide
+__device__ __forceinline__ void cluster_sync() {
+  asm volatile("barrier.cluster.arrive.release.aligned;\nbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+// address of the same shared-memory object in the CTA of cluster rank `rank`
+__device__ __forceinline__ uint32_t cluster_addr(const void* p, uint32_t rank) {
+  uint32_t a;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(a) : "r"(smem_u32(p)), "r"(rank));
+  return a;
+}
+// arrive on an mbarrier of any CTA of the cluster (address from cluster_addr); releases this thread's prior writes
+__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_bar) {
+  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_bar) : "memory");
+}
+// wait side of such arrivals: acquires what the arriving threads of either CTA released
+__device__ __forceinline__ bool mbar_try_wait_cluster(uint64_t* bar, uint32_t parity) {
+  uint32_t ok;
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n"
+      "selp.u32 %0, 1, 0, p;\n"
+      "}\n"
+      : "=r"(ok)
+      : "r"(smem_u32(bar)), "r"(parity)
+      : "memory");
+  return ok != 0;
+}
+__device__ __forceinline__ void mma_f16_ss_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
+                                                uint32_t accumulate) {
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      "setp.ne.b32 p, %4, 0;\n"
+      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n"
+      "}\n" ::"r"(tmem_d),
+      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+// completion of the pair's MMAs arrives on the mbarrier at this offset in both CTAs
+__device__ __forceinline__ void commit_pair(uint64_t* bar) {
+  asm volatile(
+      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
+          smem_u32(bar)),
+      "h"((uint16_t)3)
+      : "memory");
+}
+__device__ __forceinline__ void tmem_alloc_pair(uint32_t* dst, uint32_t cols) {
+  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst)), "r"(cols)
+               : "memory");
+  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void tmem_dealloc_pair(uint32_t addr, uint32_t cols) {
+  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(addr), "r"(cols) : "memory");
+}
+
 // warp-collective: this thread's TMEM lane (= accumulator row), 32 consecutive fp32 columns
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
   uint32_t r[32];

@@ -235,7 +235,108 @@ umma_selftest_ts_kernel(const float* __restrict__ A, const float* __restrict__ B
   if (tid < 32) umma::tmem_dealloc(tbase, 256);
 }
 
+// Fourth self-test: the 2-SM MMA of a CTA pair (cluster of 2, cta_group::2), as the pair kernel of the flow layer
+// issues it: D[256 x 64] = A[256 x K] * B[64 x K]^T, CTA r holding rows [128 r, 128 r + 128) of A and rows
+// [32 r, 32 r + 32) of B -- the first or second contiguous half of a 64-row operand tile.
+//   mode 0: K = 16, SWIZZLE_32B tiles (one K step)      mode 1: K = 64, SWIZZLE_128B tiles (four K steps)
+// Both CTAs signal "operands written" to the even CTA's mbarrier (count 2) by a remote arrive; the even CTA issues
+// and commits to the mbarriers of both.
+__global__ void __launch_bounds__(128, 1)
+umma_selftest_pair_kernel(const float* __restrict__ A, const float* __restrict__ B, int mode, float* __restrict__ D,
+                          int* __restrict__ err) {
+  extern __shared__ unsigned char smem_raw[];
+  // same offsets in both CTAs: the MMA addresses the operands of the peer with the issuer's descriptors
+  unsigned char* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
+  unsigned char* a_t = smem;            // 128 rows: 4 KB (mode 0) / 16 KB (mode 1)
+  unsigned char* b_t = smem + 16384;    // 32 rows: 1 KB / 4 KB
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + 16384 + 4096);   // [0] MMA done (count 1), [1] request (count 2)
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2);
+  const int tid = threadIdx.x, K = mode == 0 ? 16 : 64;
+  const uint32_t rank = umma::cluster_rank();
+  if (tid == 0) {
+    mbar_init(&bars[0], 1);
+    mbar_init(&bars[1], 2);
+    fence_mbar_init();
+  }
+  if (tid < 32) umma::tmem_alloc_pair(tmem_slot, 64);
+  for (int r = tid; r < 128 + 32; r += 128) {
+    const bool isA = r < 128;
+    const int row = isA ? r : r - 128;
+    const float* src = isA ? A + (size_t)(128 * rank + row) * K : B + (size_t)(32 * rank + row) * K;
+    for (int c = 0; c < K / 8; ++c) {
+      __align__(16) __half h[8];
+#pragma unroll
+      for (int e = 0; e < 8; ++e) h[e] = __float2half_rn(src[c * 8 + e]);
+      const uint32_t off = mode == 0 ? umma::sw32_offset(row, c) : umma::sw128_offset(row, c);
+      *reinterpret_cast<uint4*>((isA ? a_t : b_t) + off) = *reinterpret_cast<const uint4*>(h);
+    }
+  }
+  fence_proxy_async();
+  umma::fence_before_sync();
+  umma::cluster_sync();   // mbarriers of both CTAs initialised, operands of both written
+  umma::fence_after_sync();
+  const uint32_t tbase = *tmem_slot;
+  if (tid == 0) umma::mbar_arrive_cluster(umma::cluster_addr(&bars[1], 0));
+  if (rank == 0 && tid == 0) {
+    int spins = 0;
+    while (!umma::mbar_try_wait_cluster(&bars[1], 0)) {
+      if (++spins > kSelfWaitLimit) {
+        *err = 2;
+        break;
+      }
+    }
+    umma::fence_after_sync();
+    const uint32_t idesc = umma::make_idesc_f16(256, 64);
+    if (mode == 0) {
+      umma::mma_f16_ss_pair(tbase, umma::make_desc_sw32(smem_u32(a_t)), umma::make_desc_sw32(smem_u32(b_t)), idesc, 0);
+    } else {
+      const uint64_t da = umma::make_desc_sw128(smem_u32(a_t)), db = umma::make_desc_sw128(smem_u32(b_t));
+      for (int k = 0; k < 4; ++k)
+        umma::mma_f16_ss_pair(tbase, umma::desc_advance_k(da, k), umma::desc_advance_k(db, k), idesc, k > 0);
+    }
+    umma::commit_pair(&bars[0]);
+  }
+  int spins = 0;
+  while (!mbar_try_wait(&bars[0], 0)) {
+    if (++spins > kSelfWaitLimit) {
+      if (tid == 0) *err = 1;
+      break;
+    }
+  }
+  umma::fence_after_sync();
+  const int warp = tid >> 5;
+  for (int c0 = 0; c0 < 64; c0 += 32) {
+    float v[32];
+    umma::tmem_ld32(tbase + ((uint32_t)(warp * 32) << 16) + (uint32_t)c0, v);
+#pragma unroll
+    for (int i = 0; i < 32; ++i) D[(size_t)(128 * rank + tid) * 64 + c0 + i] = v[i];
+  }
+  umma::fence_before_sync();
+  umma::cluster_sync();   // no CTA frees its columns or exits while the pair's MMA may still use them
+  if (tid < 32) umma::tmem_dealloc_pair(tbase, 64);
+}
+
 }  // namespace mfb
+
+extern "C" int mfb_selftest_umma_pair(const float* a, const float* b, int mode, float* d, int* err, void* stream) {
+  MFB_CHECK_ARG(a && b && d && err && (mode == 0 || mode == 1));
+  const size_t smem = 16384 + 4096 + 64 + 1024;
+  MFB_CUDA(cudaFuncSetAttribute(mfb::umma_selftest_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(2);
+  cfg.blockDim = dim3(128);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = (cudaStream_t)stream;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = 2;
+  attr[0].val.clusterDim.y = 1;
+  attr[0].val.clusterDim.z = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  MFB_CUDA(cudaLaunchKernelEx(&cfg, mfb::umma_selftest_pair_kernel, a, b, mode, d, err));
+  return mfb::launch_status();
+}
 
 extern "C" int mfb_selftest_umma_ts(const float* a, const float* b, int n, float* d, int* err, void* stream) {
   MFB_CHECK_ARG(a && b && d && err && (n == 64 || n == 96 || n == 128));
