@@ -154,6 +154,9 @@ int64_t mfb_kde2d_workspace_bytes(int64_t n, int d, int k, int bx, int by);
 int mfb_project_kde2d_fwd(const float* x, int64_t n, int d, const float* proj, const float* geom,
                           int k, int bx, int by, float max_sigma_over_delta, float* sums,
                           void* workspace, int64_t workspace_bytes, int flags, void* stream);
+/* 1 if mfb_project_kde2d_fwd with these arguments takes the tensor-core path (any bandwidth), 0 if it takes
+ * the windowed fixed-point path (sigma / bin spacing up to 1.0734, like mfb_project_kde2d_bwd)        */
+int mfb_kde2d_uses_tensor_cores(int64_t n, int d, int bx, int by, int flags);
 /* P <- P / (sum(P) dx dy + 1e-10)  (histogram.py:70-73) and its backward                */
 int mfb_kde2d_normalize(const float* sums, const float* geom, int k, int bx, int by,
                         float* profiles, void* stream);

@@ -37,6 +37,7 @@ SIGNATURES = {
     "mfb_project_hist1d": (c_int, [P, c_int64, c_int, P, P, c_int, c_int, P, P]),
     "mfb_kde2d_workspace_bytes": (c_int64, [c_int64, c_int, c_int, c_int, c_int]),
     "mfb_project_kde2d_fwd": (c_int, [P, c_int64, c_int, P, P, c_int, c_int, c_int, c_float, P, P, c_int64, c_int, P]),
+    "mfb_kde2d_uses_tensor_cores": (c_int, [c_int64, c_int, c_int, c_int, c_int]),
     "mfb_kde2d_normalize": (c_int, [P, P, c_int, c_int, c_int, P, P]),
     "mfb_kde2d_normalize_bwd": (c_int, [P, P, c_int, c_int, c_int, P, P, P]),
     "mfb_project_kde2d_bwd": (c_int, [P, c_int64, c_int, P, P, c_int, c_int, c_int, c_float, P, P, c_int, P]),

@@ -14,9 +14,9 @@
 // LDS/FADD/STS -- no atomics, and the accumulation order is fixed => run-to-run deterministic.
 // Each particle touches only the pair-aligned window of 2R+2 bins around its projection
 // (everything beyond ~8.9 sigma is below 1e-17 of a central tap), instead of all B; the taps
-// come from a factorised Gaussian (3 MUFU) with packed-fp32 recurrences.  Per-CTA partials are
-// merged in a fixed order by a second tiny kernel (kde1d_finish_kernel), which also normalises
-// and evaluates the KL term.  The kernel sits at its shared-memory floor (80 B read + written
+// come from recurrences whose factors are all <= 1 (4 MUFU, packed-fp32 multiplies, no overflow at
+// any bandwidth).  Per-CTA partials are merged in a fixed order by a second tiny kernel
+// (kde1d_finish_kernel), which also normalises and evaluates the KL term.  The kernel sits at its shared-memory floor (80 B read + written
 // per particle-projection); the backward kernel uses the same taps on a zero-padded table.
 #include <type_traits>
 
@@ -199,31 +199,6 @@ static KdePlan plan_kde(int64_t n, int d, int k, int b, int r) {
   return P;
 }
 
-// Gaussian taps of one particle at fractional offset f from its nearest bin centre:
-//   tap[R + j] = 2^(alpha (f - j)^2) = E0 * q^j * c_j,  E0 = 2^(alpha f^2), q = 2^(-2 alpha f),
-// c_j / c_(j-1) = 2^(alpha (2j-1)) (rj[j-1], per projection).  Three MUFU instead of 2R+1.
-template <int R>
-__device__ __forceinline__ void gauss_taps(float f, float alpha, const float (&rj)[R], float (&tap)[2 * R + 1]) {
-  const float af = alpha * f;
-  const float e0 = fast_exp2(af * f);
-  const float q = fast_exp2(-2.0f * af), qi = fast_exp2(2.0f * af);
-  tap[R] = e0;
-  float up = e0, dn = e0;
-#pragma unroll
-  for (int j = 1; j <= R; ++j) {
-    up *= q * rj[j - 1];
-    dn *= qi * rj[j - 1];
-    tap[R + j] = up;
-    tap[R - j] = dn;
-  }
-}
-
-// The same taps for a window ALIGNED to row pairs: 2R+2 slots starting at an even row, slot i at offset
-// o_i = i - (R + 1/2) from the window's centre, t in [-1, 1] = particle position relative to that centre:
-//   tap[i] = 2^(alpha (t - o_i)^2) = E_c * G^o_i * C_o_i,   E_c = 2^(alpha t^2), G = 2^(-2 alpha t), C_o = 2^(alpha o^2)
-// chalf = C_1/2 and rr[j] = C_(j+3/2) / C_(j+1/2) = 2^(alpha (2j + 2)) per projection.  The nine taps of the
-// unaligned window [fb-R, fb+R] are all inside (plus one more, 1e-18 of the centre) and land in their pair slots
-// without the shift-by-parity selects the unaligned form needed (11 FSEL per particle-projection).
 // two fp32 products for one issue slot (Blackwell FMUL2; lanes are IEEE round-to-nearest like the scalar multiply)
 __device__ __forceinline__ void mul_pair(float a0, float a1, float b0, float b1, float& c0, float& c1) {
   unsigned long long a, b, c;
@@ -233,22 +208,35 @@ __device__ __forceinline__ void mul_pair(float a0, float a1, float b0, float b1,
   asm("mov.b64 {%0, %1}, %2;" : "=f"(c0), "=f"(c1) : "l"(c));
 }
 
+// Gaussian taps of one particle for a window ALIGNED to row pairs: 2R+2 slots starting at an even row, slot i at offset
+// o_i = i - (R + 1/2) from the window's centre, t in [-1, 1] = particle position relative to that centre:
+//   tap[i] = 2^(alpha (t - o_i)^2),  alpha = -log2(e) / (2 (sigma / delta)^2) < 0.
+// The two centre taps (o = -1/2, +1/2) are evaluated directly; one slot further out multiplies by the ratio
+//   up (slot R+1+j from R+j):     2^(alpha (2j - 2t)) = su * rr[j-2],
+//   down (slot R-j from R-j+1):   2^(alpha (2j + 2t)) = sd * rr[j-2],
+// with su = 2^(alpha (2 - 2t)), sd = 2^(alpha (2 + 2t)) and rr[i] = 2^(2 alpha (i + 1)) per projection.  Every factor is
+// <= 1, so no intermediate overflows however narrow the kernel is; a tap below the fp32 range underflows to zero, which is
+// its correctly rounded value.  Four MUFU instead of 2R+2.  The nine taps of the unaligned window [fb-R, fb+R] are all
+// inside (plus one more, 1e-18 of the centre) and land in their pair slots without shift-by-parity selects.
 template <int R>
-__device__ __forceinline__ void gauss_taps_pairs(float t, float alpha, float chalf, const float (&rr)[R],
-                                                 float (&tap)[2 * R + 2]) {
-  const float at = alpha * t;
-  const float base = fast_exp2(at * t) * chalf;
-  const float h = fast_exp2(-at), hi = fast_exp2(at);     // G^(1/2), G^(-1/2)
-  float g, gi, up, dn;
-  mul_pair(h, hi, h, hi, g, gi);
-  mul_pair(base, base, h, hi, up, dn);
+__device__ __forceinline__ void gauss_taps_pairs(float t, float alpha, const float (&rr)[R - 1], float (&tap)[2 * R + 2]) {
+  static_assert(R >= 2, "window radius");
+  float qu, qd;
+  mul_pair(t - 0.5f, t + 0.5f, t - 0.5f, t + 0.5f, qu, qd);
+  mul_pair(qu, qd, alpha, alpha, qu, qd);
+  float up = fast_exp2(qu), dn = fast_exp2(qd);
+  const float a2 = 2.0f * alpha;
+  const float su = fast_exp2(fmaf(-a2, t, a2)), sd = fast_exp2(fmaf(a2, t, a2));
   tap[R + 1] = up;
   tap[R] = dn;
+  mul_pair(up, dn, su, sd, up, dn);
+  tap[R + 2] = up;
+  tap[R - 1] = dn;
 #pragma unroll
-  for (int j = 1; j <= R; ++j) {
-    float gr, gir;
-    mul_pair(g, gi, rr[j - 1], rr[j - 1], gr, gir);
-    mul_pair(up, dn, gr, gir, up, dn);
+  for (int j = 2; j <= R; ++j) {
+    float ru, rd;
+    mul_pair(su, sd, rr[j - 2], rr[j - 2], ru, rd);
+    mul_pair(up, dn, ru, rd, up, dn);
     tap[R + 1 + j] = up;
     tap[R - j] = dn;
   }
@@ -296,10 +284,10 @@ kde1d_deposit_kernel(const float* __restrict__ x, int64_t n, int d_rt, const flo
   __syncthreads();
 
   float w[kMaxDim];
-  float c0s = 0.f, inv_delta = 0.f, alpha = 0.f, chalf = 0.f;
-  float rr[R];
+  float c0s = 0.f, inv_delta = 0.f, alpha = 0.f;
+  float rr[R - 1];
 #pragma unroll
-  for (int j = 0; j < R; ++j) rr[j] = 0.f;
+  for (int j = 0; j < R - 1; ++j) rr[j] = 0.f;
   if (active) {
 #pragma unroll
     for (int i = 0; i < kMaxDim; ++i) w[i] = i < d ? proj[(size_t)k * d + i] : 0.f;
@@ -308,9 +296,8 @@ kde1d_deposit_kernel(const float* __restrict__ x, int64_t n, int d_rt, const flo
     c0s = g[0] * inv_delta;
     float r = g[1] / g[2];
     alpha = -0.5f * r * r * kLog2e;
-    chalf = exp2f(0.25f * alpha);
 #pragma unroll
-    for (int j = 0; j < R; ++j) rr[j] = exp2f(alpha * (float)(2 * j + 2));
+    for (int j = 0; j < R - 1; ++j) rr[j] = exp2f(alpha * (float)(2 * j + 2));
   }
   MpTerms mpt;
   if constexpr (kMP) {
@@ -360,7 +347,7 @@ kde1d_deposit_kernel(const float* __restrict__ x, int64_t n, int d_rt, const flo
       // mantissa bits, no FRND / F2I
       const float shifted = fmaf(0.5f, ar, 12582912.0f);
       const float fp = shifted - 12582912.0f;
-      gauss_taps_pairs<R>(fmaf(-2.0f, fp, ar), alpha, chalf, rr, taps[q]);
+      gauss_taps_pairs<R>(fmaf(-2.0f, fp, ar), alpha, rr, taps[q]);
       dst[q] = __float_as_uint(shifted) * 256u + cthread;
     }
 #pragma unroll
@@ -713,7 +700,7 @@ kde1d_bwd_kernel(const float* __restrict__ x, int64_t n, int d_rt, const float* 
   float* s_g = sm;                          // [K][BP]
   float* s_w = s_g + (((size_t)K * BP + 3) & ~(size_t)3);   // [K][d]; 16-byte aligned so that s_q is
   float4* s_q = reinterpret_cast<float4*>(s_w + (((size_t)K * d + 3) & ~(size_t)3));  // [K] c0, inv_delta, alpha, beta
-  float* s_rr = reinterpret_cast<float*>(s_q + K);   // [K][R]: 2^(alpha (2 j + 1)), ratios of the tap recurrence
+  float* s_rr = reinterpret_cast<float*>(s_q + K);   // [K][R]: 2^(2 alpha j), steps of the tap ratios
   float* s_mp = s_rr + (size_t)K * R;                // [K][2d + 4] (multipole variant only)
   for (int i = threadIdx.x; i < K * BP; i += blockDim.x) {
     const int kk = i / BP, b = i % BP - kPad;
@@ -728,7 +715,7 @@ kde1d_bwd_kernel(const float* __restrict__ x, int64_t n, int d_rt, const float* 
     const float r = g[1] / g[2];
     const float alpha = -0.5f * r * r * kLog2e;
     s_q[k] = make_float4(g[0], 1.0f / g[1], alpha, -g[1] / (g[2] * g[2]));
-    for (int j = 0; j < R; ++j) s_rr[(size_t)k * R + j] = exp2f(alpha * (float)(2 * j + 1));
+    for (int j = 0; j < R; ++j) s_rr[(size_t)k * R + j] = exp2f(alpha * (float)(2 * j));
   }
   __syncthreads();
   const float lo = -(float)(R + 2), hi = (float)(B + R + 1);
@@ -767,24 +754,25 @@ kde1d_bwd_kernel(const float* __restrict__ x, int64_t n, int d_rt, const float* 
       const float4 q = s_q[k];
       float a = (u - q.x) * q.y;
       a = fminf(fmaxf(a, lo), hi);
-      // nearest bin through the 1.5 * 2^23 rounding constant (no FRND / F2I), taps by the factorised Gaussian of the
-      // forward kernel: value at offset j = E G^j C_j, E = 2^(alpha f^2), G = 2^(-2 alpha f), C_(j+1) / C_j = rr[j] --
-      // three MUFU per particle-projection instead of 2R+1, the up / down recurrences as packed multiplies
+      // nearest bin through the 1.5 * 2^23 rounding constant (no FRND / F2I), taps by recurrences as in the forward
+      // kernel: the value at offset 0 is 2^(alpha f^2), the ratio from offset j to j+1 is 2^(alpha (2j + 1 - 2f)) =
+      // su rr[j] (up) and from -j to -(j+1) 2^(alpha (2j + 1 + 2f)) = sd rr[j] (down), su = 2^(alpha (1 - 2f)),
+      // sd = 2^(alpha (1 + 2f)).  |f| <= 1/2 keeps every factor <= 1 (no overflow at any bandwidth); three MUFU per
+      // particle-projection instead of 2R+1, the up / down recurrences as packed multiplies
       const float shifted = a + 12582912.0f;
       const float fb = shifted - 12582912.0f;
       const float f = a - fb;
       const float* grow = s_g + (size_t)k * BP + ((__float_as_int(shifted) - 0x4B400000) + kPad);
       const float af = q.z * f;
       const float e0 = fast_exp2(af * f);
-      const float gup = fast_exp2(-2.0f * af), gdn = fast_exp2(2.0f * af);
+      const float su = fast_exp2(fmaf(-2.0f, af, q.z)), sd = fast_exp2(fmaf(2.0f, af, q.z));
       const float* rr = s_rr + (size_t)k * R;
       float acc = grow[0] * (e0 * f);
       float up = e0, dn = e0;
 #pragma unroll
       for (int j = 0; j < R; ++j) {
-        const float rj = rr[j];
-        float ru, rd;
-        mul_pair(gup, gdn, rj, rj, ru, rd);
+        float ru = su, rd = sd;
+        if (j > 0) mul_pair(su, sd, rr[j], rr[j], ru, rd);
         mul_pair(up, dn, ru, rd, up, dn);
         float wu, wd;
         mul_pair(up, dn, f - (float)(j + 1), f + (float)(j + 1), wu, wd);

@@ -54,9 +54,12 @@ __device__ __forceinline__ void window(const Axis& ax, float u, int nb, int& b0,
   }
 }
 
-// The same window by the factorised Gaussian of the 1-D kernels (kde1d.cu): value at offset j = E G^j C_j with
-// E = 2^(alpha f^2), G = 2^(-2 alpha f), C_(j+1) / C_j = 2^(alpha (2 j + 1)) -- three MUFU per axis instead of 2R+1 --
-// and the nearest bin through the 1.5 * 2^23 rounding constant.
+// The same window by the tap recurrences of the 1-D kernels (kde1d.cu): the value at offset 0 is E = 2^(alpha f^2), the
+// ratio from offset j-1 to j is 2^(alpha (2j - 1 - 2f)) = su c_j (up) and from -(j-1) to -j 2^(alpha (2j - 1 + 2f)) =
+// sd c_j (down), su = 2^(alpha (1 - 2f)), sd = 2^(alpha (1 + 2f)), c_j = 2^(2 alpha (j - 1)).  |f| <= 1/2 keeps every
+// factor <= 1, so nothing overflows at any bandwidth -- three MUFU per axis instead of 2R+1 --, the c_j do not depend on
+// the particle (the compiler keeps them across the particles of a screen), and the nearest bin comes through the
+// 1.5 * 2^23 rounding constant.
 template <int R>
 __device__ __forceinline__ void window_fact(const Axis& ax, float u, int nb, int& b0, float (&val)[2 * R + 1],
                                             float (&tt)[2 * R + 1]) {
@@ -66,15 +69,20 @@ __device__ __forceinline__ void window_fact(const Axis& ax, float u, int nb, int
   const float fb = shifted - 12582912.0f;
   b0 = __float_as_int(shifted) - 0x4B400000;
   const float f = a - fb, af = ax.alpha * f;
-  const float e0 = fast_exp2(af * f), gup = fast_exp2(-2.0f * af), gdn = fast_exp2(2.0f * af);
+  const float e0 = fast_exp2(af * f);
+  const float su = fast_exp2(fmaf(-2.0f, af, ax.alpha)), sd = fast_exp2(fmaf(2.0f, af, ax.alpha));
+  const float c2 = exp2f(2.0f * ax.alpha);
   val[R] = e0;
   tt[R] = f;
-  float up = e0, dn = e0, c = exp2f(ax.alpha);          // c = C_1 / C_0; the ratio of ratios is 2^(2 alpha)
-  const float c2 = c * c;
+  float up = e0 * su, dn = e0 * sd, c = c2;
+  val[R + 1] = up;
+  val[R - 1] = dn;
+  tt[R + 1] = f - 1.0f;
+  tt[R - 1] = f + 1.0f;
 #pragma unroll
-  for (int j = 1; j <= R; ++j) {
-    up *= gup * c;
-    dn *= gdn * c;
+  for (int j = 2; j <= R; ++j) {
+    up *= su * c;
+    dn *= sd * c;
     c *= c2;
     val[R + j] = up;
     val[R - j] = dn;
@@ -393,6 +401,10 @@ int64_t mfb_kde2d_workspace_bytes(int64_t n, int d, int k, int bx, int by) {
   return (int64_t)k * bx * by * 16 + kde2d_tc_partial_bytes(k, bx, by);
 }
 
+int mfb_kde2d_uses_tensor_cores(int64_t n, int d, int bx, int by, int flags) {
+  return !(flags & MFB_FLAG_NO_TENSOR_CORES) && kde2d_tc_supported(n, d, bx, by) ? 1 : 0;
+}
+
 int mfb_project_kde2d_fwd(const float* x, int64_t n, int d, const float* proj, const float* geom, int k, int bx,
                           int by, float max_sigma_over_delta, float* sums, void* workspace,
                           int64_t workspace_bytes, int flags, void* stream) {
@@ -404,7 +416,7 @@ int mfb_project_kde2d_fwd(const float* x, int64_t n, int d, const float* proj, c
   if (smem > 200 * 1024) return MFB_E_UNSUPPORTED;
   cudaStream_t st = (cudaStream_t)stream;
   unsigned long long* acc = (unsigned long long*)workspace;
-  if (!(flags & MFB_FLAG_NO_TENSOR_CORES) && kde2d_tc_supported(n, d, bx, by) &&
+  if (mfb_kde2d_uses_tensor_cores(n, d, bx, by, flags) &&
       workspace_bytes >= len * 16 + kde2d_tc_partial_bytes(k, bx, by)) {
     float* partial = reinterpret_cast<float*>(reinterpret_cast<unsigned char*>(workspace) + len * 16);
     return kde2d_tc_forward(x, n, d, proj, geom, k, bx, by, sums, acc, partial, st);

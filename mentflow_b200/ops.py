@@ -8,6 +8,7 @@ thread, so nothing here caches streams or keeps global state).  Differentiable o
 from __future__ import annotations
 
 import ctypes
+import math
 from typing import Optional
 
 import torch
@@ -45,6 +46,39 @@ def _check_f32(name: str, t: torch.Tensor) -> torch.Tensor:
 
 
 # --------------------------------------------------------------------------------------
+# supported bandwidths
+# --------------------------------------------------------------------------------------
+# A KDE kernel deposits a particle into the R bins on either side of its nearest bin, R = the smallest integer
+# >= 8.85 sigma / delta - 1/2 (kde1d.cu window_radius): the taps it drops are below 1e-17 of the centre.  The windows are
+# compiled for R = 4, 9 and 13 in 1-D, R = 4 and 9 for the 2-D fixed-point deposit and the 2-D backward; the 2-D
+# tensor-core forward evaluates dense kernel rows and takes any bandwidth.  Wider kernels are refused here, before
+# anything is launched, instead of failing inside the library with a generic error code.
+KDE1D_MAX_RADIUS = 13
+KDE2D_MAX_RADIUS = 9
+
+
+def kde_window_radius(ratio: float) -> int:
+    """Window radius the kernels use for sigma / bin spacing = ``ratio`` (<= 0 stands for the default 0.5)."""
+    r = ctypes.c_float(ratio).value          # the C ABI takes the ratio as a float
+    if r <= 0.0:
+        r = 0.5
+    return max(1, math.ceil(8.85 * r - 0.5))
+
+
+def kde_max_ratio(radius: int) -> float:
+    """Largest sigma / bin spacing whose window fits ``radius`` bins."""
+    return (radius + 0.5) / 8.85
+
+
+def check_kde_ratio(ratio: float, max_radius: int, what: str) -> None:
+    """ValueError unless a kernel compiled up to ``max_radius`` covers sigma / bin spacing = ``ratio``."""
+    if kde_window_radius(ratio) > max_radius:
+        raise ValueError(f"{what}: KDE bandwidth too wide: sigma / bin spacing = {float(ratio):.4g}, the supported limit "
+                         f"is {kde_max_ratio(max_radius):.4f} (a window of {max_radius} bins on either side); "
+                         "use a smaller bandwidth or wider bins")
+
+
+# --------------------------------------------------------------------------------------
 # projection + KDE, 1-D screens
 # --------------------------------------------------------------------------------------
 def _check_mp(mp: torch.Tensor, k: int, d: int) -> torch.Tensor:
@@ -59,6 +93,7 @@ def kde1d_sums(x: torch.Tensor, proj: torch.Tensor, geom: torch.Tensor, ratio: f
     """S[k, b] = sum_n exp(-0.5 ((u_kn - c_b) / sigma_k)^2)  (unnormalised), u_kn = proj_k . x_n, plus the
     multipole terms of ``mp`` (K, 2D+4) when given (see ``simulate.multipole_terms``)."""
     lib = _lib.load()
+    check_kde_ratio(ratio, KDE1D_MAX_RADIUS, "1-D KDE")
     x, proj, geom = _check_f32("x", x), _check_f32("proj", proj), _check_f32("geom", geom)
     n, d = x.shape
     k = proj.shape[0]
@@ -100,6 +135,7 @@ def kde1d_normalize_bwd(sums, n_total, geom, gprof):
 
 def kde1d_grad_x(x, proj, geom, ratio, gsums, out: Optional[torch.Tensor] = None, mp: Optional[torch.Tensor] = None):
     lib = _lib.load()
+    check_kde_ratio(ratio, KDE1D_MAX_RADIUS, "1-D KDE backward")
     n, d = x.shape
     k, b = gsums.shape
     acc = 1 if out is not None else 0
@@ -121,6 +157,7 @@ KL_PAD = 1.0e-12   # loss.py:15-17
 def kde1d_loss_forward(x, proj, geom, ratio, nbins, n_total, meas):
     """Deposit + merge + normalise (+ KL against ``meas``) in two launches: (sums, profiles, kl)."""
     lib = _lib.load()
+    check_kde_ratio(ratio, KDE1D_MAX_RADIUS, "1-D KDE")
     x, proj, geom = _check_f32("x", x), _check_f32("proj", proj), _check_f32("geom", geom)
     n, d = x.shape
     k = proj.shape[0]
@@ -164,6 +201,7 @@ def kde1d_loss_forward_p2p(peer, x, proj, geom, ratio, nbins, tail, n_total, mea
     """Sharded forward tail in two launches: deposit, then merge + cross-rank sum over NVLink peer memory +
     normalisation (+ KL).  Returns (sums, profiles, kl, tail_sum)."""
     lib = _lib.load()
+    check_kde_ratio(ratio, KDE1D_MAX_RADIUS, "1-D KDE")
     x, proj, geom = _check_f32("x", x), _check_f32("proj", proj), _check_f32("geom", geom)
     n, d = x.shape
     k = proj.shape[0]
@@ -220,6 +258,7 @@ class ProjectKDE1D(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, proj, geom, ratio, nbins, reducer, meas, mp=None):
         ctx.set_materialize_grads(False)
+        check_kde_ratio(ratio, KDE1D_MAX_RADIUS, "1-D KDE")      # before any launch or cross-rank exchange
         x = _check_f32("x", x)
         n_total = float(x.shape[0])
         if meas is not None:
@@ -321,14 +360,16 @@ def kde2d_sums(x, proj, geom, ratio, bx, by):
     x, proj, geom = _check_f32("x", x), _check_f32("proj", proj), _check_f32("geom", geom)
     n, d = x.shape
     k = proj.shape[0]
+    flags = 0 if KDE2D_USE_TENSOR_CORES else FLAG_NO_TENSOR_CORES
+    if not lib.mfb_kde2d_uses_tensor_cores(n, d, bx, by, flags):     # the windowed fixed-point deposit
+        check_kde_ratio(ratio, KDE2D_MAX_RADIUS, "2-D KDE (fixed-point deposit)")
     sums = torch.empty((k, bx, by), dtype=torch.float32, device=x.device)
     with torch.cuda.device(x.device):
         # workspace = the two int64 planes, then the per-CTA partial screens of the tensor-core path
         wbytes = int(lib.mfb_kde2d_workspace_bytes(n, d, k, bx, by))
         work = torch.empty((wbytes + 7) // 8, dtype=torch.int64, device=x.device)
         _lib.check(lib.mfb_project_kde2d_fwd(_ptr(x), n, d, _ptr(proj), _ptr(geom), k, bx, by, float(ratio),
-                                             _ptr(sums), _ptr(work), wbytes,
-                                             0 if KDE2D_USE_TENSOR_CORES else FLAG_NO_TENSOR_CORES, _stream()),
+                                             _ptr(sums), _ptr(work), wbytes, flags, _stream()),
                    "project_kde2d_fwd")
     acc = work[: 2 * k * bx * by].view(2, k, bx, by)
     return sums, acc
@@ -362,6 +403,7 @@ class ProjectKDE2D(torch.autograd.Function):
     @staticmethod
     def backward(ctx, gprof):
         lib = _lib.load()
+        check_kde_ratio(ctx.ratio, KDE2D_MAX_RADIUS, "2-D KDE backward")
         x, proj, geom, sums = ctx.saved_tensors
         k, bx, by = sums.shape
         gprof = _check_f32("gprof", gprof)
@@ -378,6 +420,9 @@ class ProjectKDE2D(torch.autograd.Function):
 
 
 def project_kde2d(x, proj, geom, ratio, bx, by, reducer=None):
+    if torch.is_grad_enabled() and x.requires_grad:
+        # the backward is windowed at any batch size: refuse now rather than in backward()
+        check_kde_ratio(ratio, KDE2D_MAX_RADIUS, "2-D KDE backward (x requires grad)")
     return ProjectKDE2D.apply(x, proj, geom, ratio, bx, by, reducer)
 
 

@@ -63,7 +63,14 @@ def test_kde2d_gradient_matches_reference_autograd(golden):
     assert (x.grad.cpu() - ref).abs().max() <= TOL * ref.abs().max()
 
 
-@pytest.mark.parametrize("n,d,k,bx,by", [(1, 4, 1, 8, 8), (999, 6, 15, 85, 85), (200000, 4, 6, 85, 85), (5000, 3, 2, 20, 31)])
+@pytest.mark.parametrize("n,d,k,bx,by", [(1, 4, 1, 8, 8), (999, 6, 15, 85, 85), (200000, 4, 6, 85, 85), (5000, 3, 2, 20, 31),
+                                         # limits of the tensor-core path: the largest screen it takes and one bin more
+                                         (5000, 4, 3, 128, 96), (5000, 4, 2, 129, 96), (5000, 4, 2, 128, 97),
+                                         # either side of the batch size that selects it, and a ragged 64-particle tile
+                                         (4095, 6, 3, 32, 32), (4096, 6, 3, 32, 32), (4097, 6, 3, 32, 32),
+                                         # five screens' accumulators are resident in TMEM at a time
+                                         (8192, 4, 5, 40, 40), (8192, 4, 6, 40, 40), (8192, 4, 10, 40, 40),
+                                         (8192, 4, 11, 40, 40)])
 def test_kde2d_vs_oracle_shapes(n, d, k, bx, by):
     gen = torch.Generator().manual_seed(n + k)
     x = torch.randn(n, d, generator=gen)
@@ -76,6 +83,10 @@ def test_kde2d_vs_oracle_shapes(n, d, k, bx, by):
     ref = torch.stack([hp.kde_profile_2d(x @ w[i, 0], x @ w[i, 1], ex, ey, sx, sy, chunk=20000)
                        for i in range(k)])
     assert profile_err(prof, ref) < TOL
+    # screens up to 128 x 96 bins and batches of at least 4096 particles run on the tensor cores
+    from mentflow_b200 import _lib
+    tc = bool(_lib.load().mfb_kde2d_uses_tensor_cores(n, d, bx, by, 0 if ops.KDE2D_USE_TENSOR_CORES else 1))
+    assert tc == (ops.KDE2D_USE_TENSOR_CORES and n >= 4096 and bx <= 128 and by <= 96)
 
 
 def test_kde2d_tensor_core_and_fixed_point_paths_agree():

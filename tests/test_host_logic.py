@@ -141,6 +141,31 @@ def test_diagnostic_interface_and_no_cpu_fallback():
         gen.forward(torch.randn(4, 2))
 
 
+def test_kde_window_radius_and_bandwidth_limits():
+    """The window radius the kernels pick from sigma / bin spacing (kde1d.cu window_radius), the boundaries of the
+    compiled templates, and the refusal of wider kernels before anything needs the GPU."""
+    from mentflow_b200 import ops
+    assert ops.kde_window_radius(0.5) == 4 and ops.kde_window_radius(0.0) == 4      # <= 0: the default 0.5
+    assert ops.kde_window_radius(0.05) == 1
+    assert ops.kde_window_radius(0.505) == 4 and ops.kde_window_radius(0.515) == 5
+    assert ops.kde_window_radius(1.07) == 9 and ops.kde_window_radius(1.08) == 10
+    assert ops.kde_window_radius(1.52) == 13 and ops.kde_window_radius(1.53) == 14
+    for radius in (4, 9, 13):
+        top = ops.kde_max_ratio(radius)
+        assert ops.kde_window_radius(top * (1 - 1e-6)) == radius and ops.kde_window_radius(top * (1 + 1e-6)) == radius + 1
+    assert abs(ops.kde_max_ratio(ops.KDE1D_MAX_RADIUS) - 1.5254) < 1e-4
+    assert abs(ops.kde_max_ratio(ops.KDE2D_MAX_RADIUS) - 1.0734) < 1e-4
+    ops.check_kde_ratio(1.52, ops.KDE1D_MAX_RADIUS, "1-D")
+    with pytest.raises(ValueError, match="1.5254"):
+        ops.check_kde_ratio(1.53, ops.KDE1D_MAX_RADIUS, "1-D")
+    with pytest.raises(ValueError, match="1.0734"):
+        ops.check_kde_ratio(1.08, ops.KDE2D_MAX_RADIUS, "2-D")
+    # the reference's default absolute bandwidth (1.0) on typical bins is refused with the limit, not a library error
+    from mentflow_b200.diagnostics.histogram import kde_histogram_1d
+    with pytest.raises(ValueError, match="bandwidth too wide"):
+        kde_histogram_1d(torch.randn(100), torch.linspace(-3.5, 3.5, 65))
+
+
 def test_projection_vectors_follow_transform_and_direction():
     m = torch.randn(4, 4)
     e = torch.linspace(-1, 1, 9)
