@@ -322,6 +322,32 @@ int mfb_ment_integrate_nd(int d, const float* meas_coords, int nb_meas, int meas
                           const float* proj2, const float* cx2, const float* cy2, const float* tables2, int k2,
                           int bx, int by, float prior_neg_half_inv_s2, float prior_log_norm, float* pred,
                           void* stream);
+/* The same behind thin multipole kicks: every transfer map is linear or a chain linear* -> MultipoleTransform (order
+ * 3, 4 or 5, normal or skew) -> linear* (simulate/transform.py:35-146; experiments/rec_2d/nonlinear).  Measured
+ * coordinate of a row: proj . x + a Re(z^m) + b Im(z^m), z = wa . x + i wb . x, m = order - 1, with
+ * mp[k][2 d + 4] = [wa (d) | wb (d) | a | b | order | 0] for the 1-D screens and mp2[k2][2][2 d + 4] for the two rows
+ * of each 2-D screen (they share wa, wb and the order).  A row of a linear map has order 0 and adds no kick.
+ * _integrate_nd_mp maps the screen back with the folded inverse of the screen's chain,
+ *   x = linv u + p Re(zi^m) + q Im(zi^m),  zi = r0 . u + i r2 . u,
+ * inv_mp[4 d + 2] = [r0 (d) | r2 (d) | p (d) | q (d) | order | 0] (order 0: a linear map, x = linv u; linv = M^-1).
+ * The host folds matrices, kick strength / (order-1)! and the reference's quirks into these terms
+ * (simulate.multipole_terms, simulate.multipole_inverse_terms).  mp / mp2 must be given when k / k2 > 0.  */
+int mfb_ment_prob_nd_mp(const float* x, int64_t g, int d, const float* proj, const float* coords, const float* tables,
+                        int k, int b, const float* mp, const float* proj2, const float* cx2, const float* cy2,
+                        const float* tables2, int k2, int bx, int by, const float* mp2, float prior_neg_half_inv_s2,
+                        float prior_log_norm, float* out, void* stream);
+int mfb_ment_prob_grid_nd_mp(int d, const int32_t* shape_host, const float* first_centre_host, const float* step_host,
+                             const float* proj, const float* coords, const float* tables, int k, int b, const float* mp,
+                             const float* proj2, const float* cx2, const float* cy2, const float* tables2, int k2,
+                             int bx, int by, const float* mp2, float prior_neg_half_inv_s2, float prior_log_norm,
+                             float* out, void* stream);
+int mfb_ment_integrate_nd_mp(int d, const float* meas_coords, int nb_meas, int meas_axis, const float* meas_coords2,
+                             int nb_meas2, int meas_axis2, int n_int_axes, const int32_t* int_shape_host,
+                             const float* int_first_host, const float* int_step_host, const float* linv,
+                             const float* inv_mp, const float* proj, const float* coords, const float* tables, int k,
+                             int b, const float* mp, const float* proj2, const float* cx2, const float* cy2,
+                             const float* tables2, int k2, int bx, int by, const float* mp2,
+                             float prior_neg_half_inv_s2, float prior_log_norm, float* pred, void* stream);
 /* sample.py:27-57: cdf of (rho + pad) over the cells in double, then `size` draws: cell by
  * inverse-CDF search with a Philox4x32-10 stream (seed, offset), uniform position inside the
  * cell (+ 0.5*U(-delta,delta) when jitter != 0).  workspace[0] (device double) = total mass. */

@@ -67,6 +67,12 @@ SIGNATURES = {
                                       c_float, P, P]),
     "mfb_ment_integrate_nd": (c_int, [c_int, P, c_int, c_int, P, c_int, c_int, c_int, P, P, P, P, P, P, P, c_int, c_int,
                                       P, P, P, P, c_int, c_int, c_int, c_float, c_float, P, P]),
+    "mfb_ment_prob_nd_mp": (c_int, [P, c_int64, c_int, P, P, P, c_int, c_int, P, P, P, P, P, c_int, c_int, c_int, P,
+                                    c_float, c_float, P, P]),
+    "mfb_ment_prob_grid_nd_mp": (c_int, [c_int, P, P, P, P, P, P, c_int, c_int, P, P, P, P, P, c_int, c_int, c_int, P,
+                                         c_float, c_float, P, P]),
+    "mfb_ment_integrate_nd_mp": (c_int, [c_int, P, c_int, c_int, P, c_int, c_int, c_int, P, P, P, P, P, P, P, P,
+                                         c_int, c_int, P, P, P, P, P, c_int, c_int, c_int, P, c_float, c_float, P, P]),
     "mfb_randn_offset_increment": (c_int64, [c_int64]),
     "mfb_randn_philox": (c_int, [P, c_int64, c_uint64, c_uint64, P]),
     "mfb_randn_philox_state": (c_int, [P, c_int64, P, c_int, P]),

@@ -1,5 +1,10 @@
-// Classical MENT: density rho(x) = prior(x) * prod_k h_k(w_k . x), its integration / sampling
+// Classical MENT: density rho(x) = prior(x) * prod_k h_k(u_k(x)), its integration / sampling
 // and the Gauss-Seidel update of the Lagrange tables.
+//
+// u_k(x) = w_k . x for a linear transfer map.  Behind a chain linear* -> MultipoleTransform -> linear* (the kMP
+// instantiations) u_k(x) = w_k . x + a_k Re(z^m) + b_k Im(z^m), z = wa . x + i wb . x (multipole.cuh); rows of linear
+// maps in such a model carry order 0 and skip the kick.  Integrate mode then maps the screen back with the folded
+// inverse of the chain, x = L u + p Re(zi^m) + q Im(zi^m), zi = r0 . u + i r2 . u.
 //
 // Replaces (reference file:line, relative to mentflow/):
 //   ment.py:239-249, 227-234, 45-52   MENT.prob: per measurement a full matmul, a device->numpy
@@ -10,10 +15,16 @@
 //   ment.py:267-317                   _simulate_integrate: Python loop over measured pixels
 //   ment.py:360-367                   Python per-bin loop of the Gauss-Seidel update
 #include "common.cuh"
+#include "multipole.cuh"
 
 namespace mfb {
 
 constexpr int kMentThreads = 256;
+// Minimum resident CTAs per SM of the kernels with multipole terms: 5 (<= 51 registers) stops ptxas from spilling in
+// the kick's complex powers, where with no minimum it picks 40 - 48 registers and spills in the 5-D and 6-D variants.
+// The linear kernels keep no minimum (0).
+template <bool kMP>
+constexpr int ment_min_ctas() { return kMP ? 5 : 0; }
 
 struct MentGrid {            // regular grid of cell centres (GridSampler) or an integration grid
   int ndim;
@@ -53,6 +64,34 @@ struct Tables2D {
   const float* cy;      // [k][by]
   const float* tab;     // [k][bx][by]
 };
+// (kMP) the multipole rows of the 2-D screens travel beside Tables2D as mp2[k][2][2D+4]: the two rows of a screen share
+// wa, wb and the order, each has its own a, b.
+
+// z^m of the mp row `row` (layout of multipole.cuh) at x, and u + a Re(z^m) + b Im(z^m).  mp_z is false for order 0
+// (a linear map in a model with kicks): the kick is skipped, since 0 * z^m would turn a huge z into NaN.
+// kLdg: the row is in global memory.
+template <bool kLdg>
+__device__ __forceinline__ float mp_load(const float* __restrict__ p) {
+  if constexpr (kLdg) return __ldg(p); else return *p;
+}
+template <int D, bool kLdg>
+__device__ __forceinline__ bool mp_z(const float* __restrict__ row, const float (&x)[D], float& zr, float& zi) {
+  const int m = (int)mp_load<kLdg>(row + 2 * D + 2) - 1;
+  if (m < 1) return false;
+  float xm = 0.f, ym = 0.f;
+#pragma unroll
+  for (int i = 0; i < D; ++i) {
+    xm = fmaf(mp_load<kLdg>(row + i), x[i], xm);
+    ym = fmaf(mp_load<kLdg>(row + D + i), x[i], ym);
+  }
+  float pr, pi;
+  zpow(xm, ym, m, zr, zi, pr, pi);
+  return true;
+}
+template <int D, bool kLdg>
+__device__ __forceinline__ float mp_add(const float* __restrict__ row, float zr, float zi, float u) {
+  return fmaf(mp_load<kLdg>(row + 2 * D + 1), zi, fmaf(mp_load<kLdg>(row + 2 * D), zr, u));
+}
 
 // interval index and normalised distance on one axis (scipy find_indices: searchsorted - 1, clipped)
 __device__ __forceinline__ bool axis_locate(const float* __restrict__ c, int B, float u, int& i, double& w) {
@@ -67,8 +106,9 @@ __device__ __forceinline__ bool axis_locate(const float* __restrict__ c, int B, 
   return true;
 }
 
-template <int D>
-__device__ __forceinline__ float tables2d_product(const float (&x)[D], const Tables2D& t2) {
+template <int D, bool kMP = false>
+__device__ __forceinline__ float tables2d_product(const float (&x)[D], const Tables2D& t2,
+                                                  const float* __restrict__ mp2 = nullptr) {
   float prob = 1.0f;
   for (int k = 0; k < t2.k; ++k) {
     const float* pr = t2.proj + (size_t)k * 2 * D;
@@ -77,6 +117,14 @@ __device__ __forceinline__ float tables2d_product(const float (&x)[D], const Tab
     for (int i = 0; i < D; ++i) {
       ux = fmaf(__ldg(pr + i), x[i], ux);
       uy = fmaf(__ldg(pr + D + i), x[i], uy);
+    }
+    if constexpr (kMP) {
+      const float* row = mp2 + (size_t)k * 2 * MFB_MP_STRIDE(D);
+      float zr, zi;
+      if (mp_z<D, true>(row, x, zr, zi)) {
+        ux = mp_add<D, true>(row, zr, zi, ux);
+        uy = mp_add<D, true>(row + MFB_MP_STRIDE(D), zr, zi, uy);
+      }
     }
     int ix, iy;
     double wx, wy;
@@ -95,16 +143,21 @@ __device__ __forceinline__ float tables2d_product(const float (&x)[D], const Tab
   return prob;
 }
 
-template <int D>
+template <int D, bool kMP = false>
 __device__ __forceinline__ float ment_density(const float (&x)[D], const float* __restrict__ s_proj,
                                               const float* __restrict__ s_c, const float* __restrict__ s_h,
                                               const float* __restrict__ s_inv, const double* __restrict__ s_dinv, int K,
-                                              int B, MentPrior prior) {
+                                              int B, MentPrior prior, const float* __restrict__ s_mp = nullptr) {
   float prob = 1.0f;
   for (int k = 0; k < K; ++k) {
     float u = 0.f;
 #pragma unroll
     for (int i = 0; i < D; ++i) u = fmaf(s_proj[k * D + i], x[i], u);
+    if constexpr (kMP) {
+      const float* row = s_mp + (size_t)k * MFB_MP_STRIDE(D);
+      float zr, zi;
+      if (mp_z<D, false>(row, x, zr, zi)) u = mp_add<D, false>(row, zr, zi, u);
+    }
     float h = lagrange_eval(s_c + (size_t)k * B, s_h + (size_t)k * B, s_dinv + (size_t)k * B, B, s_inv[k], u);
     h = fminf(fmaxf(h, 0.0f), 1.0e10f);   // ment.py:246
     prob *= h;
@@ -130,12 +183,19 @@ __device__ __forceinline__ void load_tables(float* s_proj, float* s_c, float* s_
     s_inv[k] = (float)(B - 1) / (coords[(size_t)k * B + B - 1] - coords[(size_t)k * B]);
 }
 
+// (kMP) the multipole rows of the 1-D screens, [K][2D+4], follow the tables in shared memory
+__device__ __forceinline__ float* mp_smem(double* s_dinv, int K, int B) {
+  return reinterpret_cast<float*>(s_dinv + (size_t)K * B);
+}
+
 // MODE 0: explicit points x[G][D];  MODE 1: points of a regular grid generated from the index
-template <int D, int MODE>
-__global__ void __launch_bounds__(kMentThreads)
+// kMP: mp[K][2D+4] and mp2[K2][2][2D+4] add the multipole terms to the projections
+template <int D, int MODE, bool kMP = false>
+__global__ void __launch_bounds__(kMentThreads, ment_min_ctas<kMP>())
 ment_prob_kernel(const float* __restrict__ x, int64_t G, MentGrid grid, const float* __restrict__ proj,
                  const float* __restrict__ coords, const float* __restrict__ tables, int K, int B,
-                 MentPrior prior, const Tables2D t2, float* __restrict__ out) {
+                 MentPrior prior, const Tables2D t2, float* __restrict__ out, const float* __restrict__ mp = nullptr,
+                 const float* __restrict__ mp2 = nullptr) {
   extern __shared__ __align__(16) float sm[];
   float* s_proj = sm;
   float* s_c = s_proj + (((size_t)K * D + 3) & ~(size_t)3);
@@ -143,6 +203,11 @@ ment_prob_kernel(const float* __restrict__ x, int64_t G, MentGrid grid, const fl
   float* s_inv = s_h + (size_t)K * B;
   double* s_dinv = reinterpret_cast<double*>(s_inv + ((K + 1) & ~1));
   load_tables(s_proj, s_c, s_h, s_inv, s_dinv, proj, coords, tables, K, B, D);
+  float* s_mp = nullptr;
+  if constexpr (kMP) {
+    s_mp = mp_smem(s_dinv, K, B);
+    for (int i = threadIdx.x; i < K * MFB_MP_STRIDE(D); i += blockDim.x) s_mp[i] = mp[i];
+  }
   __syncthreads();
   for (int64_t g = (int64_t)blockIdx.x * kMentThreads + threadIdx.x; g < G; g += (int64_t)gridDim.x * kMentThreads) {
     float xr[D];
@@ -158,21 +223,25 @@ ment_prob_kernel(const float* __restrict__ x, int64_t G, MentGrid grid, const fl
         xr[i] = fmaf((float)idx, grid.step[i], grid.lo[i]);
       }
     }
-    float rho = ment_density<D>(xr, s_proj, s_c, s_h, s_inv, s_dinv, K, B, prior);
-    if (t2.k > 0) rho *= tables2d_product<D>(xr, t2);
+    float rho = ment_density<D, kMP>(xr, s_proj, s_c, s_h, s_inv, s_dinv, K, B, prior, s_mp);
+    if (t2.k > 0) rho *= tables2d_product<D, kMP>(xr, t2, mp2);
     out[g] = rho;
   }
 }
 
 // integrate mode (ment.py:267-317) for a 1-D screen: pred[b] = sum_q rho(Minv [c_b ; t_q])
 // one CTA per measured pixel, deterministic block reduction
-template <int D>
-__global__ void __launch_bounds__(kMentThreads)
+// kMP: the density has multipole rows (mp, mp2 as in ment_prob_kernel), minv is L of the folded inverse and
+// imp[4D+2] = [r0 | r2 | p | q | order | 0] its kick (order 0: a linear map, x = L u)
+template <int D, bool kMP = false>
+__global__ void __launch_bounds__(kMentThreads, ment_min_ctas<kMP>())
 ment_integrate_kernel(const float* __restrict__ meas_coords, int nb_meas, int meas_axis,
                       const float* __restrict__ meas_coords2, int nb_meas2, int meas_axis2, MentGrid igrid,
                       const float* __restrict__ minv /* [D][D] */, const float* __restrict__ proj,
                       const float* __restrict__ coords, const float* __restrict__ tables, int K, int B,
-                      MentPrior prior, const Tables2D t2, float* __restrict__ pred) {
+                      MentPrior prior, const Tables2D t2, float* __restrict__ pred,
+                      const float* __restrict__ mp = nullptr, const float* __restrict__ mp2 = nullptr,
+                      const float* __restrict__ imp = nullptr) {
   extern __shared__ __align__(16) float sm[];
   float* s_proj = sm;
   float* s_c = s_proj + (((size_t)K * D + 3) & ~(size_t)3);
@@ -183,6 +252,14 @@ ment_integrate_kernel(const float* __restrict__ meas_coords, int nb_meas, int me
   double* s_dinv = reinterpret_cast<double*>(s_inv + ((K + 1) & ~1));
   load_tables(s_proj, s_c, s_h, s_inv, s_dinv, proj, coords, tables, K, B, D);
   for (int i = threadIdx.x; i < D * D; i += blockDim.x) s_minv[i] = minv[i];
+  float* s_mp = nullptr;
+  float* s_imp = nullptr;
+  if constexpr (kMP) {
+    s_mp = mp_smem(s_dinv, K, B);
+    s_imp = s_mp + (size_t)K * MFB_MP_STRIDE(D);
+    for (int i = threadIdx.x; i < K * MFB_MP_STRIDE(D); i += blockDim.x) s_mp[i] = mp[i];
+    for (int i = threadIdx.x; i < 4 * D + 2; i += blockDim.x) s_imp[i] = imp[i];
+  }
   __syncthreads();
   int64_t Q = 1;
   for (int i = 0; i < igrid.ndim; ++i) Q *= igrid.shape[i];
@@ -217,8 +294,24 @@ ment_integrate_kernel(const float* __restrict__ meas_coords, int nb_meas, int me
       for (int j = 0; j < D; ++j) s = fmaf(u[j], s_minv[i * D + j], s);
       xr[i] = s;
     }
-    float rho = ment_density<D>(xr, s_proj, s_c, s_h, s_inv, s_dinv, K, B, prior);
-    if (t2.k > 0) rho *= tables2d_product<D>(xr, t2);
+    if constexpr (kMP) {
+      // kick of the inverse map: zi = r0 . u + i r2 . u, x += p Re(zi^m) + q Im(zi^m)
+      const int m = (int)s_imp[4 * D] - 1;
+      if (m >= 1) {
+        float xm = 0.f, ym = 0.f;
+#pragma unroll
+        for (int j = 0; j < D; ++j) {
+          xm = fmaf(s_imp[j], u[j], xm);
+          ym = fmaf(s_imp[D + j], u[j], ym);
+        }
+        float zr, zi, pr, pi;
+        zpow(xm, ym, m, zr, zi, pr, pi);
+#pragma unroll
+        for (int i = 0; i < D; ++i) xr[i] = fmaf(s_imp[3 * D + i], zi, fmaf(s_imp[2 * D + i], zr, xr[i]));
+      }
+    }
+    float rho = ment_density<D, kMP>(xr, s_proj, s_c, s_h, s_inv, s_dinv, K, B, prior, s_mp);
+    if (t2.k > 0) rho *= tables2d_product<D, kMP>(xr, t2, mp2);
     dacc += (double)rho;
   }
   (void)acc;
@@ -460,6 +553,10 @@ __global__ void gs_update_kernel(float* __restrict__ table, const float* __restr
 static size_t ment_smem(int K, int B, int d) {
   return ((((size_t)K * d + 3) & ~(size_t)3) + 2 * (size_t)K * B + ((K + 1) & ~1)) * 4 + (size_t)K * B * 8 + 16;
 }
+// kMP: the 1-D screens' multipole rows and the inverse kick of integrate mode follow (mp_smem)
+static size_t ment_smem_mp(int K, int B, int d) {
+  return ment_smem(K, B, d) + ((size_t)K * MFB_MP_STRIDE(d) + 4 * (size_t)d + 2) * 4;
+}
 
 static MentGrid make_grid(int ndim, const int32_t* shape, const float* lo, const float* step) {
   MentGrid g;
@@ -472,21 +569,24 @@ static MentGrid make_grid(int ndim, const int32_t* shape, const float* lo, const
   return g;
 }
 
-template <int D>
+template <int D, bool kMP = false>
 static int launch_prob(int mode, const float* x, int64_t G, const MentGrid& grid, const float* proj,
                        const float* coords, const float* tables, int K, int B, MentPrior prior, float* out,
-                       cudaStream_t st, const Tables2D& t2 = Tables2D{0, 0, 0, nullptr, nullptr, nullptr, nullptr}) {
-  const size_t smem = ment_smem(K, B, D);
+                       cudaStream_t st, const Tables2D& t2 = Tables2D{0, 0, 0, nullptr, nullptr, nullptr, nullptr},
+                       const float* mp = nullptr, const float* mp2 = nullptr) {
+  const size_t smem = kMP ? ment_smem_mp(K, B, D) : ment_smem(K, B, D);
   if (smem > 200 * 1024) return MFB_E_UNSUPPORTED;
   int64_t blocks = (G + kMentThreads - 1) / kMentThreads;
   int64_t cap = (int64_t)sm_count() * 8;
   const int gridx = (int)(blocks < cap ? blocks : cap);
   if (mode == 0) {
-    MFB_CUDA(cudaFuncSetAttribute(ment_prob_kernel<D, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ment_prob_kernel<D, 0><<<gridx, kMentThreads, smem, st>>>(x, G, grid, proj, coords, tables, K, B, prior, t2, out);
+    MFB_CUDA(cudaFuncSetAttribute(ment_prob_kernel<D, 0, kMP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    ment_prob_kernel<D, 0, kMP><<<gridx, kMentThreads, smem, st>>>(x, G, grid, proj, coords, tables, K, B, prior, t2, out,
+                                                                   mp, mp2);
   } else {
-    MFB_CUDA(cudaFuncSetAttribute(ment_prob_kernel<D, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ment_prob_kernel<D, 1><<<gridx, kMentThreads, smem, st>>>(x, G, grid, proj, coords, tables, K, B, prior, t2, out);
+    MFB_CUDA(cudaFuncSetAttribute(ment_prob_kernel<D, 1, kMP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    ment_prob_kernel<D, 1, kMP><<<gridx, kMentThreads, smem, st>>>(x, G, grid, proj, coords, tables, K, B, prior, t2, out,
+                                                                   mp, mp2);
   }
   return launch_status();
 }
@@ -497,16 +597,17 @@ static int check_tables2d(const Tables2D& t2) {
   return 0;
 }
 
-template <int D>
+template <int D, bool kMP = false>
 static int launch_integrate(const float* mc, int nb, int ax, const float* mc2, int nb2, int ax2, const MentGrid& grid,
                             const float* minv, const float* proj, const float* coords, const float* tables, int k, int b,
-                            MentPrior pr, const Tables2D& t2, float* pred, cudaStream_t st) {
-  const size_t smem = ment_smem(k, b, D);
+                            MentPrior pr, const Tables2D& t2, float* pred, cudaStream_t st, const float* mp = nullptr,
+                            const float* mp2 = nullptr, const float* imp = nullptr) {
+  const size_t smem = kMP ? ment_smem_mp(k, b, D) : ment_smem(k, b, D);
   if (smem > 200 * 1024) return MFB_E_UNSUPPORTED;
-  MFB_CUDA(cudaFuncSetAttribute(ment_integrate_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  MFB_CUDA(cudaFuncSetAttribute(ment_integrate_kernel<D, kMP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int pixels = ax2 >= 0 ? nb * nb2 : nb;
-  ment_integrate_kernel<D><<<pixels, kMentThreads, smem, st>>>(mc, nb, ax, mc2, nb2, ax2, grid, minv, proj, coords, tables,
-                                                              k, b, pr, t2, pred);
+  ment_integrate_kernel<D, kMP><<<pixels, kMentThreads, smem, st>>>(mc, nb, ax, mc2, nb2, ax2, grid, minv, proj, coords,
+                                                                   tables, k, b, pr, t2, pred, mp, mp2, imp);
   return launch_status();
 }
 
@@ -624,6 +725,85 @@ int mfb_ment_integrate(int d, const float* meas_coords, int nb_meas, int meas_ax
   return mfb_ment_integrate_nd(d, meas_coords, nb_meas, meas_axis, nullptr, 0, -1, n_int_axes, int_shape_host,
                                int_first_host, int_step_host, minv, proj, coords, tables, k, b, nullptr, nullptr,
                                nullptr, nullptr, 0, 0, 0, prior_neg_half_inv_s2, prior_log_norm, pred, stream);
+}
+
+int mfb_ment_prob_nd_mp(const float* x, int64_t g, int d, const float* proj, const float* coords, const float* tables,
+                        int k, int b, const float* mp, const float* proj2, const float* cx2, const float* cy2,
+                        const float* tables2, int k2, int bx, int by, const float* mp2, float prior_neg_half_inv_s2,
+                        float prior_log_norm, float* out, void* stream) {
+  MFB_CHECK_ARG(x && out && g >= 0 && k >= 0 && d >= 1 && d <= kMaxDim);
+  MFB_CHECK_ARG(k == 0 || (proj && coords && tables && mp && b >= 2));
+  const Tables2D t2{k2, bx, by, proj2, cx2, cy2, tables2};
+  if (check_tables2d(t2)) return MFB_E_BADARG;
+  MFB_CHECK_ARG(k2 == 0 || mp2);
+  if (g == 0) return 0;
+  if (k == 0) b = 2;
+  MentPrior pr{prior_neg_half_inv_s2, prior_log_norm};
+  MentGrid grid = make_grid(0, nullptr, nullptr, nullptr);
+  cudaStream_t st = (cudaStream_t)stream;
+#define MFB_CALL(DD) launch_prob<DD, true>(0, x, g, grid, proj, coords, tables, k, b, pr, out, st, t2, mp, mp2)
+  MFB_DISPATCH_D(d, MFB_CALL)
+#undef MFB_CALL
+}
+
+int mfb_ment_prob_grid_nd_mp(int d, const int32_t* shape_host, const float* first_centre_host, const float* step_host,
+                             const float* proj, const float* coords, const float* tables, int k, int b, const float* mp,
+                             const float* proj2, const float* cx2, const float* cy2, const float* tables2, int k2,
+                             int bx, int by, const float* mp2, float prior_neg_half_inv_s2, float prior_log_norm,
+                             float* out, void* stream) {
+  MFB_CHECK_ARG(shape_host && first_centre_host && step_host && out);
+  MFB_CHECK_ARG(k >= 0 && d >= 1 && d <= kMaxDim);
+  MFB_CHECK_ARG(k == 0 || (proj && coords && tables && mp && b >= 2));
+  const Tables2D t2{k2, bx, by, proj2, cx2, cy2, tables2};
+  if (check_tables2d(t2)) return MFB_E_BADARG;
+  MFB_CHECK_ARG(k2 == 0 || mp2);
+  if (k == 0) b = 2;
+  int64_t g = 1;
+  for (int i = 0; i < d; ++i) {
+    MFB_CHECK_ARG(shape_host[i] >= 1);
+    g *= shape_host[i];
+  }
+  MentPrior pr{prior_neg_half_inv_s2, prior_log_norm};
+  MentGrid grid = make_grid(d, shape_host, first_centre_host, step_host);
+  cudaStream_t st = (cudaStream_t)stream;
+#define MFB_CALL(DD) launch_prob<DD, true>(1, nullptr, g, grid, proj, coords, tables, k, b, pr, out, st, t2, mp, mp2)
+  MFB_DISPATCH_D(d, MFB_CALL)
+#undef MFB_CALL
+}
+
+int mfb_ment_integrate_nd_mp(int d, const float* meas_coords, int nb_meas, int meas_axis, const float* meas_coords2,
+                             int nb_meas2, int meas_axis2, int n_int_axes, const int32_t* int_shape_host,
+                             const float* int_first_host, const float* int_step_host, const float* linv,
+                             const float* inv_mp, const float* proj, const float* coords, const float* tables, int k,
+                             int b, const float* mp, const float* proj2, const float* cx2, const float* cy2,
+                             const float* tables2, int k2, int bx, int by, const float* mp2,
+                             float prior_neg_half_inv_s2, float prior_log_norm, float* pred, void* stream) {
+  MFB_CHECK_ARG(meas_coords && linv && inv_mp && pred && int_shape_host && int_first_host && int_step_host);
+  MFB_CHECK_ARG(k >= 0 && (k == 0 || (proj && coords && tables && mp && b >= 2)));
+  const int n_meas = meas_axis2 >= 0 ? 2 : 1;
+  MFB_CHECK_ARG(d >= 2 && d <= kMaxDim && n_int_axes == d - n_meas && n_int_axes >= 1);
+  MFB_CHECK_ARG(meas_axis >= 0 && meas_axis < d && nb_meas >= 1 && meas_axis2 < d && meas_axis2 != meas_axis);
+  MFB_CHECK_ARG(meas_axis2 < 0 || (meas_coords2 && nb_meas2 >= 1));
+  const Tables2D t2{k2, bx, by, proj2, cx2, cy2, tables2};
+  if (check_tables2d(t2)) return MFB_E_BADARG;
+  MFB_CHECK_ARG(k2 == 0 || mp2);
+  if (k == 0) b = 2;
+  MentPrior pr{prior_neg_half_inv_s2, prior_log_norm};
+  MentGrid grid = make_grid(n_int_axes, int_shape_host, int_first_host, int_step_host);
+  cudaStream_t st = (cudaStream_t)stream;
+#define MFB_CALL(DD)                                                                                                 \
+  launch_integrate<DD, true>(meas_coords, nb_meas, meas_axis, meas_coords2, nb_meas2, meas_axis2, grid, linv, proj, \
+                             coords, tables, k, b, pr, t2, pred, st, mp, mp2, inv_mp)
+  switch (d) {
+    case 2: return MFB_CALL(2);
+    case 3: return MFB_CALL(3);
+    case 4: return MFB_CALL(4);
+    case 5: return MFB_CALL(5);
+    case 6: return MFB_CALL(6);
+    case 7: return MFB_CALL(7);
+    default: return MFB_CALL(8);
+  }
+#undef MFB_CALL
 }
 
 int64_t mfb_cdf_workspace_bytes(int64_t g) {

@@ -9,6 +9,14 @@ update is one elementwise kernel.  One- and two-dimensional screens (Histogram1D
 experiments/config/rec_nd_1d_ment.yaml, rec_nd_2d_ment.yaml) may be mixed; within each family the
 screens must have the same number of bins.
 
+Transfer maps are linear (``LinearTransform``, or a ``CompositeTransform`` of them) or a chain
+linear* -> MultipoleTransform (order 3, 4 or 5, normal or skew) -> linear* (experiments/rec_2d/nonlinear), in
+any mix.  Behind a kick the projection of a screen is ``w . x + a Re(z^m) + b Im(z^m)``
+(``simulate.multipole_terms``), evaluated inside the density kernels; integrate mode maps the screen back
+with the chain's folded inverse (``simulate.multipole_inverse_terms``), and sample mode predicts profiles
+through ``simulate.forward`` (1-D screens behind a kick fused, 2-D ones object by object).  Other maps
+raise ``NotImplementedError``.
+
 Sharded over GPUs (``mentflow_b200.distributed.shard_model``; BASELINE config 5): every rank evaluates
 the same density, draws ITS slice of the ``n_samples`` particles from the same Philox stream (particle s
 always uses counter s, whichever rank draws it), and the unnormalised profile sums are all-reduced before
@@ -25,7 +33,8 @@ from .diagnostics import Histogram1D, Histogram2D
 from .loss import kl_divergence
 from .prior import Gaussian, Uniform
 from .simulate import forward as simulate_forward
-from .simulate.simulate import _linear_matrix
+from .simulate.simulate import _linear_matrix, _multipole_chain, multipole_inverse_terms, multipole_terms
+from .simulate.transform import LinearTransform
 from .utils import coords_from_edges, get_grid_points, unravel
 
 
@@ -119,40 +128,77 @@ class MENT:
     def _slots(self):
         return [(i, j) for i in range(len(self.diagnostics)) for j in range(len(self.diagnostics[i]))]
 
+    def _transfer(self, index: int):
+        """(matrix, chain) of transform ``index``: the matrix of a linear map (None for the identity) and no chain, or
+        no matrix and the (pre, kick, post) of a linear* -> MultipoleTransform -> linear* chain."""
+        transform = self.transforms[index]
+        matrix = _linear_matrix(transform)
+        if matrix is not NotImplemented:
+            return matrix, None
+        chain = _multipole_chain(transform)
+        if chain is None or self.ndim == 3:
+            raise NotImplementedError(
+                "MENT on the CUDA path supports linear transfer maps (LinearTransform or a CompositeTransform of them) "
+                "and chains linear* -> MultipoleTransform(order 3, 4 or 5) -> linear* in D = 2 or D >= 4; "
+                f"transform {index} is {type(transform).__name__}")
+        return None, chain
+
     def _pack(self, device):
         """Static part of the kernel arguments: projection rows and bin centres of every table, the 1-D and
-        the 2-D screens as two families."""
+        the 2-D screens as two families; with a multipole kick anywhere in the model, the multipole rows of every
+        screen as well (order 0 behind linear maps)."""
         if self._packed is not None and self._packed["device"] == device:
             return self._packed
-        slots1, proj1, coords1 = [], [], []
-        slots2, proj2, cx2, cy2 = [], [], [], []
+        slots1, proj1, coords1, mp1 = [], [], [], []
+        slots2, proj2, cx2, cy2, mp2 = [], [], [], [], []
+        nd = self.ndim
         for i, j in self._slots():
             d = self.diagnostics[i][j]
-            matrix = _linear_matrix(self.transforms[i])
-            if matrix is NotImplemented:
-                raise NotImplementedError("MENT on the CUDA path needs linear transforms")
+            matrix, chain = self._transfer(i)
+            if chain is not None:
+                # measured rows of the linear part after the kick, folded through the kick and the part before it
+                pre, kick, post = chain
+                post32 = post.to(torch.float32) if post is not None else None
+                rows = (d.projection_vectors(post32, nd, "cpu") if isinstance(d, Histogram2D)
+                        else d.projection_vector(post32, nd, "cpu")[None])
+                terms = [multipole_terms(r, pre, kick, nd) for r in rows]
+                vec = torch.stack([w for w, _ in terms]).to(device)
+                mp = torch.stack([m for _, m in terms]).to(device)
             if isinstance(d, Histogram2D):
                 slots2.append((i, j))
-                proj2.append(d.projection_vectors(matrix, self.ndim, device))
+                proj2.append(d.projection_vectors(matrix, nd, device) if chain is None else vec)
+                mp2.append(mp if chain is not None else None)
                 cx2.append(coords_from_edges(d.edges_x.to(torch.float32)).to(device))
                 cy2.append(coords_from_edges(d.edges_y.to(torch.float32)).to(device))
             else:
                 slots1.append((i, j))
-                proj1.append(d.projection_vector(matrix, self.ndim, device))
+                proj1.append(d.projection_vector(matrix, nd, device) if chain is None else vec[0])
+                mp1.append(mp[0] if chain is not None else None)
                 coords1.append(coords_from_edges(d.edges.to(torch.float32)).to(device))
         for family in (coords1, cx2, cy2):
             if len({int(c.shape[0]) for c in family}) > 1:
                 raise NotImplementedError("all screens of one kind in a MENT model must have the same number of bins")
+        kicked = any(m is not None for m in mp1 + mp2)
+
+        def stack_mp(rows, shape):
+            if not kicked or not rows:
+                return None
+            return torch.stack([m if m is not None else torch.zeros(shape, dtype=torch.float32, device=device)
+                                for m in rows]).contiguous()
+
         self._packed = {"device": device, "slots1": slots1, "slots2": slots2,
                         "proj": torch.stack(proj1).contiguous() if proj1 else None,
                         "coords": torch.stack(coords1).contiguous() if coords1 else None,
                         "proj2": torch.stack(proj2).contiguous() if proj2 else None,
                         "cx2": torch.stack(cx2).contiguous() if cx2 else None,
-                        "cy2": torch.stack(cy2).contiguous() if cy2 else None}
+                        "cy2": torch.stack(cy2).contiguous() if cy2 else None,
+                        "mp": stack_mp(mp1, (2 * nd + 4,)), "mp2": stack_mp(mp2, (2, 2 * nd + 4)),
+                        "kicked": kicked, "inverse": {}}
         return self._packed
 
     def _groups(self, device):
-        """(g1, g2) for ``ops.ment_prob_nd``: the current tables of the two screen families."""
+        """(g1, g2) for ``ops.ment_prob_nd``: the current tables of the two screen families, followed by their
+        multipole rows when the model has a kick."""
         pk = self._pack(device)
 
         def stack(slots):
@@ -161,7 +207,30 @@ class MENT:
 
         g1 = (pk["proj"], pk["coords"], stack(pk["slots1"])) if pk["slots1"] else None
         g2 = (pk["proj2"], pk["cx2"], pk["cy2"], stack(pk["slots2"])) if pk["slots2"] else None
+        if pk["kicked"]:
+            g1 = g1 + (pk["mp"],) if g1 is not None else None
+            g2 = g2 + (pk["mp2"],) if g2 is not None else None
         return g1, g2
+
+    def _inverse(self, index: int, device):
+        """(minv, inv_mp) mapping screen coordinates of transform ``index`` back to x: the inverse matrix of a linear
+        map (``matrix_inv`` of a LinearTransform, the inverse of the product of a linear CompositeTransform) and no
+        kick, or L and the kick terms of a multipole chain (``multipole_inverse_terms``, kept with the packed rows)."""
+        matrix, chain = self._transfer(index)
+        if chain is None:
+            transform = self.transforms[index]
+            if isinstance(transform, LinearTransform):
+                minv = transform.matrix_inv
+            elif matrix is None:
+                minv = torch.eye(self.ndim)
+            else:
+                minv = torch.linalg.inv(matrix)
+            return minv.to(device=device, dtype=torch.float32).contiguous(), None
+        cache = self._pack(device)["inverse"]
+        if index not in cache:
+            lin, imp = multipole_inverse_terms(*chain, self.ndim)
+            cache[index] = (lin.to(device).contiguous(), imp.to(device).contiguous())
+        return cache[index]
 
     def _prior_args(self) -> Tuple[float, float]:
         if isinstance(self.prior, Gaussian):
@@ -232,26 +301,26 @@ class MENT:
         return coords[0] if len(coords) == 1 else self.send(get_grid_points(*coords))
 
     def _simulate_integrate(self, index: int, diag_index: int) -> torch.Tensor:
-        """pred[b] = sum over the integration grid of rho(M^-1 [pixel; grid]) (ment.py:267-317)."""
+        """pred[b] = sum over the integration grid of rho(T^-1 [pixel; grid]) (ment.py:267-317)."""
         limits = self.integration_limits[index][diag_index]
         shape = [int(s) for s in self.integration_shape[index][diag_index]]
         diagnostic = self.diagnostics[index][diag_index]
-        transform = self.transforms[index]
         device = torch.device(self.device if self.device is not None else "cuda")
         g1, g2 = self._groups(device)
         a, b = self._prior_args()
         first = [float(limits[k][0]) for k in range(len(shape))]
         step = [(float(limits[k][1]) - float(limits[k][0])) / max(shape[k] - 1, 1) for k in range(len(shape))]
-        minv = transform.matrix_inv.to(device=device, dtype=torch.float32).contiguous()
+        minv, inv_mp = self._inverse(index, device)
         if isinstance(diagnostic, Histogram2D):
             cx = coords_from_edges(diagnostic.edges_x.to(torch.float32)).to(device)
             cy = coords_from_edges(diagnostic.edges_y.to(torch.float32)).to(device)
             ax, ay = diagnostic.axis
-            pred = ops.ment_integrate_nd(self.ndim, cx, ax, cy, ay, shape, first, step, minv, g1, g2, a, b)
+            pred = ops.ment_integrate_nd(self.ndim, cx, ax, cy, ay, shape, first, step, minv, g1, g2, a, b,
+                                         inv_mp=inv_mp)
         else:
             meas_coords = coords_from_edges(diagnostic.edges.to(torch.float32)).to(device)
             pred = ops.ment_integrate_nd(self.ndim, meas_coords, diagnostic.axis, None, -1, shape, first, step, minv,
-                                         g1, g2, a, b)
+                                         g1, g2, a, b, inv_mp=inv_mp)
         return self.normalize_projection(pred, index, diag_index)
 
     def _simulate_sample(self, index: int, diag_index: int) -> torch.Tensor:

@@ -179,6 +179,38 @@ def multipole_terms(row: torch.Tensor, pre: Optional[torch.Tensor], kick: Multip
     return w.to(torch.float32), mp.to(torch.float32)
 
 
+def multipole_inverse_terms(pre: Optional[torch.Tensor], kick: MultipoleTransform, post: Optional[torch.Tensor],
+                            ndim: int, dtype=torch.float32):
+    """(L, imp): the inverse of ``post . kick . pre`` as ``x = L u + p Re(z^m) + q Im(z^m)``, z = r0 . u + i r2 . u,
+    m = order - 1, imp = [r0 | r2 | p | q | order | 0] (the integrate mode of classical MENT).
+
+    Follows CompositeTransform.inverse: post^-1, then the kick's inverse (momentum reversal, kick, momentum reversal:
+    simulate/transform.py:145-146), then pre^-1.  With A = pre^-1 and B = post^-1, r0 / r2 are rows 0 / 2 of B; the
+    normal kick gives p = k A[:, 1], q = -k A[:, 3] and L = A Q B, where Q is the identity except that row 3 is e1 for
+    D > 2 (the reference's U[:, 3] = X[:, 1] + ... quirk); the skew kick gives p = -k A[:, 3], q = -k A[:, 1] and L = A B.
+    Columns 3.. are absent for D = 2.  Evaluated in float64 on the host, returned as ``dtype``."""
+    eye = torch.eye(ndim, dtype=torch.float64)
+    a_inv = eye if pre is None else torch.linalg.inv(pre.to(torch.float64))
+    b_inv = eye if post is None else torch.linalg.inv(post.to(torch.float64))
+    k = kick.coefficient()
+    zero = torch.zeros(ndim, dtype=torch.float64)
+    r0 = b_inv[0]
+    r2 = b_inv[2] if ndim > 2 else zero
+    c1 = a_inv[:, 1]
+    c3 = a_inv[:, 3] if ndim > 2 else zero
+    if kick.skew:
+        p, q = -k * c3, -k * c1
+        lin = a_inv @ b_inv
+    else:
+        p, q = k * c1, -k * c3
+        quirk = eye.clone()
+        if ndim > 2:
+            quirk[3] = eye[1]
+        lin = a_inv @ quirk @ b_inv
+    imp = torch.cat([r0, r2, p, q, torch.tensor([float(kick.order), 0.0], dtype=torch.float64)])
+    return lin.to(dtype), imp.to(dtype)
+
+
 def _tensor_key(t):
     """identity + in-place version of a tensor (None-safe)"""
     return (id(t), getattr(t, "_version", 0)) if t is not None else None
