@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define MFB_ABI_VERSION 2
+#define MFB_ABI_VERSION 3
 
 #define MFB_E_BADARG (-1)      /* null pointer / non-positive size / unsupported shape   */
 #define MFB_E_UNSUPPORTED (-2) /* combination not compiled (e.g. D > 8, hidden != 64)    */
@@ -227,15 +227,9 @@ int64_t mfb_nsf_layer_param_om_floats(int d, int hidden_units, int hidden_layers
 /* The backward of a layer runs as three tcgen05 kernels for hidden_layers = 3, bins = 20 (nsf_tc.cu kBwd,
  * nsf_tc_bwd.cu) and on CUDA-core kernels otherwise, or when `flags` has MFB_FLAG_NO_TENSOR_CORES.   */
 int64_t mfb_nsf_layer_bwd_workspace_bytes(int64_t n, int d, int hidden_layers);
-int mfb_nsf_layer_bwd(const float* v, const float* gy, const float* glogq, int64_t n, int d,
-                      int hidden_units, int hidden_layers, int bins, const float* params,
-                      const float* params_om, const int32_t* order_host, int first_layer, float* gv,
-                      float* gparams, int accumulate, void* workspace, int64_t workspace_bytes,
-                      int flags, void* stream);
-
-/* The same with the layer's tcgen05 operand image that mfb_nsf_tc_prepare built for the forward pass of
- * this step (tc_image, mfb_nsf_tc_image_bytes bytes, 16-byte aligned; NULL = build it here): a
- * training step then builds each image once instead of twice.                              */
+/* tc_image: the layer's tcgen05 operand image that mfb_nsf_tc_prepare built for the forward pass of
+ * this step (mfb_nsf_tc_image_bytes bytes, 16-byte aligned; NULL = build it here): a training
+ * step then builds each image once instead of twice.                                      */
 int mfb_nsf_layer_bwd_img(const float* v, const float* gy, const float* glogq, int64_t n, int d,
                           int hidden_units, int hidden_layers, int bins, const float* params,
                           const float* params_om, const int32_t* order_host, int first_layer,
@@ -278,76 +272,52 @@ int mfb_f64_split(const double* in, int n, float* out_hi_lo, void* stream);
 int mfb_f64_join(const float* in_hi_lo, int n, double* out, void* stream);
 
 /* ---- classical MENT (ment.py, sample.py) --------------------------------------------------
- * rho(x) = exp(log prior(x)) * prod_k clamp(h_k(proj_k . x), 0, 1e10); h_k = linear interpolation
- * of tables[k][0..b) on the bin centres coords[k][0..b), 0 outside the first/last centre,
- * evaluated in double like scipy's RegularGridInterpolator (ment.py:45-52, 227-249).
- * prior: log p(x) = prior_neg_half_inv_s2 * |x|^2 + prior_log_norm (Gaussian prior.py:25-26;
- * a flat prior passes 0 and its log constant).                                            */
-int mfb_ment_prob(const float* x, int64_t g, int d, const float* proj, const float* coords,
-                  const float* tables, int k, int b, float prior_neg_half_inv_s2,
+ * rho(x) = exp(log prior(x)) * prod clamp(h(u(x)), 0, 1e10) over two families of Lagrange tables, evaluated in
+ * double like scipy's RegularGridInterpolator and 0 outside the box of the bin centres (ment.py:36-52, 227-249);
+ * either family may be empty (k = 0 / k2 = 0):
+ *   1-D screens: h_k linear on tables[k][0..b) at the bin centres coords[k][0..b), u = proj[k] . x;
+ *   2-D screens (LagrangeFunction over an N-D RegularGridInterpolator; experiments/config/rec_nd_2d_ment.yaml):
+ *     h bilinear on tables2[k2][bx][by] at the bin-centre grids cx2[k2][bx] x cy2[k2][by], u = proj2[k2][2][d] . x
+ *     (the two measured rows of each transfer matrix).
+ * prior: log p(x) = prior_neg_half_inv_s2 * |x|^2 + prior_log_norm (Gaussian prior.py:25-26; a flat prior passes 0
+ * and its log constant).
+ *
+ * Multipole kicks: every transfer map is linear or a chain linear* -> MultipoleTransform (order 3, 4 or 5, normal or
+ * skew) -> linear* (simulate/transform.py:35-146; experiments/rec_2d/nonlinear).  The measured coordinate of a row is
+ * then proj . x + a Re(z^m) + b Im(z^m), z = wa . x + i wb . x, m = order - 1, with mp[k][2 d + 4] = [wa (d) | wb (d) |
+ * a | b | order | 0] for the 1-D screens and mp2[k2][2][2 d + 4] for the two rows of each 2-D screen (they share wa,
+ * wb and the order).  A row of a linear map has order 0 and adds no kick.  The host folds matrices, kick
+ * strength / (order-1)! and the reference's quirks into these terms (simulate.multipole_terms,
+ * simulate.multipole_inverse_terms).
+ * With mp, mp2 and (integrate) inv_mp all NULL every map is linear.  If any of them is given the kernels with kicks
+ * run; mp is then required when k > 0, mp2 when k2 > 0 and inv_mp by the integration, otherwise MFB_E_BADARG.  */
+/* rho at explicit points x[g][d]                                                          */
+int mfb_ment_prob(const float* x, int64_t g, int d, const float* proj, const float* coords, const float* tables,
+                  int k, int b, const float* mp, const float* proj2, const float* cx2, const float* cy2,
+                  const float* tables2, int k2, int bx, int by, const float* mp2, float prior_neg_half_inv_s2,
                   float prior_log_norm, float* out, void* stream);
-/* same on the cell centres of a regular grid generated from the index ('ij' order, last axis
- * fastest) instead of res^D x D materialised points (sample.py:99-104 GridSampler).  shape /
- * first_centre / step are HOST arrays of d entries.                                       */
-int mfb_ment_prob_grid(int d, const int32_t* shape_host, const float* first_centre_host,
-                       const float* step_host, const float* proj, const float* coords,
-                       const float* tables, int k, int b, float prior_neg_half_inv_s2,
-                       float prior_log_norm, float* out, void* stream);
-/* integrate mode for a 1-D screen (ment.py:267-317): pred[i] = sum over the integration grid of
- * rho(Minv [meas_coords[i] on meas_axis ; grid point on the other axes]).                 */
-int mfb_ment_integrate(int d, const float* meas_coords, int nb_meas, int meas_axis, int n_int_axes,
-                       const int32_t* int_shape_host, const float* int_first_host,
-                       const float* int_step_host, const float* minv, const float* proj,
-                       const float* coords, const float* tables, int k, int b,
-                       float prior_neg_half_inv_s2, float prior_log_norm, float* pred, void* stream);
-/* The same three entry points with two-dimensional screens as well (ment.py:36-49: LagrangeFunction over an N-D
- * RegularGridInterpolator; experiments/config/rec_nd_2d_ment.yaml): k2 tables tables2[k2][bx][by] on the bin-centre
- * grids cx2[k2][bx] x cy2[k2][by], bilinear, zero outside the box of the centres, evaluated in double like scipy;
- * proj2[k2][2][d] are the two measured rows of each transfer matrix.  rho = prior * prod(1-D tables) * prod(2-D
- * tables); either family may be empty (k = 0 / k2 = 0).  _integrate_nd: meas_axis2 >= 0 selects a 2-D screen
- * (pred[nb_meas][nb_meas2], integration over the other d-2 axes), meas_axis2 = -1 a 1-D one.              */
-int mfb_ment_prob_nd(const float* x, int64_t g, int d, const float* proj, const float* coords, const float* tables,
-                     int k, int b, const float* proj2, const float* cx2, const float* cy2, const float* tables2,
-                     int k2, int bx, int by, float prior_neg_half_inv_s2, float prior_log_norm, float* out,
-                     void* stream);
-int mfb_ment_prob_grid_nd(int d, const int32_t* shape_host, const float* first_centre_host, const float* step_host,
-                          const float* proj, const float* coords, const float* tables, int k, int b,
-                          const float* proj2, const float* cx2, const float* cy2, const float* tables2, int k2,
-                          int bx, int by, float prior_neg_half_inv_s2, float prior_log_norm, float* out,
-                          void* stream);
-int mfb_ment_integrate_nd(int d, const float* meas_coords, int nb_meas, int meas_axis, const float* meas_coords2,
-                          int nb_meas2, int meas_axis2, int n_int_axes, const int32_t* int_shape_host,
-                          const float* int_first_host, const float* int_step_host, const float* minv,
-                          const float* proj, const float* coords, const float* tables, int k, int b,
-                          const float* proj2, const float* cx2, const float* cy2, const float* tables2, int k2,
-                          int bx, int by, float prior_neg_half_inv_s2, float prior_log_norm, float* pred,
-                          void* stream);
-/* The same behind thin multipole kicks: every transfer map is linear or a chain linear* -> MultipoleTransform (order
- * 3, 4 or 5, normal or skew) -> linear* (simulate/transform.py:35-146; experiments/rec_2d/nonlinear).  Measured
- * coordinate of a row: proj . x + a Re(z^m) + b Im(z^m), z = wa . x + i wb . x, m = order - 1, with
- * mp[k][2 d + 4] = [wa (d) | wb (d) | a | b | order | 0] for the 1-D screens and mp2[k2][2][2 d + 4] for the two rows
- * of each 2-D screen (they share wa, wb and the order).  A row of a linear map has order 0 and adds no kick.
- * _integrate_nd_mp maps the screen back with the folded inverse of the screen's chain,
+/* rho on the cell centres of a regular grid generated from the index ('ij' order, last axis fastest) instead of
+ * res^D x D materialised points (sample.py:99-104 GridSampler).  shape / first_centre / step are HOST arrays of d
+ * entries.                                                                                */
+int mfb_ment_prob_grid(int d, const int32_t* shape_host, const float* first_centre_host, const float* step_host,
+                       const float* proj, const float* coords, const float* tables, int k, int b, const float* mp,
+                       const float* proj2, const float* cx2, const float* cy2, const float* tables2, int k2,
+                       int bx, int by, const float* mp2, float prior_neg_half_inv_s2, float prior_log_norm,
+                       float* out, void* stream);
+/* integrate mode (ment.py:267-317): pred[i] = sum over the integration grid (n_int_axes = d - 1 or d - 2 HOST
+ * arrays) of rho(x(u)), u = meas_coords[i] on meas_axis and the grid point on the other axes.  meas_axis2 >= 0
+ * selects a 2-D screen: pred[nb_meas][nb_meas2], meas_coords2 on meas_axis2; meas_axis2 = -1 a 1-D one.
+ * The screen is mapped back with the folded inverse of its transfer map,
  *   x = linv u + p Re(zi^m) + q Im(zi^m),  zi = r0 . u + i r2 . u,
- * inv_mp[4 d + 2] = [r0 (d) | r2 (d) | p (d) | q (d) | order | 0] (order 0: a linear map, x = linv u; linv = M^-1).
- * The host folds matrices, kick strength / (order-1)! and the reference's quirks into these terms
- * (simulate.multipole_terms, simulate.multipole_inverse_terms).  mp / mp2 must be given when k / k2 > 0.  */
-int mfb_ment_prob_nd_mp(const float* x, int64_t g, int d, const float* proj, const float* coords, const float* tables,
-                        int k, int b, const float* mp, const float* proj2, const float* cx2, const float* cy2,
-                        const float* tables2, int k2, int bx, int by, const float* mp2, float prior_neg_half_inv_s2,
-                        float prior_log_norm, float* out, void* stream);
-int mfb_ment_prob_grid_nd_mp(int d, const int32_t* shape_host, const float* first_centre_host, const float* step_host,
-                             const float* proj, const float* coords, const float* tables, int k, int b, const float* mp,
-                             const float* proj2, const float* cx2, const float* cy2, const float* tables2, int k2,
-                             int bx, int by, const float* mp2, float prior_neg_half_inv_s2, float prior_log_norm,
-                             float* out, void* stream);
-int mfb_ment_integrate_nd_mp(int d, const float* meas_coords, int nb_meas, int meas_axis, const float* meas_coords2,
-                             int nb_meas2, int meas_axis2, int n_int_axes, const int32_t* int_shape_host,
-                             const float* int_first_host, const float* int_step_host, const float* linv,
-                             const float* inv_mp, const float* proj, const float* coords, const float* tables, int k,
-                             int b, const float* mp, const float* proj2, const float* cx2, const float* cy2,
-                             const float* tables2, int k2, int bx, int by, const float* mp2,
-                             float prior_neg_half_inv_s2, float prior_log_norm, float* pred, void* stream);
+ * inv_mp[4 d + 2] = [r0 (d) | r2 (d) | p (d) | q (d) | order | 0] (order 0, or inv_mp NULL: a linear map, x = linv u;
+ * linv = M^-1).  d >= 2.                                                                  */
+int mfb_ment_integrate(int d, const float* meas_coords, int nb_meas, int meas_axis, const float* meas_coords2,
+                       int nb_meas2, int meas_axis2, int n_int_axes, const int32_t* int_shape_host,
+                       const float* int_first_host, const float* int_step_host, const float* linv,
+                       const float* inv_mp, const float* proj, const float* coords, const float* tables, int k,
+                       int b, const float* mp, const float* proj2, const float* cx2, const float* cy2,
+                       const float* tables2, int k2, int bx, int by, const float* mp2,
+                       float prior_neg_half_inv_s2, float prior_log_norm, float* pred, void* stream);
 /* sample.py:27-57: cdf of (rho + pad) over the cells in double, then `size` draws: cell by
  * inverse-CDF search with a Philox4x32-10 stream (seed, offset), uniform position inside the
  * cell (+ 0.5*U(-delta,delta) when jitter != 0).  workspace[0] (device double) = total mass. */

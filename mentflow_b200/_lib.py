@@ -13,6 +13,8 @@ LIB_PATH = os.environ.get("MENTFLOW_B200_LIB") or os.path.join(PKG_DIR, "libment
 
 P = c_void_p  # every device pointer crosses the ABI as a plain address
 
+ABI_VERSION = 3  # MFB_ABI_VERSION of the header SIGNATURES mirrors
+
 # name -> (restype, argtypes); mirrors include/mentflow_b200.h line by line
 SIGNATURES = {
     "mfb_abi_version": (c_int, []),
@@ -53,26 +55,14 @@ SIGNATURES = {
     "mfb_nsf_tc_layer_inv": (c_int, [P, c_int64, c_int, c_int, c_int, c_int, P, P, P, c_int, P, P, P]),
     "mfb_nsf_layer_param_om_floats": (c_int64, [c_int, c_int, c_int]),
     "mfb_nsf_layer_bwd_workspace_bytes": (c_int64, [c_int64, c_int, c_int]),
-    "mfb_nsf_layer_bwd": (c_int, [P, P, P, c_int64, c_int, c_int, c_int, c_int, P, P, P, c_int, P, P, c_int, P,
-                                  c_int64, c_int, P]),
     "mfb_nsf_layer_bwd_img": (c_int, [P, P, P, c_int64, c_int, c_int, c_int, c_int, P, P, P, c_int, P, P, P, c_int, P,
                                       c_int64, c_int, P]),
-    "mfb_ment_prob": (c_int, [P, c_int64, c_int, P, P, P, c_int, c_int, c_float, c_float, P, P]),
-    "mfb_ment_prob_grid": (c_int, [c_int, P, P, P, P, P, P, c_int, c_int, c_float, c_float, P, P]),
-    "mfb_ment_integrate": (c_int, [c_int, P, c_int, c_int, c_int, P, P, P, P, P, P, P, c_int, c_int, c_float,
+    "mfb_ment_prob": (c_int, [P, c_int64, c_int, P, P, P, c_int, c_int, P, P, P, P, P, c_int, c_int, c_int, P, c_float,
+                              c_float, P, P]),
+    "mfb_ment_prob_grid": (c_int, [c_int, P, P, P, P, P, P, c_int, c_int, P, P, P, P, P, c_int, c_int, c_int, P, c_float,
                                    c_float, P, P]),
-    "mfb_ment_prob_nd": (c_int, [P, c_int64, c_int, P, P, P, c_int, c_int, P, P, P, P, c_int, c_int, c_int, c_float,
-                                 c_float, P, P]),
-    "mfb_ment_prob_grid_nd": (c_int, [c_int, P, P, P, P, P, P, c_int, c_int, P, P, P, P, c_int, c_int, c_int, c_float,
-                                      c_float, P, P]),
-    "mfb_ment_integrate_nd": (c_int, [c_int, P, c_int, c_int, P, c_int, c_int, c_int, P, P, P, P, P, P, P, c_int, c_int,
-                                      P, P, P, P, c_int, c_int, c_int, c_float, c_float, P, P]),
-    "mfb_ment_prob_nd_mp": (c_int, [P, c_int64, c_int, P, P, P, c_int, c_int, P, P, P, P, P, c_int, c_int, c_int, P,
-                                    c_float, c_float, P, P]),
-    "mfb_ment_prob_grid_nd_mp": (c_int, [c_int, P, P, P, P, P, P, c_int, c_int, P, P, P, P, P, c_int, c_int, c_int, P,
-                                         c_float, c_float, P, P]),
-    "mfb_ment_integrate_nd_mp": (c_int, [c_int, P, c_int, c_int, P, c_int, c_int, c_int, P, P, P, P, P, P, P, P,
-                                         c_int, c_int, P, P, P, P, P, c_int, c_int, c_int, P, c_float, c_float, P, P]),
+    "mfb_ment_integrate": (c_int, [c_int, P, c_int, c_int, P, c_int, c_int, c_int, P, P, P, P, P, P, P, P, c_int, c_int,
+                                   P, P, P, P, P, c_int, c_int, c_int, P, c_float, c_float, P, P]),
     "mfb_randn_offset_increment": (c_int64, [c_int64]),
     "mfb_randn_philox": (c_int, [P, c_int64, c_uint64, c_uint64, P]),
     "mfb_randn_philox_state": (c_int, [P, c_int64, P, c_int, P]),
@@ -118,6 +108,10 @@ def load():
             raise LibraryMissing(f"{LIB_PATH} does not export {name}; rebuild it") from e
         fn.restype = res
         fn.argtypes = args
+    # a library built from other sources may export the same names with other argument lists
+    version = lib.mfb_abi_version()
+    if version != ABI_VERSION:
+        raise LibraryMissing(f"{LIB_PATH} has ABI version {version}, this package needs {ABI_VERSION}; rebuild it")
     _lib = lib
     return lib
 

@@ -569,45 +569,42 @@ static MentGrid make_grid(int ndim, const int32_t* shape, const float* lo, const
   return g;
 }
 
-template <int D, bool kMP = false>
-static int launch_prob(int mode, const float* x, int64_t G, const MentGrid& grid, const float* proj,
-                       const float* coords, const float* tables, int K, int B, MentPrior prior, float* out,
-                       cudaStream_t st, const Tables2D& t2 = Tables2D{0, 0, 0, nullptr, nullptr, nullptr, nullptr},
-                       const float* mp = nullptr, const float* mp2 = nullptr) {
-  const size_t smem = kMP ? ment_smem_mp(K, B, D) : ment_smem(K, B, D);
+// The 1-D family (k tables of b bins) and the 2-D family t2; behind kicks a non-empty family needs its multipole rows
+static bool tables_ok(int k, int b, const float* proj, const float* coords, const float* tables, const float* mp,
+                      const Tables2D& t2, const float* mp2, bool kick) {
+  if (k < 0 || (k > 0 && !(proj && coords && tables && b >= 2))) return false;
+  if (t2.k < 0 || (t2.k > 0 && !(t2.proj && t2.cx && t2.cy && t2.tab && t2.bx >= 2 && t2.by >= 2))) return false;
+  return !kick || ((k == 0 || mp) && (t2.k == 0 || mp2));
+}
+
+template <int D>
+static int launch_prob(int mode, bool kick, const float* x, int64_t G, const MentGrid& grid, const float* proj,
+                       const float* coords, const float* tables, int K, int B, const float* mp, const Tables2D& t2,
+                       const float* mp2, MentPrior prior, float* out, cudaStream_t st) {
+  const size_t smem = kick ? ment_smem_mp(K, B, D) : ment_smem(K, B, D);
   if (smem > 200 * 1024) return MFB_E_UNSUPPORTED;
   int64_t blocks = (G + kMentThreads - 1) / kMentThreads;
   int64_t cap = (int64_t)sm_count() * 8;
   const int gridx = (int)(blocks < cap ? blocks : cap);
-  if (mode == 0) {
-    MFB_CUDA(cudaFuncSetAttribute(ment_prob_kernel<D, 0, kMP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ment_prob_kernel<D, 0, kMP><<<gridx, kMentThreads, smem, st>>>(x, G, grid, proj, coords, tables, K, B, prior, t2, out,
-                                                                   mp, mp2);
-  } else {
-    MFB_CUDA(cudaFuncSetAttribute(ment_prob_kernel<D, 1, kMP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ment_prob_kernel<D, 1, kMP><<<gridx, kMentThreads, smem, st>>>(x, G, grid, proj, coords, tables, K, B, prior, t2, out,
-                                                                   mp, mp2);
-  }
+  const auto kernel = mode == 0 ? (kick ? ment_prob_kernel<D, 0, true> : ment_prob_kernel<D, 0, false>)
+                                : (kick ? ment_prob_kernel<D, 1, true> : ment_prob_kernel<D, 1, false>);
+  MFB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kernel<<<gridx, kMentThreads, smem, st>>>(x, G, grid, proj, coords, tables, K, B, prior, t2, out, mp, mp2);
   return launch_status();
 }
 
-static int check_tables2d(const Tables2D& t2) {
-  if (t2.k < 0) return MFB_E_BADARG;
-  if (t2.k > 0 && !(t2.proj && t2.cx && t2.cy && t2.tab && t2.bx >= 2 && t2.by >= 2)) return MFB_E_BADARG;
-  return 0;
-}
-
-template <int D, bool kMP = false>
-static int launch_integrate(const float* mc, int nb, int ax, const float* mc2, int nb2, int ax2, const MentGrid& grid,
-                            const float* minv, const float* proj, const float* coords, const float* tables, int k, int b,
-                            MentPrior pr, const Tables2D& t2, float* pred, cudaStream_t st, const float* mp = nullptr,
-                            const float* mp2 = nullptr, const float* imp = nullptr) {
-  const size_t smem = kMP ? ment_smem_mp(k, b, D) : ment_smem(k, b, D);
+template <int D>
+static int launch_integrate(bool kick, const float* mc, int nb, int ax, const float* mc2, int nb2, int ax2,
+                            const MentGrid& grid, const float* minv, const float* imp, const float* proj,
+                            const float* coords, const float* tables, int k, int b, const float* mp,
+                            const Tables2D& t2, const float* mp2, MentPrior pr, float* pred, cudaStream_t st) {
+  const size_t smem = kick ? ment_smem_mp(k, b, D) : ment_smem(k, b, D);
   if (smem > 200 * 1024) return MFB_E_UNSUPPORTED;
-  MFB_CUDA(cudaFuncSetAttribute(ment_integrate_kernel<D, kMP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const auto kernel = kick ? ment_integrate_kernel<D, true> : ment_integrate_kernel<D, false>;
+  MFB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int pixels = ax2 >= 0 ? nb * nb2 : nb;
-  ment_integrate_kernel<D, kMP><<<pixels, kMentThreads, smem, st>>>(mc, nb, ax, mc2, nb2, ax2, grid, minv, proj, coords,
-                                                                   tables, k, b, pr, t2, pred, mp, mp2, imp);
+  kernel<<<pixels, kMentThreads, smem, st>>>(mc, nb, ax, mc2, nb2, ax2, grid, minv, proj, coords, tables, k, b, pr, t2,
+                                             pred, mp, mp2, imp);
   return launch_status();
 }
 
@@ -617,95 +614,23 @@ using namespace mfb;
 
 extern "C" {
 
-#define MFB_DISPATCH_D(d, CALL)          \
-  switch (d) {                           \
-    case 1: return CALL(1);              \
-    case 2: return CALL(2);              \
-    case 3: return CALL(3);              \
-    case 4: return CALL(4);              \
-    case 5: return CALL(5);              \
-    case 6: return CALL(6);              \
-    case 7: return CALL(7);              \
-    default: return CALL(8);             \
-  }
-
-int mfb_ment_prob_nd(const float* x, int64_t g, int d, const float* proj, const float* coords, const float* tables,
-                     int k, int b, const float* proj2, const float* cx2, const float* cy2, const float* tables2, int k2,
-                     int bx, int by, float prior_neg_half_inv_s2, float prior_log_norm, float* out, void* stream) {
-  MFB_CHECK_ARG(x && out && g >= 0 && k >= 0 && d >= 1 && d <= kMaxDim);
-  MFB_CHECK_ARG(k == 0 || (proj && coords && tables && b >= 2));
+// rho at the g points x (mode 0) or on the g cells of `grid` (mode 1): the body of mfb_ment_prob and mfb_ment_prob_grid
+static int ment_prob_impl(int mode, const float* x, int64_t g, const MentGrid& grid, int d, const float* proj,
+                          const float* coords, const float* tables, int k, int b, const float* mp, const float* proj2,
+                          const float* cx2, const float* cy2, const float* tables2, int k2, int bx, int by,
+                          const float* mp2, float prior_neg_half_inv_s2, float prior_log_norm, float* out,
+                          void* stream) {
+  const bool kick = mp || mp2;
+  MFB_CHECK_ARG(out && d >= 1 && d <= kMaxDim);
   const Tables2D t2{k2, bx, by, proj2, cx2, cy2, tables2};
-  if (check_tables2d(t2)) return MFB_E_BADARG;
+  MFB_CHECK_ARG(tables_ok(k, b, proj, coords, tables, mp, t2, mp2, kick));
   if (g == 0) return 0;
   if (k == 0) b = 2;
-  MentPrior pr{prior_neg_half_inv_s2, prior_log_norm};
-  MentGrid grid = make_grid(0, nullptr, nullptr, nullptr);
+  const MentPrior pr{prior_neg_half_inv_s2, prior_log_norm};
   cudaStream_t st = (cudaStream_t)stream;
-#define MFB_CALL(DD) launch_prob<DD>(0, x, g, grid, proj, coords, tables, k, b, pr, out, st, t2)
-  MFB_DISPATCH_D(d, MFB_CALL)
-#undef MFB_CALL
-}
-
-int mfb_ment_prob(const float* x, int64_t g, int d, const float* proj, const float* coords, const float* tables,
-                  int k, int b, float prior_neg_half_inv_s2, float prior_log_norm, float* out, void* stream) {
-  MFB_CHECK_ARG(proj && coords && tables && b >= 2);
-  return mfb_ment_prob_nd(x, g, d, proj, coords, tables, k, b, nullptr, nullptr, nullptr, nullptr, 0, 0, 0,
-                          prior_neg_half_inv_s2, prior_log_norm, out, stream);
-}
-
-int mfb_ment_prob_grid_nd(int d, const int32_t* shape_host, const float* first_centre_host, const float* step_host,
-                          const float* proj, const float* coords, const float* tables, int k, int b,
-                          const float* proj2, const float* cx2, const float* cy2, const float* tables2, int k2, int bx,
-                          int by, float prior_neg_half_inv_s2, float prior_log_norm, float* out, void* stream) {
-  MFB_CHECK_ARG(shape_host && first_centre_host && step_host && out);
-  MFB_CHECK_ARG(k >= 0 && d >= 1 && d <= kMaxDim);
-  MFB_CHECK_ARG(k == 0 || (proj && coords && tables && b >= 2));
-  const Tables2D t2{k2, bx, by, proj2, cx2, cy2, tables2};
-  if (check_tables2d(t2)) return MFB_E_BADARG;
-  if (k == 0) b = 2;
-  int64_t g = 1;
-  for (int i = 0; i < d; ++i) {
-    MFB_CHECK_ARG(shape_host[i] >= 1);
-    g *= shape_host[i];
-  }
-  MentPrior pr{prior_neg_half_inv_s2, prior_log_norm};
-  MentGrid grid = make_grid(d, shape_host, first_centre_host, step_host);
-  cudaStream_t st = (cudaStream_t)stream;
-#define MFB_CALL(DD) launch_prob<DD>(1, nullptr, g, grid, proj, coords, tables, k, b, pr, out, st, t2)
-  MFB_DISPATCH_D(d, MFB_CALL)
-#undef MFB_CALL
-}
-
-int mfb_ment_prob_grid(int d, const int32_t* shape_host, const float* first_centre_host, const float* step_host,
-                       const float* proj, const float* coords, const float* tables, int k, int b,
-                       float prior_neg_half_inv_s2, float prior_log_norm, float* out, void* stream) {
-  MFB_CHECK_ARG(proj && coords && tables && b >= 2);
-  return mfb_ment_prob_grid_nd(d, shape_host, first_centre_host, step_host, proj, coords, tables, k, b, nullptr, nullptr,
-                               nullptr, nullptr, 0, 0, 0, prior_neg_half_inv_s2, prior_log_norm, out, stream);
-}
-
-int mfb_ment_integrate_nd(int d, const float* meas_coords, int nb_meas, int meas_axis, const float* meas_coords2,
-                          int nb_meas2, int meas_axis2, int n_int_axes, const int32_t* int_shape_host,
-                          const float* int_first_host, const float* int_step_host, const float* minv, const float* proj,
-                          const float* coords, const float* tables, int k, int b, const float* proj2, const float* cx2,
-                          const float* cy2, const float* tables2, int k2, int bx, int by, float prior_neg_half_inv_s2,
-                          float prior_log_norm, float* pred, void* stream) {
-  MFB_CHECK_ARG(meas_coords && minv && pred && int_shape_host && int_first_host && int_step_host);
-  MFB_CHECK_ARG(k >= 0 && (k == 0 || (proj && coords && tables && b >= 2)));
-  const int n_meas = meas_axis2 >= 0 ? 2 : 1;
-  MFB_CHECK_ARG(d >= 2 && d <= kMaxDim && n_int_axes == d - n_meas && n_int_axes >= 1);
-  MFB_CHECK_ARG(meas_axis >= 0 && meas_axis < d && nb_meas >= 1 && meas_axis2 < d && meas_axis2 != meas_axis);
-  MFB_CHECK_ARG(meas_axis2 < 0 || (meas_coords2 && nb_meas2 >= 1));
-  const Tables2D t2{k2, bx, by, proj2, cx2, cy2, tables2};
-  if (check_tables2d(t2)) return MFB_E_BADARG;
-  if (k == 0) b = 2;
-  MentPrior pr{prior_neg_half_inv_s2, prior_log_norm};
-  MentGrid grid = make_grid(n_int_axes, int_shape_host, int_first_host, int_step_host);
-  cudaStream_t st = (cudaStream_t)stream;
-#define MFB_CALL(DD)                                                                                                    \
-  launch_integrate<DD>(meas_coords, nb_meas, meas_axis, meas_coords2, nb_meas2, meas_axis2, grid, minv, proj, coords, \
-                       tables, k, b, pr, t2, pred, st)
+#define MFB_CALL(DD) launch_prob<DD>(mode, kick, x, g, grid, proj, coords, tables, k, b, mp, t2, mp2, pr, out, st)
   switch (d) {
+    case 1: return MFB_CALL(1);
     case 2: return MFB_CALL(2);
     case 3: return MFB_CALL(3);
     case 4: return MFB_CALL(4);
@@ -717,83 +642,53 @@ int mfb_ment_integrate_nd(int d, const float* meas_coords, int nb_meas, int meas
 #undef MFB_CALL
 }
 
-int mfb_ment_integrate(int d, const float* meas_coords, int nb_meas, int meas_axis, int n_int_axes,
-                       const int32_t* int_shape_host, const float* int_first_host, const float* int_step_host,
-                       const float* minv, const float* proj, const float* coords, const float* tables, int k,
-                       int b, float prior_neg_half_inv_s2, float prior_log_norm, float* pred, void* stream) {
-  MFB_CHECK_ARG(proj && coords && tables && b >= 2);
-  return mfb_ment_integrate_nd(d, meas_coords, nb_meas, meas_axis, nullptr, 0, -1, n_int_axes, int_shape_host,
-                               int_first_host, int_step_host, minv, proj, coords, tables, k, b, nullptr, nullptr,
-                               nullptr, nullptr, 0, 0, 0, prior_neg_half_inv_s2, prior_log_norm, pred, stream);
+int mfb_ment_prob(const float* x, int64_t g, int d, const float* proj, const float* coords, const float* tables, int k,
+                  int b, const float* mp, const float* proj2, const float* cx2, const float* cy2, const float* tables2,
+                  int k2, int bx, int by, const float* mp2, float prior_neg_half_inv_s2, float prior_log_norm,
+                  float* out, void* stream) {
+  MFB_CHECK_ARG(x && g >= 0);
+  return ment_prob_impl(0, x, g, make_grid(0, nullptr, nullptr, nullptr), d, proj, coords, tables, k, b, mp, proj2,
+                        cx2, cy2, tables2, k2, bx, by, mp2, prior_neg_half_inv_s2, prior_log_norm, out, stream);
 }
 
-int mfb_ment_prob_nd_mp(const float* x, int64_t g, int d, const float* proj, const float* coords, const float* tables,
-                        int k, int b, const float* mp, const float* proj2, const float* cx2, const float* cy2,
-                        const float* tables2, int k2, int bx, int by, const float* mp2, float prior_neg_half_inv_s2,
-                        float prior_log_norm, float* out, void* stream) {
-  MFB_CHECK_ARG(x && out && g >= 0 && k >= 0 && d >= 1 && d <= kMaxDim);
-  MFB_CHECK_ARG(k == 0 || (proj && coords && tables && mp && b >= 2));
-  const Tables2D t2{k2, bx, by, proj2, cx2, cy2, tables2};
-  if (check_tables2d(t2)) return MFB_E_BADARG;
-  MFB_CHECK_ARG(k2 == 0 || mp2);
-  if (g == 0) return 0;
-  if (k == 0) b = 2;
-  MentPrior pr{prior_neg_half_inv_s2, prior_log_norm};
-  MentGrid grid = make_grid(0, nullptr, nullptr, nullptr);
-  cudaStream_t st = (cudaStream_t)stream;
-#define MFB_CALL(DD) launch_prob<DD, true>(0, x, g, grid, proj, coords, tables, k, b, pr, out, st, t2, mp, mp2)
-  MFB_DISPATCH_D(d, MFB_CALL)
-#undef MFB_CALL
-}
-
-int mfb_ment_prob_grid_nd_mp(int d, const int32_t* shape_host, const float* first_centre_host, const float* step_host,
-                             const float* proj, const float* coords, const float* tables, int k, int b, const float* mp,
-                             const float* proj2, const float* cx2, const float* cy2, const float* tables2, int k2,
-                             int bx, int by, const float* mp2, float prior_neg_half_inv_s2, float prior_log_norm,
-                             float* out, void* stream) {
-  MFB_CHECK_ARG(shape_host && first_centre_host && step_host && out);
-  MFB_CHECK_ARG(k >= 0 && d >= 1 && d <= kMaxDim);
-  MFB_CHECK_ARG(k == 0 || (proj && coords && tables && mp && b >= 2));
-  const Tables2D t2{k2, bx, by, proj2, cx2, cy2, tables2};
-  if (check_tables2d(t2)) return MFB_E_BADARG;
-  MFB_CHECK_ARG(k2 == 0 || mp2);
-  if (k == 0) b = 2;
+int mfb_ment_prob_grid(int d, const int32_t* shape_host, const float* first_centre_host, const float* step_host,
+                       const float* proj, const float* coords, const float* tables, int k, int b, const float* mp,
+                       const float* proj2, const float* cx2, const float* cy2, const float* tables2, int k2, int bx,
+                       int by, const float* mp2, float prior_neg_half_inv_s2, float prior_log_norm, float* out,
+                       void* stream) {
+  MFB_CHECK_ARG(shape_host && first_centre_host && step_host && d >= 1 && d <= kMaxDim);
   int64_t g = 1;
   for (int i = 0; i < d; ++i) {
     MFB_CHECK_ARG(shape_host[i] >= 1);
     g *= shape_host[i];
   }
-  MentPrior pr{prior_neg_half_inv_s2, prior_log_norm};
-  MentGrid grid = make_grid(d, shape_host, first_centre_host, step_host);
-  cudaStream_t st = (cudaStream_t)stream;
-#define MFB_CALL(DD) launch_prob<DD, true>(1, nullptr, g, grid, proj, coords, tables, k, b, pr, out, st, t2, mp, mp2)
-  MFB_DISPATCH_D(d, MFB_CALL)
-#undef MFB_CALL
+  return ment_prob_impl(1, nullptr, g, make_grid(d, shape_host, first_centre_host, step_host), d, proj, coords, tables,
+                        k, b, mp, proj2, cx2, cy2, tables2, k2, bx, by, mp2, prior_neg_half_inv_s2, prior_log_norm,
+                        out, stream);
 }
 
-int mfb_ment_integrate_nd_mp(int d, const float* meas_coords, int nb_meas, int meas_axis, const float* meas_coords2,
-                             int nb_meas2, int meas_axis2, int n_int_axes, const int32_t* int_shape_host,
-                             const float* int_first_host, const float* int_step_host, const float* linv,
-                             const float* inv_mp, const float* proj, const float* coords, const float* tables, int k,
-                             int b, const float* mp, const float* proj2, const float* cx2, const float* cy2,
-                             const float* tables2, int k2, int bx, int by, const float* mp2,
-                             float prior_neg_half_inv_s2, float prior_log_norm, float* pred, void* stream) {
-  MFB_CHECK_ARG(meas_coords && linv && inv_mp && pred && int_shape_host && int_first_host && int_step_host);
-  MFB_CHECK_ARG(k >= 0 && (k == 0 || (proj && coords && tables && mp && b >= 2)));
+int mfb_ment_integrate(int d, const float* meas_coords, int nb_meas, int meas_axis, const float* meas_coords2,
+                       int nb_meas2, int meas_axis2, int n_int_axes, const int32_t* int_shape_host,
+                       const float* int_first_host, const float* int_step_host, const float* linv, const float* inv_mp,
+                       const float* proj, const float* coords, const float* tables, int k, int b, const float* mp,
+                       const float* proj2, const float* cx2, const float* cy2, const float* tables2, int k2, int bx,
+                       int by, const float* mp2, float prior_neg_half_inv_s2, float prior_log_norm, float* pred,
+                       void* stream) {
+  const bool kick = mp || mp2 || inv_mp;
+  MFB_CHECK_ARG(meas_coords && linv && (inv_mp || !kick) && pred && int_shape_host && int_first_host && int_step_host);
   const int n_meas = meas_axis2 >= 0 ? 2 : 1;
   MFB_CHECK_ARG(d >= 2 && d <= kMaxDim && n_int_axes == d - n_meas && n_int_axes >= 1);
   MFB_CHECK_ARG(meas_axis >= 0 && meas_axis < d && nb_meas >= 1 && meas_axis2 < d && meas_axis2 != meas_axis);
   MFB_CHECK_ARG(meas_axis2 < 0 || (meas_coords2 && nb_meas2 >= 1));
   const Tables2D t2{k2, bx, by, proj2, cx2, cy2, tables2};
-  if (check_tables2d(t2)) return MFB_E_BADARG;
-  MFB_CHECK_ARG(k2 == 0 || mp2);
+  MFB_CHECK_ARG(tables_ok(k, b, proj, coords, tables, mp, t2, mp2, kick));
   if (k == 0) b = 2;
-  MentPrior pr{prior_neg_half_inv_s2, prior_log_norm};
-  MentGrid grid = make_grid(n_int_axes, int_shape_host, int_first_host, int_step_host);
+  const MentPrior pr{prior_neg_half_inv_s2, prior_log_norm};
+  const MentGrid grid = make_grid(n_int_axes, int_shape_host, int_first_host, int_step_host);
   cudaStream_t st = (cudaStream_t)stream;
-#define MFB_CALL(DD)                                                                                                 \
-  launch_integrate<DD, true>(meas_coords, nb_meas, meas_axis, meas_coords2, nb_meas2, meas_axis2, grid, linv, proj, \
-                             coords, tables, k, b, pr, t2, pred, st, mp, mp2, inv_mp)
+#define MFB_CALL(DD)                                                                                                   \
+  launch_integrate<DD>(kick, meas_coords, nb_meas, meas_axis, meas_coords2, nb_meas2, meas_axis2, grid, linv, inv_mp, \
+                       proj, coords, tables, k, b, mp, t2, mp2, pr, pred, st)
   switch (d) {
     case 2: return MFB_CALL(2);
     case 3: return MFB_CALL(3);

@@ -663,10 +663,11 @@ int64_t mfb_nsf_layer_param_om_floats(int d, int hidden_units, int hidden_layers
   return (int64_t)kH * d + (int64_t)(hidden_layers - 1) * kH * kH + (int64_t)d * kPP * kH;
 }
 
-static int layer_bwd_impl(const float* v, const float* gy, const float* glogq, int64_t n, int d, int hidden_units,
+int mfb_nsf_layer_bwd_img(const float* v, const float* gy, const float* glogq, int64_t n, int d, int hidden_units,
                           int hidden_layers, int bins, const float* params, const float* params_om,
-                          const int32_t* order_host, int first_layer, const void* tc_image, float* gv, float* gparams,
-                          int accumulate, void* workspace, int64_t workspace_bytes, int flags, void* stream) {
+                          const int32_t* order_host, int first_layer, const void* tc_image, float* gv,
+                          float* gparams, int accumulate, void* workspace, int64_t workspace_bytes, int flags,
+                          void* stream) {
   MFB_CHECK_ARG(v && gy && params && params_om && gv && gparams && workspace && n >= 1);
   if (hidden_units != kH || hidden_layers < 1 || bins < 2 || 3 * bins - 1 > kPP || d < 2 || d > 6)
     return MFB_E_UNSUPPORTED;
@@ -687,23 +688,6 @@ static int layer_bwd_impl(const float* v, const float* gy, const float* glogq, i
     default: return MFB_E_UNSUPPORTED;
   }
 #undef MFB_BWD
-}
-
-int mfb_nsf_layer_bwd(const float* v, const float* gy, const float* glogq, int64_t n, int d, int hidden_units,
-                      int hidden_layers, int bins, const float* params, const float* params_om,
-                      const int32_t* order_host, int first_layer, float* gv, float* gparams, int accumulate,
-                      void* workspace, int64_t workspace_bytes, int flags, void* stream) {
-  return layer_bwd_impl(v, gy, glogq, n, d, hidden_units, hidden_layers, bins, params, params_om, order_host,
-                        first_layer, nullptr, gv, gparams, accumulate, workspace, workspace_bytes, flags, stream);
-}
-
-int mfb_nsf_layer_bwd_img(const float* v, const float* gy, const float* glogq, int64_t n, int d, int hidden_units,
-                          int hidden_layers, int bins, const float* params, const float* params_om,
-                          const int32_t* order_host, int first_layer, const void* tc_image, float* gv,
-                          float* gparams, int accumulate, void* workspace, int64_t workspace_bytes, int flags,
-                          void* stream) {
-  return layer_bwd_impl(v, gy, glogq, n, d, hidden_units, hidden_layers, bins, params, params_om, order_host,
-                        first_layer, tc_image, gv, gparams, accumulate, workspace, workspace_bytes, flags, stream);
 }
 
 }  // extern "C"

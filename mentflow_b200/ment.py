@@ -57,12 +57,12 @@ class LagrangeFunction:
         if self.values.ndim == 1:
             u = u.reshape(-1, 1).to(torch.float32)
             one = torch.ones((1, 1), dtype=torch.float32, device=u.device)
-            return ops.ment_prob(u, one, self.coords.reshape(1, -1).to(u.device),
-                                 self.values.reshape(1, -1).to(u.device), 0.0, 0.0)
+            coords, values = (t.reshape(1, -1).to(u.device) for t in (self.coords, self.values))
+            return ops.ment_prob(u, (one, coords, values), None, 0.0, 0.0)
         u = u.reshape(-1, 2).to(torch.float32)
         eye = torch.eye(2, dtype=torch.float32, device=u.device).reshape(1, 2, 2)
         cx, cy = (c.reshape(1, -1).to(u.device) for c in self.coords)
-        return ops.ment_prob_nd(u, None, (eye, cx, cy, self.values.to(u.device)[None]), 0.0, 0.0)
+        return ops.ment_prob(u, None, (eye, cx, cy, self.values.to(u.device)[None]), 0.0, 0.0)
 
 
 class MENT:
@@ -197,7 +197,7 @@ class MENT:
         return self._packed
 
     def _groups(self, device):
-        """(g1, g2) for ``ops.ment_prob_nd``: the current tables of the two screen families, followed by their
+        """(g1, g2) for ``ops.ment_prob``: the current tables of the two screen families, followed by their
         multipole rows when the model has a kick."""
         pk = self._pack(device)
 
@@ -244,15 +244,15 @@ class MENT:
         """rho(x) (ment.py:239-249)."""
         g1, g2 = self._groups(x.device)
         a, b = self._prior_args()
-        return ops.ment_prob_nd(x, g1, g2, a, b)
+        return ops.ment_prob(x, g1, g2, a, b)
 
     def prob_on_grid(self, sampler) -> torch.Tensor:
         """rho on the cell centres of a GridSampler grid, straight from the grid index."""
         device = torch.device(self.device if self.device is not None else "cuda")
         g1, g2 = self._groups(device)
         a, b = self._prior_args()
-        return ops.ment_prob_grid_nd(list(sampler.shape), sampler.first_centres(), sampler.cell_sizes(), g1, g2, a, b,
-                                     device)
+        return ops.ment_prob_grid(list(sampler.shape), sampler.first_centres(), sampler.cell_sizes(), g1, g2, a, b,
+                                  device)
 
     def log_prob(self, x: torch.Tensor, pad: float = 1.0e-12) -> torch.Tensor:
         return torch.log(self.prob(x) + pad)
@@ -315,12 +315,12 @@ class MENT:
             cx = coords_from_edges(diagnostic.edges_x.to(torch.float32)).to(device)
             cy = coords_from_edges(diagnostic.edges_y.to(torch.float32)).to(device)
             ax, ay = diagnostic.axis
-            pred = ops.ment_integrate_nd(self.ndim, cx, ax, cy, ay, shape, first, step, minv, g1, g2, a, b,
-                                         inv_mp=inv_mp)
+            pred = ops.ment_integrate(self.ndim, cx, ax, cy, ay, shape, first, step, minv, g1, g2, a, b,
+                                      inv_mp=inv_mp)
         else:
             meas_coords = coords_from_edges(diagnostic.edges.to(torch.float32)).to(device)
-            pred = ops.ment_integrate_nd(self.ndim, meas_coords, diagnostic.axis, None, -1, shape, first, step, minv,
-                                         g1, g2, a, b, inv_mp=inv_mp)
+            pred = ops.ment_integrate(self.ndim, meas_coords, diagnostic.axis, None, -1, shape, first, step, minv,
+                                      g1, g2, a, b, inv_mp=inv_mp)
         return self.normalize_projection(pred, index, diag_index)
 
     def _simulate_sample(self, index: int, diag_index: int) -> torch.Tensor:

@@ -772,63 +772,14 @@ def _host_f32(values):
     return arr, ctypes.cast(arr, ctypes.c_void_p)
 
 
-def ment_prob(x, proj, coords, tables, neg_half_inv_s2: float, log_norm: float) -> torch.Tensor:
-    """rho at explicit points x (G, D); proj (K, D), coords / tables (K, B)."""
-    lib = _lib.load()
-    x, proj = _check_f32("x", x), _check_f32("proj", proj)
-    coords, tables = _check_f32("coords", coords), _check_f32("tables", tables)
-    g, d = x.shape
-    k, b = tables.shape
-    out = torch.empty(g, dtype=torch.float32, device=x.device)
-    with torch.cuda.device(x.device):
-        _lib.check(lib.mfb_ment_prob(_ptr(x), g, d, _ptr(proj), _ptr(coords), _ptr(tables), k, b,
-                                     float(neg_half_inv_s2), float(log_norm), _ptr(out), _stream()), "ment_prob")
-    return out
-
-
-def ment_prob_grid(shape, first_centre, step, proj, coords, tables, neg_half_inv_s2, log_norm) -> torch.Tensor:
-    """rho on the centres of a regular grid (flattened, 'ij' order) without materialising the points."""
-    lib = _lib.load()
-    proj, coords, tables = _check_f32("proj", proj), _check_f32("coords", coords), _check_f32("tables", tables)
-    d = len(shape)
-    k, b = tables.shape
-    g = 1
-    for s in shape:
-        g *= int(s)
-    out = torch.empty(g, dtype=torch.float32, device=proj.device)
-    a1, p1 = _host_i32(shape)
-    a2, p2 = _host_f32(first_centre)
-    a3, p3 = _host_f32(step)
-    with torch.cuda.device(proj.device):
-        _lib.check(lib.mfb_ment_prob_grid(d, p1, p2, p3, _ptr(proj), _ptr(coords), _ptr(tables), k, b,
-                                          float(neg_half_inv_s2), float(log_norm), _ptr(out), _stream()),
-                   "ment_prob_grid")
-    return out
-
-
-def ment_integrate(d, meas_coords, meas_axis, int_shape, int_first, int_step, minv, proj, coords, tables,
-                   neg_half_inv_s2, log_norm) -> torch.Tensor:
-    lib = _lib.load()
-    meas_coords, minv = _check_f32("meas_coords", meas_coords), _check_f32("minv", minv)
-    proj, coords, tables = _check_f32("proj", proj), _check_f32("coords", coords), _check_f32("tables", tables)
-    k, b = tables.shape
-    nb = meas_coords.shape[0]
-    pred = torch.empty(nb, dtype=torch.float32, device=proj.device)
-    a1, p1 = _host_i32(int_shape)
-    a2, p2 = _host_f32(int_first)
-    a3, p3 = _host_f32(int_step)
-    with torch.cuda.device(proj.device):
-        _lib.check(lib.mfb_ment_integrate(d, _ptr(meas_coords), nb, int(meas_axis), len(int_shape), p1, p2, p3,
-                                          _ptr(minv), _ptr(proj), _ptr(coords), _ptr(tables), k, b,
-                                          float(neg_half_inv_s2), float(log_norm), _ptr(pred), _stream()),
-                   "ment_integrate")
-    return pred
-
-
-def _ment_groups(g1, g2, device):
-    """C-ABI arguments of the two table families: g1 = (proj (K,D), coords (K,B), tables (K,B)[, mp]) or None,
-    g2 = (proj2 (K2,2,D), cx (K2,Bx), cy (K2,By), tables2 (K2,Bx,By)[, mp2]) or None.  The optional multipole rows
-    are read by ``_ment_mp_args``."""
+def _ment_tables(g1, g2, d: int, device, kick: bool = False):
+    """C-ABI arguments of the two table families in ABI order (proj, coords, tables, k, b, mp, proj2, cx, cy, tables2,
+    k2, bx, by, mp2), the tensors they point into, and whether the model has kicks.
+    g1 = (proj (K,D), coords (K,B), tables (K,B)[, mp (K,2D+4)]) or None,
+    g2 = (proj2 (K2,2,D), cx (K2,Bx), cy (K2,By), tables2 (K2,Bx,By)[, mp2 (K2,2,2D+4)]) or None.
+    The optional multipole rows have the layout of ``simulate.multipole_terms``, order 0 for the rows of linear maps.
+    The model has kicks when either family carries rows or ``kick`` is set; then a family without rows gets order-0
+    rows.  A linear model passes NULL for both."""
     keep = []
     if g1 is not None:
         proj, coords, tables = (_check_f32(n, t) for n, t in zip(("proj", "coords", "tables"), g1))
@@ -844,22 +795,14 @@ def _ment_groups(g1, g2, device):
         a2 = [_ptr(proj2), _ptr(cx), _ptr(cy), _ptr(tab2), tab2.shape[0], tab2.shape[1], tab2.shape[2]]
     else:
         a2 = [None, None, None, None, 0, 0, 0]
-    return a1, a2, keep
-
-
-def _ment_mp_args(g1, g2, d: int, device, keep: list, force: bool = False):
-    """(mp, mp2) pointers of the multipole rows carried as the optional last element of g1 (mp (K, 2D+4)) and g2
-    (mp2 (K2, 2, 2D+4)); layout of ``simulate.multipole_terms``, order 0 for the rows of linear maps.  None when
-    neither family carries rows (and not ``force``): the model is linear.  A family without rows gets order-0 rows."""
     mp1 = g1[3] if g1 is not None and len(g1) > 3 else None
     mp2 = g2[4] if g2 is not None and len(g2) > 4 else None
-    if mp1 is None and mp2 is None and not force:
-        return None
+    kick = kick or mp1 is not None or mp2 is not None
+    rows = []
     stride = 2 * d + 4
-    ptrs = []
     for mp, grp, lead, name in ((mp1, g1, (), "mp"), (mp2, g2, (2,), "mp2")):
-        if grp is None:
-            ptrs.append(None)
+        if not kick or grp is None:
+            rows.append(None)
             continue
         k = int(grp[0].shape[0])
         if mp is None:
@@ -869,53 +812,44 @@ def _ment_mp_args(g1, g2, d: int, device, keep: list, force: bool = False):
             raise ValueError(f"MENT multipole rows {name} must have shape {(k,) + lead + (stride,)}, "
                              f"got {tuple(mp.shape)}")
         keep.append(mp)
-        ptrs.append(_ptr(mp))
-    return ptrs
+        rows.append(_ptr(mp))
+    return a1 + [rows[0]] + a2 + [rows[1]], keep, kick
 
 
-def ment_prob_nd(x, g1, g2, neg_half_inv_s2: float, log_norm: float) -> torch.Tensor:
-    """rho at explicit points with one- and two-dimensional Lagrange tables (see ``_ment_groups``); with multipole
-    rows in g1 / g2 the projections take the kicks (``_ment_mp_args``)."""
+def ment_prob(x, g1, g2, neg_half_inv_s2: float, log_norm: float) -> torch.Tensor:
+    """rho at explicit points x (G, D) with one- and two-dimensional Lagrange tables and, when g1 / g2 carry
+    multipole rows, the kicks (see ``_ment_tables``)."""
     lib = _lib.load()
     x = _check_f32("x", x)
     g, d = x.shape
-    a1, a2, keep = _ment_groups(g1, g2, x.device)
-    mp = _ment_mp_args(g1, g2, d, x.device, keep)
+    args, keep, _ = _ment_tables(g1, g2, d, x.device)
     out = torch.empty(g, dtype=torch.float32, device=x.device)
     with torch.cuda.device(x.device):
-        if mp is None:
-            _lib.check(lib.mfb_ment_prob_nd(_ptr(x), g, d, *a1, *a2, float(neg_half_inv_s2), float(log_norm),
-                                            _ptr(out), _stream()), "ment_prob_nd")
-        else:
-            _lib.check(lib.mfb_ment_prob_nd_mp(_ptr(x), g, d, *a1, mp[0], *a2, mp[1], float(neg_half_inv_s2),
-                                               float(log_norm), _ptr(out), _stream()), "ment_prob_nd_mp")
+        _lib.check(lib.mfb_ment_prob(_ptr(x), g, d, *args, float(neg_half_inv_s2), float(log_norm), _ptr(out),
+                                     _stream()), "ment_prob")
     return out
 
 
-def ment_prob_grid_nd(shape, first_centre, step, g1, g2, neg_half_inv_s2, log_norm, device) -> torch.Tensor:
+def ment_prob_grid(shape, first_centre, step, g1, g2, neg_half_inv_s2, log_norm, device) -> torch.Tensor:
+    """rho on the centres of a regular grid (flattened, 'ij' order) without materialising the points."""
     lib = _lib.load()
     d = len(shape)
     g = 1
     for s_ in shape:
         g *= int(s_)
-    a1, a2, keep = _ment_groups(g1, g2, device)
-    mp = _ment_mp_args(g1, g2, d, device, keep)
+    args, keep, _ = _ment_tables(g1, g2, d, device)
     out = torch.empty(g, dtype=torch.float32, device=device)
     h1, p1 = _host_i32(shape)
     h2, p2 = _host_f32(first_centre)
     h3, p3 = _host_f32(step)
     with torch.cuda.device(device):
-        if mp is None:
-            _lib.check(lib.mfb_ment_prob_grid_nd(d, p1, p2, p3, *a1, *a2, float(neg_half_inv_s2), float(log_norm),
-                                                 _ptr(out), _stream()), "ment_prob_grid_nd")
-        else:
-            _lib.check(lib.mfb_ment_prob_grid_nd_mp(d, p1, p2, p3, *a1, mp[0], *a2, mp[1], float(neg_half_inv_s2),
-                                                    float(log_norm), _ptr(out), _stream()), "ment_prob_grid_nd_mp")
+        _lib.check(lib.mfb_ment_prob_grid(d, p1, p2, p3, *args, float(neg_half_inv_s2), float(log_norm), _ptr(out),
+                                          _stream()), "ment_prob_grid")
     return out
 
 
-def ment_integrate_nd(d, meas_coords, meas_axis, meas_coords2, meas_axis2, int_shape, int_first, int_step, minv, g1, g2,
-                      neg_half_inv_s2, log_norm, inv_mp: Optional[torch.Tensor] = None) -> torch.Tensor:
+def ment_integrate(d, meas_coords, meas_axis, meas_coords2, meas_axis2, int_shape, int_first, int_step, minv, g1, g2,
+                   neg_half_inv_s2, log_norm, inv_mp: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Integration-mode prediction of one screen: 1-D (meas_axis2 = -1) -> (B,), 2-D -> (Bx, By).  The screen is mapped
     back with ``minv``; with ``inv_mp`` (4D+2,) = [r0 | r2 | p | q | order | 0] (``simulate.multipole_inverse_terms``)
     the map back is ``minv u + p Re(z^m) + q Im(z^m)``, z = r0 . u + i r2 . u.  Multipole rows in g1 / g2 or an
@@ -929,9 +863,8 @@ def ment_integrate_nd(d, meas_coords, meas_axis, meas_coords2, meas_axis2, int_s
     if meas_axis2 >= 0:
         meas_coords2 = _check_f32("meas_coords2", meas_coords2)
         nb2 = meas_coords2.shape[0]
-    a1, a2, keep = _ment_groups(g1, g2, minv.device)
-    mp = _ment_mp_args(g1, g2, d, minv.device, keep, force=inv_mp is not None)
-    if mp is not None:
+    args, keep, kick = _ment_tables(g1, g2, d, minv.device, kick=inv_mp is not None)
+    if kick:
         if inv_mp is None:
             inv_mp = torch.zeros(4 * d + 2, dtype=torch.float32, device=minv.device)
         inv_mp = _check_f32("inv_mp", inv_mp)
@@ -943,16 +876,10 @@ def ment_integrate_nd(d, meas_coords, meas_axis, meas_coords2, meas_axis2, int_s
     h3, p3 = _host_f32(int_step)
     mc2 = _ptr(meas_coords2) if meas_axis2 >= 0 else None
     with torch.cuda.device(minv.device):
-        if mp is None:
-            _lib.check(lib.mfb_ment_integrate_nd(d, _ptr(meas_coords), nb, int(meas_axis), mc2, nb2, int(meas_axis2),
-                                                 len(int_shape), p1, p2, p3, _ptr(minv), *a1, *a2,
-                                                 float(neg_half_inv_s2), float(log_norm), _ptr(pred), _stream()),
-                       "ment_integrate_nd")
-        else:
-            _lib.check(lib.mfb_ment_integrate_nd_mp(d, _ptr(meas_coords), nb, int(meas_axis), mc2, nb2,
-                                                    int(meas_axis2), len(int_shape), p1, p2, p3, _ptr(minv),
-                                                    _ptr(inv_mp), *a1, mp[0], *a2, mp[1], float(neg_half_inv_s2),
-                                                    float(log_norm), _ptr(pred), _stream()), "ment_integrate_nd_mp")
+        _lib.check(lib.mfb_ment_integrate(d, _ptr(meas_coords), nb, int(meas_axis), mc2, nb2, int(meas_axis2),
+                                          len(int_shape), p1, p2, p3, _ptr(minv), _ptr(inv_mp), *args,
+                                          float(neg_half_inv_s2), float(log_norm), _ptr(pred), _stream()),
+                   "ment_integrate")
     return pred
 
 

@@ -16,7 +16,7 @@ from oracle.zuko_nsf import layer_order, masked_mlp_masks
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_library_exports_every_declared_symbol():
+def test_library_exports_every_declared_symbol_at_the_header_abi_version():
     header = open(os.path.join(ROOT, "include", "mentflow_b200.h")).read()
     declared = set(re.findall(r"\b(mfb_[a-z0-9_]+)\s*\(", header))
     assert declared, "no declarations parsed"
@@ -24,7 +24,8 @@ def test_library_exports_every_declared_symbol():
     for name in sorted(declared):
         assert hasattr(lib, name), f"{name} declared in the header but not exported"
     assert declared == set(_lib.SIGNATURES), "ctypes table and header disagree"
-    assert lib.mfb_abi_version() == 2
+    version = int(re.search(r"#define MFB_ABI_VERSION (\d+)", header).group(1))
+    assert lib.mfb_abi_version() == version == _lib.ABI_VERSION == 3
     assert b"workspace" in lib.mfb_error_string(-3)
 
 
@@ -212,6 +213,45 @@ def test_tensor_core_flow_host_side_contract():
     rc = lib.mfb_nsf_tc_layer_fwd(dummy, 10, 6, 64, 2, 20, dummy, ctypes.cast(bad_order, ctypes.c_void_p), None, 1,
                                   dummy, None, None)
     assert rc == -2                                             # hidden_layers = 2 is not compiled for tcgen05
+
+
+def test_ment_entry_points_refuse_bad_arguments(monkeypatch):
+    """Argument checks of the classical MENT entry points (dummy device pointers: every call fails before any CUDA
+    call), and the refusal of a library built for another ABI version."""
+    import ctypes
+    lib = _lib.load()
+    dummy = ctypes.c_void_p(16)
+    shape = (ctypes.c_int32 * 4)(8, 8, 8, 8)
+    first = (ctypes.c_float * 4)(0.0, 0.0, 0.0, 0.0)
+    step = (ctypes.c_float * 4)(0.1, 0.1, 0.1, 0.1)
+    hp = [ctypes.cast(a, ctypes.c_void_p) for a in (shape, first, step)]
+
+    def tables(mp=None, mp2=None):
+        # 1-D family: k = 3 tables of 8 bins; 2-D family: k2 = 2 tables of 8 x 8 bins
+        return [dummy, dummy, dummy, 3, 8, mp, dummy, dummy, dummy, dummy, 2, 8, 8, mp2]
+
+    def prob(*t):
+        return lib.mfb_ment_prob(dummy, 100, 4, *t, 0.0, 0.0, dummy, None)
+
+    def prob_grid(*t):
+        return lib.mfb_ment_prob_grid(4, *hp, *t, 0.0, 0.0, dummy, None)
+
+    def integrate(*t, ax2=1, inv_mp=dummy):
+        return lib.mfb_ment_integrate(4, dummy, 8, 0, dummy, 8, ax2, 2, *hp, dummy, inv_mp, *t, 0.0, 0.0, dummy, None)
+
+    # a 2-D screen measured twice on one axis
+    assert integrate(*tables(), ax2=0, inv_mp=None) == -1
+    # with kicks, a non-empty family needs its multipole rows
+    for call in (prob, prob_grid, integrate):
+        assert call(*tables(mp=None, mp2=dummy)) == -1
+        assert call(*tables(mp=dummy, mp2=None)) == -1
+    # with kicks, integrate mode needs the inverse kick
+    assert integrate(*tables(mp=dummy, mp2=dummy), inv_mp=None) == -1
+    # names of this ABI exist in older libraries with other argument lists: another version is refused
+    monkeypatch.setattr(_lib, "ABI_VERSION", _lib.ABI_VERSION - 1)
+    monkeypatch.setattr(_lib, "_lib", None)
+    with pytest.raises(_lib.LibraryMissing, match="ABI version"):
+        _lib.load()
 
 
 def test_graphed_loss_chunk_plan():
