@@ -17,6 +17,8 @@
 #include "common.cuh"
 #include "multipole.cuh"
 
+#include <type_traits>
+
 namespace mfb {
 
 constexpr int kMentThreads = 256;
@@ -325,89 +327,134 @@ ment_integrate_kernel(const float* __restrict__ meas_coords, int nb_meas, int me
   }
 }
 
-// ---- inclusive scan of (rho + pad) in double: 3 passes -----------------------------------------
+// ---- inclusive scan of (rho + pad): an exact integer prefix -----------------------------------
+// A prefix summed in double in two different associations (tile offsets from tree-summed tile sums, entries inside a
+// tile from serial thread sums) decreases at tile starts by a few ulps, and its total misses the last entry.  So the
+// scan runs on integers instead: every cell is worth units = rn((rho + pad) * scale) with scale = 2^e chosen from the
+// float64 total so that the total sits in [2^61, 2^62), the units are summed exactly in uint64 (the order no longer
+// matters), and cdf = units / scale.  Hence, by construction: the cdf is non-decreasing, the total is cdf[G-1] bit
+// for bit, a cell of zero weight has cdf[i] == cdf[i-1], and the result is the same on every run.  Resolution 2^-62 of
+// the total.  Passes: float64 tile sums -> scale -> unit tile sums -> exclusive unit prefix -> cdf.
 constexpr int kScanThreads = 256;
 constexpr int kScanItems = 16;  // per thread
 constexpr int kScanTile = kScanThreads * kScanItems;
 
-__global__ void __launch_bounds__(kScanThreads)
-scan_tile_sums_kernel(const float* __restrict__ rho, int64_t G, double pad, double* __restrict__ tile_sums) {
-  __shared__ double red[kScanThreads / 32];
-  const int64_t base = (int64_t)blockIdx.x * kScanTile + (int64_t)threadIdx.x * kScanItems;
-  double s = 0.0;
+__device__ __forceinline__ uint64_t warp_sum_u64(uint64_t v) {
 #pragma unroll
-  for (int i = 0; i < kScanItems; ++i)
-    if (base + i < G) s += (double)rho[base + i] + pad;
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  return v;
+}
+
+// kUnits = false: the float64 sum of (rho + pad) over each tile (only the total is used: it picks the scale);
+// kUnits = true: the exact sum of the units of each tile, written over the float64 sums as uint64.
+template <bool kUnits>
+__global__ void __launch_bounds__(kScanThreads)
+scan_tile_sums_kernel(const float* __restrict__ rho, int64_t G, double pad, const double* __restrict__ scale,
+                      double* __restrict__ tile_sums) {
+  using T = typename std::conditional<kUnits, uint64_t, double>::type;
+  __shared__ T red[kScanThreads / 32];
+  const int64_t base = (int64_t)blockIdx.x * kScanTile + (int64_t)threadIdx.x * kScanItems;
+  const double sc = kUnits ? *scale : 1.0;
+  T s = 0;
+#pragma unroll
+  for (int i = 0; i < kScanItems; ++i) {
+    if (base + i < G) {
+      const double v = (double)rho[base + i] + pad;
+      if constexpr (kUnits) s += __double2ull_rn(v * sc); else s += v;
+    }
+  }
+  if constexpr (kUnits) s = warp_sum_u64(s); else s = warp_sum(s);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = s;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    T t = 0;
+    for (int i = 0; i < kScanThreads / 32; ++i) t += red[i];
+    reinterpret_cast<T*>(tile_sums)[blockIdx.x] = t;
+  }
+}
+
+// scale = 2^(62 - e) for a float64 total in [2^(e-1), 2^e): the units of all cells add up to just below 2^62 (the
+// float64 total is off by a relative G * 2^-53 at most, the rounding of the units by G / 2: far from 2^64).  An empty
+// or non-finite total keeps scale 1; a total below 2^-961 (a subnormal pad) gets 2^1023, the largest power of two.
+__global__ void __launch_bounds__(1024)
+scan_scale_kernel(const double* __restrict__ tile_sums, int64_t ntiles, double* __restrict__ scale) {
+  __shared__ double red[32];
+  double s = 0.0;
+  for (int64_t i = threadIdx.x; i < ntiles; i += 1024) s += tile_sums[i];
   s = warp_sum(s);
   if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = s;
   __syncthreads();
   if (threadIdx.x == 0) {
     double t = 0.0;
-    for (int i = 0; i < kScanThreads / 32; ++i) t += red[i];
-    tile_sums[blockIdx.x] = t;
+    for (int i = 0; i < 32; ++i) t += red[i];
+    int e = 0;
+    frexp(t, &e);
+    *scale = (t > 0.0 && isfinite(t)) ? ldexp(1.0, min(62 - e, 1023)) : 1.0;
   }
 }
 
-// exclusive prefix of the tile sums, one block of 1024 threads: every thread adds its contiguous chunk serially, the
-// 1024 chunk sums are scanned with a fixed shuffle / shared-memory tree (deterministic), then the chunk is written
-// back as exclusive offsets.  (A single thread walking 4096 tiles took 244 us of a 3.3 ms MENT update.)
+// exclusive prefix of the unit tile sums, one block of 1024 threads: every thread adds its contiguous chunk serially, the
+// 1024 chunk sums are scanned with a shuffle / shared-memory tree, then the chunk is written back as exclusive offsets.
+// Integer sums: any order gives the same offsets.  (A single thread walking 4096 tiles took 244 us of a 3.3 ms MENT
+// update.)  total = units of all cells / scale, exactly as scan_apply_kernel converts cdf[G-1].
 __global__ void __launch_bounds__(1024)
-scan_tile_offsets_kernel(double* __restrict__ tile_sums, int64_t ntiles, double* __restrict__ total) {
-  __shared__ double warp_tot[32];
+scan_tile_offsets_kernel(uint64_t* __restrict__ tile_sums, int64_t ntiles, const double* __restrict__ scale,
+                         double* __restrict__ total) {
+  __shared__ uint64_t warp_tot[32];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int64_t chunk = (ntiles + 1023) / 1024;
   const int64_t i0 = (int64_t)tid * chunk, i1 = (i0 + chunk < ntiles) ? i0 + chunk : ntiles;
-  double s = 0.0;
+  uint64_t s = 0;
   for (int64_t i = i0; i < i1; ++i) s += tile_sums[i];
   // inclusive scan of the chunk sums over the block
-  double inc = s;
+  uint64_t inc = s;
 #pragma unroll
   for (int o = 1; o < 32; o <<= 1) {
-    const double up = __shfl_up_sync(0xffffffffu, inc, o);
+    const uint64_t up = __shfl_up_sync(0xffffffffu, inc, o);
     if (lane >= o) inc += up;
   }
   if (lane == 31) warp_tot[warp] = inc;
   __syncthreads();
   if (warp == 0) {
-    double w = warp_tot[lane];
+    uint64_t w = warp_tot[lane];
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
-      const double up = __shfl_up_sync(0xffffffffu, w, o);
+      const uint64_t up = __shfl_up_sync(0xffffffffu, w, o);
       if (lane >= o) w += up;
     }
     warp_tot[lane] = w;   // inclusive over warps
   }
   __syncthreads();
-  const double before_warp = warp > 0 ? warp_tot[warp - 1] : 0.0;
-  double run = before_warp + (inc - s);   // exclusive prefix of this thread's chunk
+  uint64_t run = (warp > 0 ? warp_tot[warp - 1] : 0) + (inc - s);   // exclusive prefix of this thread's chunk
   for (int64_t i = i0; i < i1; ++i) {
-    const double v = tile_sums[i];
+    const uint64_t v = tile_sums[i];
     tile_sums[i] = run;
     run += v;
   }
-  if (tid == 1023) *total = warp_tot[31];
+  if (tid == 1023) *total = __ull2double_rn(warp_tot[31]) * (1.0 / *scale);
 }
 
 __global__ void __launch_bounds__(kScanThreads)
-scan_apply_kernel(const float* __restrict__ rho, int64_t G, double pad, const double* __restrict__ tile_offsets,
-                  double* __restrict__ cdf) {
-  __shared__ double s_thread[kScanThreads];
+scan_apply_kernel(const float* __restrict__ rho, int64_t G, double pad, const double* __restrict__ scale,
+                  const uint64_t* __restrict__ tile_offsets, double* __restrict__ cdf) {
+  __shared__ uint64_t s_thread[kScanThreads];
   const int64_t base = (int64_t)blockIdx.x * kScanTile + (int64_t)threadIdx.x * kScanItems;
-  double loc[kScanItems];
-  double s = 0.0;
+  const double sc = *scale, inv = 1.0 / sc;   // powers of two: exact
+  uint64_t loc[kScanItems];
+  uint64_t s = 0;
 #pragma unroll
   for (int i = 0; i < kScanItems; ++i) {
-    if (base + i < G) s += (double)rho[base + i] + pad;
+    if (base + i < G) s += __double2ull_rn(((double)rho[base + i] + pad) * sc);
     loc[i] = s;
   }
   s_thread[threadIdx.x] = s;
   __syncthreads();
   // exclusive prefix over the 256 thread sums (serial per thread over <= 255 values: tiny)
-  double off = tile_offsets[blockIdx.x];
+  uint64_t off = tile_offsets[blockIdx.x];
   for (int t = 0; t < (int)threadIdx.x; ++t) off += s_thread[t];
 #pragma unroll
   for (int i = 0; i < kScanItems; ++i)
-    if (base + i < G) cdf[base + i] = off + loc[i];
+    if (base + i < G) cdf[base + i] = __ull2double_rn(off + loc[i]) * inv;
 }
 
 // ---- Philox4x32-10 -------------------------------------------------------------------------------------
@@ -489,7 +536,11 @@ cdf_sample_kernel(const double* __restrict__ cdf, int64_t G, const double* __res
     // first index with cdf > target.  Plain bisection wastes three quarters of every 32-byte sector it fetches (the
     // kernel is bound by L2 sector requests, 22 per sample); the pivot levels pack four keys per sector: level l holds
     // the last cdf entry of every group of 4^l cells, one sector per level decides among four children -- 12 requests
-    // for 16^6 cells, the top six from L1.  The cell found is the bisection's.
+    // for 16^6 cells, the top six from L1.  The cdf is non-decreasing and tot == cdf[G-1] (exact integer prefix,
+    // scan_tile_sums_kernel), so the keys of every level are non-decreasing, counting the keys <= target picks the
+    // first child whose last key exceeds the target, and the cell found is the bisection's: the first with cdf > target,
+    // which has positive weight.  Only uu * tot == tot (uu rounds to 1 with probability 2^-53) leaves no key above the
+    // target; the descent then ends on the last cell, G - 1.
     int64_t grp = 0;
     for (int l = lv.n - 1; l >= 1; --l) {
       const double* keys = pivots + lv.off[l] + 4 * grp;
@@ -499,7 +550,7 @@ cdf_sample_kernel(const double* __restrict__ cdf, int64_t G, const double* __res
       int i = (k01.x <= target) ? 1 : 0;
       i += (left > 1 && k01.y <= target) ? 1 : 0;
       i += (left > 2 && k23.x <= target) ? 1 : 0;
-      i = (i < left - 1) ? i : (int)(left - 1);            // the last valid key of a group always covers the target
+      i = (i < left - 1) ? i : (int)(left - 1);            // the group's last key (>= its parent's key > target) covers it
       i = i < 3 ? i : 3;
       grp = 4 * grp + i;
     }
@@ -704,21 +755,26 @@ int mfb_ment_integrate(int d, const float* meas_coords, int nb_meas, int meas_ax
 int64_t mfb_cdf_workspace_bytes(int64_t g) {
   if (g < 1) return 0;
   const int64_t ntiles = (g + kScanTile - 1) / kScanTile;
-  return (((ntiles + 2) + 3) & ~(int64_t)3) * 8 + cdf_levels(g).total * 8;   // total | tile offsets | pivot levels
+  return (((ntiles + 2) + 3) & ~(int64_t)3) * 8 + cdf_levels(g).total * 8;   // total | tile sums | scale | pivot levels
 }
 
-/* cdf[i] = sum_{j<=i} (rho[j] + pad) in double; total written to workspace[0] (device) */
+/* cdf[i] = sum_{j<=i} (rho[j] + pad), an exact prefix at 2^-62 of the total (scan_tile_sums_kernel); the total,
+   written to workspace[0] (device), is cdf[g-1] */
 int mfb_cdf_build(const float* rho, int64_t g, double pad, double* cdf, void* workspace, int64_t workspace_bytes,
                   void* stream) {
   MFB_CHECK_ARG(rho && cdf && workspace && g >= 1);
   if (workspace_bytes < mfb_cdf_workspace_bytes(g)) return MFB_E_WORKSPACE;
   const int64_t ntiles = (g + kScanTile - 1) / kScanTile;
   double* total = (double*)workspace;
-  double* tiles = total + 1;
+  double* tiles = total + 1;            // float64 tile sums, then the uint64 unit sums, then their exclusive prefix
+  double* scale = tiles + ntiles;
   cudaStream_t st = (cudaStream_t)stream;
-  scan_tile_sums_kernel<<<(int)ntiles, kScanThreads, 0, st>>>(rho, g, pad, tiles);
-  scan_tile_offsets_kernel<<<1, 1024, 0, st>>>(tiles, ntiles, total);
-  scan_apply_kernel<<<(int)ntiles, kScanThreads, 0, st>>>(rho, g, pad, tiles, cdf);
+  scan_tile_sums_kernel<false><<<(int)ntiles, kScanThreads, 0, st>>>(rho, g, pad, nullptr, tiles);
+  scan_scale_kernel<<<1, 1024, 0, st>>>(tiles, ntiles, scale);
+  scan_tile_sums_kernel<true><<<(int)ntiles, kScanThreads, 0, st>>>(rho, g, pad, scale, tiles);
+  uint64_t* units = reinterpret_cast<uint64_t*>(tiles);
+  scan_tile_offsets_kernel<<<1, 1024, 0, st>>>(units, ntiles, scale, total);
+  scan_apply_kernel<<<(int)ntiles, kScanThreads, 0, st>>>(rho, g, pad, scale, units, cdf);
   const CdfLevels lv = cdf_levels(g);
   if (lv.total > 0) {
     double* pivots = (double*)workspace + (((ntiles + 2) + 3) & ~(int64_t)3);

@@ -9,118 +9,10 @@ import torch
 
 import mentflow_b200 as mf
 from mentflow_b200.simulate.transform import CompositeTransform, LinearTransform, MultipoleTransform
-from mfb_testutil import t32
-from oracle import hotpath as hp
+from mfb_testutil import (check_density as _check_density, integrate_check as _integrate_check, oracle_prob,
+                          positive_tables as _positive_tables, t32)
 
 pytestmark = pytest.mark.gpu
-
-
-# ---------------------------------------------------------------------------------------------- float64 oracle
-def _cpu64(t):
-    """float64 CPU copy of a transfer map."""
-    if isinstance(t, LinearTransform):
-        return LinearTransform(t.matrix.detach().to("cpu", torch.float64))
-    if isinstance(t, CompositeTransform):
-        return CompositeTransform(*[_cpu64(s) for s in t.transforms])
-    return MultipoleTransform(order=t.order, strength=t.strength, skew=t.skew)
-
-
-def _h(diag, table, u):
-    """Lagrange function of ``diag`` at the transformed points u (float64), as the reference's interpolator."""
-    if isinstance(diag, mf.diagnostics.Histogram2D):
-        cx, cy = (hp.centres(e.cpu()) for e in (diag.edges_x, diag.edges_y))
-        return hp.lagrange_interp_2d(table.cpu(), cx, cy, u[:, list(diag.axis)])
-    return hp.lagrange_interp(table.cpu(), hp.centres(diag.edges.cpu()), u[:, diag.axis])
-
-
-def oracle_prob(model, x):
-    """hp.ment_prob with transform.forward in float64 in place of the matrix."""
-    x = x.detach().cpu().double()
-    prob = torch.ones(x.shape[0], dtype=torch.float32)
-    for i, t in enumerate(model.transforms):
-        u = _cpu64(t)(x)
-        for j, diag in enumerate(model.diagnostics[i]):
-            h = _h(diag, model.lagrange_functions[i][j].values, u)
-            prob = prob * torch.clamp(h.type(torch.float32), 0.0, 1.0e10)
-    return prob * torch.exp(hp.gaussian_log_prob(x, float(model.prior.scale)).float())
-
-
-def oracle_integrate(model, i, j):
-    """Normalised integrate-mode prediction: sum over the integration grid of rho(transform.inverse(points))."""
-    diag = model.diagnostics[i][j]
-    limits, shape = model.integration_limits[i][j], model.integration_shape[i][j]
-    grid = [torch.linspace(float(lo), float(hi), int(n), dtype=torch.float64) for (lo, hi), n in zip(limits, shape)]
-    if isinstance(diag, mf.diagnostics.Histogram2D):
-        meas = [hp.centres(diag.edges_x.cpu()).double(), hp.centres(diag.edges_y.cpu()).double()]
-        axes = list(diag.axis)
-    else:
-        meas = [hp.centres(diag.edges.cpu()).double()]
-        axes = [diag.axis]
-    d = model.ndim
-    others = [a for a in range(d) if a not in axes]
-    mesh = torch.meshgrid(*meas, *grid, indexing="ij")
-    u = torch.zeros(mesh[0].numel(), d, dtype=torch.float64)
-    for a, m in zip(axes + others, mesh):
-        u[:, a] = m.reshape(-1)
-    x = _cpu64(model.transforms[i]).inverse(u)
-    rho = oracle_prob(model, x).double().reshape(*[m.numel() for m in meas], -1).sum(dim=-1)
-    if isinstance(diag, mf.diagnostics.Histogram2D):
-        vol = float(diag.edges_x[1] - diag.edges_x[0]) * float(diag.edges_y[1] - diag.edges_y[0])
-    else:
-        vol = float(diag.edges[1] - diag.edges[0])
-    return (rho / rho.sum() / vol).float()
-
-
-def oracle_sweeps(model, n, lr=1.0, thresh=1.0e-10):
-    """``n`` Gauss-Seidel sweeps of integrate mode on the oracle (model's tables are read, not changed)."""
-    saved = [[lf.values.clone() for lf in row] for row in model.lagrange_functions]
-    out = None
-    try:
-        for _ in range(n):
-            for i in range(len(model.transforms)):
-                for j in range(len(model.diagnostics[i])):
-                    pred = oracle_integrate(model, i, j)
-                    lf = model.lagrange_functions[i][j]
-                    meas = model.measurements[i][j].cpu()
-                    new = hp.gauss_seidel_table(lf.values.cpu(), meas, pred, lr, thresh)
-                    lf.set_values(new.to(lf.values.device))
-        out = [[lf.values.cpu().clone() for lf in row] for row in model.lagrange_functions]
-    finally:
-        for row, vals in zip(model.lagrange_functions, saved):
-            for lf, v in zip(row, vals):
-                lf.set_values(v)
-    return out
-
-
-def _positive_tables(model, seed):
-    """Positive random tables, zero on the outermost centres so that h is continuous (a point whose fp32 and float64
-    projections straddle the last centre would otherwise see a jump)."""
-    gen = torch.Generator().manual_seed(seed)
-    for row in model.lagrange_functions:
-        for lf in row:
-            v = torch.rand(lf.values.shape, generator=gen) + 0.2
-            if v.ndim == 1:
-                v[0] = v[-1] = 0.0
-            else:
-                v[0], v[-1], v[:, 0], v[:, -1] = 0.0, 0.0, 0.0, 0.0
-            lf.set_values(v.cuda())
-
-
-def _check_density(model, x, want_x):
-    """prob at explicit points, prob_on_grid and prob at the materialised grid points against the float64 oracle.
-    The kernels project in fp32: where a factor sits near the zero end of its table its relative error is that of
-    the projection over the distance to the end (a fp32 emulation of the kernels' arithmetic reaches 7e-7 of the
-    maximum there), hence an absolute tolerance of 2e-6 of the maximum at the explicit points as on the grid."""
-    prob = model.prob(x.cuda()).cpu()
-    assert int((want_x > 0).sum()) > 0.2 * want_x.numel()               # not vacuous
-    assert torch.allclose(prob, want_x, rtol=1e-4, atol=2e-6 * float(want_x.max()))
-    grid = model.prob_on_grid(model.sampler).cpu()
-    pts = model.sampler.get_grid_points()
-    refg = oracle_prob(model, pts)
-    assert int((refg > 0).sum()) > 0.05 * refg.numel()
-    # grid points come from the index (lo + i*step) instead of fp32 linspace centres: 1-ulp shifts
-    assert torch.allclose(grid, refg, rtol=1e-4, atol=2e-6 * float(refg.max()))
-    assert torch.allclose(model.prob(pts).cpu(), refg, rtol=1e-4, atol=2e-6 * float(refg.max()))
 
 
 # ---------------------------------------------------------------------------------------------- rec_2d/nonlinear
@@ -196,26 +88,6 @@ def test_random_chains_density_matches_float64(d, flip):
 
 
 # ---------------------------------------------------------------------------------------------- integrate mode
-def _integrate_check(model, slots):
-    """simulate(i, j) against the oracle, then two Gauss-Seidel sweeps against the oracle's sweeps.  A screen's own
-    pixels sit exactly on its bin centres: where the table is 0 next to a nonzero value, fp32 rounding of the pixel's
-    own projection (a few 1e-7) turns h = 0 into slope x rounding, up to ~1e-5 of the maximum prediction.  Such entries
-    stay 0 through the update (0 x anything), so the tables keep the tight tolerances."""
-    for i, j in slots:
-        pred = model.simulate(i, j).cpu()
-        want = oracle_integrate(model, i, j)
-        assert pred.shape == want.shape and int((want > 0).sum()) > 5
-        assert torch.allclose(pred, want, rtol=1e-4, atol=1e-5 * float(want.max())), (i, j)
-    want = oracle_sweeps(model, 2)
-    model.gauss_seidel_update(lr=1.0, thresh=1.0e-10)
-    model.gauss_seidel_step(lr=1.0, thresh=1.0e-10)
-    for row_g, row_w in zip(model.lagrange_functions, want):
-        for lf, w in zip(row_g, row_w):
-            got = lf.values.cpu()
-            assert torch.allclose(got, w, rtol=2e-4, atol=1e-6)
-            assert torch.equal(got == 0, w == 0)
-
-
 def test_integrate_mode_nonlinear_setup_matches_float64(golden):
     """Tables zero on the outermost centres: a screen's own pixels sit exactly on its centres, and T(T^-1(c)) lands a
     rounding error above or below the last centre, where a nonzero end value would make h jump to 0."""
