@@ -271,6 +271,22 @@ int mfb_loss_tail(const float* d, int k, const float* h, float mu, float* out, v
 int mfb_f64_split(const double* in, int n, float* out_hi_lo, void* stream);
 int mfb_f64_join(const float* in_hi_lo, int n, double* out, void* stream);
 
+/* ---- k-nearest-neighbour entropy (KNNEntropyEstimator) ----------------------------------------
+ * x[n][d], 1 <= d <= 8, 1 <= k <= 16, k < n < 2^31.  r[i] = distance from x_i to its k-th nearest OTHER particle
+ * (self excluded by index, so a duplicate is a neighbour at distance 0), idx[i] = that particle's index, neighbours
+ * ordered by (r^2, j): ties go to the smaller index.  A particle without k others at a finite distance (NaN or inf
+ * coordinates, r^2 overflowing) gets r[i] = inf, idx[i] = i.  logsum[0] = sum_i log(r_i + pad) in double.  All
+ * pairs in fp32 direct differences; deterministic (no floating-point atomics).  d > 8 or k > 16: MFB_E_UNSUPPORTED. */
+int64_t mfb_knn_workspace_bytes(int64_t n, int d, int k);
+int mfb_knn_kth(const float* x, int64_t n, int d, int k, double pad, float* r, int32_t* idx, double* logsum,
+                void* workspace, int64_t workspace_bytes, void* stream);
+/* gx[n][d] = glogsum[0] * d logsum / dx with the neighbours held fixed:
+ *   w_i (x_i - x_idx[i]) + sum over j with idx[j] = i, ascending j, of w_j (x_i - x_j),  w_j = 1 / (r_j (r_j + pad)),
+ * 0 where r_j = 0.  sorted_idx[n] = idx stably sorted, perm[n] (int64) the positions it came from.            */
+int mfb_knn_kth_bwd(const float* x, int64_t n, int d, const float* r, const int32_t* idx,
+                    const int32_t* sorted_idx, const int64_t* perm, double pad, const double* glogsum,
+                    float* gx, void* stream);
+
 /* ---- classical MENT (ment.py, sample.py) --------------------------------------------------
  * rho(x) = exp(log prior(x)) * prod clamp(h(u(x)), 0, 1e10) over two families of Lagrange tables, evaluated in
  * double like scipy's RegularGridInterpolator and 0 outside the box of the bin centres (ment.py:36-52, 227-249);

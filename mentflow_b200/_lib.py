@@ -82,6 +82,9 @@ SIGNATURES = {
     "mfb_f64_join": (c_int, [P, c_int, P, P]),
     "mfb_mc_entropy": (c_int, [P, c_double, c_double, c_double, P, P]),
     "mfb_loss_tail": (c_int, [P, c_int, P, c_float, P, P]),
+    "mfb_knn_workspace_bytes": (c_int64, [c_int64, c_int, c_int]),
+    "mfb_knn_kth": (c_int, [P, c_int64, c_int, c_int, c_double, P, P, P, P, c_int64, P]),
+    "mfb_knn_kth_bwd": (c_int, [P, c_int64, c_int, P, P, P, P, c_double, P, P, P]),
 }
 
 _lib = None

@@ -152,12 +152,39 @@ class CovarianceEntropyEstimator(EntropyEstimator):
         return _CovEntropy.apply(x, float(self.pad), -3.0 * float(np.log(2.0 * np.pi * np.e)), self.reducer)
 
 
+def _digamma_int(n: int) -> float:
+    """psi(n) for an integer n >= 1: the harmonic sum below 10, the asymptotic series (error < 1e-16) above."""
+    if n < 10:
+        return -0.5772156649015329 + sum(1.0 / m for m in range(1, n))
+    x = float(n)
+    x2 = 1.0 / (x * x)
+    return math.log(x) - 0.5 / x - x2 * (1.0 / 12 - x2 * (1.0 / 120 - x2 * (1.0 / 252 - x2 * (1.0 / 240 - x2 / 132))))
+
+
+def knn_entropy_constant(n: int, d: int, k: int) -> float:
+    """psi(N) - psi(k) + log V_d, V_d = pi^(d/2) / Gamma(d/2 + 1) the volume of the unit d-ball."""
+    log_vd = 0.5 * d * math.log(math.pi) - math.lgamma(0.5 * d + 1.0)
+    return _digamma_int(n) - _digamma_int(k) + log_vd
+
+
 class KNNEntropyEstimator(EntropyEstimator):
-    def __init__(self, prior: Any = None, k: int = 5) -> None:
+    """-H, H = psi(N) - psi(k) + log V_d + (d/N) sum_i log(r_i + pad), r_i the distance from x_i to its k-th nearest
+    other particle (Kozachenko-Leonenko).  Works from the particles alone: ``log_prob`` is ignored.  The distances come
+    from an all-pairs CUDA kernel (O(N^2 d), ops.knn_kth); the gradient holds the neighbours fixed, as autograd
+    through cdist + topk would.  Sharded particles are refused: the neighbours within a shard are not those within
+    the union."""
+
+    def __init__(self, prior: Any = None, k: int = 5, pad: float = 1.0e-12) -> None:
         if prior is not None:
             raise ValueError("This class cannot estimate relative entropy (prior != None).")
         super().__init__(prior=prior)
         self.k = k
+        self.pad = pad
 
-    def forward(self, x, log_prob=None):
-        raise NotImplementedError
+    def forward(self, x: torch.Tensor, log_prob: torch.Tensor = None) -> torch.Tensor:
+        if self.reducer is not None and getattr(self.reducer, "world_size", 1) > 1:
+            raise NotImplementedError("KNNEntropyEstimator does not support sharded particles: the nearest neighbours "
+                                      "within one rank's shard are not those within the whole batch")
+        _, _, logsum = ops.knn_kth(x, self.k, self.pad)
+        n, d = x.shape
+        return (-(knn_entropy_constant(n, d, self.k) + (d / n) * logsum)).to(torch.float32)

@@ -594,6 +594,69 @@ def f64_join(pairs: torch.Tensor) -> torch.Tensor:
 
 
 # --------------------------------------------------------------------------------------
+# k-th nearest neighbour (k-NN entropy)
+# --------------------------------------------------------------------------------------
+KNN_MAX_K = 16
+KNN_MAX_DIM = 8
+
+
+class KNNKth(torch.autograd.Function):
+    """(r, idx, logsum) of ``knn_kth``; only ``logsum`` carries a gradient, with the neighbours held fixed."""
+
+    @staticmethod
+    def forward(ctx, x, k, pad):
+        lib = _lib.load()
+        x = _check_f32("x", x.detach())
+        n, d = x.shape
+        r = torch.empty(n, dtype=torch.float32, device=x.device)
+        idx = torch.empty(n, dtype=torch.int32, device=x.device)
+        logsum = torch.empty((), dtype=torch.float64, device=x.device)
+        with torch.cuda.device(x.device):
+            wbytes = lib.mfb_knn_workspace_bytes(n, d, k)
+            work = torch.empty(max(wbytes, 16), dtype=torch.uint8, device=x.device)
+            _lib.check(lib.mfb_knn_kth(_ptr(x), n, d, k, float(pad), _ptr(r), _ptr(idx), _ptr(logsum), _ptr(work),
+                                       wbytes, _stream()), "knn_kth")
+        ctx.save_for_backward(x, r, idx)
+        ctx.pad = float(pad)
+        ctx.mark_non_differentiable(r, idx)
+        return r, idx, logsum
+
+    @staticmethod
+    def backward(ctx, _gr, _gidx, glogsum):
+        x, r, idx = ctx.saved_tensors
+        n, d = x.shape
+        sorted_idx, perm = torch.sort(idx, stable=True)     # particle i's incoming neighbours, ascending j
+        g = glogsum.to(torch.float64).contiguous()
+        gx = torch.empty_like(x)
+        lib = _lib.load()
+        with torch.cuda.device(x.device):
+            _lib.check(lib.mfb_knn_kth_bwd(_ptr(x), n, d, _ptr(r), _ptr(idx), _ptr(sorted_idx), _ptr(perm), ctx.pad,
+                                           _ptr(g), _ptr(gx), _stream()), "knn_kth_bwd")
+        return gx, None, None
+
+
+def knn_kth(x: torch.Tensor, k: int, pad: float = 1.0e-12):
+    """Distance ``r`` (float32, (N,)) from every particle to its k-th nearest other particle, that neighbour's index
+    ``idx`` (int32; ties go to the smaller index) and ``logsum`` = sum log(r + pad) (float64 0-dim tensor, the only
+    differentiable output).  A particle without k others at a finite distance (NaN or inf coordinates) gets r = inf and
+    idx = its own index, which carries no gradient.  All pairs on the GPU: O(N^2 d)."""
+    if not isinstance(x, torch.Tensor) or x.dim() != 2:
+        raise ValueError("knn_kth: x must be a (N, d) tensor")
+    n, d = x.shape
+    k = int(k)
+    if not 1 <= k <= KNN_MAX_K:
+        raise ValueError(f"knn_kth: k = {k} is outside [1, {KNN_MAX_K}]")
+    if k >= n:
+        raise ValueError(f"knn_kth: k = {k} needs more than k particles (got N = {n})")
+    if not 1 <= d <= KNN_MAX_DIM:
+        raise ValueError(f"knn_kth: d = {d} is outside [1, {KNN_MAX_DIM}]")
+    if n >= 2 ** 31:
+        raise ValueError(f"knn_kth: N = {n} does not fit the int32 neighbour indices")
+    _check_f32("x", x)
+    return KNNKth.apply(x, k, float(pad))
+
+
+# --------------------------------------------------------------------------------------
 # zuko-layout parameters <-> packed blocks
 # --------------------------------------------------------------------------------------
 class PackParameters(torch.autograd.Function):
