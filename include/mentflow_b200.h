@@ -287,6 +287,27 @@ int mfb_knn_kth_bwd(const float* x, int64_t n, int d, const float* r, const int3
                     const int32_t* sorted_idx, const int64_t* perm, double pad, const double* glogsum,
                     float* gx, void* stream);
 
+/* ---- sliced Wasserstein distance (loss.py sliced_wasserstein_distance; POT's ot.sliced_wasserstein_distance) ------
+ * x[n][d], 1 <= d <= 8, 1 <= n < 2^31; theta[nproj][d] the directions.  u_k = x theta_k, each an fp32 fused
+ * multiply-add chain from zero in ascending coordinate order, sorted stably (ties keep the smaller index, -0 and +0
+ * compare equal, every NaN sorts last) by an 8-bit LSD radix sort per direction.  The directions are processed in
+ * chunks of as many as workspace_bytes holds, at least one: mfb_swd_workspace_bytes(n, c) is the size for chunks of
+ * c directions (c <= 65535).  Results do not depend on the chunking, bit for bit.
+ * sorted[nproj][n] = the sorted u_k, perm[nproj][n] (may be NULL) = the particle index of each entry.            */
+int64_t mfb_swd_workspace_bytes(int64_t n, int nproj_chunk);
+int mfb_swd_sort(const float* x, int64_t n, int d, const float* theta, int nproj, float* sorted, int32_t* perm,
+                 void* workspace, int64_t workspace_bytes, void* stream);
+/* wpp[k] (double) = W_p^p between the samples' projections u_k and the reference projections y_sorted[k][0..m)
+ * (ascending, e.g. from mfb_swd_sort): sum over rank pairs (i, j) of len_ij |u_(i) - v_(j)|^p, len_ij the overlap
+ * of [i/n, (i+1)/n) and [j/m, (j+1)/m) computed exactly in int64; p >= 1 finite.  grad_coef[nproj][n] (may be NULL)
+ * receives dW_p^p(k)/du_{k,i} at each particle's own index, with the ranks held fixed.  Per-CTA double partials are
+ * added in a fixed order: no floating-point atomics.                                                               */
+int mfb_swd_wpp(const float* x, int64_t n, int d, const float* theta, int nproj, const float* y_sorted, int64_t m,
+                double p, double* wpp, float* grad_coef, void* workspace, int64_t workspace_bytes, void* stream);
+/* gx[n][d] = sum over k ascending of gwpp[k] theta_k grad_coef[k][n] (gwpp: nproj doubles on the device)      */
+int mfb_swd_bwd(const float* grad_coef, int64_t n, int d, const float* theta, int nproj, const double* gwpp,
+                float* gx, void* stream);
+
 /* ---- classical MENT (ment.py, sample.py) --------------------------------------------------
  * rho(x) = exp(log prior(x)) * prod clamp(h(u(x)), 0, 1e10) over two families of Lagrange tables, evaluated in
  * double like scipy's RegularGridInterpolator and 0 outside the box of the bin centres (ment.py:36-52, 227-249);

@@ -657,6 +657,123 @@ def knn_kth(x: torch.Tensor, k: int, pad: float = 1.0e-12):
 
 
 # --------------------------------------------------------------------------------------
+# sliced Wasserstein distance: projections, stable radix sort, 1-D quantile integral
+# --------------------------------------------------------------------------------------
+SWD_MAX_DIM = 8
+SWD_MAX_CHUNK = 65535               # directions per chunk (the library's grid limit)
+SWD_WORKSPACE_CAP = 1 << 30         # bytes of sort workspace per call; the directions are sorted in chunks that fit
+                                    # (about 16.5 bytes per particle and direction)
+
+
+def check_swd_points(name: str, t, d: Optional[int] = None) -> None:
+    """Refuse anything but a (N, d) tensor with 1 <= d <= 8, 1 <= N < 2^31 (and d equal to ``d`` when given)."""
+    if not isinstance(t, torch.Tensor) or t.dim() != 2:
+        raise ValueError(f"{name} must be a (N, d) tensor")
+    n, dd = t.shape
+    if not 1 <= dd <= SWD_MAX_DIM:
+        raise ValueError(f"{name}: d = {dd} is outside [1, {SWD_MAX_DIM}]")
+    if d is not None and dd != d:
+        raise ValueError(f"{name} has d = {dd}, the samples have d = {d}")
+    if not 1 <= n < 2 ** 31:
+        raise ValueError(f"{name}: N = {n} is outside [1, 2^31)")
+
+
+def check_swd_p(p) -> float:
+    p = float(p)
+    if not (math.isfinite(p) and p >= 1.0):
+        raise ValueError(f"p = {p} must be finite and >= 1")
+    return p
+
+
+def _swd_theta(theta, d: int) -> None:
+    if not isinstance(theta, torch.Tensor) or theta.dim() != 2 or theta.shape[1] != d or theta.shape[0] < 1:
+        raise ValueError(f"theta must be a (P, {d}) tensor of directions with P >= 1")
+    if theta.requires_grad:
+        raise ValueError("theta requires grad, but the sliced Wasserstein kernels differentiate only x")
+
+
+def _swd_workspace(lib, n: int, nproj: int, device):
+    per = int(lib.mfb_swd_workspace_bytes(n, 1))
+    chunk = max(1, min(nproj, SWD_MAX_CHUNK, SWD_WORKSPACE_CAP // per))
+    wbytes = int(lib.mfb_swd_workspace_bytes(n, chunk))
+    return torch.empty(wbytes, dtype=torch.uint8, device=device), wbytes
+
+
+def swd_sort(x: torch.Tensor, theta: torch.Tensor):
+    """Projections u = x theta_k (fp32 fused multiply-add chains from zero, coordinates in ascending order) of every
+    direction (row of ``theta``, (P, d)), sorted stably: returns ``sorted`` ((P, N) float32) and ``perm`` ((P, N)
+    int32, the particle index of each entry; ties keep index order, -0 and +0 compare equal, NaN sorts last).  An
+    8-bit LSD radix sort on the GPU; not differentiable."""
+    check_swd_points("x", x)
+    n, d = x.shape
+    _swd_theta(theta, d)
+    x = _check_f32("x", x.detach())
+    theta = _check_f32("theta", theta)
+    nproj = theta.shape[0]
+    lib = _lib.load()
+    sorted_ = torch.empty((nproj, n), dtype=torch.float32, device=x.device)
+    perm = torch.empty((nproj, n), dtype=torch.int32, device=x.device)
+    with torch.cuda.device(x.device):
+        work, wbytes = _swd_workspace(lib, n, nproj, x.device)
+        _lib.check(lib.mfb_swd_sort(_ptr(x), n, d, _ptr(theta), nproj, _ptr(sorted_), _ptr(perm), _ptr(work), wbytes,
+                                    _stream()), "swd_sort")
+    return sorted_, perm
+
+
+class SWDWpp(torch.autograd.Function):
+    """(P,) float64 W_p^p of ``swd_wpp``; only x gets a gradient, with the ranks held fixed."""
+
+    @staticmethod
+    def forward(ctx, x, theta, y_sorted, p):
+        lib = _lib.load()
+        n, d = x.shape
+        nproj, m = y_sorted.shape
+        wpp = torch.empty(nproj, dtype=torch.float64, device=x.device)
+        gcoef = torch.empty((nproj, n), dtype=torch.float32, device=x.device) if ctx.needs_input_grad[0] else None
+        with torch.cuda.device(x.device):
+            work, wbytes = _swd_workspace(lib, n, nproj, x.device)
+            _lib.check(lib.mfb_swd_wpp(_ptr(x), n, d, _ptr(theta), nproj, _ptr(y_sorted), m, p, _ptr(wpp), _ptr(gcoef),
+                                       _ptr(work), wbytes, _stream()), "swd_wpp")
+        if gcoef is not None:
+            ctx.save_for_backward(gcoef, theta)
+        return wpp
+
+    @staticmethod
+    def backward(ctx, gwpp):
+        gcoef, theta = ctx.saved_tensors
+        nproj, n = gcoef.shape
+        d = theta.shape[1]
+        gw = gwpp.to(torch.float64).contiguous()
+        gx = torch.empty((n, d), dtype=torch.float32, device=gcoef.device)
+        lib = _lib.load()
+        with torch.cuda.device(gcoef.device):
+            _lib.check(lib.mfb_swd_bwd(_ptr(gcoef), n, d, _ptr(theta), nproj, _ptr(gw), _ptr(gx), _stream()),
+                       "swd_bwd")
+        return gx, None, None, None
+
+
+def swd_wpp(x: torch.Tensor, theta: torch.Tensor, y_sorted: torch.Tensor, p: float) -> torch.Tensor:
+    """W_p^p (the p-th power, as POT's ``wasserstein_1d``) between the projections of x on every direction (row of
+    ``theta``, (P, d)) and the ascending reference projections ``y_sorted`` ((P, M), e.g. ``swd_sort(y, theta)[0]``),
+    both sets uniformly weighted: (P,) float64.  Differentiable w.r.t. x only (ranks held fixed, the derivative of
+    |0| is 0); the forward keeps a (P, N) float32 coefficient table for the backward when x requires grad."""
+    check_swd_points("x", x)
+    n, d = x.shape
+    _swd_theta(theta, d)
+    p = check_swd_p(p)
+    if not isinstance(y_sorted, torch.Tensor) or y_sorted.dim() != 2 or y_sorted.shape[0] != theta.shape[0]:
+        raise ValueError("y_sorted must be a (P, M) tensor, one sorted row per direction")
+    if not 1 <= y_sorted.shape[1] < 2 ** 31:
+        raise ValueError(f"y_sorted: M = {y_sorted.shape[1]} is outside [1, 2^31)")
+    if y_sorted.requires_grad:
+        raise ValueError("y_sorted requires grad, but the sliced Wasserstein kernels differentiate only x")
+    x = _check_f32("x", x)                  # a contiguous copy, if one is made, stays on the autograd graph
+    theta = _check_f32("theta", theta)
+    y_sorted = _check_f32("y_sorted", y_sorted)
+    return SWDWpp.apply(x, theta, y_sorted, p)
+
+
+# --------------------------------------------------------------------------------------
 # zuko-layout parameters <-> packed blocks
 # --------------------------------------------------------------------------------------
 class PackParameters(torch.autograd.Function):
