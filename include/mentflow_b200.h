@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define MFB_ABI_VERSION 3
+#define MFB_ABI_VERSION 4
 
 #define MFB_E_BADARG (-1)      /* null pointer / non-positive size / unsupported shape   */
 #define MFB_E_UNSUPPORTED (-2) /* combination not compiled (e.g. D > 8, hidden != 64)    */
@@ -61,25 +61,29 @@ int mfb_sm_count(void);
  * x[n][d]; proj[K][d] (row `axis` of M_k, or M_k^T d_hat); out partial sums are reduced
  * deterministically into sums[K][B] = S_kb = sum_n K_nb (unnormalised; this is what ranks
  * all-reduce).  max_sigma_over_delta = largest sigma/delta of the K screens (host value; sets
- * the deposit window: bins further than ~8.9 sigma from a particle are skipped).         */
+ * the deposit window: bins further than ~8.9 sigma from a particle are skipped).
+ *
+ * Multipole kicks (CompositeTransform(linear.., MultipoleTransform, linear..) followed by
+ * Histogram1D, simulate/transform.py:35-55,78-146; experiments/rec_2d/nonlinear/setup.py:24-44):
+ * the projection, its backward and the exact histogram take optional rows mp[K][2 d + 4] =
+ * [wa (d) | wb (d) | a | b | order | 0], and the projected coordinate becomes
+ *   u = proj_k . x + a_k Re(z^m) + b_k Im(z^m),  z = wa_k . x + i wb_k . x,  m = order - 1.
+ * mp NULL selects the linear kernels.  The host side folds the matrices, the kick strength /
+ * (order-1)! and the reference's U[:,3] = X[:,1] + .. quirk into proj, a and b
+ * (simulate.multipole_terms).
+ *
+ * mfb_project_kde1d_fwd deposits and merges in two launches.  profiles NULL: sums only (n = 0
+ * gives zeros; n_total is ignored, meas and kl must be NULL).  profiles given: n >= 1,
+ * n_total > 0, and the merge kernel also normalises (diagnostics/histogram.py:39-43:
+ * p = (S/N) / (sum_b (S_b/N) * delta + 1e-10), N = n_total) and -- when meas[K][B] is given --
+ * evaluates kl[k] = sum_b (xlogy(t,t) - t log(p + pad)) / B (core.py:89-117 with
+ * loss.py:15-17); kl is NULL iff meas is NULL.  sums[K][B] is the unnormalised input of
+ * mfb_kde1d_finish and of the backward.                                                   */
 int64_t mfb_kde1d_workspace_bytes(int64_t n, int d, int k, int b);
-int mfb_project_kde1d_fwd(const float* x, int64_t n, int d, const float* proj, const float* geom,
-                          int k, int b, float max_sigma_over_delta, float* sums, void* workspace,
-                          int64_t workspace_bytes, void* stream);
-/* diagnostics/histogram.py:39-43: p = (S/N) / (sum_b (S_b/N) * delta + 1e-10)            */
-int mfb_kde1d_normalize(const float* sums, double n_total, const float* geom, int k, int b,
-                        float* profiles, void* stream);
-/* backward of the normalisation: gsums = dL/dS given gprof = dL/dp  (SURVEY App. B.10)  */
-int mfb_kde1d_normalize_bwd(const float* sums, double n_total, const float* geom, int k, int b,
-                            const float* gprof, float* gsums, void* stream);
-/* Fused forward tail for the training loss (core.py:89-117 with loss.py:15-17): deposit, merge,
- * normalise and -- when meas[K][B] is given -- kl[k] = sum_b (xlogy(t,t) - t log(p + pad)) / B in
- * two launches.  sums[K][B] (unnormalised, kept for the backward), profiles[K][B], kl[K] (NULL iff
- * meas is NULL).  Workspace as for mfb_project_kde1d_fwd.                                  */
-int mfb_project_kde1d_loss_fwd(const float* x, int64_t n, int d, const float* proj, const float* geom,
-                               int k, int b, float max_sigma_over_delta, double n_total,
-                               const float* meas, float pad, float* sums, float* profiles, float* kl,
-                               void* workspace, int64_t workspace_bytes, void* stream);
+int mfb_project_kde1d_fwd(const float* x, int64_t n, int d, const float* proj, const float* mp,
+                          const float* geom, int k, int b, float max_sigma_over_delta, double n_total,
+                          const float* meas, float pad, float* sums, float* profiles, float* kl,
+                          void* workspace, int64_t workspace_bytes, void* stream);
 /* The same tail from already merged (e.g. all-reduced across ranks) sums.                   */
 int mfb_kde1d_finish(const float* sums, double n_total, const float* geom, int k, int b,
                      const float* meas, float pad, float* profiles, float* kl, void* stream);
@@ -102,41 +106,26 @@ int mfb_kde1d_finish_p2p(const uint64_t* peer_blocks_host, int rank, int world, 
                          const float* geom, int k, int b, const float* meas, float pad, float* sums,
                          float* profiles, float* kl, double* tail_out, void* stream);
 /* deposit + (merge of the deposit's partials, cross-rank sum, normalise, KL) in two launches: the sharded counterpart
- * of mfb_project_kde1d_loss_fwd; workspace as for mfb_project_kde1d_fwd.                                       */
+ * of mfb_project_kde1d_fwd with profiles, linear maps only.                                                    */
 int mfb_project_kde1d_loss_fwd_p2p(const float* x, int64_t n, int d, const float* proj, const float* geom, int k,
                                    int b, float max_sigma_over_delta, double n_total, const float* meas, float pad,
                                    const uint64_t* peer_blocks_host, int rank, int world, uint32_t* state,
                                    const double* local_tail, int tail_doubles, float* sums, float* profiles,
                                    float* kl, double* tail_out, void* workspace, int64_t workspace_bytes,
                                    void* stream);
-/* dL/dx[n][d] (+)= sum_k proj_k * sum_b gsums[k][b] K_nb (-(u-c_b)/sigma^2); accumulate!=0
- * adds into gx instead of overwriting it.                                               */
-int mfb_project_kde1d_bwd(const float* x, int64_t n, int d, const float* proj, const float* geom,
-                          int k, int b, float max_sigma_over_delta, const float* gsums, float* gx,
-                          int accumulate, void* stream);
-
-/* ---- the same three kernels behind a thin multipole kick -------------------------------
- * Replaces CompositeTransform(linear.., MultipoleTransform, linear..) followed by Histogram1D
- * (simulate/transform.py:35-55,78-146; experiments/rec_2d/nonlinear/setup.py:24-44):
- *   u = proj_k . x + a_k Re(z^m) + b_k Im(z^m),  z = wa_k . x + i wb_k . x,  m = order - 1.
- * mp[K][2 d + 4] = [wa (d) | wb (d) | a | b | order | 0]; everything else as in the functions
- * without _mp.  The host side folds the matrices, the kick strength / (order-1)! and the
- * reference's U[:,3] = X[:,1] + .. quirk into proj, a and b (simulate.multipole_terms).     */
-int mfb_project_kde1d_mp_fwd(const float* x, int64_t n, int d, const float* proj, const float* mp,
-                             const float* geom, int k, int b, float max_sigma_over_delta, float* sums,
-                             void* workspace, int64_t workspace_bytes, void* stream);
-int mfb_project_kde1d_mp_bwd(const float* x, int64_t n, int d, const float* proj, const float* mp,
-                             const float* geom, int k, int b, float max_sigma_over_delta,
-                             const float* gsums, float* gx, int accumulate, void* stream);
-int mfb_project_hist1d_mp(const float* x, int64_t n, int d, const float* proj, const float* mp,
-                          const float* edges, int k, int b, int64_t* counts, void* stream);
+/* dL/dx[n][d] (+)= sum_k du_k/dx * sum_b gsums[k][b] K_nb (-(u-c_b)/sigma^2), du_k/dx = proj_k
+ * without mp; accumulate!=0 adds into gx instead of overwriting it.                       */
+int mfb_project_kde1d_bwd(const float* x, int64_t n, int d, const float* proj, const float* mp,
+                          const float* geom, int k, int b, float max_sigma_over_delta,
+                          const float* gsums, float* gx, int accumulate, void* stream);
 
 /* ---- fused projection + exact histogram, 1-D screens -----------------------------------
  * Replaces diagnostics/diagnostics.py:128-131 (torch.histogram(x_proj, edges)): bin i holds
  * edges[i] <= u < edges[i+1], last bin closed, everything else dropped.  edges[K][B+1];
- * counts[K][B] int64, ADDED to (zero them first; integer adds => bit-reproducible).     */
-int mfb_project_hist1d(const float* x, int64_t n, int d, const float* proj, const float* edges,
-                       int k, int b, int64_t* counts, void* stream);
+ * counts[K][B] int64, ADDED to (zero them first; integer adds => bit-reproducible).  mp as
+ * for the KDE (NULL: linear).                                                             */
+int mfb_project_hist1d(const float* x, int64_t n, int d, const float* proj, const float* mp,
+                       const float* edges, int k, int b, int64_t* counts, void* stream);
 
 /* ---- 2-D screens ------------------------------------------------------------------------
  * diagnostics/diagnostics.py:179-191 -> histogram.py:89-101, 47-74: P = Kx^T Ky.

@@ -13,7 +13,7 @@ LIB_PATH = os.environ.get("MENTFLOW_B200_LIB") or os.path.join(PKG_DIR, "libment
 
 P = c_void_p  # every device pointer crosses the ABI as a plain address
 
-ABI_VERSION = 3  # MFB_ABI_VERSION of the header SIGNATURES mirrors
+ABI_VERSION = 4  # MFB_ABI_VERSION of the header SIGNATURES mirrors
 
 # name -> (restype, argtypes); mirrors include/mentflow_b200.h line by line
 SIGNATURES = {
@@ -21,22 +21,16 @@ SIGNATURES = {
     "mfb_error_string": (c_char_p, [c_int]),
     "mfb_sm_count": (c_int, []),
     "mfb_kde1d_workspace_bytes": (c_int64, [c_int64, c_int, c_int, c_int]),
-    "mfb_project_kde1d_fwd": (c_int, [P, c_int64, c_int, P, P, c_int, c_int, c_float, P, P, c_int64, P]),
-    "mfb_kde1d_normalize": (c_int, [P, c_double, P, c_int, c_int, P, P]),
-    "mfb_kde1d_normalize_bwd": (c_int, [P, c_double, P, c_int, c_int, P, P, P]),
-    "mfb_project_kde1d_loss_fwd": (c_int, [P, c_int64, c_int, P, P, c_int, c_int, c_float, c_double, P, c_float, P, P, P,
-                                           P, c_int64, P]),
+    "mfb_project_kde1d_fwd": (c_int, [P, c_int64, c_int, P, P, P, c_int, c_int, c_float, c_double, P, c_float, P, P, P,
+                                      P, c_int64, P]),
     "mfb_kde1d_finish": (c_int, [P, c_double, P, c_int, c_int, P, c_float, P, P, P]),
     "mfb_kde1d_p2p_block_floats": (c_int64, [c_int, c_int, c_int]),
     "mfb_kde1d_finish_p2p": (c_int, [P, c_int, c_int, P, P, P, c_int, c_double, P, c_int, c_int, P, c_float, P, P, P, P, P]),
     "mfb_project_kde1d_loss_fwd_p2p": (c_int, [P, c_int64, c_int, P, P, c_int, c_int, c_float, c_double, P, c_float, P,
                                                c_int, c_int, P, P, c_int, P, P, P, P, P, c_int64, P]),
     "mfb_kde1d_finish_bwd": (c_int, [P, c_double, P, c_int, c_int, P, c_float, P, P, P, P]),
-    "mfb_project_kde1d_bwd": (c_int, [P, c_int64, c_int, P, P, c_int, c_int, c_float, P, P, c_int, P]),
-    "mfb_project_kde1d_mp_fwd": (c_int, [P, c_int64, c_int, P, P, P, c_int, c_int, c_float, P, P, c_int64, P]),
-    "mfb_project_kde1d_mp_bwd": (c_int, [P, c_int64, c_int, P, P, P, c_int, c_int, c_float, P, P, c_int, P]),
-    "mfb_project_hist1d_mp": (c_int, [P, c_int64, c_int, P, P, P, c_int, c_int, P, P]),
-    "mfb_project_hist1d": (c_int, [P, c_int64, c_int, P, P, c_int, c_int, P, P]),
+    "mfb_project_kde1d_bwd": (c_int, [P, c_int64, c_int, P, P, P, c_int, c_int, c_float, P, P, c_int, P]),
+    "mfb_project_hist1d": (c_int, [P, c_int64, c_int, P, P, P, c_int, c_int, P, P]),
     "mfb_kde2d_workspace_bytes": (c_int64, [c_int64, c_int, c_int, c_int, c_int]),
     "mfb_project_kde2d_fwd": (c_int, [P, c_int64, c_int, P, P, c_int, c_int, c_int, c_float, P, P, c_int64, c_int, P]),
     "mfb_kde2d_uses_tensor_cores": (c_int, [c_int64, c_int, c_int, c_int, c_int]),

@@ -352,17 +352,7 @@ kde1d_deposit_kernel(const float* __restrict__ x, int64_t n, int d_rt, const flo
   }
 }
 
-// sums[k][b] = sum over CTAs (fixed order)
-__global__ void reduce_partials_kernel(const float* __restrict__ partial, int nparts, int64_t len,
-                                       float* __restrict__ sums) {
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < len; i += (int64_t)gridDim.x * blockDim.x) {
-    float s = 0.f;
-    for (int c = 0; c < nparts; ++c) s += partial[(size_t)c * len + i];
-    sums[i] = s;
-  }
-}
-
-// ---- normalisation and its backward: one CTA per projection ---------------------------------
+// ---- merge, normalisation and KL, forward and backward: one CTA per projection ---------------
 __device__ __forceinline__ float block_sum_256(float v, float* red) {
   // deterministic: warp shuffle tree, then thread 0 adds the 8 warp sums in order
   v = warp_sum(v);
@@ -379,39 +369,10 @@ __device__ __forceinline__ float block_sum_256(float v, float* red) {
   return t;
 }
 
-__global__ void __launch_bounds__(256)
-kde1d_normalize_kernel(const float* __restrict__ sums, float inv_n, const float* __restrict__ geom, int B,
-                       float* __restrict__ prof) {
-  __shared__ float red[33];
-  const int k = blockIdx.x;
-  const float delta = geom[(size_t)k * MFB_GEOM_STRIDE + 3];  // the reference's c[1]-c[0]
-  float acc = 0.f;
-  for (int b = threadIdx.x; b < B; b += blockDim.x) acc += sums[(size_t)k * B + b] * inv_n * delta;
-  const float z = block_sum_256(acc, red) + 1.0e-10f;
-  for (int b = threadIdx.x; b < B; b += blockDim.x) prof[(size_t)k * B + b] = sums[(size_t)k * B + b] * inv_n / z;
-}
-
-__global__ void __launch_bounds__(256)
-kde1d_normalize_bwd_kernel(const float* __restrict__ sums, float inv_n, const float* __restrict__ geom, int B,
-                           const float* __restrict__ gprof, float* __restrict__ gsums) {
-  __shared__ float red[33];
-  const int k = blockIdx.x;
-  const float delta = geom[(size_t)k * MFB_GEOM_STRIDE + 3];  // the reference's c[1]-c[0]
-  float acc = 0.f;
-  for (int b = threadIdx.x; b < B; b += blockDim.x) acc += sums[(size_t)k * B + b] * inv_n * delta;
-  const float z = block_sum_256(acc, red) + 1.0e-10f;
-  float dot = 0.f;  // sum_j gp_j p_j
-  for (int b = threadIdx.x; b < B; b += blockDim.x)
-    dot += gprof[(size_t)k * B + b] * (sums[(size_t)k * B + b] * inv_n / z);
-  const float g = block_sum_256(dot, red);
-  for (int b = threadIdx.x; b < B; b += blockDim.x)
-    gsums[(size_t)k * B + b] = (gprof[(size_t)k * B + b] / z - delta * g / z) * inv_n;
-}
-
 // ---- fused tail of the forward pass: merge per-CTA partials, normalise, KL against the measurement ----
-// One CTA per projection.  Replaces reduce_partials + normalize + the ~8 elementwise/reduce kernels of
-// loss.py:15-17 evaluated on (K, B) tensors.  Sum order is fixed (partials c = g, g+G, ... per group g,
-// groups combined in order), so the result is run-to-run deterministic.
+// One CTA per projection.  Replaces the merge, the normalisation of histogram.py:39-43 and the ~8
+// elementwise/reduce kernels of loss.py:15-17 evaluated on (K, B) tensors.  Sum order is fixed
+// (partials c = g, g+G, ... per group g, groups combined in order), so the result is run-to-run deterministic.
 constexpr int kFinishThreads = 256;
 
 __device__ __forceinline__ void merge_partials_to_smem(const float* __restrict__ partial, int nparts, int64_t len,
@@ -605,7 +566,7 @@ kde1d_finish_p2p_kernel(const __grid_constant__ PeerSet peers, int rank, int wor
 }
 
 // gradient of (profiles, KL) w.r.t. the unnormalised sums:  gp_b = gprof_b - gkl * t_b / (p_b + pad) / B,
-// then the normalisation backward of kde1d_normalize_bwd_kernel
+// then the normalisation backward  gsums_b = (gp_b / z - delta sum_j gp_j p_j / z) / N
 __global__ void __launch_bounds__(kFinishThreads)
 kde1d_finish_bwd_kernel(const float* __restrict__ sums, float inv_n, const float* __restrict__ geom, int B,
                         const float* __restrict__ meas, float pad, const float* __restrict__ gprof,
@@ -866,19 +827,6 @@ static int launch_kde1d_deposit(int r, const KdePlan& L, const float* x, int64_t
   return launch_status();
 }
 
-// deposit of all projections into the per-CTA partials; mp != nullptr selects the multipole variant
-// (runtime dimension: the non-linear configurations are low-dimensional)
-static int deposit_dispatch(int r, const KdePlan& L, const float* x, int64_t n, int d, const float* proj,
-                            const float* geom, int k, int b, float* partial, cudaStream_t st, const float* mp) {
-  if (mp) return launch_kde1d_deposit<0, true>(r, L, x, n, d, proj, geom, k, b, partial, st, mp);
-  switch (d) {
-    case 2: return launch_kde1d_deposit<2>(r, L, x, n, d, proj, geom, k, b, partial, st);
-    case 4: return launch_kde1d_deposit<4>(r, L, x, n, d, proj, geom, k, b, partial, st);
-    case 6: return launch_kde1d_deposit<6>(r, L, x, n, d, proj, geom, k, b, partial, st);
-    default: return launch_kde1d_deposit<0>(r, L, x, n, d, proj, geom, k, b, partial, st);
-  }
-}
-
 template <int D, bool kMP = false>
 static int launch_kde1d_bwd(int r, int grid, size_t smem, const float* x, int64_t n, int d, const float* proj,
                             const float* geom, int k, int b, const float* gsums, float* gx, int acc,
@@ -905,6 +853,29 @@ using namespace mfb;
 // passes the largest sigma/delta ratio of the launch (<= 0 means the default bandwidth 0.5).
 static int radius_from_hint(float hint) { return window_radius(hint > 0.f ? hint : 0.5); }
 
+// the window radius of the kernel template that serves radius r (launches refuse r > 13)
+static int compiled_radius(int r) { return r <= 4 ? 4 : (r <= 9 ? 9 : 13); }
+
+// deposit of all projections (n >= 1) into the per-CTA partials [nparts][k][b] in the workspace; mp != nullptr
+// selects the multipole variant (runtime dimension: the non-linear configurations are low-dimensional)
+static int kde1d_deposit(const float* x, int64_t n, int d, const float* proj, const float* mp, const float* geom,
+                         int k, int b, float max_sigma_over_delta, void* workspace, int64_t workspace_bytes,
+                         cudaStream_t st, int* nparts) {
+  const int r = radius_from_hint(max_sigma_over_delta);
+  KdePlan L = plan_kde(n, d, k, b, compiled_radius(r));
+  if (L.smem > 227 * 1024) return MFB_E_UNSUPPORTED;
+  if (workspace_bytes < (int64_t)L.grid_x * k * b * 4) return MFB_E_WORKSPACE;
+  *nparts = L.grid_x;
+  float* partial = (float*)workspace;
+  if (mp) return launch_kde1d_deposit<0, true>(r, L, x, n, d, proj, geom, k, b, partial, st, mp);
+  switch (d) {
+    case 2: return launch_kde1d_deposit<2>(r, L, x, n, d, proj, geom, k, b, partial, st);
+    case 4: return launch_kde1d_deposit<4>(r, L, x, n, d, proj, geom, k, b, partial, st);
+    case 6: return launch_kde1d_deposit<6>(r, L, x, n, d, proj, geom, k, b, partial, st);
+    default: return launch_kde1d_deposit<0>(r, L, x, n, d, proj, geom, k, b, partial, st);
+  }
+}
+
 extern "C" {
 
 int64_t mfb_kde1d_workspace_bytes(int64_t n, int d, int k, int b) {
@@ -916,67 +887,23 @@ int64_t mfb_kde1d_workspace_bytes(int64_t n, int d, int k, int b) {
   return gx * k * b * 4;
 }
 
-static int kde1d_fwd_impl(const float* x, int64_t n, int d, const float* proj, const float* mp, const float* geom,
-                         int k, int b, float max_sigma_over_delta, float* sums, void* workspace,
-                         int64_t workspace_bytes, void* stream) {
+int mfb_project_kde1d_fwd(const float* x, int64_t n, int d, const float* proj, const float* mp, const float* geom,
+                          int k, int b, float max_sigma_over_delta, double n_total, const float* meas, float pad,
+                          float* sums, float* profiles, float* kl, void* workspace, int64_t workspace_bytes,
+                          void* stream) {
   MFB_CHECK_ARG(x && proj && geom && sums && workspace);
   MFB_CHECK_ARG(n >= 0 && d >= 1 && d <= kMaxDim && k >= 1 && b >= 2);
+  MFB_CHECK_ARG((meas != nullptr) == (kl != nullptr));
+  MFB_CHECK_ARG(profiles ? n >= 1 && n_total > 0 : meas == nullptr);
   cudaStream_t st = (cudaStream_t)stream;
   if (n == 0) return (int)cudaMemsetAsync(sums, 0, (size_t)k * b * 4, st);
-  const int r = radius_from_hint(max_sigma_over_delta);
-  const int rr = r <= 4 ? 4 : (r <= 9 ? 9 : 13);   // compiled window radii
-  KdePlan L = plan_kde(n, d, k, b, rr);
-  if (L.smem > 227 * 1024) return MFB_E_UNSUPPORTED;
-  if (workspace_bytes < (int64_t)L.grid_x * k * b * 4) return MFB_E_WORKSPACE;
-  float* partial = (float*)workspace;
-  int rc = deposit_dispatch(r, L, x, n, d, proj, geom, k, b, partial, st, mp);
-  if (rc) return rc;
-  const int64_t len = (int64_t)k * b;
-  if (finish_smem(b) > 48 * 1024) {   // very wide screens: the plain merge
-    int rgrid = (int)((len + 255) / 256);
-    reduce_partials_kernel<<<rgrid, 256, 0, st>>>(partial, L.grid_x, len, sums);
-    return launch_status();
-  }
-  MFB_CUDA(launch_pdl(kde1d_finish_kernel, dim3(k), dim3(kFinishThreads), finish_smem(b), st, partial, L.grid_x, len, 1.f, geom, b, nullptr, 0.f,
-                                                                 sums, nullptr, nullptr));
-  return launch_status();
-}
-
-int mfb_project_kde1d_fwd(const float* x, int64_t n, int d, const float* proj, const float* geom, int k, int b,
-                          float max_sigma_over_delta, float* sums, void* workspace, int64_t workspace_bytes,
-                          void* stream) {
-  return kde1d_fwd_impl(x, n, d, proj, nullptr, geom, k, b, max_sigma_over_delta, sums, workspace, workspace_bytes,
-                        stream);
-}
-
-int mfb_project_kde1d_mp_fwd(const float* x, int64_t n, int d, const float* proj, const float* mp, const float* geom,
-                             int k, int b, float max_sigma_over_delta, float* sums, void* workspace,
-                             int64_t workspace_bytes, void* stream) {
-  MFB_CHECK_ARG(mp);
-  return kde1d_fwd_impl(x, n, d, proj, mp, geom, k, b, max_sigma_over_delta, sums, workspace, workspace_bytes,
-                        stream);
-}
-
-int mfb_project_kde1d_loss_fwd(const float* x, int64_t n, int d, const float* proj, const float* geom, int k, int b,
-                               float max_sigma_over_delta, double n_total, const float* meas, float pad,
-                               float* sums, float* profiles, float* kl, void* workspace, int64_t workspace_bytes,
-                               void* stream) {
-  MFB_CHECK_ARG(x && proj && geom && sums && profiles && workspace);
-  MFB_CHECK_ARG((meas != nullptr) == (kl != nullptr));
-  MFB_CHECK_ARG(n >= 1 && d >= 1 && d <= kMaxDim && k >= 1 && b >= 2 && n_total > 0);
   if (finish_smem(b) > 48 * 1024) return MFB_E_UNSUPPORTED;
-  cudaStream_t st = (cudaStream_t)stream;
-  const int r = radius_from_hint(max_sigma_over_delta);
-  const int rr = r <= 4 ? 4 : (r <= 9 ? 9 : 13);
-  KdePlan L = plan_kde(n, d, k, b, rr);
-  if (L.smem > 227 * 1024) return MFB_E_UNSUPPORTED;
-  if (workspace_bytes < (int64_t)L.grid_x * k * b * 4) return MFB_E_WORKSPACE;
-  float* partial = (float*)workspace;
-  int rc = deposit_dispatch(r, L, x, n, d, proj, geom, k, b, partial, st, nullptr);
+  int nparts = 0;
+  int rc = kde1d_deposit(x, n, d, proj, mp, geom, k, b, max_sigma_over_delta, workspace, workspace_bytes, st, &nparts);
   if (rc) return rc;
-  MFB_CUDA(launch_pdl(kde1d_finish_kernel, dim3(k), dim3(kFinishThreads), finish_smem(b), st, partial, L.grid_x, (int64_t)k * b,
-                                                                 (float)(1.0 / n_total), geom, b, meas, pad, sums,
-                                                                 profiles, kl));
+  const float inv_n = profiles ? (float)(1.0 / n_total) : 1.f;   // without profiles the kernel stops after the merge
+  MFB_CUDA(launch_pdl(kde1d_finish_kernel, dim3(k), dim3(kFinishThreads), finish_smem(b), st, workspace, nparts,
+                      (int64_t)k * b, inv_n, geom, b, meas, pad, sums, profiles, kl));
   return launch_status();
 }
 
@@ -1006,7 +933,7 @@ int mfb_kde1d_finish_p2p(const uint64_t* peer_blocks_host, int rank, int world, 
 }
 
 /* deposit + (merge, cross-rank sum, normalise, KL) in two launches: the sharded counterpart of
- * mfb_project_kde1d_loss_fwd */
+ * mfb_project_kde1d_fwd with profiles */
 int mfb_project_kde1d_loss_fwd_p2p(const float* x, int64_t n, int d, const float* proj, const float* geom, int k, int b,
                                    float max_sigma_over_delta, double n_total, const float* meas, float pad,
                                    const uint64_t* peer_blocks_host, int rank, int world, uint32_t* state,
@@ -1019,20 +946,16 @@ int mfb_project_kde1d_loss_fwd_p2p(const float* x, int64_t n, int d, const float
   MFB_CHECK_ARG(tail_doubles >= 0 && tail_doubles <= 32 && (tail_doubles == 0 || (local_tail && tail_out)));
   if (finish_smem(b) > 48 * 1024 || k > 1024) return MFB_E_UNSUPPORTED;
   cudaStream_t st = (cudaStream_t)stream;
-  const int r = radius_from_hint(max_sigma_over_delta);
-  const int rr = r <= 4 ? 4 : (r <= 9 ? 9 : 13);
-  KdePlan L = plan_kde(n, d, k, b, rr);
-  if (L.smem > 227 * 1024) return MFB_E_UNSUPPORTED;
-  if (workspace_bytes < (int64_t)L.grid_x * k * b * 4) return MFB_E_WORKSPACE;
-  float* partial = (float*)workspace;
-  int rc = deposit_dispatch(r, L, x, n, d, proj, geom, k, b, partial, st, nullptr);
+  int nparts = 0;
+  int rc = kde1d_deposit(x, n, d, proj, nullptr, geom, k, b, max_sigma_over_delta, workspace, workspace_bytes, st,
+                         &nparts);
   if (rc) return rc;
   PeerSet ps;
   for (int i = 0; i < kMaxRanks; ++i) ps.buf[i] = i < world ? reinterpret_cast<float*>(peer_blocks_host[i]) : nullptr;
   const int64_t parity = (int64_t)k * b + 2 * (int64_t)tail_doubles;
   kde1d_finish_p2p_kernel<<<k, kFinishThreads, finish_smem(b), st>>>(
-      ps, rank, world, state, parity, partial, L.grid_x, local_tail, tail_doubles, (float)(1.0 / n_total), geom, k, b,
-      meas, pad, sums, profiles, kl, tail_out);
+      ps, rank, world, state, parity, (const float*)workspace, nparts, local_tail, tail_doubles,
+      (float)(1.0 / n_total), geom, k, b, meas, pad, sums, profiles, kl, tail_out);
   return launch_status();
 }
 
@@ -1055,31 +978,16 @@ int mfb_kde1d_finish_bwd(const float* sums, double n_total, const float* geom, i
   return launch_status();
 }
 
-int mfb_kde1d_normalize(const float* sums, double n_total, const float* geom, int k, int b, float* profiles,
-                        void* stream) {
-  MFB_CHECK_ARG(sums && geom && profiles && k >= 1 && b >= 2 && n_total > 0);
-  kde1d_normalize_kernel<<<k, 256, 0, (cudaStream_t)stream>>>(sums, (float)(1.0 / n_total), geom, b, profiles);
-  return launch_status();
-}
-
-int mfb_kde1d_normalize_bwd(const float* sums, double n_total, const float* geom, int k, int b,
-                            const float* gprof, float* gsums, void* stream) {
-  MFB_CHECK_ARG(sums && geom && gprof && gsums && k >= 1 && b >= 2 && n_total > 0);
-  kde1d_normalize_bwd_kernel<<<k, 256, 0, (cudaStream_t)stream>>>(sums, (float)(1.0 / n_total), geom, b, gprof,
-                                                                  gsums);
-  return launch_status();
-}
-
-static int kde1d_bwd_impl(const float* x, int64_t n, int d, const float* proj, const float* mp, const float* geom,
-                         int k, int b, float max_sigma_over_delta, const float* gsums, float* gx, int accumulate,
-                         void* stream) {
+int mfb_project_kde1d_bwd(const float* x, int64_t n, int d, const float* proj, const float* mp, const float* geom,
+                          int k, int b, float max_sigma_over_delta, const float* gsums, float* gx, int accumulate,
+                          void* stream) {
   MFB_CHECK_ARG(x && proj && geom && gsums && gx);
   MFB_CHECK_ARG(n >= 0 && d >= 1 && d <= kMaxDim && k >= 1 && b >= 2);
   if (n == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
   const int r = radius_from_hint(max_sigma_over_delta);
   // projections are processed in chunks whose gradient table fits in shared memory
-  const int rt = r <= 4 ? 4 : (r <= 9 ? 9 : 13);                      // the template radius the launch picks
+  const int rt = compiled_radius(r);
   const size_t bp = (size_t)b + 2 * (2 * rt + 2);                       // padded gradient row
   const size_t per_k = bp * 4 + (size_t)d * 4 + 16 + (size_t)rt * 4 + (mp ? (size_t)MFB_MP_STRIDE(d) * 4 : 0);
   int kchunk = (int)((160 * 1024) / per_k);
@@ -1118,19 +1026,7 @@ static int kde1d_bwd_impl(const float* x, int64_t n, int d, const float* proj, c
   return 0;
 }
 
-int mfb_project_kde1d_bwd(const float* x, int64_t n, int d, const float* proj, const float* geom, int k, int b,
-                          float max_sigma_over_delta, const float* gsums, float* gx, int accumulate, void* stream) {
-  return kde1d_bwd_impl(x, n, d, proj, nullptr, geom, k, b, max_sigma_over_delta, gsums, gx, accumulate, stream);
-}
-
-int mfb_project_kde1d_mp_bwd(const float* x, int64_t n, int d, const float* proj, const float* mp, const float* geom,
-                             int k, int b, float max_sigma_over_delta, const float* gsums, float* gx, int accumulate,
-                             void* stream) {
-  MFB_CHECK_ARG(mp);
-  return kde1d_bwd_impl(x, n, d, proj, mp, geom, k, b, max_sigma_over_delta, gsums, gx, accumulate, stream);
-}
-
-static int hist1d_impl(const float* x, int64_t n, int d, const float* proj, const float* mp, const float* edges, int k,
+int mfb_project_hist1d(const float* x, int64_t n, int d, const float* proj, const float* mp, const float* edges, int k,
                        int b, int64_t* counts, void* stream) {
   MFB_CHECK_ARG(x && proj && edges && counts);
   MFB_CHECK_ARG(n >= 0 && d >= 1 && d <= kMaxDim && k >= 1 && b >= 1);
@@ -1162,17 +1058,6 @@ static int hist1d_impl(const float* x, int64_t n, int d, const float* proj, cons
   }
 #undef MFB_LAUNCH_D
   return launch_status();
-}
-
-int mfb_project_hist1d(const float* x, int64_t n, int d, const float* proj, const float* edges, int k, int b,
-                       int64_t* counts, void* stream) {
-  return hist1d_impl(x, n, d, proj, nullptr, edges, k, b, counts, stream);
-}
-
-int mfb_project_hist1d_mp(const float* x, int64_t n, int d, const float* proj, const float* mp, const float* edges,
-                          int k, int b, int64_t* counts, void* stream) {
-  MFB_CHECK_ARG(mp);
-  return hist1d_impl(x, n, d, proj, mp, edges, k, b, counts, stream);
 }
 
 }  // extern "C"

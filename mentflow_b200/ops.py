@@ -88,88 +88,55 @@ def _check_mp(mp: torch.Tensor, k: int, d: int) -> torch.Tensor:
     return mp
 
 
+KL_PAD = 1.0e-12   # loss.py:15-17
+
+
+def _kde1d_fwd(x, proj, geom, ratio, mp, sums, n_total=1.0, meas=None, prof=None, kl=None):
+    """Deposit + merge into ``sums`` (K, B); with ``prof`` also normalise by ``n_total`` (+ KL against ``meas``)."""
+    lib = _lib.load()
+    check_kde_ratio(ratio, KDE1D_MAX_RADIUS, "1-D KDE")
+    x, proj, geom = _check_f32("x", x), _check_f32("proj", proj), _check_f32("geom", geom)
+    n, d = x.shape
+    k, nbins = sums.shape
+    if mp is not None:
+        mp = _check_mp(mp, k, d)
+    with torch.cuda.device(x.device):
+        wbytes = lib.mfb_kde1d_workspace_bytes(n, d, k, nbins)
+        work = torch.empty(max(wbytes, 16), dtype=torch.uint8, device=x.device)
+        _lib.check(lib.mfb_project_kde1d_fwd(_ptr(x), n, d, _ptr(proj), _ptr(mp), _ptr(geom), k, nbins, float(ratio),
+                                             float(n_total), _ptr(meas), KL_PAD, _ptr(sums), _ptr(prof), _ptr(kl),
+                                             _ptr(work), wbytes, _stream()), "project_kde1d_fwd")
+
+
 def kde1d_sums(x: torch.Tensor, proj: torch.Tensor, geom: torch.Tensor, ratio: float, nbins: int,
                mp: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """S[k, b] = sum_n exp(-0.5 ((u_kn - c_b) / sigma_k)^2)  (unnormalised), u_kn = proj_k . x_n, plus the
     multipole terms of ``mp`` (K, 2D+4) when given (see ``simulate.multipole_terms``)."""
-    lib = _lib.load()
-    check_kde_ratio(ratio, KDE1D_MAX_RADIUS, "1-D KDE")
-    x, proj, geom = _check_f32("x", x), _check_f32("proj", proj), _check_f32("geom", geom)
-    n, d = x.shape
-    k = proj.shape[0]
-    sums = out if out is not None else torch.empty((k, nbins), dtype=torch.float32, device=x.device)
-    with torch.cuda.device(x.device):
-        wbytes = lib.mfb_kde1d_workspace_bytes(n, d, k, nbins)
-        work = torch.empty(max(wbytes, 16), dtype=torch.uint8, device=x.device)
-        if mp is None:
-            _lib.check(lib.mfb_project_kde1d_fwd(_ptr(x), n, d, _ptr(proj), _ptr(geom), k, nbins, float(ratio),
-                                                 _ptr(sums), _ptr(work), wbytes, _stream()), "project_kde1d_fwd")
-        else:
-            mp = _check_mp(mp, k, d)
-            _lib.check(lib.mfb_project_kde1d_mp_fwd(_ptr(x), n, d, _ptr(proj), _ptr(mp), _ptr(geom), k, nbins,
-                                                    float(ratio), _ptr(sums), _ptr(work), wbytes, _stream()),
-                       "project_kde1d_mp_fwd")
+    sums = out if out is not None else torch.empty((proj.shape[0], nbins), dtype=torch.float32, device=x.device)
+    _kde1d_fwd(x, proj, geom, ratio, mp, sums)
     return sums
 
 
-def kde1d_normalize(sums: torch.Tensor, n_total: float, geom: torch.Tensor) -> torch.Tensor:
-    lib = _lib.load()
-    k, b = sums.shape
-    prof = torch.empty_like(sums)
-    with torch.cuda.device(sums.device):
-        _lib.check(lib.mfb_kde1d_normalize(_ptr(sums), float(n_total), _ptr(geom), k, b, _ptr(prof), _stream()),
-                   "kde1d_normalize")
-    return prof
-
-
-def kde1d_normalize_bwd(sums, n_total, geom, gprof):
-    lib = _lib.load()
-    k, b = sums.shape
-    gprof = _check_f32("gprof", gprof)
-    gsums = torch.empty_like(sums)
-    with torch.cuda.device(sums.device):
-        _lib.check(lib.mfb_kde1d_normalize_bwd(_ptr(sums), float(n_total), _ptr(geom), k, b, _ptr(gprof),
-                                               _ptr(gsums), _stream()), "kde1d_normalize_bwd")
-    return gsums
-
-
-def kde1d_grad_x(x, proj, geom, ratio, gsums, out: Optional[torch.Tensor] = None, mp: Optional[torch.Tensor] = None):
+def kde1d_grad_x(x, proj, geom, ratio, gsums, mp: Optional[torch.Tensor] = None):
     lib = _lib.load()
     check_kde_ratio(ratio, KDE1D_MAX_RADIUS, "1-D KDE backward")
     n, d = x.shape
     k, b = gsums.shape
-    acc = 1 if out is not None else 0
-    gx = out if out is not None else torch.empty_like(x)
+    if mp is not None:
+        mp = _check_mp(mp, k, d)
+    gx = torch.empty_like(x)
     with torch.cuda.device(x.device):
-        if mp is None:
-            _lib.check(lib.mfb_project_kde1d_bwd(_ptr(x), n, d, _ptr(proj), _ptr(geom), k, b, float(ratio),
-                                                 _ptr(gsums), _ptr(gx), acc, _stream()), "project_kde1d_bwd")
-        else:
-            mp = _check_mp(mp, k, d)
-            _lib.check(lib.mfb_project_kde1d_mp_bwd(_ptr(x), n, d, _ptr(proj), _ptr(mp), _ptr(geom), k, b, float(ratio),
-                                                    _ptr(gsums), _ptr(gx), acc, _stream()), "project_kde1d_mp_bwd")
+        _lib.check(lib.mfb_project_kde1d_bwd(_ptr(x), n, d, _ptr(proj), _ptr(mp), _ptr(geom), k, b, float(ratio),
+                                             _ptr(gsums), _ptr(gx), 0, _stream()), "project_kde1d_bwd")
     return gx
 
 
-KL_PAD = 1.0e-12   # loss.py:15-17
-
-
-def kde1d_loss_forward(x, proj, geom, ratio, nbins, n_total, meas):
+def kde1d_loss_forward(x, proj, geom, ratio, nbins, n_total, meas, mp=None):
     """Deposit + merge + normalise (+ KL against ``meas``) in two launches: (sums, profiles, kl)."""
-    lib = _lib.load()
-    check_kde_ratio(ratio, KDE1D_MAX_RADIUS, "1-D KDE")
-    x, proj, geom = _check_f32("x", x), _check_f32("proj", proj), _check_f32("geom", geom)
-    n, d = x.shape
-    k = proj.shape[0]
-    sums = torch.empty((k, nbins), dtype=torch.float32, device=x.device)
+    sums = torch.empty((proj.shape[0], nbins), dtype=torch.float32, device=x.device)
     prof = torch.empty_like(sums)
-    kl = torch.empty(k, dtype=torch.float32, device=x.device) if meas is not None else None
-    with torch.cuda.device(x.device):
-        wbytes = lib.mfb_kde1d_workspace_bytes(n, d, k, nbins)
-        work = torch.empty(max(wbytes, 16), dtype=torch.uint8, device=x.device)
-        _lib.check(lib.mfb_project_kde1d_loss_fwd(_ptr(x), n, d, _ptr(proj), _ptr(geom), k, nbins, float(ratio),
-                                                  float(n_total), _ptr(meas), KL_PAD, _ptr(sums), _ptr(prof),
-                                                  _ptr(kl), _ptr(work), wbytes, _stream()), "project_kde1d_loss_fwd")
+    kl = torch.empty(proj.shape[0], dtype=torch.float32, device=x.device) if meas is not None else None
+    _kde1d_fwd(x, proj, geom, ratio, mp, sums, n_total, meas, prof, kl)
     return sums, prof, kl
 
 
@@ -243,9 +210,6 @@ def kde1d_finish_p2p(peer, sums_local, tail, n_total, geom, meas):
     return sums, prof, kl, tail_out
 
 
-_FINISH_MAX_BINS = 6000   # shared-memory bound of the fused tail kernel
-
-
 class ProjectKDE1D(torch.autograd.Function):
     """profiles[k, b] of K one-dimensional screens, differentiable w.r.t. the particles.
 
@@ -263,24 +227,21 @@ class ProjectKDE1D(torch.autograd.Function):
         n_total = float(x.shape[0])
         if meas is not None:
             meas = _check_f32("meas", meas)
-        if reducer is None and mp is None and x.shape[0] > 0 and nbins <= _FINISH_MAX_BINS:
-            sums, prof, kl = kde1d_loss_forward(x, proj, geom, ratio, nbins, n_total, meas)
+        peer = getattr(reducer, "peer", None)
+        if reducer is None and x.shape[0] > 0:
+            sums, prof, kl = kde1d_loss_forward(x, proj, geom, ratio, nbins, n_total, meas, mp)
+        elif (peer is not None and mp is None and x.shape[0] > 0 and proj.shape[0] <= 1024 and nbins <= 4096
+                and (proj.shape[0] * nbins) % 2 == 0):
+            # sharded: the cross-rank sum happens inside the tail kernel, over NVLink peer memory
+            n_total = reducer.global_count(n_total)
+            stash = reducer.take_stash()
+            sums, prof, kl, tail_sum = kde1d_loss_forward_p2p(peer, x, proj, geom, ratio, nbins, stash, n_total, meas)
+            if stash is not None:
+                reducer.set_stash_result(tail_sum)
+            reducer.calls += 1
         else:
             # sharded: the unnormalised sums are all-reduced before the non-linear tail; float64 partial sums
             # another op stashed on the reducer (the entropy moments) ride at the end of the same buffer
-            peer = getattr(reducer, "peer", None)
-            if (peer is not None and mp is None and x.shape[0] > 0 and proj.shape[0] <= 1024 and nbins <= 4096
-                    and (proj.shape[0] * nbins) % 2 == 0):
-                # the cross-rank sum happens inside the tail kernel, over NVLink peer memory
-                n_total = reducer.global_count(n_total)
-                stash = reducer.take_stash()
-                sums, prof, kl, tail_sum = kde1d_loss_forward_p2p(peer, x, proj, geom, ratio, nbins, stash, n_total, meas)
-                if stash is not None:
-                    reducer.set_stash_result(tail_sum)
-                reducer.calls += 1
-                ctx.save_for_backward(x, proj, geom, sums, meas, None, mp)
-                ctx.ratio, ctx.n_total = ratio, n_total
-                return prof if meas is None else (prof, kl)
             tail = reducer.tail_floats() if hasattr(reducer, "tail_floats") else 0
             if tail:
                 flat = torch.empty(proj.shape[0] * nbins + tail, dtype=torch.float32, device=x.device)
@@ -290,14 +251,8 @@ class ProjectKDE1D(torch.autograd.Function):
                 sums = kde1d_sums(x, proj, geom, ratio, nbins, mp)
                 if reducer is not None:
                     n_total = reducer(sums, n_total)
-            if nbins <= _FINISH_MAX_BINS:
-                prof, kl = kde1d_finish(sums, n_total, geom, meas)
-            else:
-                prof = kde1d_normalize(sums, n_total, geom)
-                kl = None
-                if meas is not None:
-                    kl = (torch.xlogy(meas, meas) - meas * torch.log(prof + KL_PAD)).sum(dim=1) / nbins
-        ctx.save_for_backward(x, proj, geom, sums, meas, prof if nbins > _FINISH_MAX_BINS else None, mp)
+            prof, kl = kde1d_finish(sums, n_total, geom, meas)
+        ctx.save_for_backward(x, proj, geom, sums, meas, mp)
         ctx.ratio, ctx.n_total = ratio, n_total
         if meas is None:
             return prof
@@ -305,16 +260,10 @@ class ProjectKDE1D(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, gprof, gkl=None):
-        x, proj, geom, sums, meas, prof, mp = ctx.saved_tensors
+        x, proj, geom, sums, meas, mp = ctx.saved_tensors
         if gprof is None and gkl is None:
             return None, None, None, None, None, None, None, None
-        if prof is not None:       # wide screens: torch expression for the KL part
-            if gkl is not None:
-                extra = -(gkl / sums.shape[1])[:, None] * meas / (prof + KL_PAD)
-                gprof = extra if gprof is None else gprof + extra
-            gsums = kde1d_normalize_bwd(sums, ctx.n_total, geom, gprof)
-        else:
-            gsums = kde1d_finish_bwd(sums, ctx.n_total, geom, meas, gprof, gkl if meas is not None else None)
+        gsums = kde1d_finish_bwd(sums, ctx.n_total, geom, meas, gprof, gkl if meas is not None else None)
         gx = kde1d_grad_x(x, proj, geom, ctx.ratio, gsums, mp=mp)
         return gx, None, None, None, None, None, None, None
 
@@ -339,14 +288,11 @@ def project_hist1d(x: torch.Tensor, proj: torch.Tensor, edges: torch.Tensor,
         counts = torch.zeros((k, b), dtype=torch.int64, device=x.device)
     if n == 0:              # nothing to count
         return counts
+    if mp is not None:
+        mp = _check_mp(mp, k, d)
     with torch.cuda.device(x.device):
-        if mp is None:
-            _lib.check(lib.mfb_project_hist1d(_ptr(x), n, d, _ptr(proj), _ptr(edges), k, b, _ptr(counts), _stream()),
-                       "project_hist1d")
-        else:
-            mp = _check_mp(mp, k, d)
-            _lib.check(lib.mfb_project_hist1d_mp(_ptr(x), n, d, _ptr(proj), _ptr(mp), _ptr(edges), k, b, _ptr(counts),
-                                                 _stream()), "project_hist1d_mp")
+        _lib.check(lib.mfb_project_hist1d(_ptr(x), n, d, _ptr(proj), _ptr(mp), _ptr(edges), k, b, _ptr(counts),
+                                          _stream()), "project_hist1d")
     return counts
 
 

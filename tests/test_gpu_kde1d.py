@@ -144,19 +144,27 @@ def test_full_size_properties():
     counts = ops.project_hist1d(x, w, edges.cuda()[None].repeat(k, 1))
     n_in = ((x @ w.T >= edges[0]) & (x @ w.T <= edges[-1])).sum(dim=0)
     assert (counts.sum(dim=1) - n_in).abs().max() <= 2
-    prof = ops.kde1d_normalize(full.float(), n, geom)
+    prof = ops.kde1d_finish(full.float(), n, geom, None)[0]
     assert torch.allclose(prof.sum(dim=1) * delta, torch.ones(k, device="cuda"), atol=1e-5)
 
 
-@pytest.mark.parametrize("n,d,k,nb", [(1, 6, 3, 64), (4097, 4, 11, 37), (70001, 6, 100, 64), (3000, 2, 5, 300),
-                                      (2000, 3, 2, 1000)])
-def test_fused_loss_tail_matches_separate_kernels_and_torch_kl(n, d, k, nb):
-    """deposit + merge + normalise + KL in two launches (mfb_project_kde1d_loss_fwd / _finish / _finish_bwd)
-    vs the separate normalise kernel and the torch expression of loss.py:15-17, values and gradients."""
+@pytest.mark.parametrize("n,d,k,nb,kick", [pytest.param(*c, False, id="-".join(map(str, c))) for c in
+                                           [(1, 6, 3, 64), (4097, 4, 11, 37), (70001, 6, 100, 64), (3000, 2, 5, 300),
+                                            (2000, 3, 2, 1000)]] + [pytest.param(30001, 4, 7, 64, True, id="30001-4-7-64-kick")])
+def test_fused_loss_tail_matches_separate_kernels_and_torch_kl(n, d, k, nb, kick):
+    """deposit + merge + normalise + KL in two launches (mfb_project_kde1d_fwd with profiles / _finish / _finish_bwd)
+    vs the torch expression of loss.py:15-17, values and gradients; ``kick``: screens behind a multipole kick."""
     gen = torch.Generator().manual_seed(7 * n + k)
     x = torch.randn(n, d, generator=gen).cuda()
     w = torch.randn(k, d, generator=gen)
     w = (w / w.norm(dim=1, keepdim=True)).cuda()
+    mp = None
+    if kick:                                      # kick -> screen row, orders 3, 4, 5, normal and skew
+        from mentflow_b200.simulate.simulate import multipole_terms
+        terms = [multipole_terms(w[i], None, mf.simulate.MultipoleTransform(3 + i % 3, 0.5 - 0.15 * i, i % 2 == 1), d)
+                 for i in range(k)]
+        w = torch.stack([t[0] for t in terms]).cuda()
+        mp = torch.stack([t[1] for t in terms]).cuda()
     edges = torch.linspace(-3.5, 3.5, nb + 1)
     geom = geom_rows(edges, 0.5, k)[0].cuda()
     meas = torch.rand(k, nb, generator=gen)
@@ -164,14 +172,14 @@ def test_fused_loss_tail_matches_separate_kernels_and_torch_kl(n, d, k, nb):
     meas = (meas / meas.sum(dim=1, keepdim=True) * nb / 7.0).cuda()
 
     xa = x.clone().requires_grad_(True)
-    prof_a, kl_a = ops.project_kde1d(xa, w, geom, 0.5, nb, None, meas)
+    prof_a, kl_a = ops.project_kde1d(xa, w, geom, 0.5, nb, None, meas, mp)
     xb = x.clone().requires_grad_(True)
-    prof_b = ops.project_kde1d(xb, w, geom, 0.5, nb)
+    prof_b = ops.project_kde1d(xb, w, geom, 0.5, nb, mp=mp)
     kl_b = mf.loss.kl_divergence_batched(prof_b, meas)
     assert float((prof_a - prof_b).abs().max()) <= 2e-6 * float(prof_b.abs().max())
     assert torch.allclose(kl_a, kl_b, rtol=2e-5, atol=1e-6)
     # the merged sums agree with the stand-alone merge bit for bit (same kernel, same order)
-    sums = ops.kde1d_sums(x, w, geom, 0.5, nb)
+    sums = ops.kde1d_sums(x, w, geom, 0.5, nb, mp)
     prof_c, kl_c = ops.kde1d_finish(sums, float(n), geom, meas)
     assert torch.equal(prof_c, prof_a) and torch.equal(kl_c, kl_a)
 
@@ -183,10 +191,10 @@ def test_fused_loss_tail_matches_separate_kernels_and_torch_kl(n, d, k, nb):
     assert float((xa.grad - xb.grad).abs().max()) <= 1e-4 * scale
     # KL only (no gradient through the profiles): the materialised-zero path is skipped
     xc = x.clone().requires_grad_(True)
-    _, kl_only = ops.project_kde1d(xc, w, geom, 0.5, nb, None, meas)
+    _, kl_only = ops.project_kde1d(xc, w, geom, 0.5, nb, None, meas, mp)
     kl_only.sum().backward()
     xd = x.clone().requires_grad_(True)
-    mf.loss.kl_divergence_batched(ops.project_kde1d(xd, w, geom, 0.5, nb), meas).sum().backward()
+    mf.loss.kl_divergence_batched(ops.project_kde1d(xd, w, geom, 0.5, nb, mp=mp), meas).sum().backward()
     assert float((xc.grad - xd.grad).abs().max()) <= 1e-4 * float(xd.grad.abs().max())
 
 

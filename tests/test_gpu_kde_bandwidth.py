@@ -363,6 +363,12 @@ def test_bandwidth_beyond_the_compiled_windows_is_refused_before_launch():
     diag = mf.diagnostics.Histogram1D(axis=0, edges=edges[0], bandwidth=1.6).to(DEV)
     with pytest.raises(ValueError, match="bandwidth too wide"):
         mf.simulate.forward(x, [mf.simulate.LinearTransform(torch.eye(4, device=DEV))], [[diag]])
+    # the private bins of the 1-D deposit fill shared memory at about 1800 bins: wider screens are refused
+    geom, _, ratio = geom_1d([torch.linspace(-4.0, 4.0, 8193)] * 3, [0.5] * 3)
+    with pytest.raises(RuntimeError, match="not supported"):
+        ops.kde1d_sums(x, w, geom.cuda(), ratio, 8192)
+    with pytest.raises(RuntimeError, match="not supported"):
+        ops.project_kde1d(x.clone().requires_grad_(True), w, geom.cuda(), ratio, 8192)
 
     # 2-D: the tensor-core forward takes any width, the fixed-point deposit and the backward stop at R = 9
     screens = SCREEN_EDGES_2D[:2]

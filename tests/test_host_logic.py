@@ -25,7 +25,7 @@ def test_library_exports_every_declared_symbol_at_the_header_abi_version():
         assert hasattr(lib, name), f"{name} declared in the header but not exported"
     assert declared == set(_lib.SIGNATURES), "ctypes table and header disagree"
     version = int(re.search(r"#define MFB_ABI_VERSION (\d+)", header).group(1))
-    assert lib.mfb_abi_version() == version == _lib.ABI_VERSION == 3
+    assert lib.mfb_abi_version() == version == _lib.ABI_VERSION == 4
     assert b"workspace" in lib.mfb_error_string(-3)
 
 
@@ -252,6 +252,25 @@ def test_ment_entry_points_refuse_bad_arguments(monkeypatch):
     monkeypatch.setattr(_lib, "_lib", None)
     with pytest.raises(_lib.LibraryMissing, match="ABI version"):
         _lib.load()
+
+
+def test_kde1d_forward_refuses_inconsistent_outputs():
+    """Argument checks of mfb_project_kde1d_fwd's two modes (sums only / sums + profiles (+ KL)); dummy device
+    pointers: every call fails before any CUDA call."""
+    import ctypes
+    lib = _lib.load()
+    dummy = ctypes.c_void_p(16)
+
+    def fwd(n=1000, n_total=1000.0, meas=None, profiles=None, kl=None):
+        return lib.mfb_project_kde1d_fwd(dummy, n, 4, dummy, None, dummy, 3, 64, 0.5, n_total, meas, 1e-12, dummy,
+                                         profiles, kl, dummy, 1 << 20, None)
+
+    assert fwd(meas=dummy, profiles=dummy) == -1                 # meas without kl
+    assert fwd(profiles=dummy, kl=dummy) == -1                   # kl without meas
+    assert fwd(meas=dummy, kl=dummy) == -1                       # meas / kl without profiles
+    assert fwd(n=0, profiles=dummy) == -1                        # profiles of no particles
+    assert fwd(n_total=0.0, profiles=dummy) == -1
+    assert fwd(n_total=-1.0, profiles=dummy, meas=dummy, kl=dummy) == -1
 
 
 def test_graphed_loss_chunk_plan():
