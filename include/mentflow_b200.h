@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define MFB_ABI_VERSION 4
+#define MFB_ABI_VERSION 5
 
 #define MFB_E_BADARG (-1)      /* null pointer / non-positive size / unsupported shape   */
 #define MFB_E_UNSUPPORTED (-2) /* combination not compiled (e.g. D > 8, hidden != 64)    */
@@ -160,70 +160,62 @@ int mfb_project_hist2d(const float* x, int64_t n, int d, const float* proj, cons
                        const float* edges_y, int k, int bx, int by, int64_t* counts, void* stream);
 
 /* ---- neural spline flow (zuko 1.3.1 NSF as built by generate/build.py:36-46) ------------
- * One autoregressive layer per call: y = RQS(MaskedMLP(v))(v), logq_out = logq_in - ladj.
- * Replaces generate/flows/zuko.py:24-29 (rsample_and_log_prob / transform.inv) layer by layer.
- * params: packed fp32 block of one layer (layout: mfb_nsf_layer_param_floats / nsf.cu).
- * first_layer != 0: logq_in is ignored and replaced by log N(v; 0, I).
- * logq_in/logq_out may be NULL (sample only).  order_host: HOST array of d ints, the
- * layer's autoregressive order (feature with order 0 has a bias-only spline); may be NULL.*/
+ * One autoregressive layer per call, in each of three directions: forward, inverse and backward.
+ * params: packed fp32 block of one layer (layout: mfb_nsf_layer_param_floats / nsf.cu), pre-masked.
+ * order_host: HOST array of d ints, the layer's autoregressive order (the feature with order 0 has a
+ * bias-only spline).  params and order_host are required in every direction.
+ *
+ * tc_image selects the implementation.  NULL: fp32 CUDA-core kernels, every shape.  Otherwise the
+ * layer's operand image from mfb_nsf_tc_prepare (mfb_nsf_tc_image_bytes bytes, 16-byte aligned) and
+ * the tcgen05 kernels: the conditioner's masked GEMMs run as tcgen05.mma tiles over fp16 (hi, lo)
+ * splits of the fp32 operands with fp32 accumulators in TMEM, the spline is the epilogue.  They are
+ * compiled for hidden_units = 64, hidden_layers = 3, bins = 20, d = 2..6 (mfb_nsf_tc_supported) and
+ * need an order that is a permutation.  With tc_image, another shape returns MFB_E_UNSUPPORTED; an
+ * order that is not a permutation or an unaligned image returns MFB_E_BADARG.
+ *
+ * mfb_nsf_tc_prepare turns the packed parameters of n_layers layers (layer l at
+ * params + l * layer_stride_floats; all-zero masked blocks are skipped) into n_layers operand images
+ * of mfb_nsf_tc_image_bytes bytes each; orders_host = HOST array [n_layers][d].                  */
 int64_t mfb_nsf_layer_param_floats(int d, int hidden_units, int hidden_layers, int bins);
-int mfb_nsf_layer_fwd(const float* v, int64_t n, int d, int hidden_units, int hidden_layers,
-                      int bins, const float* params, const int32_t* order_host, const float* logq_in,
-                      int first_layer, float* y, float* logq_out, void* stream);
-
-/* Tensor-core version of mfb_nsf_layer_fwd (same reference lines): the conditioner's masked GEMMs
- * run as tcgen05.mma tiles over fp16 (hi, lo) splits of the fp32 operands with fp32 accumulators
- * in TMEM, the spline is the epilogue.  Compiled for hidden_units = 64, hidden_layers = 3,
- * bins = 20, d = 2..6 (mfb_nsf_tc_supported); other shapes use mfb_nsf_layer_fwd.
- * mfb_nsf_tc_prepare turns the packed fp32 parameters of n_layers layers (layer l at
- * params + l * layer_stride_floats; they MUST be pre-masked: all-zero blocks are skipped) into
- * n_layers operand images of mfb_nsf_tc_image_bytes bytes each; orders_host = HOST array
- * [n_layers][d].  mfb_nsf_tc_layer_fwd then runs one layer from its image.                  */
 int mfb_nsf_tc_supported(int d, int hidden_units, int hidden_layers, int bins);
 int64_t mfb_nsf_tc_image_bytes(int d, int hidden_layers);
-int64_t mfb_nsf_tc_prepare_workspace_bytes(int n_layers);
 int mfb_nsf_tc_prepare(const float* params, int64_t layer_stride_floats, int n_layers, int d,
                        int hidden_units, int hidden_layers, int bins, const int32_t* orders_host,
-                       void* images, void* workspace, int64_t workspace_bytes, void* stream);
-int mfb_nsf_tc_layer_fwd(const float* v, int64_t n, int d, int hidden_units, int hidden_layers,
-                         int bins, const void* image, const int32_t* order_host,
-                         const float* logq_in, int first_layer, float* y, float* logq_out,
-                         void* stream);
+                       void* images, void* stream);
 
-/* Density direction of one layer: v = A^-1(y) (d conditioner sweeps per particle) and
- * ladj_out = ladj_in + log|det dA/dv|(v).  Replaces generate/flows/zuko.py:21-22,31-32,43-50
- * (log_prob / inverse / inverse_steps).  Call the layers in REVERSE order; with last_layer != 0
- * (the flow's first layer) ladj_out receives log q(x) = log N(v;0,I) - sum ladj instead.
- * ladj_in / ladj_out may be NULL.  order_host is required (HOST array of d ints).          */
-int mfb_nsf_layer_inv(const float* y, int64_t n, int d, int hidden_units, int hidden_layers,
-                      int bins, const float* params, const int32_t* order_host, const float* ladj_in,
-                      int last_layer, float* v, float* ladj_out, void* stream);
-/* The same on the tensor cores, from one layer's operand image of mfb_nsf_tc_prepare (shapes of
- * mfb_nsf_tc_supported): the feature first in the order inverts its bias-only spline, every further
- * feature takes one pass of the conditioner (first layer, two hidden GEMMs, its own output tile) and
- * the inverse spline in registers -- S x 4 GEMM round trips per 128-particle tile instead of D sweeps. */
-int mfb_nsf_tc_layer_inv(const float* y, int64_t n, int d, int hidden_units, int hidden_layers, int bins,
-                         const void* image, const int32_t* order_host, const float* ladj_in, int last_layer,
-                         float* v, float* ladj_out, void* stream);
+/* Forward: y = RQS(MaskedMLP(v))(v), logq_out = logq_in - ladj.  Replaces generate/flows/zuko.py:24-29
+ * (rsample_and_log_prob / transform.inv) layer by layer.  first_layer != 0: logq_in is ignored and
+ * replaced by log N(v; 0, I).  logq_in/logq_out may be NULL (sample only).                       */
+int mfb_nsf_layer_fwd(const float* v, int64_t n, int d, int hidden_units, int hidden_layers, int bins,
+                      const float* params, const void* tc_image, const int32_t* order_host,
+                      const float* logq_in, int first_layer, float* y, float* logq_out, void* stream);
 
-/* Backward of one layer (replaces torch autograd through the zuko graph).  Activations are
- * recomputed from the layer input v.  gy = dL/dy [n][d], glogq = dL/dlogq_out [n] (may be NULL);
- * outputs gv = dL/dv [n][d] and gparams = dL/dparams in the packed forward layout (added to
- * when accumulate != 0).  params_om: the same masked weights in out-major layout
+/* Inverse (density direction): v = A^-1(y) and ladj_out = ladj_in + log|det dA/dv|(v).  Replaces
+ * generate/flows/zuko.py:21-22,31-32,43-50 (log_prob / inverse / inverse_steps).  Call the layers in
+ * REVERSE order; with last_layer != 0 (the flow's first layer) ladj_out receives
+ * log q(x) = log N(v;0,I) - sum ladj instead.  ladj_in / ladj_out may be NULL.  The CUDA-core kernel
+ * makes d conditioner sweeps per particle.  The tcgen05 kernel inverts the bias-only spline of the
+ * feature first in the order, then gives every further feature one pass of the conditioner (first
+ * layer, two hidden GEMMs, its own output tile) and the inverse spline in registers: S x 4 GEMM round
+ * trips per 128-particle tile instead of d sweeps.                                               */
+int mfb_nsf_layer_inv(const float* y, int64_t n, int d, int hidden_units, int hidden_layers, int bins,
+                      const float* params, const void* tc_image, const int32_t* order_host,
+                      const float* ladj_in, int last_layer, float* v, float* ladj_out, void* stream);
+
+/* Backward (replaces torch autograd through the zuko graph).  Activations are recomputed from the
+ * layer input v.  gy = dL/dy [n][d], glogq = dL/dlogq_out [n] (may be NULL); outputs gv = dL/dv
+ * [n][d] and gparams = dL/dparams in the packed forward layout (added to when accumulate != 0).
+ * params_om: the same masked weights in out-major layout
  * W1 [64][d] | Wl [64 out][64 in] x (L-1) | Wout [d*64 (59->64 padded rows)][64 in], no biases
- * (mfb_nsf_layer_param_om_floats floats).  dL/dlogq_in = glogq (pass-through).           */
+ * (mfb_nsf_layer_param_om_floats floats).  dL/dlogq_in = glogq (pass-through).  With tc_image the
+ * layer runs as three tcgen05 kernels (nsf_tc.cu kBwd, nsf_tc_bwd.cu); a training step passes the
+ * images it built for its forward pass.                                                          */
 int64_t mfb_nsf_layer_param_om_floats(int d, int hidden_units, int hidden_layers);
-/* The backward of a layer runs as three tcgen05 kernels for hidden_layers = 3, bins = 20 (nsf_tc.cu kBwd,
- * nsf_tc_bwd.cu) and on CUDA-core kernels otherwise, or when `flags` has MFB_FLAG_NO_TENSOR_CORES.   */
 int64_t mfb_nsf_layer_bwd_workspace_bytes(int64_t n, int d, int hidden_layers);
-/* tc_image: the layer's tcgen05 operand image that mfb_nsf_tc_prepare built for the forward pass of
- * this step (mfb_nsf_tc_image_bytes bytes, 16-byte aligned; NULL = build it here): a training
- * step then builds each image once instead of twice.                                      */
-int mfb_nsf_layer_bwd_img(const float* v, const float* gy, const float* glogq, int64_t n, int d,
-                          int hidden_units, int hidden_layers, int bins, const float* params,
-                          const float* params_om, const int32_t* order_host, int first_layer,
-                          const void* tc_image, float* gv, float* gparams, int accumulate,
-                          void* workspace, int64_t workspace_bytes, int flags, void* stream);
+int mfb_nsf_layer_bwd(const float* v, const float* gy, const float* glogq, int64_t n, int d, int hidden_units,
+                      int hidden_layers, int bins, const float* params, const float* params_om,
+                      const void* tc_image, const int32_t* order_host, int first_layer, float* gv,
+                      float* gparams, int accumulate, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* ---- parameter layouts --------------------------------------------------------------------
  * zuko keeps every MaskedLinear as weight [out][in] + a 0/1 mask applied on each call (zuko/nn.py, reached from

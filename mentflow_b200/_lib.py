@@ -13,7 +13,7 @@ LIB_PATH = os.environ.get("MENTFLOW_B200_LIB") or os.path.join(PKG_DIR, "libment
 
 P = c_void_p  # every device pointer crosses the ABI as a plain address
 
-ABI_VERSION = 4  # MFB_ABI_VERSION of the header SIGNATURES mirrors
+ABI_VERSION = 5  # MFB_ABI_VERSION of the header SIGNATURES mirrors
 
 # name -> (restype, argtypes); mirrors include/mentflow_b200.h line by line
 SIGNATURES = {
@@ -39,18 +39,15 @@ SIGNATURES = {
     "mfb_project_kde2d_bwd": (c_int, [P, c_int64, c_int, P, P, c_int, c_int, c_int, c_float, P, P, c_int, P]),
     "mfb_project_hist2d": (c_int, [P, c_int64, c_int, P, P, P, c_int, c_int, c_int, P, P]),
     "mfb_nsf_layer_param_floats": (c_int64, [c_int, c_int, c_int, c_int]),
-    "mfb_nsf_layer_fwd": (c_int, [P, c_int64, c_int, c_int, c_int, c_int, P, P, P, c_int, P, P, P]),
     "mfb_nsf_tc_supported": (c_int, [c_int, c_int, c_int, c_int]),
     "mfb_nsf_tc_image_bytes": (c_int64, [c_int, c_int]),
-    "mfb_nsf_tc_prepare_workspace_bytes": (c_int64, [c_int]),
-    "mfb_nsf_tc_prepare": (c_int, [P, c_int64, c_int, c_int, c_int, c_int, c_int, P, P, P, c_int64, P]),
-    "mfb_nsf_tc_layer_fwd": (c_int, [P, c_int64, c_int, c_int, c_int, c_int, P, P, P, c_int, P, P, P]),
-    "mfb_nsf_layer_inv": (c_int, [P, c_int64, c_int, c_int, c_int, c_int, P, P, P, c_int, P, P, P]),
-    "mfb_nsf_tc_layer_inv": (c_int, [P, c_int64, c_int, c_int, c_int, c_int, P, P, P, c_int, P, P, P]),
+    "mfb_nsf_tc_prepare": (c_int, [P, c_int64, c_int, c_int, c_int, c_int, c_int, P, P, P]),
+    "mfb_nsf_layer_fwd": (c_int, [P, c_int64, c_int, c_int, c_int, c_int, P, P, P, P, c_int, P, P, P]),
+    "mfb_nsf_layer_inv": (c_int, [P, c_int64, c_int, c_int, c_int, c_int, P, P, P, P, c_int, P, P, P]),
     "mfb_nsf_layer_param_om_floats": (c_int64, [c_int, c_int, c_int]),
     "mfb_nsf_layer_bwd_workspace_bytes": (c_int64, [c_int64, c_int, c_int]),
-    "mfb_nsf_layer_bwd_img": (c_int, [P, P, P, c_int64, c_int, c_int, c_int, c_int, P, P, P, c_int, P, P, P, c_int, P,
-                                      c_int64, c_int, P]),
+    "mfb_nsf_layer_bwd": (c_int, [P, P, P, c_int64, c_int, c_int, c_int, c_int, P, P, P, P, c_int, P, P, c_int, P,
+                                  c_int64, P]),
     "mfb_ment_prob": (c_int, [P, c_int64, c_int, P, P, P, c_int, c_int, P, P, P, P, P, c_int, c_int, c_int, P, c_float,
                               c_float, P, P]),
     "mfb_ment_prob_grid": (c_int, [c_int, P, P, P, P, P, P, c_int, c_int, P, P, P, P, P, c_int, c_int, c_int, P, c_float,

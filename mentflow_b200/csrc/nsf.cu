@@ -11,7 +11,7 @@
 // (pre-masked, transposed) weights resident in shared memory for the lifetime of a persistent
 // CTA, activations of the current layer in registers, outputs of a layer staged through a
 // per-thread column of shared memory (conflict free).  Spline parameters never touch HBM.
-#include "nsf_common.cuh"
+#include "nsf_tc_common.cuh"
 
 namespace mfb {
 
@@ -151,15 +151,17 @@ int64_t mfb_nsf_layer_param_floats(int d, int hidden_units, int hidden_layers, i
 }
 
 int mfb_nsf_layer_fwd(const float* v, int64_t n, int d, int hidden_units, int hidden_layers, int bins,
-                      const float* params, const int32_t* order_host, const float* logq_in, int first_layer,
-                      float* y, float* logq_out, void* stream) {
-  MFB_CHECK_ARG(v && params && y && n >= 0);
+                      const float* params, const void* tc_image, const int32_t* order_host, const float* logq_in,
+                      int first_layer, float* y, float* logq_out, void* stream) {
+  MFB_CHECK_ARG(v && params && order_host && y && n >= 0);
   if (hidden_units != kH || hidden_layers < 1 || bins < 2 || 3 * bins - 1 > kPP) return MFB_E_UNSUPPORTED;
   MFB_CHECK_ARG(first_layer || !logq_out || logq_in);
-  if (n == 0) return 0;
-  FeatureOrder ord;
-  for (int i = 0; i < kMaxDim; ++i) ord.v[i] = (order_host && i < d) ? order_host[i] : 1;
   cudaStream_t st = (cudaStream_t)stream;
+  if (tc_image)
+    return nsf_tc_fwd(v, n, d, hidden_layers, bins, tc_image, order_host, logq_in, first_layer, y, logq_out, st);
+  if (n == 0) return 0;
+  FeatureOrder ord = {};
+  for (int i = 0; i < d && i < kMaxDim; ++i) ord.v[i] = order_host[i];
   switch (d) {
     case 2: return launch_nsf_fwd<2>(v, n, hidden_layers, bins, params, ord, logq_in, first_layer, y, logq_out, st);
     case 3: return launch_nsf_fwd<3>(v, n, hidden_layers, bins, params, ord, logq_in, first_layer, y, logq_out, st);

@@ -19,7 +19,7 @@
 // Gradients land directly in the packed parameter layout of the forward kernel, so the host
 // maps them back to zuko-layout tensors (and applies the masks) by plain autograd through
 // NSFGenerator.packed_parameters().
-#include "nsf_common.cuh"
+#include "nsf_tc_common.cuh"
 
 namespace mfb {
 
@@ -482,12 +482,6 @@ int64_t nsf_tc_dgrad_image_bytes(int d);
 int nsf_tc_dgrad(const float* gphi, const float* gmax, const uint32_t* masks, const float* gvd, int64_t n, int d,
                  int hidden_layers, const float* params, const int32_t* order, float* gz, float* gv, void* image,
                  int* gmaxes, cudaStream_t st);
-// tcgen05 recompute + spline forward/backward (nsf_tc.cu); image: mfb_nsf_tc_image_bytes scratch the operand
-// image is built in, unless ready_image (the image mfb_nsf_tc_prepare built for the forward pass) is given
-int nsf_tc_spline_bwd(const float* v, const float* gy, const float* glogq, int64_t n, int d, int hidden_layers,
-                      int bins, const float* params, const int32_t* order, int first_layer, float* acts,
-                      float* gphi, uint32_t* masks, float* gvd, float* gmax, int* gmaxes, void* image, const void* ready_image,
-                      cudaStream_t st);
 // tcgen05 weight + bias gradients of the whole layer (nsf_tc_bwd.cu)
 int64_t nsf_tc_wgrad_partial_floats(int d);
 int nsf_tc_wgrad(const float* gphi, const float* gz, const float* acts, const float* v, int64_t n, int d,
@@ -517,10 +511,7 @@ static BwdPlan plan_bwd(int64_t n, int d, int hidden_layers) {
   P.gvd = take(n * d);
   P.gmax = take(n);
   P.gmaxes = take(8);
-  {
-    int64_t ib = nsf_tc_dgrad_image_bytes(d), fb = mfb_nsf_tc_image_bytes(d, 3);
-    P.image = take(((ib > fb ? ib : fb) + 3) / 4 + 256);   // operand image scratch (+ slack to align it to 1 KB)
-  }
+  P.image = take((nsf_tc_dgrad_image_bytes(d) + 3) / 4 + 256);   // dgrad operand image (+ slack to align it to 1 KB)
   const int sms = sm_count();
   int nsplit = (4 * sms + d - 1) / d;
   int64_t tiles = (n + kWgTileP - 1) / kWgTileP;
@@ -539,9 +530,8 @@ static BwdPlan plan_bwd(int64_t n, int d, int hidden_layers) {
 
 template <int D>
 static int run_layer_bwd(const float* v, const float* gy, const float* glogq, int64_t n, int hidden_layers, int nb,
-                         const float* params, const float* params_om, const FeatureOrder& order, int first,
-                         float* gv, float* gparams, int accumulate, float* ws, cudaStream_t st,
-                         const void* ready_image = nullptr, int flags = 0) {
+                         const float* params, const float* params_om, const void* tc_image, const int32_t* order_host,
+                         int first, float* gv, float* gparams, int accumulate, float* ws, cudaStream_t st) {
   const BwdPlan P = plan_bwd(n, D, hidden_layers);
   const int64_t np = nsf_param_floats(D, hidden_layers);
   float* acts = ws + P.acts;
@@ -553,43 +543,33 @@ static int run_layer_bwd(const float* v, const float* gy, const float* glogq, in
   const int sms = sm_count();
   int* gmaxes = reinterpret_cast<int*>(ws + P.gmaxes);
   MFB_CUDA(cudaMemsetAsync(gmaxes, 0, 8 * sizeof(int), st));
-  // 1. recompute + spline backward: on the tensor cores where compiled, else the CUDA-core kernel
-  bool tc_spline = false;
-  if (hidden_layers == 3 && !(flags & MFB_FLAG_NO_TENSOR_CORES)) {
-    int32_t ord[kMaxDim];
-    for (int i = 0; i < D; ++i) ord[i] = order.v[i];
+  if (tc_image) {
+    // 1. recompute + spline backward, 1b. data gradients of the whole conditioner (ga[l] = dL/d(pre-activation) of
+    //    hidden layer l, gv = dL/dv), 1c. every weight and bias gradient of the layer: three tensor-core kernels
+    //    that share the tile-major workspace layout
+    uint32_t* masks = reinterpret_cast<uint32_t*>(ws + P.masks);
+    int rc = nsf_tc_spline_bwd(v, gy, glogq, n, D, tc_image, order_host, first, acts, gphi, masks, gvd, ws + P.gmax,
+                               gmaxes, st);
+    if (rc) return rc;
     unsigned char* image = reinterpret_cast<unsigned char*>(((uintptr_t)(ws + P.image) + 1023) & ~(uintptr_t)1023);
-    int rc = nsf_tc_spline_bwd(v, gy, glogq, n, D, hidden_layers, nb, params, ord, first, acts, gphi,
-                               reinterpret_cast<uint32_t*>(ws + P.masks), gvd, ws + P.gmax, gmaxes, image, ready_image, st);
-    if (rc == 0) tc_spline = true;
-    else if (rc != MFB_E_UNSUPPORTED) return rc;
+    rc = nsf_tc_dgrad(gphi, ws + P.gmax, masks, gvd, n, D, hidden_layers, params, order_host, ga, gv, image, gmaxes, st);
+    if (rc) return rc;
+    rc = nsf_tc_wgrad(gphi, ga, acts, v, n, D, hidden_layers, order_host, gmaxes, partial, gparams, accumulate, st);
+    return rc ? rc : launch_status();
   }
-  if (!tc_spline) {
+  // 1. recompute + spline backward on the CUDA cores
+  {
+    FeatureOrder order = {};
+    for (int i = 0; i < D; ++i) order.v[i] = order_host[i];
     const size_t smem = (size_t)((np + 3) & ~(int64_t)3) * 4 + (size_t)kPP * kNsfThreads * 4;
     if (smem > 227 * 1024) return MFB_E_UNSUPPORTED;
     MFB_CUDA(cudaFuncSetAttribute(nsf_bwd_spline_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int64_t tiles = (n + kNsfThreads - 1) / kNsfThreads;
     int grid = (int)(tiles < sms ? tiles : sms);
     nsf_bwd_spline_kernel<D><<<grid, kNsfThreads, smem, st>>>(v, gy, glogq, n, hidden_layers, nb, params, np, order,
-                                                              first, acts, gphi, gvd, ws + P.gmax,
-                                                              reinterpret_cast<int*>(ws + P.gmaxes));
+                                                              first, acts, gphi, gvd, ws + P.gmax, gmaxes);
     int rc = launch_status();
     if (rc) return rc;
-  }
-  // 1b. data gradients of the whole conditioner on the tensor cores (three hidden layers):
-  //     ga[l] = dL/d(pre-activation) of hidden layer l, gv = dL/dv
-  bool tc_chain = false;
-  if (tc_spline) {   // the three tensor-core kernels share the tile-major workspace layout: all or none
-    int32_t ord[kMaxDim];
-    for (int i = 0; i < D; ++i) ord[i] = order.v[i];
-    unsigned char* image = reinterpret_cast<unsigned char*>(((uintptr_t)(ws + P.image) + 1023) & ~(uintptr_t)1023);
-    int rc = nsf_tc_dgrad(gphi, ws + P.gmax, reinterpret_cast<const uint32_t*>(ws + P.masks), gvd, n, D, hidden_layers, params,
-                          ord, ga, gv, image, gmaxes, st);
-    if (rc) return rc;
-    tc_chain = true;
-    // 1c. every weight and bias gradient of the layer in one tensor-core kernel
-    rc = nsf_tc_wgrad(gphi, ga, acts, v, n, D, hidden_layers, ord, gmaxes, partial, gparams, accumulate, st);
-    return rc ? rc : launch_status();
   }
   // packed (forward) layout offsets
   const int64_t off_w1 = 0, off_b1 = (int64_t)D * kH, off_hid = off_b1 + kH;
@@ -608,13 +588,12 @@ static int run_layer_bwd(const float* v, const float* gy, const float* glogq, in
     nsf_wgrad_reduce_kernel<<<(D * kH * kH + 255) / 256, 256, 0, st>>>(partial, P.nsplit, D, (int64_t)kH * kPP,
                                                                         gparams + off_wout, accumulate);
     nsf_rowsum_kernel<<<D * kPP, 256, 0, st>>>(gphi, n, gparams + off_bout, 0, kPP, 0, accumulate);
-    if (!tc_chain)
-      nsf_dgrad_kernel<<<dgrid, kBwdThreads, dsmem, st>>>(gphi, D * kPP, n, params_om + om_wout, h_last, ga);
+    nsf_dgrad_kernel<<<dgrid, kBwdThreads, dsmem, st>>>(gphi, D * kPP, n, params_om + om_wout, h_last, ga);
     int rc = launch_status();
     if (rc) return rc;
   }
   // hidden layers, last to first: gcur holds dL/d(pre-activation) of hidden layer l+1 (index l+1 in acts)
-  float* gcur = tc_chain ? ga + (size_t)(hidden_layers - 1) * kH * n : ga;
+  float* gcur = ga;
   float* gnext = gb;
   for (int l = hidden_layers - 2; l >= 0; --l) {
     const float* h_prev = acts + (size_t)l * kH * n;
@@ -623,10 +602,6 @@ static int run_layer_bwd(const float* v, const float* gy, const float* glogq, in
     nsf_wgrad_kernel<<<grid, 256, 0, st>>>(h_prev, gcur, n, P.per_split, partial);
     nsf_wgrad_reduce_kernel<<<(kH * kH + 255) / 256, 256, 0, st>>>(partial, P.nsplit, 1, 0, gw, accumulate);
     nsf_rowsum_kernel<<<kH, 256, 0, st>>>(gcur, n, gw + kH * kH, 0, kH, 0, accumulate);
-    if (tc_chain) {
-      gcur = ga + (size_t)l * kH * n;   // already computed by the tcgen05 chain
-      continue;
-    }
     nsf_dgrad_kernel<<<dgrid, kBwdThreads, dsmem, st>>>(gcur, kH, n, params_om + om_hid + (int64_t)l * kH * kH,
                                                          h_prev, gnext);
     int rc = launch_status();
@@ -642,7 +617,7 @@ static int run_layer_bwd(const float* v, const float* gy, const float* glogq, in
     nsf_wgrad_in_kernel<D><<<gridw, 256, 0, st>>>(v, gcur, n, per_cta, partial);
     nsf_sum_partials_kernel<<<(D * kH + 255) / 256, 256, 0, st>>>(partial, gridw, D * kH, gparams + off_w1, accumulate);
     nsf_rowsum_kernel<<<kH, 256, 0, st>>>(gcur, n, gparams + off_b1, 0, kH, 0, accumulate);
-    if (!tc_chain) nsf_bwd_input_kernel<D><<<dgrid, 256, 0, st>>>(gvd, gcur, n, params_om + om_w1, gv);
+    nsf_bwd_input_kernel<D><<<dgrid, 256, 0, st>>>(gvd, gcur, n, params_om + om_w1, gv);
   }
   return launch_status();
 }
@@ -663,22 +638,23 @@ int64_t mfb_nsf_layer_param_om_floats(int d, int hidden_units, int hidden_layers
   return (int64_t)kH * d + (int64_t)(hidden_layers - 1) * kH * kH + (int64_t)d * kPP * kH;
 }
 
-int mfb_nsf_layer_bwd_img(const float* v, const float* gy, const float* glogq, int64_t n, int d, int hidden_units,
-                          int hidden_layers, int bins, const float* params, const float* params_om,
-                          const int32_t* order_host, int first_layer, const void* tc_image, float* gv,
-                          float* gparams, int accumulate, void* workspace, int64_t workspace_bytes, int flags,
-                          void* stream) {
-  MFB_CHECK_ARG(v && gy && params && params_om && gv && gparams && workspace && n >= 1);
+int mfb_nsf_layer_bwd(const float* v, const float* gy, const float* glogq, int64_t n, int d, int hidden_units,
+                      int hidden_layers, int bins, const float* params, const float* params_om, const void* tc_image,
+                      const int32_t* order_host, int first_layer, float* gv, float* gparams, int accumulate,
+                      void* workspace, int64_t workspace_bytes, void* stream) {
+  MFB_CHECK_ARG(v && gy && params && params_om && order_host && gv && gparams && workspace && n >= 1);
   if (hidden_units != kH || hidden_layers < 1 || bins < 2 || 3 * bins - 1 > kPP || d < 2 || d > 6)
     return MFB_E_UNSUPPORTED;
+  if (tc_image) {
+    const int rc = nsf_tc_check(d, hidden_layers, bins, tc_image, order_host);
+    if (rc) return rc;
+  }
   if (workspace_bytes < mfb_nsf_layer_bwd_workspace_bytes(n, d, hidden_layers)) return MFB_E_WORKSPACE;
-  FeatureOrder ord;
-  for (int i = 0; i < kMaxDim; ++i) ord.v[i] = (order_host && i < d) ? order_host[i] : 1;
   cudaStream_t st = (cudaStream_t)stream;
   float* ws = (float*)workspace;
-#define MFB_BWD(DD)                                                                                              \
-  return run_layer_bwd<DD>(v, gy, glogq, n, hidden_layers, bins, params, params_om, ord, first_layer, gv, gparams, \
-                           accumulate, ws, st, tc_image, flags)
+#define MFB_BWD(DD)                                                                                                 \
+  return run_layer_bwd<DD>(v, gy, glogq, n, hidden_layers, bins, params, params_om, tc_image, order_host, first_layer, \
+                           gv, gparams, accumulate, ws, st)
   switch (d) {
     case 2: MFB_BWD(2);
     case 3: MFB_BWD(3);

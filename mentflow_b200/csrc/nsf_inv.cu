@@ -8,7 +8,7 @@
 // particle with the weights in shared memory; sweep s only updates the features whose order
 // is >= s (the others are already exact), and the last sweep also yields log dy/dv, so the
 // extra forward pass disappears.
-#include "nsf_common.cuh"
+#include "nsf_tc_common.cuh"
 
 namespace mfb {
 
@@ -191,14 +191,16 @@ static int launch_nsf_inv(const float* y, int64_t n, int hidden_layers, int nb, 
 using namespace mfb;
 
 extern "C" int mfb_nsf_layer_inv(const float* y, int64_t n, int d, int hidden_units, int hidden_layers, int bins,
-                                 const float* params, const int32_t* order_host, const float* ladj_in,
-                                 int last_layer, float* v, float* ladj_out, void* stream) {
-  MFB_CHECK_ARG(y && params && v && n >= 0);
+                                 const float* params, const void* tc_image, const int32_t* order_host,
+                                 const float* ladj_in, int last_layer, float* v, float* ladj_out, void* stream) {
+  MFB_CHECK_ARG(y && params && order_host && v && n >= 0);
   if (hidden_units != kH || hidden_layers < 1 || bins < 2 || 3 * bins - 1 > kPP) return MFB_E_UNSUPPORTED;
-  if (n == 0) return 0;
-  FeatureOrder ord;
-  for (int i = 0; i < kMaxDim; ++i) ord.v[i] = (order_host && i < d) ? order_host[i] : i;
   cudaStream_t st = (cudaStream_t)stream;
+  if (tc_image)
+    return nsf_tc_inv(y, n, d, hidden_layers, bins, tc_image, order_host, ladj_in, last_layer, v, ladj_out, st);
+  if (n == 0) return 0;
+  FeatureOrder ord = {};
+  for (int i = 0; i < d && i < kMaxDim; ++i) ord.v[i] = order_host[i];
   switch (d) {
     case 2: return launch_nsf_inv<2>(y, n, hidden_layers, bins, params, ord, ladj_in, last_layer, v, ladj_out, st);
     case 3: return launch_nsf_inv<3>(y, n, hidden_layers, bins, params, ord, ladj_in, last_layer, v, ladj_out, st);

@@ -1168,32 +1168,55 @@ static int launch_inverse(const float* y, int64_t n, const unsigned char* image,
 
 }  // namespace tc
 
-// First stage of the layer backward on the tensor cores (called from nsf_bwd.cu): builds the operand
-// image of the layer into `image` (mfb_nsf_tc_image_bytes bytes, 1 KB aligned), then recompute + spline
-// forward/backward.  MFB_E_UNSUPPORTED for shapes the tcgen05 kernels are not compiled for.
-int nsf_tc_spline_bwd(const float* v, const float* gy, const float* glogq, int64_t n, int d, int hidden_layers,
-                      int bins, const float* params, const int32_t* order, int first_layer, float* acts,
-                      float* gphi, uint32_t* masks, float* gvd, float* gmax, int* gmaxes, void* image, const void* ready_image,
-                      cudaStream_t st) {
+int nsf_tc_check(int d, int hidden_layers, int bins, const void* image, const int32_t* order) {
   if (!(d >= 2 && d <= 6 && hidden_layers == 3 && bins == 20)) return MFB_E_UNSUPPORTED;
   if (!tc::valid_order(d, order)) return MFB_E_BADARG;
-  tc::PrepArgs args = {};
-  int cls[kH];
-  tc::hidden_classes(d, cls, args.perm);
+  if ((reinterpret_cast<uintptr_t>(image) & 15u) != 0) return MFB_E_BADARG;   // loaded with a bulk copy
+  return 0;
+}
+
+int nsf_tc_fwd(const float* v, int64_t n, int d, int hidden_layers, int bins, const void* image,
+               const int32_t* order, const float* logq_in, int first_layer, float* y, float* logq_out,
+               cudaStream_t st) {
+  const int rc = nsf_tc_check(d, hidden_layers, bins, image, order);
+  if (rc || n == 0) return rc;
   tc::Meta meta;
-  tc::make_meta(d, order, &meta, &args.layer[0]);
-  const unsigned char* img = reinterpret_cast<const unsigned char*>(ready_image);
-  if (img == nullptr) {   // no image from the forward pass: build it in the scratch buffer
-    unsigned char* scratch = reinterpret_cast<unsigned char*>(image);
-    MFB_CUDA(cudaMemsetAsync(scratch, 0, (size_t)tc::image_bytes(d, hidden_layers), st));
-    tc::nsf_tc_prepare_kernel<<<dim3(1, tc::kPrepSlices), 256, 0, st>>>(params, 0, d, hidden_layers, bins, args, 0,
-                                                                        scratch, tc::image_bytes(d, hidden_layers));
-    int rc = launch_status();
-    if (rc) return rc;
-    img = scratch;
-  } else if ((reinterpret_cast<uintptr_t>(img) & 15u) != 0) {
-    return MFB_E_BADARG;    // the image is loaded with a bulk copy: 16-byte aligned
+  tc::make_meta(d, order, &meta, nullptr);
+  const unsigned char* img = reinterpret_cast<const unsigned char*>(image);
+  switch (d) {
+    case 2: return tc::launch_layer<2>(v, n, img, meta, logq_in, first_layer, y, logq_out, st);
+    case 3: return tc::launch_layer<3>(v, n, img, meta, logq_in, first_layer, y, logq_out, st);
+    case 4: return tc::launch_layer<4>(v, n, img, meta, logq_in, first_layer, y, logq_out, st);
+    case 5: return tc::launch_layer<5>(v, n, img, meta, logq_in, first_layer, y, logq_out, st);
+    case 6: return tc::launch_layer<6>(v, n, img, meta, logq_in, first_layer, y, logq_out, st);
+    default: return MFB_E_UNSUPPORTED;
   }
+}
+
+int nsf_tc_inv(const float* y, int64_t n, int d, int hidden_layers, int bins, const void* image,
+               const int32_t* order, const float* ladj_in, int last_layer, float* v, float* ladj_out,
+               cudaStream_t st) {
+  const int rc = nsf_tc_check(d, hidden_layers, bins, image, order);
+  if (rc || n == 0) return rc;
+  tc::Meta meta;
+  tc::make_meta(d, order, &meta, nullptr);
+  const unsigned char* img = reinterpret_cast<const unsigned char*>(image);
+  switch (d) {
+    case 2: return tc::launch_inverse<2>(y, n, img, meta, ladj_in, last_layer, v, ladj_out, st);
+    case 3: return tc::launch_inverse<3>(y, n, img, meta, ladj_in, last_layer, v, ladj_out, st);
+    case 4: return tc::launch_inverse<4>(y, n, img, meta, ladj_in, last_layer, v, ladj_out, st);
+    case 5: return tc::launch_inverse<5>(y, n, img, meta, ladj_in, last_layer, v, ladj_out, st);
+    case 6: return tc::launch_inverse<6>(y, n, img, meta, ladj_in, last_layer, v, ladj_out, st);
+    default: return MFB_E_UNSUPPORTED;
+  }
+}
+
+int nsf_tc_spline_bwd(const float* v, const float* gy, const float* glogq, int64_t n, int d, const void* image,
+                      const int32_t* order, int first_layer, float* acts, float* gphi, uint32_t* masks, float* gvd,
+                      float* gmax, int* gmaxes, cudaStream_t st) {
+  tc::Meta meta;
+  tc::make_meta(d, order, &meta, nullptr);
+  const unsigned char* img = reinterpret_cast<const unsigned char*>(image);
   const tc::BwdIO bio = {gy, glogq, acts, gphi, masks, gvd, gmax, gmaxes};
   switch (d) {
     case 2: return tc::launch_layer_bwd<2>(v, n, img, meta, first_layer, bio, st);
@@ -1226,13 +1249,8 @@ int64_t mfb_nsf_tc_image_bytes(int d, int hidden_layers) {
   return tc::image_bytes(d, hidden_layers);
 }
 
-int64_t mfb_nsf_tc_prepare_workspace_bytes(int n_layers) { (void)n_layers; return 0; }   /* kept for ABI stability */
-
 int mfb_nsf_tc_prepare(const float* params, int64_t layer_stride_floats, int n_layers, int d, int hidden_units,
-                       int hidden_layers, int bins, const int32_t* orders_host, void* images, void* workspace,
-                       int64_t workspace_bytes, void* stream) {
-  (void)workspace;
-  (void)workspace_bytes;
+                       int hidden_layers, int bins, const int32_t* orders_host, void* images, void* stream) {
   MFB_CHECK_ARG(params && orders_host && images && n_layers > 0);
   if (!mfb_nsf_tc_supported(d, hidden_units, hidden_layers, bins)) return MFB_E_UNSUPPORTED;
   cudaStream_t st = (cudaStream_t)stream;
@@ -1255,49 +1273,6 @@ int mfb_nsf_tc_prepare(const float* params, int64_t layer_stride_floats, int n_l
     if (rc) return rc;
   }
   return 0;
-}
-
-int mfb_nsf_tc_layer_fwd(const float* v, int64_t n, int d, int hidden_units, int hidden_layers, int bins,
-                         const void* image, const int32_t* order_host, const float* logq_in, int first_layer,
-                         float* y, float* logq_out, void* stream) {
-  MFB_CHECK_ARG(v && image && y && order_host && n >= 0);
-  if (!mfb_nsf_tc_supported(d, hidden_units, hidden_layers, bins)) return MFB_E_UNSUPPORTED;
-  MFB_CHECK_ARG(first_layer || !logq_out || logq_in);
-  if (!tc::valid_order(d, order_host)) return MFB_E_BADARG;
-  if (n == 0) return 0;
-  tc::Meta meta;
-  tc::make_meta(d, order_host, &meta, nullptr);
-  cudaStream_t st = (cudaStream_t)stream;
-  const unsigned char* img = reinterpret_cast<const unsigned char*>(image);
-  switch (d) {
-    case 2: return tc::launch_layer<2>(v, n, img, meta, logq_in, first_layer, y, logq_out, st);
-    case 3: return tc::launch_layer<3>(v, n, img, meta, logq_in, first_layer, y, logq_out, st);
-    case 4: return tc::launch_layer<4>(v, n, img, meta, logq_in, first_layer, y, logq_out, st);
-    case 5: return tc::launch_layer<5>(v, n, img, meta, logq_in, first_layer, y, logq_out, st);
-    case 6: return tc::launch_layer<6>(v, n, img, meta, logq_in, first_layer, y, logq_out, st);
-    default: return MFB_E_UNSUPPORTED;
-  }
-}
-
-int mfb_nsf_tc_layer_inv(const float* y, int64_t n, int d, int hidden_units, int hidden_layers, int bins,
-                         const void* image, const int32_t* order_host, const float* ladj_in, int last_layer, float* v,
-                         float* ladj_out, void* stream) {
-  MFB_CHECK_ARG(y && image && v && order_host && n >= 0);
-  if (!mfb_nsf_tc_supported(d, hidden_units, hidden_layers, bins)) return MFB_E_UNSUPPORTED;
-  if (!tc::valid_order(d, order_host)) return MFB_E_BADARG;
-  if (n == 0) return 0;
-  tc::Meta meta;
-  tc::make_meta(d, order_host, &meta, nullptr);
-  cudaStream_t st = (cudaStream_t)stream;
-  const unsigned char* img = reinterpret_cast<const unsigned char*>(image);
-  switch (d) {
-    case 2: return tc::launch_inverse<2>(y, n, img, meta, ladj_in, last_layer, v, ladj_out, st);
-    case 3: return tc::launch_inverse<3>(y, n, img, meta, ladj_in, last_layer, v, ladj_out, st);
-    case 4: return tc::launch_inverse<4>(y, n, img, meta, ladj_in, last_layer, v, ladj_out, st);
-    case 5: return tc::launch_inverse<5>(y, n, img, meta, ladj_in, last_layer, v, ladj_out, st);
-    case 6: return tc::launch_inverse<6>(y, n, img, meta, ladj_in, last_layer, v, ladj_out, st);
-    default: return MFB_E_UNSUPPORTED;
-  }
 }
 
 }  // extern "C"

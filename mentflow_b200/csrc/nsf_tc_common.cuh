@@ -198,4 +198,23 @@ static void hidden_classes(int d, int* cls, int* perm) {
 }
 
 }  // namespace tc
+
+// The tcgen05 layer kernels of nsf_tc.cu, run from one layer's operand image (mfb_nsf_tc_prepare); the C entry points
+// of nsf.cu, nsf_inv.cu and nsf_bwd.cu call them when they are given an image.  order: HOST array of d ints.
+// nsf_tc_check: MFB_E_UNSUPPORTED for a shape the kernels are not compiled for (mfb_nsf_tc_supported), MFB_E_BADARG
+// for an order that is not a permutation or an image that is not 16-byte aligned (it is loaded with a bulk copy).
+int nsf_tc_check(int d, int hidden_layers, int bins, const void* image, const int32_t* order);
+// the layer forward and inverse; each runs nsf_tc_check first
+int nsf_tc_fwd(const float* v, int64_t n, int d, int hidden_layers, int bins, const void* image,
+               const int32_t* order, const float* logq_in, int first_layer, float* y, float* logq_out,
+               cudaStream_t st);
+int nsf_tc_inv(const float* y, int64_t n, int d, int hidden_layers, int bins, const void* image,
+               const int32_t* order, const float* ladj_in, int last_layer, float* v, float* ladj_out,
+               cudaStream_t st);
+// first stage of the layer backward: recompute + spline forward/backward into the tile-major workspace matrices of
+// nsf_bwd.cu.  The caller has run nsf_tc_check.
+int nsf_tc_spline_bwd(const float* v, const float* gy, const float* glogq, int64_t n, int d, const void* image,
+                      const int32_t* order, int first_layer, float* acts, float* gphi, uint32_t* masks, float* gvd,
+                      float* gmax, int* gmaxes, cudaStream_t st);
+
 }  // namespace mfb

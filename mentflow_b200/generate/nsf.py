@@ -230,9 +230,8 @@ class NSFGenerator(GenerativeModel):
         if self._pack_key != key:
             with torch.no_grad():
                 packed = self.packed_parameters()
-                images = None
-                if ops.nsf_tc_supported(self.features, self.hidden_units, self.hidden_layers, self.bins, self._orders):
-                    images = ops.nsf_tc_images(packed, self._orders, self.hidden_units, self.hidden_layers, self.bins)
+                images = ops.nsf_direction_images(ops.NSF_USE_TENSOR_CORES, packed, self._orders, self.hidden_units,
+                                                  self.hidden_layers, self.bins)
             self._pack_key, self._pack_cache = key, (packed, images)
         return self._pack_cache
 

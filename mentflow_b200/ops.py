@@ -422,9 +422,20 @@ def nsf_tc_images(packed, orders, hidden_units, hidden_layers, bins):
     order_arr = (ctypes.c_int32 * (t_layers * d))(*[int(o) for order in orders for o in order])
     with torch.cuda.device(packed.device):
         _lib.check(lib.mfb_nsf_tc_prepare(_ptr(packed), packed.stride(0), t_layers, d, hidden_units, hidden_layers,
-                                          bins, ctypes.cast(order_arr, ctypes.c_void_p), _ptr(images), None, 0,
-                                          _stream()), "nsf_tc_prepare")
+                                          bins, ctypes.cast(order_arr, ctypes.c_void_p), _ptr(images), _stream()),
+                   "nsf_tc_prepare")
     return images
+
+
+def nsf_direction_images(use, packed, orders, hidden_units, hidden_layers, bins, images=None):
+    """The operand images one direction of the flow runs its layers from, or None for the fp32 CUDA-core kernels.
+    None unless ``use`` (the direction's switch) is set and the tcgen05 kernels are compiled for this shape and
+    these orders; then ``images`` when the caller has them for these weights, else built here."""
+    d = len(orders[0])
+    if not (use and orders_autoregressive(orders) and _lib.load().mfb_nsf_tc_supported(d, hidden_units, hidden_layers,
+                                                                                        bins)):
+        return None
+    return images if images is not None else nsf_tc_images(packed, orders, hidden_units, hidden_layers, bins)
 
 
 def nsf_layer_forward(v, params, order, hidden_units, hidden_layers, bins, logq_in, first_layer,
@@ -433,6 +444,7 @@ def nsf_layer_forward(v, params, order, hidden_units, hidden_layers, bins, logq_
     ``nsf_tc_images``) the tensor-core kernel runs, otherwise the fp32 CUDA-core kernel."""
     lib = _lib.load()
     v = _check_f32("v", v)
+    params = _check_f32("params", params)
     n, d = v.shape
     y = torch.empty_like(v)
     logq_out = torch.empty(n, dtype=torch.float32, device=v.device) if want_logq else None
@@ -440,28 +452,16 @@ def nsf_layer_forward(v, params, order, hidden_units, hidden_layers, bins, logq_
         return y, logq_out
     order_arr = (ctypes.c_int32 * d)(*[int(o) for o in order])
     with torch.cuda.device(v.device):
-        if image is not None:
-            _lib.check(lib.mfb_nsf_tc_layer_fwd(_ptr(v), n, d, hidden_units, hidden_layers, bins, _ptr(image),
-                                                ctypes.cast(order_arr, ctypes.c_void_p), _ptr(logq_in),
-                                                1 if first_layer else 0, _ptr(y), _ptr(logq_out), _stream()),
-                       "nsf_tc_layer_fwd")
-        else:
-            params = _check_f32("params", params)
-            _lib.check(lib.mfb_nsf_layer_fwd(_ptr(v), n, d, hidden_units, hidden_layers, bins, _ptr(params),
-                                             ctypes.cast(order_arr, ctypes.c_void_p), _ptr(logq_in),
-                                             1 if first_layer else 0, _ptr(y), _ptr(logq_out), _stream()),
-                       "nsf_layer_fwd")
+        _lib.check(lib.mfb_nsf_layer_fwd(_ptr(v), n, d, hidden_units, hidden_layers, bins, _ptr(params), _ptr(image),
+                                         ctypes.cast(order_arr, ctypes.c_void_p), _ptr(logq_in),
+                                         1 if first_layer else 0, _ptr(y), _ptr(logq_out), _stream()),
+                   "nsf_layer_fwd")
     return y, logq_out
 
 
-def _nsf_run_layers(z, packed, orders, hidden_units, hidden_layers, bins, want_logq, images=None):
-    """All layers in sampling order; returns ([z, y_1, ..., x], log q).  ``images``: operand images
-    of the tensor-core kernel when the caller has them cached for these weights."""
-    d = z.shape[1]
-    if not nsf_tc_supported(d, hidden_units, hidden_layers, bins, orders):
-        images = None
-    elif images is None:
-        images = nsf_tc_images(packed, orders, hidden_units, hidden_layers, bins)
+def _nsf_run_layers(z, packed, orders, hidden_units, hidden_layers, bins, want_logq, images):
+    """All layers in sampling order; returns ([z, y_1, ..., x], log q).  ``images``: the forward's
+    operand images (``nsf_direction_images``), None for the CUDA-core kernel."""
     steps, logq = [z], None
     for t, order in enumerate(orders):
         y, logq = nsf_layer_forward(steps[-1], packed[t], order, hidden_units, hidden_layers, bins, logq,
@@ -776,8 +776,6 @@ class NSFForward(torch.autograd.Function):
         orders, hidden_units, hidden_layers, bins, want_logq, images = meta
         z = _check_f32("z", z)
         packed = _check_f32("packed", packed)
-        if images is None and NSF_USE_TENSOR_CORES and nsf_tc_supported(z.shape[1], hidden_units, hidden_layers, bins, orders):
-            images = nsf_tc_images(packed, orders, hidden_units, hidden_layers, bins)
         steps, logq = _nsf_run_layers(z, packed, orders, hidden_units, hidden_layers, bins, want_logq, images)
         ctx.meta = meta
         ctx.images = images        # the backward kernels read the same operand images (~1 MB, not rebuilt)
@@ -812,7 +810,7 @@ def nsf_backward(inputs, packed, packed_om, orders, hidden_units, hidden_layers,
     gz = torch.empty_like(inputs[0])
     if n == 0:
         return gz, gpacked
-    bwd_flags = 0 if (NSF_BWD_USE_TENSOR_CORES and orders_autoregressive(orders)) else FLAG_NO_TENSOR_CORES
+    images = nsf_direction_images(NSF_BWD_USE_TENSOR_CORES, packed, orders, hidden_units, hidden_layers, bins, images)
     chunk = min(n, NSF_BWD_CHUNK)
     with torch.cuda.device(dev):
         wbytes = lib.mfb_nsf_layer_bwd_workspace_bytes(chunk, d, hidden_layers)
@@ -824,13 +822,12 @@ def nsf_backward(inputs, packed, packed_om, orders, hidden_units, hidden_layers,
             for t in range(len(orders) - 1, -1, -1):
                 order_arr = (ctypes.c_int32 * d)(*[int(o) for o in orders[t]])
                 out = gz[start:start + m] if t == 0 else torch.empty((m, d), dtype=torch.float32, device=dev)
-                _lib.check(lib.mfb_nsf_layer_bwd_img(_ptr(inputs[t][start:start + m]), _ptr(g), _ptr(gl), m, d,
-                                                     hidden_units, hidden_layers, bins, _ptr(packed[t]),
-                                                     _ptr(packed_om[t]), ctypes.cast(order_arr, ctypes.c_void_p),
-                                                     1 if t == 0 else 0, _ptr(images[t]) if images is not None else None,
-                                                     _ptr(out), _ptr(gpacked[t]), 1 if start > 0 else 0, _ptr(work),
-                                                     wbytes, bwd_flags,
-                                                     _stream()), "nsf_layer_bwd")
+                _lib.check(lib.mfb_nsf_layer_bwd(_ptr(inputs[t][start:start + m]), _ptr(g), _ptr(gl), m, d,
+                                                 hidden_units, hidden_layers, bins, _ptr(packed[t]), _ptr(packed_om[t]),
+                                                 None if images is None else _ptr(images[t]),
+                                                 ctypes.cast(order_arr, ctypes.c_void_p), 1 if t == 0 else 0,
+                                                 _ptr(out), _ptr(gpacked[t]), 1 if start > 0 else 0, _ptr(work),
+                                                 wbytes, _stream()), "nsf_layer_bwd")
                 g = out
     return gz, gpacked
 
@@ -838,6 +835,8 @@ def nsf_backward(inputs, packed, packed_om, orders, hidden_units, hidden_layers,
 def nsf_forward(z, packed, packed_om, orders, hidden_units, hidden_layers, bins, want_logq=True, want_steps=False,
                 images=None):
     """Returns (x, logq or None, steps or None)."""
+    images = nsf_direction_images(NSF_USE_TENSOR_CORES, packed.detach(), orders, hidden_units, hidden_layers, bins,
+                                  images)
     if want_steps or not (torch.is_grad_enabled() and (z.requires_grad or packed.requires_grad)):
         # nothing to differentiate: skip the autograd.Function bookkeeping
         z = _check_f32("z", z.detach())
@@ -861,6 +860,9 @@ def nsf_inverse(x, packed, orders, hidden_units, hidden_layers, bins, want_logq=
     x = _check_f32("x", x.detach())
     packed = _check_f32("packed", packed.detach())
     n, d = x.shape
+    if images is not None:     # the inverse runs from the forward's images only: it builds none of its own
+        images = nsf_direction_images(NSF_INV_USE_TENSOR_CORES, packed, orders, hidden_units, hidden_layers, bins,
+                                      images)
     steps = [x]
     acc = None
     with torch.cuda.device(x.device):
@@ -872,14 +874,10 @@ def nsf_inverse(x, packed, orders, hidden_units, hidden_layers, bins, want_logq=
                 acc = out
                 steps.append(v)
                 continue
-            if images is not None and NSF_INV_USE_TENSOR_CORES:
-                _lib.check(lib.mfb_nsf_tc_layer_inv(_ptr(steps[-1]), n, d, hidden_units, hidden_layers, bins,
-                                                    _ptr(images[t]), ctypes.cast(order_arr, ctypes.c_void_p), _ptr(acc),
-                                                    1 if t == 0 else 0, _ptr(v), _ptr(out), _stream()), "nsf_tc_layer_inv")
-            else:
-                _lib.check(lib.mfb_nsf_layer_inv(_ptr(steps[-1]), n, d, hidden_units, hidden_layers, bins, _ptr(packed[t]),
-                                                 ctypes.cast(order_arr, ctypes.c_void_p), _ptr(acc), 1 if t == 0 else 0,
-                                                 _ptr(v), _ptr(out), _stream()), "nsf_layer_inv")
+            _lib.check(lib.mfb_nsf_layer_inv(_ptr(steps[-1]), n, d, hidden_units, hidden_layers, bins, _ptr(packed[t]),
+                                             None if images is None else _ptr(images[t]),
+                                             ctypes.cast(order_arr, ctypes.c_void_p), _ptr(acc), 1 if t == 0 else 0,
+                                             _ptr(v), _ptr(out), _stream()), "nsf_layer_inv")
             acc = out
             steps.append(v)
     return steps[-1], acc, (steps if want_steps else None)

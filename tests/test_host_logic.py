@@ -25,7 +25,7 @@ def test_library_exports_every_declared_symbol_at_the_header_abi_version():
         assert hasattr(lib, name), f"{name} declared in the header but not exported"
     assert declared == set(_lib.SIGNATURES), "ctypes table and header disagree"
     version = int(re.search(r"#define MFB_ABI_VERSION (\d+)", header).group(1))
-    assert lib.mfb_abi_version() == version == _lib.ABI_VERSION == 4
+    assert lib.mfb_abi_version() == version == _lib.ABI_VERSION == 5
     assert b"workspace" in lib.mfb_error_string(-3)
 
 
@@ -193,8 +193,9 @@ def test_kl_matches_torch_kl_div():
 
 
 def test_tensor_core_flow_host_side_contract():
-    """Host-only parts of the tcgen05 flow entry points (no kernel is launched): which shapes are
-    compiled, the operand-image size, argument checking."""
+    """Host-only parts of the flow entry points (dummy device pointers: every call fails before any CUDA call): which
+    shapes the tcgen05 kernels are compiled for, the operand-image size, and the argument checks of the forward,
+    inverse and backward when they are given an operand image."""
     import ctypes
     from mentflow_b200 import _lib
     lib = _lib.load()
@@ -206,13 +207,30 @@ def test_tensor_core_flow_host_side_contract():
     # image + three 32 KB activation buffers + particle staging + barriers must fit one SM (227 KB)
     assert sizes[-1] + 3 * 32768 + 3 * 2 * 128 * 6 * 4 + 256 + 1024 <= 227 * 1024
     assert lib.mfb_nsf_tc_image_bytes(7, 3) == 0
-    bad_order = (ctypes.c_int32 * 6)(0, 1, 2, 3, 4, 4)          # not a permutation
+    good_order = ctypes.cast((ctypes.c_int32 * 6)(5, 4, 3, 2, 1, 0), ctypes.c_void_p)
+    bad_order = ctypes.cast((ctypes.c_int32 * 6)(0, 1, 2, 3, 4, 4), ctypes.c_void_p)      # not a permutation
     dummy = ctypes.c_void_p(16)
-    rc = lib.mfb_nsf_tc_prepare(dummy, 1, 1, 6, 64, 3, 20, ctypes.cast(bad_order, ctypes.c_void_p), dummy, None, 0, None)
-    assert rc == -1 and b"bad argument" in lib.mfb_error_string(rc)
-    rc = lib.mfb_nsf_tc_layer_fwd(dummy, 10, 6, 64, 2, 20, dummy, ctypes.cast(bad_order, ctypes.c_void_p), None, 1,
-                                  dummy, None, None)
-    assert rc == -2                                             # hidden_layers = 2 is not compiled for tcgen05
+    assert lib.mfb_nsf_tc_prepare(dummy, 1, 1, 6, 64, 3, 20, bad_order, dummy, None) == -1
+    assert b"bad argument" in lib.mfb_error_string(-1)
+
+    def fwd(hidden_layers, image, order):
+        return lib.mfb_nsf_layer_fwd(dummy, 10, 6, 64, hidden_layers, 20, dummy, image, order, None, 1, dummy, None,
+                                     None)
+
+    def inv(hidden_layers, image, order):
+        return lib.mfb_nsf_layer_inv(dummy, 10, 6, 64, hidden_layers, 20, dummy, image, order, None, 1, dummy, None,
+                                     None)
+
+    def bwd(hidden_layers, image, order):
+        return lib.mfb_nsf_layer_bwd(dummy, dummy, None, 10, 6, 64, hidden_layers, 20, dummy, dummy, image, order, 1,
+                                     dummy, dummy, 0, dummy, 0, None)
+
+    for call in (fwd, inv, bwd):
+        assert call(2, dummy, good_order) == -2              # hidden_layers = 2 is not compiled for tcgen05
+        assert call(3, dummy, bad_order) == -1               # the tcgen05 kernels need a permutation
+        assert call(3, ctypes.c_void_p(24), good_order) == -1    # the image is loaded with a bulk copy: 16-byte aligned
+        assert call(3, None, None) == -1                     # the order is required, with or without an image
+        assert call(3, dummy, None) == -1
 
 
 def test_ment_entry_points_refuse_bad_arguments(monkeypatch):
