@@ -289,6 +289,26 @@ int mfb_swd_wpp(const float* x, int64_t n, int d, const float* theta, int nproj,
 int mfb_swd_bwd(const float* grad_coef, int64_t n, int d, const float* theta, int nproj, const double* gwpp,
                 float* gx, void* stream);
 
+/* ---- tanh-MLP generator (generate/nn.py NNGenerator) -------------------------------------------------------------
+ * x[n][dout] = W_out t_L + b_out, t_l = tanh(W_l t_{l-1} + b_l), t_0 = z[n][din]; hidden_layers = L tanh layers of
+ * hidden_units.  Weights in nn.Linear layout: w_in[H][din], b_in[H], w_hid[L-1][H][H], b_hid[L-1][H] (both may be NULL
+ * when L = 1), w_out[dout][H], b_out[dout].  fp32 on the CUDA cores, accurate tanh.  Compiled for 1 <= din, dout <= 8,
+ * H = 64, 1 <= L <= 8 (mfb_nn_supported); another shape returns MFB_E_UNSUPPORTED, a NULL required pointer or n < 1
+ * MFB_E_BADARG, both before any launch.                                                                             */
+int mfb_nn_supported(int din, int dout, int hidden_units, int hidden_layers);
+int mfb_nn_fwd(const float* z, int64_t n, int din, int dout, int hidden_units, int hidden_layers, const float* w_in,
+               const float* b_in, const float* w_hid, const float* b_hid, const float* w_out, const float* b_out,
+               float* x, void* stream);
+/* Backward from z and gx = dL/dx: the forward is recomputed on chip.  gz[n][din] = dL/dz (may be NULL); the six
+ * parameter gradients are written (not accumulated) in the weights' layouts.  Per-CTA partials in the workspace are
+ * added in CTA order: no floating-point atomics, repeated calls are bitwise equal.  0 from the size query: shape not
+ * supported.                                                                                                        */
+int64_t mfb_nn_bwd_workspace_bytes(int64_t n, int din, int dout, int hidden_units, int hidden_layers);
+int mfb_nn_bwd(const float* z, const float* gx, int64_t n, int din, int dout, int hidden_units, int hidden_layers,
+               const float* w_in, const float* b_in, const float* w_hid, const float* b_hid, const float* w_out,
+               const float* b_out, float* gz, float* gw_in, float* gb_in, float* gw_hid, float* gb_hid, float* gw_out,
+               float* gb_out, void* workspace, int64_t workspace_bytes, void* stream);
+
 /* ---- classical MENT (ment.py, sample.py) --------------------------------------------------
  * rho(x) = exp(log prior(x)) * prod clamp(h(u(x)), 0, 1e10) over two families of Lagrange tables, evaluated in
  * double like scipy's RegularGridInterpolator and 0 outside the box of the bin centres (ment.py:36-52, 227-249);

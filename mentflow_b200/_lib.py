@@ -80,6 +80,11 @@ SIGNATURES = {
     "mfb_swd_sort": (c_int, [P, c_int64, c_int, P, c_int, P, P, P, c_int64, P]),
     "mfb_swd_wpp": (c_int, [P, c_int64, c_int, P, c_int, P, c_int64, c_double, P, P, P, c_int64, P]),
     "mfb_swd_bwd": (c_int, [P, c_int64, c_int, P, c_int, P, P, P]),
+    "mfb_nn_supported": (c_int, [c_int, c_int, c_int, c_int]),
+    "mfb_nn_fwd": (c_int, [P, c_int64, c_int, c_int, c_int, c_int, P, P, P, P, P, P, P, P]),
+    "mfb_nn_bwd_workspace_bytes": (c_int64, [c_int64, c_int, c_int, c_int, c_int]),
+    "mfb_nn_bwd": (c_int, [P, P, c_int64, c_int, c_int, c_int, c_int, P, P, P, P, P, P, P, P, P, P, P, P, P, P,
+                           c_int64, P]),
 }
 
 _lib = None

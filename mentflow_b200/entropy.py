@@ -71,6 +71,10 @@ class MonteCarloEntropyEstimator(EntropyEstimator):
     """H = mean(log q) - mean(log prior(x))  (entropy.py:53-62)."""
 
     def forward(self, x: torch.Tensor, log_prob: torch.Tensor) -> torch.Tensor:
+        if log_prob is None:
+            raise ValueError("MonteCarloEntropyEstimator needs the generator's log-density, and this generator has "
+                             "none (log_prob is None): use CovarianceEntropyEstimator, KNNEntropyEstimator or "
+                             "EmptyEntropyEstimator, which work from the particles alone")
         if self.prior is None:
             return _MCEntropy.apply(x, log_prob, 0.0, 0.0, self.reducer)
         if isinstance(self.prior, Gaussian):
@@ -84,7 +88,8 @@ class MonteCarloEntropyEstimator(EntropyEstimator):
         """Compute the local sums and leave them on the reducer; None if this configuration cannot defer
         (no reducer, unequal shards, a prior evaluated by foreign code)."""
         red = self.reducer
-        if (red is None or not hasattr(red, "stash") or red.world_size == 1 or red.global_count(x.shape[0]) is None
+        if (log_prob is None or red is None or not hasattr(red, "stash") or red.world_size == 1
+                or red.global_count(x.shape[0]) is None
                 or not (self.prior is None or isinstance(self.prior, Gaussian))):
             return None
         m = ops.moments(x.detach(), log_prob.detach(), with_cov=False)
@@ -131,7 +136,8 @@ class _CovEntropy(torch.autograd.Function):
     def backward(ctx, g):
         x, mean, cov, eps = ctx.saved_tensors
         scale = -(eps / (eps + ctx.pad)) / (ctx.n - 1.0) * g.double()
-        a = (torch.linalg.inv(cov) * scale).to(torch.float32)          # symmetric D x D
+        # inv_ex: the same inverse without the error check's host sync, so a CUDA graph can capture the backward
+        a = (torch.linalg.inv_ex(cov)[0] * scale).to(torch.float32)    # symmetric D x D
         gx = torch.addmm(-(mean.to(torch.float32) @ a)[None, :], x, a)  # (x - mean) @ a
         return gx, None, None, None
 

@@ -2,6 +2,7 @@
 import torch
 
 from .base import GenerativeModel
+from .nn import NNGenerator
 from .nsf import NSFGenerator
 
 
@@ -19,9 +20,19 @@ def build_flow(name: str, input_features: int, output_features: int, hidden_laye
                         transforms=transforms, bins=bins, device=device, passes=passes)
 
 
+def build_nn(input_features: int, output_features: int, hidden_layers: int, hidden_units: int, transforms=None,
+             dropout: float = 0.0, activation: str = "tanh", device=None, **kws) -> NNGenerator:
+    """The reference's common generator options (``transforms`` is a flow option and is ignored) plus the network's
+    ``dropout`` and ``activation``."""
+    if kws:
+        raise TypeError(f"unsupported NN generator options: {sorted(kws)}")
+    return NNGenerator(input_features, output_features, hidden_layers=hidden_layers, hidden_units=hidden_units,
+                       dropout=dropout, activation=activation, device=device)
+
+
 def build_generator(name: str, device: torch.device = None, **kws) -> GenerativeModel:
     if name == "nn":
-        raise NotImplementedError("the plain NN generator has no density and is outside the accelerated path")
+        return build_nn(device=device, **kws)
     if name in ("bpf", "ffjord", "gf", "gmm", "maf", "nag", "nsf", "sospf", "unaf"):
         return build_flow(name=name, device=device, **kws)
     raise ValueError(f"Invalid generative model name '{name}'")

@@ -40,7 +40,8 @@ class GraphedLoss:
         # particles one launch of the flow kernel processes per pass over the SMs (one 128-row tile
         # per compute warpgroup, three per SM): pieces of whole waves leave no ragged tail per piece
         self._wave = max(1, _lib.load().mfb_sm_count()) * 3 * 128
-        self.z = torch.empty((self.batch_size, gen.features), dtype=torch.float32, device=dev)
+        zdim = getattr(gen, "input_features", None) or gen.features   # the NN generator's noise is not x-sized
+        self.z = torch.empty((self.batch_size, zdim), dtype=torch.float32, device=dev)
         self.graph: Optional[torch.cuda.CUDAGraph] = None
         self._key = None
         self._held = None
@@ -146,7 +147,10 @@ class GraphedLoss:
             xs.append(x_c)
             lqs.append(lq_c)
         cur.wait_stream(cp)
-        x, logq = (xs[0], lqs[0]) if len(xs) == 1 else (torch.cat(xs), torch.cat(lqs))
+        if len(xs) == 1:
+            x, logq = xs[0], lqs[0]
+        else:   # a generator without a density returns log q = None
+            x, logq = torch.cat(xs), (None if lqs[0] is None else torch.cat(lqs))
         return self.model.loss_from_particles(x, logq)
 
     def _capture_host(self, z_host) -> None:

@@ -722,6 +722,59 @@ def swd_wpp(x: torch.Tensor, theta: torch.Tensor, y_sorted: torch.Tensor, p: flo
 # --------------------------------------------------------------------------------------
 # zuko-layout parameters <-> packed blocks
 # --------------------------------------------------------------------------------------
+# --------------------------------------------------------------------------------------
+# tanh-MLP generator (generate/nn.py): fused forward, recomputing backward
+# --------------------------------------------------------------------------------------
+def nn_supported(din: int, dout: int, hidden_units: int, hidden_layers: int) -> bool:
+    return bool(_lib.load().mfb_nn_supported(int(din), int(dout), int(hidden_units), int(hidden_layers)))
+
+
+class NNForward(torch.autograd.Function):
+    """x = MLP(z) from the six stacked parameter tensors; one library call each way."""
+
+    @staticmethod
+    def forward(ctx, z, w_in, b_in, w_hid, b_hid, w_out, b_out):
+        lib = _lib.load()
+        z = _check_f32("z", z.detach())
+        params = [_check_f32(name, t.detach()) for name, t in
+                  zip(("w_in", "b_in", "w_hid", "b_hid", "w_out", "b_out"), (w_in, b_in, w_hid, b_hid, w_out, b_out))]
+        n, din = z.shape
+        hidden, dout, layers = w_in.shape[0], w_out.shape[0], w_hid.shape[0] + 1
+        x = torch.empty((n, dout), dtype=torch.float32, device=z.device)
+        if n > 0:
+            with torch.cuda.device(z.device):
+                _lib.check(lib.mfb_nn_fwd(_ptr(z), n, din, dout, hidden, layers, *[_ptr(t) for t in params], _ptr(x),
+                                          _stream()), "nn_fwd")
+        ctx.save_for_backward(z, *params)
+        ctx.dims = (din, dout, hidden, layers)
+        return x
+
+    @staticmethod
+    def backward(ctx, gx):
+        z, *params = ctx.saved_tensors
+        din, dout, hidden, layers = ctx.dims
+        n = z.shape[0]
+        grads = [torch.zeros_like(t) for t in params]
+        gz = torch.zeros_like(z) if ctx.needs_input_grad[0] else None
+        if n > 0:
+            gx = _check_f32("grad_x", gx)
+            lib = _lib.load()
+            with torch.cuda.device(z.device):
+                wbytes = lib.mfb_nn_bwd_workspace_bytes(n, din, dout, hidden, layers)
+                work = torch.empty(max(wbytes, 16), dtype=torch.uint8, device=z.device)
+                _lib.check(lib.mfb_nn_bwd(_ptr(z), _ptr(gx), n, din, dout, hidden, layers, *[_ptr(t) for t in params],
+                                          _ptr(gz), *[_ptr(g) for g in grads], _ptr(work), wbytes, _stream()), "nn_bwd")
+        return (gz, *[g if need else None for g, need in zip(grads, ctx.needs_input_grad[1:])])
+
+
+def nn_forward(z, w_in, b_in, w_hid, b_hid, w_out, b_out) -> torch.Tensor:
+    """(N, Dout) particles of the tanh MLP for (N, Din) base noise z; differentiable w.r.t. z and the parameters."""
+    if not isinstance(z, torch.Tensor) or z.dim() != 2 or z.shape[1] != w_in.shape[1]:
+        raise ValueError(f"nn_forward: z must be a (N, {w_in.shape[1]}) tensor")
+    _check_f32("z", z)
+    return NNForward.apply(z, w_in, b_in, w_hid, b_hid, w_out, b_out)
+
+
 class PackParameters(torch.autograd.Function):
     """(packed (T, floats_per_layer), packed_om (T, om_floats)) from the zuko-layout tensors of the whole flow in one
     launch; backward = one launch the other way (masked entries get exactly zero gradient).  ``packed_om`` is the
