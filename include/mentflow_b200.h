@@ -170,8 +170,10 @@ int mfb_project_hist2d(const float* x, int64_t n, int d, const float* proj, cons
  * the tcgen05 kernels: the conditioner's masked GEMMs run as tcgen05.mma tiles over fp16 (hi, lo)
  * splits of the fp32 operands with fp32 accumulators in TMEM, the spline is the epilogue.  They are
  * compiled for hidden_units = 64, hidden_layers = 3, bins = 20, d = 2..6 (mfb_nsf_tc_supported) and
- * need an order that is a permutation.  With tc_image, another shape returns MFB_E_UNSUPPORTED; an
- * order that is not a permutation or an unaligned image returns MFB_E_BADARG.
+ * need an order that is a permutation.  They bulk-copy tiles of the layer input v (forward and
+ * backward), so there v must be 16-byte aligned as well.  With tc_image, another shape returns
+ * MFB_E_UNSUPPORTED; an order that is not a permutation, an unaligned image or an unaligned v
+ * returns MFB_E_BADARG.
  *
  * mfb_nsf_tc_prepare turns the packed parameters of n_layers layers (layer l at
  * params + l * layer_stride_floats; all-zero masked blocks are skipped) into n_layers operand images

@@ -646,7 +646,7 @@ int mfb_nsf_layer_bwd(const float* v, const float* gy, const float* glogq, int64
   if (hidden_units != kH || hidden_layers < 1 || bins < 2 || 3 * bins - 1 > kPP || d < 2 || d > 6)
     return MFB_E_UNSUPPORTED;
   if (tc_image) {
-    const int rc = nsf_tc_check(d, hidden_layers, bins, tc_image, order_host);
+    const int rc = nsf_tc_check(d, hidden_layers, bins, tc_image, order_host, v);
     if (rc) return rc;
   }
   if (workspace_bytes < mfb_nsf_layer_bwd_workspace_bytes(n, d, hidden_layers)) return MFB_E_WORKSPACE;

@@ -1168,17 +1168,18 @@ static int launch_inverse(const float* y, int64_t n, const unsigned char* image,
 
 }  // namespace tc
 
-int nsf_tc_check(int d, int hidden_layers, int bins, const void* image, const int32_t* order) {
+int nsf_tc_check(int d, int hidden_layers, int bins, const void* image, const int32_t* order, const void* rows) {
   if (!(d >= 2 && d <= 6 && hidden_layers == 3 && bins == 20)) return MFB_E_UNSUPPORTED;
   if (!tc::valid_order(d, order)) return MFB_E_BADARG;
   if ((reinterpret_cast<uintptr_t>(image) & 15u) != 0) return MFB_E_BADARG;   // loaded with a bulk copy
+  if ((reinterpret_cast<uintptr_t>(rows) & 15u) != 0) return MFB_E_BADARG;    // tiles of rows: bulk copies too
   return 0;
 }
 
 int nsf_tc_fwd(const float* v, int64_t n, int d, int hidden_layers, int bins, const void* image,
                const int32_t* order, const float* logq_in, int first_layer, float* y, float* logq_out,
                cudaStream_t st) {
-  const int rc = nsf_tc_check(d, hidden_layers, bins, image, order);
+  const int rc = nsf_tc_check(d, hidden_layers, bins, image, order, v);
   if (rc || n == 0) return rc;
   tc::Meta meta;
   tc::make_meta(d, order, &meta, nullptr);
@@ -1196,7 +1197,7 @@ int nsf_tc_fwd(const float* v, int64_t n, int d, int hidden_layers, int bins, co
 int nsf_tc_inv(const float* y, int64_t n, int d, int hidden_layers, int bins, const void* image,
                const int32_t* order, const float* ladj_in, int last_layer, float* v, float* ladj_out,
                cudaStream_t st) {
-  const int rc = nsf_tc_check(d, hidden_layers, bins, image, order);
+  const int rc = nsf_tc_check(d, hidden_layers, bins, image, order, nullptr);   // y is read row by row
   if (rc || n == 0) return rc;
   tc::Meta meta;
   tc::make_meta(d, order, &meta, nullptr);

@@ -202,8 +202,10 @@ static void hidden_classes(int d, int* cls, int* perm) {
 // The tcgen05 layer kernels of nsf_tc.cu, run from one layer's operand image (mfb_nsf_tc_prepare); the C entry points
 // of nsf.cu, nsf_inv.cu and nsf_bwd.cu call them when they are given an image.  order: HOST array of d ints.
 // nsf_tc_check: MFB_E_UNSUPPORTED for a shape the kernels are not compiled for (mfb_nsf_tc_supported), MFB_E_BADARG
-// for an order that is not a permutation or an image that is not 16-byte aligned (it is loaded with a bulk copy).
-int nsf_tc_check(int d, int hidden_layers, int bins, const void* image, const int32_t* order);
+// for an order that is not a permutation, or for an image or particle rows that are not 16-byte aligned (both are
+// loaded with bulk copies).  rows: the layer input the kernel bulk-copies (v of the forward and the backward), or
+// NULL where the kernel reads its rows with ordinary loads (y of the inverse).
+int nsf_tc_check(int d, int hidden_layers, int bins, const void* image, const int32_t* order, const void* rows);
 // the layer forward and inverse; each runs nsf_tc_check first
 int nsf_tc_fwd(const float* v, int64_t n, int d, int hidden_layers, int bins, const void* image,
                const int32_t* order, const float* logq_in, int first_layer, float* y, float* logq_out,

@@ -853,6 +853,12 @@ class NSFForward(torch.autograd.Function):
 NSF_BWD_CHUNK = 1 << 20   # particles per backward pass: bounds the recompute workspace (~2.9 KB/particle)
 
 
+def nsf_bwd_chunk(n: int) -> int:
+    """Particles per backward pass for a batch of ``n``: NSF_BWD_CHUNK rounded down to a multiple of 128 (at least
+    128), so that every chunk starts on a 16-byte aligned row for every D (the tcgen05 kernels bulk-copy their rows)."""
+    return min(n, max(128, NSF_BWD_CHUNK // 128 * 128))
+
+
 def nsf_backward(inputs, packed, packed_om, orders, hidden_units, hidden_layers, bins, gx, glogq, images=None):
     """(dL/dz, dL/dpacked) given the per-layer inputs saved by the forward pass.  ``images``: the tcgen05
     operand images of the same packed weights (``nsf_tc_images``), reused instead of being rebuilt."""
@@ -864,7 +870,7 @@ def nsf_backward(inputs, packed, packed_om, orders, hidden_units, hidden_layers,
     if n == 0:
         return gz, gpacked
     images = nsf_direction_images(NSF_BWD_USE_TENSOR_CORES, packed, orders, hidden_units, hidden_layers, bins, images)
-    chunk = min(n, NSF_BWD_CHUNK)
+    chunk = nsf_bwd_chunk(n)
     with torch.cuda.device(dev):
         wbytes = lib.mfb_nsf_layer_bwd_workspace_bytes(chunk, d, hidden_layers)
         work = torch.empty(wbytes, dtype=torch.uint8, device=dev)

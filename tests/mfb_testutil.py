@@ -40,6 +40,128 @@ def generator_from_golden(g, device="cpu"):
     return gen.to(device)
 
 
+# ------------------------------------------------------------------------------------ flow gradients
+def nsf_case(d, n, scale, hidden_layers=3, transforms=5, bins=20, seed=0, wide=False):
+    """A seeded flow and its inputs: (NSFGenerator on the CPU with every parameter x ``scale``, its float64 oracle,
+    z (n, d), and the upstream gradients a = dL/dx (n, d), b = dL/dlog q (n,) of L = sum(x a) + sum(log q b))."""
+    import mentflow_b200 as mf
+    torch.manual_seed(seed)
+    gen = mf.generate.NSFGenerator(d, hidden_layers=hidden_layers, transforms=transforms, bins=bins)
+    with torch.no_grad():
+        for p in gen.parameters():
+            p.mul_(scale)
+    ref = oracle_from_generator(gen)      # before the draws below: building it advances the generator
+    z = torch.randn(n, d)
+    if wide:      # the whole spline box and beyond: first / last bins, identity outside [-5, 5]
+        z = (torch.rand(n, d) - 0.5) * 13.0
+    a, b = torch.randn(n, d), torch.randn(n)
+    return gen, ref, z, a, b
+
+
+def nsf_loss(x, lq, a, b, loss):
+    """"both": sum(x a) + sum(log q b); "x": sum(x a) (log q not computed); "logq": sum(log q b) (dL/dx = 0)."""
+    if loss == "x":
+        return (x * a).sum()
+    if loss == "logq":
+        return (lq * b).sum()
+    return (x * a).sum() + (lq * b).sum()
+
+
+def nsf_kernel_grads(gen, z, a, b, loss="both"):
+    """dL/dz and dL/dtheta of ``nsf_loss`` through the CUDA flow ``gen``: {"z", "w_in", "b_in", "w_hid", "b_hid",
+    "w_out", "b_out"}, each as the kernels left it (the x-only loss runs gen.forward, which computes no log q)."""
+    for p in gen.parameters():
+        p.grad = None
+    zc = z.cuda().requires_grad_(True)
+    if loss == "x":
+        x, lq = gen.forward(zc), None
+    else:
+        x, lq = gen.forward_and_log_prob(zc)
+    nsf_loss(x, lq, a.cuda(), b.cuda(), loss).backward()
+    out = {"z": zc.grad}
+    for name in ("w_in", "b_in", "w_hid", "b_hid", "w_out", "b_out"):
+        out[name] = getattr(gen, name).grad
+    return out
+
+
+def nsf_named_grads(g, hidden_layers, transforms):
+    """``nsf_kernel_grads`` split per layer under the names of ``nsf_oracle_grads``."""
+    out = {"z": g["z"]}
+    for t in range(transforms):
+        out[f"w_in{t}"], out[f"b_in{t}"] = g["w_in"][t], g["b_in"][t]
+        for l in range(hidden_layers - 1):
+            out[f"w_hid{t}.{l}"], out[f"b_hid{t}.{l}"] = g["w_hid"][t, l], g["b_hid"][t, l]
+        out[f"w_out{t}"], out[f"b_out{t}"] = g["w_out"][t], g["b_out"][t]
+    return out
+
+
+def nsf_oracle_grads(flow, z, a, b, loss="both"):
+    """Autograd of ``nsf_loss`` through the oracle ``flow`` in its own dtype: {"z", "w_in{t}", "b_in{t}",
+    "w_hid{t}.{l}", "b_hid{t}.{l}", "w_out{t}", "b_out{t}"} (float64), masked weights' entries zeroed; and
+    {"w_in{t}", "w_hid{t}.{l}", "w_out{t}"}: the masks."""
+    dtype = next(flow.parameters()).dtype
+    for q in flow.parameters():
+        q.grad = None
+    zz = z.to(dtype).clone().requires_grad_(True)
+    x, lq = flow.forward_and_log_prob(zz)
+    nsf_loss(x, lq, a.to(dtype), b.to(dtype), loss).backward()
+    out, masks = {"z": zz.grad.double()}, {}
+    for t in range(len(flow.layers)):
+        lin = [m for m in flow.layers[t].hyper if hasattr(m, "weight")]
+        names = [f"in{t}"] + [f"hid{t}.{l}" for l in range(len(lin) - 2)] + [f"out{t}"]
+        for name, m in zip(names, lin):
+            gw = torch.zeros_like(m.weight) if m.weight.grad is None else m.weight.grad
+            gb = torch.zeros_like(m.bias) if m.bias.grad is None else m.bias.grad
+            out["w_" + name], out["b_" + name] = (gw * m.mask).double(), gb.double()
+            masks["w_" + name] = m.mask.detach().bool()
+    return out, masks
+
+
+def nsf_relu_kink_particles(flow, z, margin=1e-6):
+    """Boolean mask of the particles whose forward pass through the oracle ``flow`` puts some hidden pre-activation
+    within ``margin`` of the ReLU kink, relative to the sum of the magnitudes of its terms (|b| + sum |w h|).  An fp32
+    evaluation may take the other branch there: the particle's whole upstream gradient then moves between the unit's
+    parameter gradients, while its dL/dz barely changes."""
+    near, hooks = torch.zeros(z.shape[0], dtype=torch.bool), []
+
+    def check(m, inputs, out):
+        nonlocal near
+        h = inputs[0]
+        size = h.abs() @ (m.weight * m.mask).abs().T + m.bias.abs()
+        near = near | (out.abs() <= margin * size).any(dim=1)
+
+    for layer in flow.layers:
+        lin = [m for m in layer.hyper if hasattr(m, "weight")]
+        hooks += [m.register_forward_hook(check) for m in lin[:-1]]      # the output layer feeds no ReLU
+    try:
+        with torch.no_grad():
+            flow.forward_and_log_prob(z.to(next(flow.parameters()).dtype))
+    finally:
+        for hk in hooks:
+            hk.remove()
+    return near
+
+
+def grads_case(d, n, scale, hidden_layers=3, transforms=5, bins=20, seed=0, keep=None, wide=False, loss="both",
+               upstream=None):
+    """{name: (CUDA flow's gradient, float64 oracle autograd's)} for the seeded ``nsf_case``.  ``upstream(a, b)``
+    returns the upstream gradients to use instead of a, b; ``keep``: boolean mask of the particles to keep."""
+    gen, ref, z, a, b = nsf_case(d, n, scale, hidden_layers, transforms, bins, seed, wide)
+    if upstream is not None:
+        a, b = upstream(a, b)
+    if keep is not None:
+        z, a, b = z[keep], a[keep], b[keep]
+    got = nsf_named_grads(nsf_kernel_grads(gen.to("cuda"), z, a, b, loss), hidden_layers, transforms)
+    want, _ = nsf_oracle_grads(ref, z, a, b, loss)
+    return {k: (got[k], want[k]) for k in want}
+
+
+def grad_rel(got, want):
+    """|got - want| relative to the largest entry of ``want`` (the metric of every flow-gradient test)."""
+    want = want.double().cpu()
+    return (got.double().cpu() - want).abs() / want.abs().max().clamp_min(1e-30)
+
+
 def rel_err(a, b):
     """max |a-b| / max(1, |b|) elementwise (SURVEY 8c metric for x and log q)."""
     a, b = a.double().cpu(), b.double().cpu()

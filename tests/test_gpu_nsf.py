@@ -17,7 +17,7 @@ import pytest
 import torch
 
 import mentflow_b200 as mf
-from mfb_testutil import err_stats, generator_from_golden, oracle_from_generator, rel_err, t32
+from mfb_testutil import generator_from_golden, grad_rel, grads_case, oracle_from_generator, rel_err, t32
 
 pytestmark = pytest.mark.gpu
 TOL = 1.0e-4
@@ -249,44 +249,6 @@ def test_sampling_statistics_full_size():
     assert rel_err(x1[idx], xr) < TOL and rel_err(l1[idx], lr) < TOL
 
 
-def _grads_case(d, n, scale, hidden_layers=3, transforms=5, bins=20, seed=0, keep=None, wide=False):
-    torch.manual_seed(seed)
-    gen = mf.generate.NSFGenerator(d, hidden_layers=hidden_layers, transforms=transforms, bins=bins)
-    with torch.no_grad():
-        for p in gen.parameters():
-            p.mul_(scale)
-    ref = oracle_from_generator(gen)
-    gen = gen.to("cuda")
-    z = torch.randn(n, d)
-    if wide:      # the whole spline box and beyond: first / last bins, identity outside [-5, 5]
-        z = (torch.rand(n, d) - 0.5) * 13.0
-    a, b = torch.randn(n, d), torch.randn(n)
-    if keep is not None:
-        z, a, b = z[keep], a[keep], b[keep]
-    zc = z.cuda().requires_grad_(True)
-    x, lq = gen.forward_and_log_prob(zc)
-    ((x * a.cuda()).sum() + (lq * b.cuda()).sum()).backward()
-    zr = z.double().requires_grad_(True)
-    xr, lr = ref.forward_and_log_prob(zr)
-    ((xr * a.double()).sum() + (lr * b.double()).sum()).backward()
-    out = {"z": (zc.grad, zr.grad)}
-    for t in range(transforms):
-        lin = [m for m in ref.layers[t].hyper if hasattr(m, "weight")]
-        out[f"w_in{t}"] = (gen.w_in.grad[t], lin[0].weight.grad * lin[0].mask)
-        out[f"b_in{t}"] = (gen.b_in.grad[t], lin[0].bias.grad)
-        for l in range(hidden_layers - 1):
-            out[f"w_hid{t}.{l}"] = (gen.w_hid.grad[t, l], lin[l + 1].weight.grad * lin[l + 1].mask)
-            out[f"b_hid{t}.{l}"] = (gen.b_hid.grad[t, l], lin[l + 1].bias.grad)
-        out[f"w_out{t}"] = (gen.w_out.grad[t], lin[-1].weight.grad * lin[-1].mask)
-        out[f"b_out{t}"] = (gen.b_out.grad[t], lin[-1].bias.grad)
-    return out
-
-
-def _rel(got, want):
-    want = want.double()
-    return (got.double().cpu() - want).abs() / want.abs().max().clamp_min(1e-30)
-
-
 @pytest.mark.parametrize("d,n,scale,hl,tr,bins", [(6, 3000, 1.0, 3, 5, 20), (2, 1000, 1.5, 3, 5, 20),
                                                   (4, 777, 1.0, 2, 3, 8), (3, 513, 1.0, 1, 2, 12),
                                                   (6, 40000, 1.5, 3, 2, 20)])
@@ -300,13 +262,13 @@ def test_backward_matches_oracle_autograd(d, n, scale, hl, tr, bins):
     their dL/dz (they must be rare); pass 2 repeats the comparison without them and requires
     every gradient tensor to agree."""
     seed = d + n
-    first = _grads_case(d, n, scale, hl, tr, bins, seed=seed)
-    per_particle = _rel(*first["z"]).max(dim=1).values
+    first = grads_case(d, n, scale, hl, tr, bins, seed=seed)
+    per_particle = grad_rel(*first["z"]).max(dim=1).values
     suspects = per_particle > 1e-4
     assert int(suspects.sum()) <= 2 + n // 100, f"{int(suspects.sum())} of {n} particles disagree in dL/dz"
-    grads = _grads_case(d, n, scale, hl, tr, bins, seed=seed, keep=~suspects)
+    grads = grads_case(d, n, scale, hl, tr, bins, seed=seed, keep=~suspects)
     for name, (got, want) in grads.items():
-        e = _rel(got, want).flatten()
+        e = grad_rel(got, want).flatten()
         assert float(e.max()) < 1e-3, f"{name}: max {float(e.max()):.2e}"
         assert float(e.median()) < 2e-5, f"{name}: median {float(e.median()):.2e}"
     got, want = grads["w_out0"]
@@ -318,13 +280,13 @@ def test_backward_edge_bins_and_outside_the_box(d, n):
     """Inputs spread over [-6.5, 6.5]^D: particles in the first and last bins (whose outer knot has no derivative
     parameter: the compact dL/dphi rows carry a zero there), outside the box (identity: no parameter gradient) and a
     last tile with a single row (n = 16 x 128 + 1)."""
-    first = _grads_case(d, n, 1.0, seed=5 + d, wide=True)
-    per_particle = _rel(*first["z"]).max(dim=1).values
+    first = grads_case(d, n, 1.0, seed=5 + d, wide=True)
+    per_particle = grad_rel(*first["z"]).max(dim=1).values
     suspects = per_particle > 1e-4
     assert int(suspects.sum()) <= 2 + n // 100, f"{int(suspects.sum())} of {n} particles disagree in dL/dz"
-    grads = _grads_case(d, n, 1.0, seed=5 + d, wide=True, keep=~suspects)
+    grads = grads_case(d, n, 1.0, seed=5 + d, wide=True, keep=~suspects)
     for name, (got, want) in grads.items():
-        e = _rel(got, want).flatten()
+        e = grad_rel(got, want).flatten()
         assert float(e.max()) < 1e-3, f"{name}: max {float(e.max()):.2e}"
         assert float(e.median()) < 2e-5, f"{name}: median {float(e.median()):.2e}"
 

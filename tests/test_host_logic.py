@@ -231,6 +231,25 @@ def test_tensor_core_flow_host_side_contract():
         assert call(3, ctypes.c_void_p(24), good_order) == -1    # the image is loaded with a bulk copy: 16-byte aligned
         assert call(3, None, None) == -1                     # the order is required, with or without an image
         assert call(3, dummy, None) == -1
+    # the tcgen05 forward and backward bulk-copy tiles of the layer input v: rows that start 4 bytes past a 16-byte
+    # boundary are refused before anything else about the batch is looked at (an empty forward, a backward without
+    # a workspace); the CUDA-core forward reads rows one by one and has nothing to do for n = 0
+    v = ctypes.c_void_p(20)
+    assert lib.mfb_nsf_layer_fwd(v, 0, 6, 64, 3, 20, dummy, dummy, good_order, None, 1, dummy, None, None) == -1
+    assert lib.mfb_nsf_layer_fwd(v, 0, 6, 64, 3, 20, dummy, None, good_order, None, 1, dummy, None, None) == 0
+    assert lib.mfb_nsf_layer_bwd(v, dummy, None, 10, 6, 64, 3, 20, dummy, dummy, dummy, good_order, 1, dummy, dummy, 0,
+                                 dummy, 0, None) == -1
+
+
+def test_flow_backward_chunks_start_on_aligned_rows(monkeypatch):
+    """nsf_backward runs a batch in chunks of NSF_BWD_CHUNK particles rounded down to a multiple of 128 (at least 128):
+    every chunk then starts on a 16-byte aligned row for every D, which the tcgen05 kernels' bulk copies need."""
+    for chunk, n, want in [(1 << 20, 5, 5), (1 << 20, 2_000_000, 1 << 20), (1000, 5000, 896), (1, 5000, 128),
+                           (0, 300, 128), (128, 100, 100), (1029, 100_000, 1024)]:
+        monkeypatch.setattr(ops, "NSF_BWD_CHUNK", chunk)
+        got = ops.nsf_bwd_chunk(n)
+        assert got == want, (chunk, n)
+        assert all(start * d * 4 % 16 == 0 for d in range(2, 7) for start in range(0, n, got))
 
 
 def test_ment_entry_points_refuse_bad_arguments(monkeypatch):
