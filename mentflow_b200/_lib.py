@@ -76,6 +76,10 @@ SIGNATURES = {
     "mfb_knn_workspace_bytes": (c_int64, [c_int64, c_int, c_int]),
     "mfb_knn_kth": (c_int, [P, c_int64, c_int, c_int, c_double, P, P, P, P, c_int64, P]),
     "mfb_knn_kth_bwd": (c_int, [P, c_int64, c_int, P, P, P, P, c_double, P, P, P]),
+    "mfb_knn_rows_workspace_bytes": (c_int64, [c_int64, c_int64, c_int, c_int]),
+    "mfb_knn_kth_rows": (c_int, [P, c_int64, c_int, c_int, c_int64, c_int64, P, P, P, c_int64, P]),
+    "mfb_knn_logsum": (c_int, [P, c_int64, c_double, P, P, c_int64, P]),
+    "mfb_knn_kth_bwd_rows": (c_int, [P, c_int64, c_int, P, P, P, P, c_int64, c_int64, c_double, P, P, P]),
     "mfb_swd_workspace_bytes": (c_int64, [c_int64, c_int]),
     "mfb_swd_sort": (c_int, [P, c_int64, c_int, P, c_int, P, P, P, c_int64, P]),
     "mfb_swd_wpp": (c_int, [P, c_int64, c_int, P, c_int, P, c_int64, c_double, P, P, P, c_int64, P]),

@@ -21,6 +21,11 @@
 // Backward of logsum (neighbour identities held fixed, as autograd through cdist + topk):
 //   d logsum / dx_i = w_i (x_i - x_n(i)) + sum_{j : n(j) = i} w_j (x_i - x_j),  w_j = 1 / (r_j (r_j + pad)), 0 at r_j = 0.
 // The caller passes n(.) stably sorted with its permutation; particle i sums its segment in ascending j.
+//
+// Row ranges (particles sharded over ranks): the search and the backward run for the queries [row0, row0 + nrows) of
+// a batch of n candidates.  A pair's r^2 and the k-th neighbour depend only on the pair and on the candidate set, so
+// the rows of a range are bit for bit those of the whole batch; knn_logpart_kernel then adds log(r + pad) of the
+// gathered r with the merge kernel's own block partials (knn_block_logpart), so the log sum is the whole batch's too.
 #include "common.cuh"
 
 namespace mfb {
@@ -157,7 +162,7 @@ __device__ __forceinline__ void scan_tile(const float* __restrict__ ts, int j0, 
 
 template <int D, int KB>
 __global__ void __launch_bounds__(kKnnThreads, 2)
-knn_partial_kernel(const float* __restrict__ x, const float* __restrict__ xt, int64_t n, int64_t npad, int k,
+knn_partial_kernel(const float* __restrict__ x, const float* __restrict__ xt, int64_t npad, int row0, int nrows, int k,
                    int ntiles, int splits, float* __restrict__ pd2, int32_t* __restrict__ pidx) {
   __shared__ __align__(128) float tile[2][D * kKnnTile];
   __shared__ __align__(8) uint64_t bar[2];
@@ -181,14 +186,15 @@ knn_partial_kernel(const float* __restrict__ x, const float* __restrict__ xt, in
   };
   if (tid == 0 && t_begin < t_end) issue(0, t_begin);
 
-  const int q0 = blockIdx.x * kKnnRows;
+  const int q0 = row0 + blockIdx.x * kKnnRows;   // global index of the CTA's first query
+  const int qend = row0 + nrows;
   int qi[2];
   uint64_t nq[2][D];
   TopK<KB> top[2];
 #pragma unroll
   for (int q = 0; q < 2; ++q) {
     qi[q] = q0 + q * kKnnThreads + tid;
-    const bool live = qi[q] < n;
+    const bool live = qi[q] < qend;
 #pragma unroll
     for (int c = 0; c < D; ++c) {
       const float v = live ? -x[(int64_t)qi[q] * D + c] : 0.f;
@@ -208,15 +214,15 @@ knn_partial_kernel(const float* __restrict__ x, const float* __restrict__ xt, in
     __syncthreads();   // everyone is done with tile[stage] before it is refilled
   }
 
-  // the k real entries, ascending, at [split][rank][query]
+  // the k real entries, ascending, at [split][rank][local query]
 #pragma unroll
   for (int q = 0; q < 2; ++q) {
-    if (qi[q] >= n) continue;
+    if (qi[q] >= qend) continue;
 #pragma unroll
     for (int s = 0; s < KB; ++s) {
       const int rank = s - (KB - k);
       if (rank >= 0) {
-        const int64_t o = ((int64_t)split * k + rank) * n + qi[q];
+        const int64_t o = ((int64_t)split * k + rank) * nrows + (qi[q] - row0);
         pd2[o] = top[q].key[s];
         pidx[o] = top[q].id[s];
       }
@@ -224,19 +230,36 @@ knn_partial_kernel(const float* __restrict__ x, const float* __restrict__ xt, in
   }
 }
 
+__device__ __forceinline__ double knn_logterm(float rv, double pad) { return log((double)rv + pad); }
+
+// one double partial of the log sum per block of kKnnThreads queries: warp sums, then the warps in order.  The merge
+// kernel and knn_logpart_kernel both call it, so a log sum of gathered rows adds exactly as one whole-batch search.
+__device__ __forceinline__ void knn_block_logpart(double lg, double* __restrict__ logpart) {
+  __shared__ double red[kKnnThreads / 32];
+  lg = warp_sum(lg);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = lg;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double s = 0.0;
+    for (int w = 0; w < kKnnThreads / 32; ++w) s += red[w];
+    logpart[blockIdx.x] = s;
+  }
+}
+
+// local queries q in [0, nrows), global index row0 + q; logpart NULL: no log sum (a row range of a sharded batch)
 template <int KB>
 __global__ void __launch_bounds__(kKnnThreads)
-knn_merge_kernel(const float* __restrict__ pd2, const int32_t* __restrict__ pidx, int64_t n, int k, int splits,
-                 double pad, float* __restrict__ r, int32_t* __restrict__ idx, double* __restrict__ logpart) {
+knn_merge_kernel(const float* __restrict__ pd2, const int32_t* __restrict__ pidx, int64_t row0, int64_t nrows, int k,
+                 int splits, double pad, float* __restrict__ r, int32_t* __restrict__ idx, double* __restrict__ logpart) {
   pdl_enter();
   const int64_t q = (int64_t)blockIdx.x * kKnnThreads + threadIdx.x;
   double lg = 0.0;
-  if (q < n) {
+  if (q < nrows) {
     TopK<KB> top;
     top.init(k);
     for (int s = 0; s < splits; ++s) {
       for (int rank = 0; rank < k; ++rank) {   // a split's list is ascending: the first miss ends it
-        const int64_t o = ((int64_t)s * k + rank) * n + q;
+        const int64_t o = ((int64_t)s * k + rank) * nrows + q;
         const float d = pd2[o];
         if (!(d < top.worst())) break;
         top.insert(d, pidx[o]);
@@ -247,18 +270,18 @@ knn_merge_kernel(const float* __restrict__ pd2, const int32_t* __restrict__ pidx
     const int nb = top.id[KB - 1];
     const float rv = nb < 0 ? __int_as_float(0x7f800000) : sqrtf(top.worst());
     r[q] = rv;
-    idx[q] = nb < 0 ? (int32_t)q : nb;
-    lg = log((double)rv + pad);
+    idx[q] = nb < 0 ? (int32_t)(row0 + q) : nb;
+    lg = knn_logterm(rv, pad);
   }
-  __shared__ double red[kKnnThreads / 32];
-  lg = warp_sum(lg);
-  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = lg;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    double s = 0.0;
-    for (int w = 0; w < kKnnThreads / 32; ++w) s += red[w];
-    logpart[blockIdx.x] = s;
-  }
+  if (logpart) knn_block_logpart(lg, logpart);
+}
+
+// the merge kernel's log partials from r of the whole batch (gathered from row ranges)
+__global__ void __launch_bounds__(kKnnThreads)
+knn_logpart_kernel(const float* __restrict__ r, int64_t n, double pad, double* __restrict__ logpart) {
+  pdl_enter();
+  const int64_t q = (int64_t)blockIdx.x * kKnnThreads + threadIdx.x;
+  knn_block_logpart(q < n ? knn_logterm(r[q], pad) : 0.0, logpart);
 }
 
 // one block: threads stride over the partials, fixed shuffle tree, fixed warp order => deterministic
@@ -284,11 +307,12 @@ __device__ __forceinline__ float knn_weight(float rv, double pad, double g) {
 template <int D>
 __global__ void __launch_bounds__(kKnnThreads)
 knn_bwd_kernel(const float* __restrict__ x, int64_t n, const float* __restrict__ r, const int32_t* __restrict__ idx,
-               const int32_t* __restrict__ sorted_idx, const int64_t* __restrict__ perm, double pad,
-               const double* __restrict__ glogsum, float* __restrict__ gx) {
+               const int32_t* __restrict__ sorted_idx, const int64_t* __restrict__ perm, int64_t row0, int64_t nrows,
+               double pad, const double* __restrict__ glogsum, float* __restrict__ gx) {
   pdl_enter();
-  const int64_t i = (int64_t)blockIdx.x * kKnnThreads + threadIdx.x;
-  if (i >= n) return;
+  const int64_t li = (int64_t)blockIdx.x * kKnnThreads + threadIdx.x;   // row of gx; i is its particle in the batch
+  if (li >= nrows) return;
+  const int64_t i = row0 + li;
   const double g = glogsum[0];
   float xi[D], acc[D];
   const float wi = knn_weight(r[i], pad, g);
@@ -312,14 +336,15 @@ knn_bwd_kernel(const float* __restrict__ x, int64_t n, const float* __restrict__
     for (int c = 0; c < D; ++c) acc[c] = fmaf(wj, xi[c] - x[j * D + c], acc[c]);
   }
 #pragma unroll
-  for (int c = 0; c < D; ++c) gx[i * D + c] = acc[c];
+  for (int c = 0; c < D; ++c) gx[li * D + c] = acc[c];
 }
 
 // ---- launch plan -----------------------------------------------------------------------------------------------
-typedef void (*KnnPartialFn)(const float*, const float*, int64_t, int64_t, int, int, int, float*, int32_t*);
-typedef void (*KnnMergeFn)(const float*, const int32_t*, int64_t, int, int, double, float*, int32_t*, double*);
-typedef void (*KnnBwdFn)(const float*, int64_t, const float*, const int32_t*, const int32_t*, const int64_t*, double,
-                         const double*, float*);
+typedef void (*KnnPartialFn)(const float*, const float*, int64_t, int, int, int, int, int, float*, int32_t*);
+typedef void (*KnnMergeFn)(const float*, const int32_t*, int64_t, int64_t, int, int, double, float*, int32_t*,
+                           double*);
+typedef void (*KnnBwdFn)(const float*, int64_t, const float*, const int32_t*, const int32_t*, const int64_t*, int64_t,
+                         int64_t, double, const double*, float*);
 
 static int knn_list_slots(int k) { return k <= 4 ? 4 : (k <= 8 ? 8 : 16); }
 
@@ -350,15 +375,18 @@ struct KnnPlan {
 };
 
 static size_t round16(size_t b) { return (b + 15) & ~(size_t)15; }
+static int64_t knn_logparts(int64_t n) { return (n + kKnnThreads - 1) / kKnnThreads; }
 
-// Splits of the candidate axis: with few queries (25,000 fill 49 CTAs of 512) the grid would leave most SMs idle, so
-// the candidate tiles are cut into `splits` ranges.  The choice rounds the CTA count up to whole waves of resident
-// CTAs (preferring fewer splits unless more are 2 % better), at least kKnnMinTilesPerSplit tiles each.
-static int knn_plan(int64_t n, int d, int k, KnnPlan& p) {
+// Queries [row0, row0 + nrows) against n candidates: the candidate tiles follow n, the query blocks and the split
+// choice follow nrows.  Splits of the candidate axis: with few queries (25,000 fill 49 CTAs of 512) the grid would
+// leave most SMs idle, so the candidate tiles are cut into `splits` ranges.  The choice rounds the CTA count up to
+// whole waves of resident CTAs (preferring fewer splits unless more are 2 % better), at least kKnnMinTilesPerSplit
+// tiles each.  with_logsum: room for the merge's log partials (the whole-batch call).
+static int knn_plan(int64_t n, int64_t nrows, int d, int k, bool with_logsum, KnnPlan& p) {
   p.ntiles = (int)((n + kKnnTile - 1) / kKnnTile);
   p.npad = (int64_t)p.ntiles * kKnnTile;
-  p.qblocks = (int)((n + kKnnRows - 1) / kKnnRows);
-  p.mblocks = (int)((n + kKnnThreads - 1) / kKnnThreads);
+  p.qblocks = (int)((nrows + kKnnRows - 1) / kKnnRows);
+  p.mblocks = (int)knn_logparts(nrows);
   int per_sm = 0;
   MFB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, knn_partial_for(d, k), kKnnThreads, 0));
   const int64_t slots = (int64_t)sm_count() * (per_sm > 0 ? per_sm : 1);
@@ -375,11 +403,11 @@ static int knn_plan(int64_t n, int d, int k, KnnPlan& p) {
     }
   }
   p.splits = best;
-  const size_t list = round16((size_t)p.splits * k * n * 4);
+  const size_t list = round16((size_t)p.splits * k * nrows * 4);
   p.off_pd2 = (size_t)d * p.npad * 4;
   p.off_pidx = p.off_pd2 + list;
   p.off_logpart = p.off_pidx + list;
-  p.bytes = p.off_logpart + (size_t)p.mblocks * 8;
+  p.bytes = p.off_logpart + (with_logsum ? (size_t)p.mblocks * 8 : 0);
   return 0;
 }
 
@@ -388,6 +416,43 @@ static int knn_check(const float* x, int64_t n, int d, int k) {
   if (d > kMaxDim || k > kKnnMaxK) return MFB_E_UNSUPPORTED;
   if (k >= n) return MFB_E_BADARG;
   return 0;
+}
+
+static bool knn_range_ok(int64_t n, int64_t row0, int64_t nrows) {
+  return row0 >= 0 && nrows >= 0 && row0 <= n && nrows <= n - row0;
+}
+
+// transpose, pair search and merge for the queries [row0, row0 + nrows); logsum NULL: no log sum
+static int knn_search(const float* x, int64_t n, int d, int k, int64_t row0, int64_t nrows, double pad, float* r,
+                      int32_t* idx, double* logsum, void* workspace, int64_t workspace_bytes, cudaStream_t st) {
+  KnnPlan p;
+  int rc = knn_plan(n, nrows, d, k, logsum != nullptr, p);
+  if (rc) return rc;
+  if (workspace_bytes < (int64_t)p.bytes) return MFB_E_WORKSPACE;
+  char* ws = (char*)workspace;
+  float* xt = (float*)ws;
+  float* pd2 = (float*)(ws + p.off_pd2);
+  int32_t* pidx = (int32_t*)(ws + p.off_pidx);
+  double* logpart = logsum ? (double*)(ws + p.off_logpart) : nullptr;
+
+  const int64_t tn = p.npad * d;
+  MFB_CUDA(launch_pdl(knn_transpose_kernel, dim3((unsigned)((tn + 255) / 256)), dim3(256), 0, st, x, n, d, p.npad, xt));
+  MFB_CUDA(launch_pdl(knn_partial_for(d, k), dim3(p.qblocks, p.splits), dim3(kKnnThreads), 0, st, x,
+                      (const float*)xt, p.npad, (int)row0, (int)nrows, k, p.ntiles, p.splits, pd2, pidx));
+  MFB_CUDA(launch_pdl(knn_merge_for(k), dim3(p.mblocks), dim3(kKnnThreads), 0, st, (const float*)pd2,
+                      (const int32_t*)pidx, row0, nrows, k, p.splits, pad, r, idx, logpart));
+  if (logsum)
+    MFB_CUDA(launch_pdl(knn_logsum_kernel, dim3(1), dim3(kKnnThreads), 0, st, (const double*)logpart, p.mblocks,
+                        logsum));
+  return launch_status();
+}
+
+static int knn_backward(const float* x, int64_t n, int d, const float* r, const int32_t* idx,
+                        const int32_t* sorted_idx, const int64_t* perm, int64_t row0, int64_t nrows, double pad,
+                        const double* glogsum, float* gx, cudaStream_t st) {
+  MFB_CUDA(launch_pdl(knn_bwd_for(d), dim3((unsigned)((nrows + kKnnThreads - 1) / kKnnThreads)), dim3(kKnnThreads), 0,
+                      st, x, n, r, idx, sorted_idx, perm, row0, nrows, pad, glogsum, gx));
+  return launch_status();
 }
 
 }  // namespace mfb
@@ -399,7 +464,7 @@ extern "C" {
 int64_t mfb_knn_workspace_bytes(int64_t n, int d, int k) {
   if (knn_check((const float*)1, n, d, k)) return 0;
   KnnPlan p;
-  if (knn_plan(n, d, k, p)) return 0;
+  if (knn_plan(n, n, d, k, true, p)) return 0;
   return (int64_t)p.bytes;
 }
 
@@ -408,34 +473,55 @@ int mfb_knn_kth(const float* x, int64_t n, int d, int k, double pad, float* r, i
   int rc = knn_check(x, n, d, k);
   if (rc) return rc;
   MFB_CHECK_ARG(r && idx && logsum && workspace);
-  KnnPlan p;
-  rc = knn_plan(n, d, k, p);
-  if (rc) return rc;
-  if (workspace_bytes < (int64_t)p.bytes) return MFB_E_WORKSPACE;
-  cudaStream_t st = (cudaStream_t)stream;
-  char* ws = (char*)workspace;
-  float* xt = (float*)ws;
-  float* pd2 = (float*)(ws + p.off_pd2);
-  int32_t* pidx = (int32_t*)(ws + p.off_pidx);
-  double* logpart = (double*)(ws + p.off_logpart);
-
-  const int64_t tn = p.npad * d;
-  MFB_CUDA(launch_pdl(knn_transpose_kernel, dim3((unsigned)((tn + 255) / 256)), dim3(256), 0, st, x, n, d, p.npad, xt));
-  MFB_CUDA(launch_pdl(knn_partial_for(d, k), dim3(p.qblocks, p.splits), dim3(kKnnThreads), 0, st, x,
-                      (const float*)xt, n, p.npad, k, p.ntiles, p.splits, pd2, pidx));
-  MFB_CUDA(launch_pdl(knn_merge_for(k), dim3(p.mblocks), dim3(kKnnThreads), 0, st, (const float*)pd2,
-                      (const int32_t*)pidx, n, k, p.splits, pad, r, idx, logpart));
-  MFB_CUDA(launch_pdl(knn_logsum_kernel, dim3(1), dim3(kKnnThreads), 0, st, (const double*)logpart, p.mblocks, logsum));
-  return launch_status();
+  return knn_search(x, n, d, k, 0, n, pad, r, idx, logsum, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 int mfb_knn_kth_bwd(const float* x, int64_t n, int d, const float* r, const int32_t* idx, const int32_t* sorted_idx,
                     const int64_t* perm, double pad, const double* glogsum, float* gx, void* stream) {
   MFB_CHECK_ARG(x && r && idx && sorted_idx && perm && glogsum && gx && n >= 2 && n <= INT32_MAX && d >= 1);
   if (d > kMaxDim) return MFB_E_UNSUPPORTED;
-  MFB_CUDA(launch_pdl(knn_bwd_for(d), dim3((unsigned)((n + kKnnThreads - 1) / kKnnThreads)), dim3(kKnnThreads), 0,
-                      (cudaStream_t)stream, x, n, r, idx, sorted_idx, perm, pad, glogsum, gx));
+  return knn_backward(x, n, d, r, idx, sorted_idx, perm, 0, n, pad, glogsum, gx, (cudaStream_t)stream);
+}
+
+int64_t mfb_knn_rows_workspace_bytes(int64_t n, int64_t nrows, int d, int k) {
+  if (knn_check((const float*)1, n, d, k) || !knn_range_ok(n, 0, nrows) || nrows == 0) return 0;
+  KnnPlan p;
+  if (knn_plan(n, nrows, d, k, false, p)) return 0;
+  return (int64_t)p.bytes;
+}
+
+int mfb_knn_kth_rows(const float* x, int64_t n, int d, int k, int64_t row0, int64_t nrows, float* r, int32_t* idx,
+                     void* workspace, int64_t workspace_bytes, void* stream) {
+  int rc = knn_check(x, n, d, k);
+  if (rc) return rc;
+  MFB_CHECK_ARG(knn_range_ok(n, row0, nrows));
+  if (nrows == 0) return 0;
+  MFB_CHECK_ARG(r && idx && workspace);
+  return knn_search(x, n, d, k, row0, nrows, 0.0, r, idx, nullptr, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+int mfb_knn_logsum(const float* r, int64_t n, double pad, double* logsum, void* workspace, int64_t workspace_bytes,
+                   void* stream) {
+  MFB_CHECK_ARG(r && logsum && workspace && n >= 1 && n <= INT32_MAX);
+  const int64_t parts = knn_logparts(n);
+  if (workspace_bytes < parts * 8) return MFB_E_WORKSPACE;
+  cudaStream_t st = (cudaStream_t)stream;
+  double* logpart = (double*)workspace;
+  MFB_CUDA(launch_pdl(knn_logpart_kernel, dim3((unsigned)parts), dim3(kKnnThreads), 0, st, r, n, pad, logpart));
+  MFB_CUDA(launch_pdl(knn_logsum_kernel, dim3(1), dim3(kKnnThreads), 0, st, (const double*)logpart, (int)parts,
+                      logsum));
   return launch_status();
+}
+
+int mfb_knn_kth_bwd_rows(const float* x, int64_t n, int d, const float* r, const int32_t* idx,
+                         const int32_t* sorted_idx, const int64_t* perm, int64_t row0, int64_t nrows, double pad,
+                         const double* glogsum, float* gx, void* stream) {
+  MFB_CHECK_ARG(x && r && idx && sorted_idx && perm && glogsum && n >= 2 && n <= INT32_MAX && d >= 1);
+  if (d > kMaxDim) return MFB_E_UNSUPPORTED;
+  MFB_CHECK_ARG(knn_range_ok(n, row0, nrows));
+  if (nrows == 0) return 0;
+  MFB_CHECK_ARG(gx);
+  return knn_backward(x, n, d, r, idx, sorted_idx, perm, row0, nrows, pad, glogsum, gx, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -5,11 +5,13 @@ exchange on the forward path is ONE small all-reduce of the *unnormalised* profi
 (K*B floats, or exact 64-bit fixed-point integers for 2-D screens / histogram counts) and of
 the entropy partial sums -- it has to happen before the non-linear normalisation and KL
 (SURVEY.md 8e).  Gradients of the flow parameters are summed after backward
-(``allreduce_gradients``).  The reference has no distributed code at all.
+(``allreduce_gradients``).  The k-NN entropy estimator is the exception: its neighbours live in the
+union batch, so it all-gathers the particles and its per-particle results (``ShardReducer.all_gather``).
+The reference has no distributed code at all.
 """
 from __future__ import annotations
 
-from typing import Iterable, Optional
+from typing import Iterable, List, Optional
 
 import torch
 import torch.distributed as dist
@@ -89,6 +91,50 @@ class ShardReducer:
         if self.world_size == 1:
             return float(n_local)
         return float(n_local) * self.world_size if self.equal_shards else None
+
+    @property
+    def rank(self) -> int:
+        return dist.get_rank(self.group) if dist.is_initialized() else 0
+
+    def shard_counts(self, n_local: int, device=None) -> List[int]:
+        """Particles of every rank, in rank order.  With ``equal_shards`` (or one rank) this needs no communication;
+        otherwise it all-gathers the counts (one small collective and a host synchronisation).  ``device``: where the
+        count tensor lives for the collective (the CUDA device for NCCL)."""
+        world = self.world_size
+        if world == 1 or self.equal_shards:
+            return [int(n_local)] * world
+        mine = torch.tensor([int(n_local)], dtype=torch.int64, device=device)
+        out = torch.empty(world, dtype=torch.int64, device=device)
+        dist.all_gather_into_tensor(out, mine, group=self.group)
+        return [int(c) for c in out.tolist()]
+
+    def all_gather(self, tensor: torch.Tensor, counts: Optional[List[int]] = None) -> torch.Tensor:
+        """Every rank's ``tensor`` concatenated along dim 0 in rank order (the union batch, rank r's rows starting at
+        the sum of the counts of ranks 0 .. r-1).  With ``equal_shards`` it is one ``all_gather_into_tensor`` and no
+        host synchronisation, so a CUDA graph can capture it.  Unequal shards take the counts (``shard_counts``,
+        gathered here when not given), gather rows padded to the largest count and drop the padding.  With one rank,
+        the tensor itself."""
+        world = self.world_size
+        if world == 1:
+            return tensor
+        tensor = tensor.contiguous()
+        rest = tuple(tensor.shape[1:])
+        if self.equal_shards:
+            out = torch.empty((world * tensor.shape[0],) + rest, dtype=tensor.dtype, device=tensor.device)
+            dist.all_gather_into_tensor(out, tensor, group=self.group)
+            return out
+        if counts is None:
+            counts = self.shard_counts(tensor.shape[0], tensor.device)
+        m = max(counts)
+        if m == 0:
+            return tensor.new_empty((0,) + rest)
+        padded = tensor
+        if tensor.shape[0] != m:
+            padded = tensor.new_zeros((m,) + rest)
+            padded[:tensor.shape[0]] = tensor
+        buf = torch.empty((world * m,) + rest, dtype=tensor.dtype, device=tensor.device)
+        dist.all_gather_into_tensor(buf, padded, group=self.group)
+        return torch.cat([buf[r * m:r * m + c] for r, c in enumerate(counts)])
 
     def __call__(self, tensor: torch.Tensor, n_local: float, flat: Optional[torch.Tensor] = None) -> float:
         """``flat``: a flat float32 buffer whose head is ``tensor`` and whose last ``tail_floats()`` entries

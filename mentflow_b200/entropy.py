@@ -173,12 +173,43 @@ def knn_entropy_constant(n: int, d: int, k: int) -> float:
     return _digamma_int(n) - _digamma_int(k) + log_vd
 
 
+class _ShardedKNNLogsum(torch.autograd.Function):
+    """sum log(r_i + pad) over the union batch of a sharded model, from this rank's particles ``x``: all-gather the
+    particles, search this rank's rows against the union, all-gather r and idx, and add the logs over the union in the
+    single-GPU order.  Every rank gets the log sum one GPU computes on the union, bit for bit.  The backward needs no
+    exchange: a particle's gradient is its own term plus those of the particles whose k-th neighbour it is, and all of
+    them are in the gathered tensors, so each rank runs the gradient kernel for its own rows."""
+
+    @staticmethod
+    def forward(ctx, x, k, pad, reducer, counts, row0):
+        rows = slice(row0, row0 + x.shape[0])
+        xu = reducer.all_gather(x.detach(), counts)
+        r_rows, idx_rows, _ = ops.knn_kth(xu, k, pad, rows=rows)
+        r = reducer.all_gather(r_rows, counts)
+        idx = reducer.all_gather(idx_rows, counts)
+        ctx.save_for_backward(xu, r, idx)
+        ctx.pad, ctx.rows = pad, rows
+        return ops.knn_logsum(r, pad)
+
+    @staticmethod
+    def backward(ctx, glogsum):
+        xu, r, idx = ctx.saved_tensors
+        return ops.knn_kth_bwd(xu, r, idx, glogsum, ctx.pad, rows=ctx.rows), None, None, None, None, None
+
+
 class KNNEntropyEstimator(EntropyEstimator):
     """-H, H = psi(N) - psi(k) + log V_d + (d/N) sum_i log(r_i + pad), r_i the distance from x_i to its k-th nearest
     other particle (Kozachenko-Leonenko).  Works from the particles alone: ``log_prob`` is ignored.  The distances come
     from an all-pairs CUDA kernel (O(N^2 d), ops.knn_kth); the gradient holds the neighbours fixed, as autograd
-    through cdist + topk would.  Sharded particles are refused: the neighbours within a shard are not those within
-    the union."""
+    through cdist + topk would.
+
+    Sharded particles (``distributed.shard_model``): N is the union of all ranks' particles, and every rank returns
+    the -H one GPU computes on the union, bit for bit.  Each rank all-gathers the particles, searches its own rows
+    against the union (a 1 / ranks share of the pair work), and all-gathers r and the neighbour indices; its backward
+    gives the gradient of its own particles without further exchange.  With equal shards nothing synchronises with the
+    host, so ``GraphedLoss`` captures it.  The reducer must offer ``all_gather``, ``shard_counts`` and ``rank`` (as
+    ``distributed.ShardReducer`` does); a reducer without ``all_gather`` is refused, because the neighbours within one
+    shard are not those within the union."""
 
     def __init__(self, prior: Any = None, k: int = 5, pad: float = 1.0e-12) -> None:
         if prior is not None:
@@ -188,9 +219,27 @@ class KNNEntropyEstimator(EntropyEstimator):
         self.pad = pad
 
     def forward(self, x: torch.Tensor, log_prob: torch.Tensor = None) -> torch.Tensor:
-        if self.reducer is not None and getattr(self.reducer, "world_size", 1) > 1:
-            raise NotImplementedError("KNNEntropyEstimator does not support sharded particles: the nearest neighbours "
-                                      "within one rank's shard are not those within the whole batch")
-        _, _, logsum = ops.knn_kth(x, self.k, self.pad)
-        n, d = x.shape
+        red = self.reducer
+        if red is not None and getattr(red, "world_size", 1) > 1:
+            if not hasattr(red, "all_gather"):
+                raise NotImplementedError("KNNEntropyEstimator needs a reducer with all_gather for sharded particles: "
+                                          "the nearest neighbours within one rank's shard are not those within the "
+                                          "whole batch")
+            logsum, n, d = self._sharded_logsum(x)
+        else:
+            _, _, logsum = ops.knn_kth(x, self.k, self.pad)
+            n, d = x.shape
         return (-(knn_entropy_constant(n, d, self.k) + (d / n) * logsum)).to(torch.float32)
+
+    def _sharded_logsum(self, x: torch.Tensor):
+        red = self.reducer
+        if not isinstance(x, torch.Tensor) or x.dim() != 2:
+            raise ValueError("KNNEntropyEstimator: x must be a (N, d) tensor")
+        n_local, d = x.shape
+        k = int(self.k)
+        counts = red.shard_counts(n_local, x.device)
+        n = sum(counts)
+        ops.knn_check(n, d, k)
+        ops._check_f32("x", x)
+        row0 = sum(counts[:red.rank])
+        return _ShardedKNNLogsum.apply(x, k, float(self.pad), red, counts, row0), n, d

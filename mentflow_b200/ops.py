@@ -570,36 +570,115 @@ class KNNKth(torch.autograd.Function):
     @staticmethod
     def backward(ctx, _gr, _gidx, glogsum):
         x, r, idx = ctx.saved_tensors
-        n, d = x.shape
-        sorted_idx, perm = torch.sort(idx, stable=True)     # particle i's incoming neighbours, ascending j
-        g = glogsum.to(torch.float64).contiguous()
-        gx = torch.empty_like(x)
-        lib = _lib.load()
-        with torch.cuda.device(x.device):
-            _lib.check(lib.mfb_knn_kth_bwd(_ptr(x), n, d, _ptr(r), _ptr(idx), _ptr(sorted_idx), _ptr(perm), ctx.pad,
-                                           _ptr(g), _ptr(gx), _stream()), "knn_kth_bwd")
-        return gx, None, None
+        return knn_kth_bwd(x, r, idx, glogsum, ctx.pad), None, None
 
 
-def knn_kth(x: torch.Tensor, k: int, pad: float = 1.0e-12):
+def knn_check(n: int, d: int, k: int, what: str = "knn_kth") -> None:
+    """ValueError unless the k-NN kernels take a batch of ``n`` particles in ``d`` dimensions at this ``k``."""
+    if not 1 <= k <= KNN_MAX_K:
+        raise ValueError(f"{what}: k = {k} is outside [1, {KNN_MAX_K}]")
+    if k >= n:
+        raise ValueError(f"{what}: k = {k} needs more than k particles (got N = {n})")
+    if not 1 <= d <= KNN_MAX_DIM:
+        raise ValueError(f"{what}: d = {d} is outside [1, {KNN_MAX_DIM}]")
+    if n >= 2 ** 31:
+        raise ValueError(f"{what}: N = {n} does not fit the int32 neighbour indices")
+
+
+def knn_rows(rows: Optional[slice], n: int, what: str = "knn_kth"):
+    """(row0, nrows) of a row range given as a slice of the batch, ``None`` for the whole batch; ValueError unless it
+    is a contiguous range inside [0, n]."""
+    if rows is None:
+        return 0, n
+    if not isinstance(rows, slice) or rows.step not in (None, 1):
+        raise ValueError(f"{what}: rows must be a slice with step 1 (got {rows!r})")
+    start = 0 if rows.start is None else int(rows.start)
+    stop = n if rows.stop is None else int(rows.stop)
+    if not 0 <= start <= stop <= n:
+        raise ValueError(f"{what}: rows [{start}, {stop}) is not a range inside [0, {n}]")
+    return start, stop - start
+
+
+def knn_kth(x: torch.Tensor, k: int, pad: float = 1.0e-12, rows: Optional[slice] = None):
     """Distance ``r`` (float32, (N,)) from every particle to its k-th nearest other particle, that neighbour's index
     ``idx`` (int32; ties go to the smaller index) and ``logsum`` = sum log(r + pad) (float64 0-dim tensor, the only
     differentiable output).  A particle without k others at a finite distance (NaN or inf coordinates) gets r = inf and
-    idx = its own index, which carries no gradient.  All pairs on the GPU: O(N^2 d)."""
+    idx = its own index, which carries no gradient.  All pairs on the GPU: O(N^2 d).
+
+    ``rows``: a slice of the batch (a rank's ``distributed.shard_slice`` of gathered particles).  Only those rows are
+    searched, against every particle of ``x``; the result is ``(r, idx, None)`` for those rows, bit for bit the rows of
+    the whole-batch call, with idx indexing ``x``.  There is no log sum (it needs every row: ``knn_logsum`` of the
+    concatenated r) and no autograd (``knn_kth_bwd`` gives the gradient of those rows)."""
     if not isinstance(x, torch.Tensor) or x.dim() != 2:
         raise ValueError("knn_kth: x must be a (N, d) tensor")
     n, d = x.shape
     k = int(k)
-    if not 1 <= k <= KNN_MAX_K:
-        raise ValueError(f"knn_kth: k = {k} is outside [1, {KNN_MAX_K}]")
-    if k >= n:
-        raise ValueError(f"knn_kth: k = {k} needs more than k particles (got N = {n})")
+    knn_check(n, d, k)
+    if rows is None:
+        _check_f32("x", x)
+        return KNNKth.apply(x, k, float(pad))
+    row0, nrows = knn_rows(rows, n)
+    x = _check_f32("x", x.detach())
+    r = torch.empty(nrows, dtype=torch.float32, device=x.device)
+    idx = torch.empty(nrows, dtype=torch.int32, device=x.device)
+    lib = _lib.load()
+    with torch.cuda.device(x.device):
+        wbytes = lib.mfb_knn_rows_workspace_bytes(n, nrows, d, k)
+        work = torch.empty(max(wbytes, 16), dtype=torch.uint8, device=x.device)
+        _lib.check(lib.mfb_knn_kth_rows(_ptr(x), n, d, k, row0, nrows, _ptr(r), _ptr(idx), _ptr(work), wbytes,
+                                        _stream()), "knn_kth_rows")
+    return r, idx, None
+
+
+def knn_logsum(r: torch.Tensor, pad: float = 1.0e-12) -> torch.Tensor:
+    """sum log(r + pad) over the k-th neighbour distances ``r`` of a whole batch (float64 0-dim tensor), added in the
+    order ``knn_kth`` adds them: for r gathered from row ranges it is bit for bit ``knn_kth``'s logsum."""
+    if not isinstance(r, torch.Tensor) or r.dim() != 1 or r.numel() < 1:
+        raise ValueError("knn_logsum: r must be a non-empty (N,) tensor")
+    if r.numel() >= 2 ** 31:
+        raise ValueError(f"knn_logsum: N = {r.numel()} does not fit the int32 neighbour indices")
+    r = _check_f32("r", r.detach())
+    n = r.numel()
+    logsum = torch.empty((), dtype=torch.float64, device=r.device)
+    wbytes = 8 * (-(-n // 256))
+    work = torch.empty(wbytes, dtype=torch.uint8, device=r.device)
+    lib = _lib.load()
+    with torch.cuda.device(r.device):
+        _lib.check(lib.mfb_knn_logsum(_ptr(r), n, float(pad), _ptr(logsum), _ptr(work), wbytes, _stream()),
+                   "knn_logsum")
+    return logsum
+
+
+def knn_kth_bwd(x: torch.Tensor, r: torch.Tensor, idx: torch.Tensor, glogsum: torch.Tensor, pad: float = 1.0e-12,
+                rows: Optional[slice] = None) -> torch.Tensor:
+    """glogsum * d logsum / dx for the rows ``rows`` of the batch (all rows for None), the neighbours held fixed:
+    bit for bit those rows of ``knn_kth``'s gradient.  ``x``, ``r`` and ``idx`` are the whole batch's (the gathered
+    particles and the concatenated results of the row ranges); ``glogsum`` is a float64 scalar tensor."""
+    if not isinstance(x, torch.Tensor) or x.dim() != 2:
+        raise ValueError("knn_kth_bwd: x must be a (N, d) tensor")
+    n, d = x.shape
     if not 1 <= d <= KNN_MAX_DIM:
-        raise ValueError(f"knn_kth: d = {d} is outside [1, {KNN_MAX_DIM}]")
-    if n >= 2 ** 31:
-        raise ValueError(f"knn_kth: N = {n} does not fit the int32 neighbour indices")
-    _check_f32("x", x)
-    return KNNKth.apply(x, k, float(pad))
+        raise ValueError(f"knn_kth_bwd: d = {d} is outside [1, {KNN_MAX_DIM}]")
+    if not 2 <= n < 2 ** 31:
+        raise ValueError(f"knn_kth_bwd: N = {n} is outside [2, 2^31)")
+    if r.shape != (n,) or idx.shape != (n,) or idx.dtype != torch.int32:
+        raise ValueError("knn_kth_bwd: r (float32) and idx (int32) must hold one entry per particle of x")
+    if r.device != x.device or idx.device != x.device:
+        raise ValueError(f"knn_kth_bwd: x, r and idx must be on one device (got {x.device}, {r.device}, {idx.device})")
+    row0, nrows = knn_rows(rows, n, "knn_kth_bwd")
+    x = _check_f32("x", x.detach())
+    gx = torch.empty((nrows, d), dtype=torch.float32, device=x.device)
+    if nrows == 0:
+        return gx
+    r = _check_f32("r", r.detach())
+    idx = idx.contiguous()
+    sorted_idx, perm = torch.sort(idx, stable=True)     # particle i's incoming neighbours, ascending j
+    g = glogsum.detach().to(device=x.device, dtype=torch.float64).reshape(()).contiguous()
+    lib = _lib.load()
+    with torch.cuda.device(x.device):
+        _lib.check(lib.mfb_knn_kth_bwd_rows(_ptr(x), n, d, _ptr(r), _ptr(idx), _ptr(sorted_idx), _ptr(perm), row0,
+                                            nrows, float(pad), _ptr(g), _ptr(gx), _stream()), "knn_kth_bwd_rows")
+    return gx
 
 
 # --------------------------------------------------------------------------------------
