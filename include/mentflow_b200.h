@@ -389,6 +389,41 @@ int mfb_cdf_build(const float* rho, int64_t g, double pad, double* cdf, void* wo
 int mfb_cdf_sample(const double* cdf, int64_t g, const void* workspace, int d,
                    const int32_t* shape_host, const float* first_edge_host, const float* cell_host,
                    int jitter, uint64_t seed, uint64_t offset, int64_t size, float* out, void* stream);
+/* ---- Metropolis-Hastings chains over rho (MetropolisHastingsSampler) ------------------------
+ * Random-walk Metropolis chains, one per GPU thread, with no sampling grid: the cost is chains x steps density
+ * evaluations whatever the dimension or resolution.  Chain c (a global 64-bit index) runs steps t = 0, 1, ...:
+ *   t = 0   x_0 = start (DEVICE array [d]) if given, else start_scale * xi_0;
+ *   t >= 1  x' = x_{t-1} + L xi_t, (L xi)_i an fp32 fmaf chain from 0 over j = 0 .. i ascending, then added to x_i;
+ *           draw u_t in (0, 1]; x_t = x' iff rho(x') is finite and rho(x') >= u_t * rho(x_{t-1}) (fp32 product),
+ *           else x_t = x_{t-1}.  A chain at zero density takes every finite proposal; a zero, NaN or inf proposal is
+ *           never taken from a point of positive density.
+ * L = chol[d][d], row-major, lower triangular: the Cholesky factor of the proposal covariance.
+ * Recorded states: x_{burnin + r thin}, r = 0 .. steps - 1 (burnin = 0: the first is the start).  Chain chain0 + i
+ * writes them to out rows i * steps + r, out[nchains * steps][d] row-major.
+ * Randomness (a chain is a pure function of seed, c, start and the model): Philox4x32-10 with
+ *   counter = (c mod 2^32, c div 2^32, t, b), key = (seed mod 2^32, seed div 2^32),
+ * blocks b = 0 .. ceil((2 ceil(d/2) + 1) / 4) - 1 giving words w[4b + q] = output word q of block b.  Pair j <
+ * ceil(d/2) is Box-Muller on (w[2j], w[2j+1]): u1 = ((w[2j] >> 8) + 1) 2^-24 in (0, 1], u2 = (w[2j+1] >> 8) 2^-24,
+ * r = sqrtf(-2 logf(u1)), xi[2j] = r cos(2 pi u2), xi[2j+1] = r sin(2 pi u2) (sincospif; dropped for odd d at the
+ * last pair).  u_t = ((w[2 ceil(d/2)] >> 8) + 1) 2^-24.  t is the counter's third word: a run needs
+ * burnin + (steps - 1) thin < 2^32.
+ * The density is mfb_ment_prob's (same tables, mp / mp2 and prior arguments), bit for bit.  accepted (device int64)
+ * is ADDED the number of proposals taken.  Arguments are checked before any launch (MFB_E_BADARG): d outside 1..8,
+ * burnin < 0, steps < 1, thin < 1, a run past 2^32 steps, chain0 + nchains past 2^64, a NULL required pointer, or a
+ * non-finite start_scale without start.  nchains = 0 launches nothing.                                     */
+int mfb_ment_mh(int d, const float* proj, const float* coords, const float* tables, int k, int b, const float* mp,
+                const float* proj2, const float* cx2, const float* cy2, const float* tables2, int k2, int bx, int by,
+                const float* mp2, float prior_neg_half_inv_s2, float prior_log_norm, uint64_t chain0,
+                int64_t nchains, const float* start, float start_scale, const float* chol, int64_t burnin,
+                int64_t steps, int64_t thin, uint64_t seed, float* out, int64_t* accepted, void* stream);
+/* The same chains one step at a time around a density the library cannot see (same words, arithmetic and rule).
+ * mfb_mh_propose: t = 0 writes the start draws x_0 of chains chain0 .. chain0 + n - 1 to xp[n][d] (x and chol may be
+ * NULL); t >= 1 writes the proposals from the current states x[n][d].  mfb_mh_accept (t >= 1): where the rule takes
+ * xp (rho_prop[n] its density), x and rho[n] become xp and rho_prop; accepted is added the count.                 */
+int mfb_mh_propose(const float* x, int64_t n, int d, uint64_t chain0, const float* start, float start_scale,
+                   const float* chol, int64_t t, uint64_t seed, float* xp, void* stream);
+int mfb_mh_accept(float* x, float* rho, const float* xp, const float* rho_prop, int64_t n, int d, uint64_t chain0,
+                  int64_t t, uint64_t seed, int64_t* accepted, void* stream);
 /* ment.py:360-367: pred[pred<thresh]=0; where meas!=0 and pred!=0: h *= 1 + lr*(meas/pred-1) */
 int mfb_gs_update(float* table, const float* meas, const float* pred, int n, float lr, float thresh,
                   void* stream);

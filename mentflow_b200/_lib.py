@@ -60,6 +60,10 @@ SIGNATURES = {
     "mfb_cdf_workspace_bytes": (c_int64, [c_int64]),
     "mfb_cdf_build": (c_int, [P, c_int64, c_double, P, P, c_int64, P]),
     "mfb_cdf_sample": (c_int, [P, c_int64, P, c_int, P, P, P, c_int, c_uint64, c_uint64, c_int64, P, P]),
+    "mfb_ment_mh": (c_int, [c_int, P, P, P, c_int, c_int, P, P, P, P, P, c_int, c_int, c_int, P, c_float, c_float,
+                            c_uint64, c_int64, P, c_float, P, c_int64, c_int64, c_int64, c_uint64, P, P, P]),
+    "mfb_mh_propose": (c_int, [P, c_int64, c_int, c_uint64, P, c_float, P, c_int64, c_uint64, P, P]),
+    "mfb_mh_accept": (c_int, [P, P, P, P, c_int64, c_int, c_uint64, c_int64, c_uint64, P, P]),
     "mfb_gs_update": (c_int, [P, P, P, c_int, c_float, c_float, P]),
     "mfb_selftest_umma": (c_int, [P, P, c_int, P, P, P]),
     "mfb_selftest_umma_ts": (c_int, [P, P, c_int, P, P, P]),

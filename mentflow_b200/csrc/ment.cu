@@ -461,8 +461,8 @@ scan_apply_kernel(const float* __restrict__ rho, int64_t G, double pad, const do
 struct Philox {
   uint32_t c[4];
 };
-__device__ __forceinline__ Philox philox4x32(uint64_t counter, uint32_t stream, uint64_t seed) {
-  uint32_t c0 = (uint32_t)counter, c1 = (uint32_t)(counter >> 32), c2 = stream, c3 = 0u;
+__device__ __forceinline__ Philox philox4x32(uint64_t counter, uint32_t stream, uint64_t seed, uint32_t word3 = 0u) {
+  uint32_t c0 = (uint32_t)counter, c1 = (uint32_t)(counter >> 32), c2 = stream, c3 = word3;
   uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
 #pragma unroll
   for (int r = 0; r < 10; ++r) {
@@ -590,6 +590,214 @@ cdf_sample_kernel(const double* __restrict__ cdf, int64_t G, const double* __res
   }
 }
 
+// ---- Metropolis-Hastings chains (MetropolisHastingsSampler) ---------------------------------------------
+// Chain c (global index), step t: the Philox blocks philox4x32(c, t, seed, b), b = 0 .. kMhBlocks - 1, give the words
+// w[4b + q].  Pair j (< ceil(D/2)) is Box-Muller on (w[2j], w[2j+1]): r = sqrt(-2 log u1), u1 in (0, 1], angle
+// 2 pi u2, u2 in [0, 1); xi[2j] = r cos, xi[2j+1] = r sin (dropped for odd D at the last pair).  The next word,
+// w[2 ceil(D/2)], is the acceptance uniform in (0, 1].  t = 0 is the start draw (its uniform is unused).
+template <int D>
+__host__ __device__ constexpr int mh_blocks() { return (2 * ((D + 1) / 2) + 1 + 3) / 4; }
+
+__device__ __forceinline__ float u01_open(uint32_t r) { return (float)((r >> 8) + 1u) * (1.0f / 16777216.0f); }  // (0,1]
+
+// Box-Muller on one pair of words
+__device__ __forceinline__ void mh_normals(uint32_t w0, uint32_t w1, float& a0, float& a1) {
+  const float r = sqrtf(-2.0f * logf(u01_open(w0)));
+  float s, co;
+  sincospif(2.0f * u01(w1), &s, &co);
+  a0 = r * co;
+  a1 = r * s;
+}
+
+// x_0: the start point, or start_scale * xi of step 0
+template <int D>
+__device__ __forceinline__ void mh_start(uint64_t c, uint64_t seed, const float* __restrict__ start, float start_scale,
+                                         float (&x)[D]) {
+  if (start) {
+#pragma unroll
+    for (int i = 0; i < D; ++i) x[i] = start[i];
+    return;
+  }
+#pragma unroll
+  for (int b = 0; b < mh_blocks<D>(); ++b) {
+    const Philox p = philox4x32(c, 0u, seed, (uint32_t)b);
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      const int j = 2 * b + h;                       // pair j: xi[2j], xi[2j+1]
+      if (2 * j < D) {
+        float a0, a1;
+        mh_normals(p.c[2 * h], p.c[2 * h + 1], a0, a1);
+        x[2 * j] = start_scale * a0;
+        if (2 * j + 1 < D) x[2 * j + 1] = start_scale * a1;
+      }
+    }
+  }
+}
+
+// proposal of step t >= 1: xp_i = x_i + (L xi)_i, (L xi)_i = fmaf chain from 0 over j = 0 .. i ascending
+// (L lower triangular, row-major [D][D]); returns the acceptance uniform.  The pairs are consumed as they are drawn:
+// pair j adds columns 2j, 2j+1 to every row, which keeps each row's chain in ascending order without holding xi.
+template <int D>
+__device__ __forceinline__ float mh_propose(uint64_t c, uint32_t t, uint64_t seed, const float* __restrict__ chol,
+                                            const float (&x)[D], float (&xp)[D]) {
+  constexpr int kPairs = (D + 1) / 2;
+#pragma unroll
+  for (int i = 0; i < D; ++i) xp[i] = 0.f;
+  float u = 0.f;
+#pragma unroll
+  for (int b = 0; b < mh_blocks<D>(); ++b) {
+    const Philox p = philox4x32(c, t, seed, (uint32_t)b);
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      const int j = 2 * b + h;
+      if (j < kPairs) {
+        float a0, a1;
+        mh_normals(p.c[2 * h], p.c[2 * h + 1], a0, a1);
+#pragma unroll
+        for (int i = 2 * j; i < D; ++i) {
+          xp[i] = fmaf(chol[i * D + 2 * j], a0, xp[i]);
+          if (2 * j + 1 <= i) xp[i] = fmaf(chol[i * D + 2 * j + 1], a1, xp[i]);
+        }
+      } else if (j == kPairs) {
+        u = u01_open(p.c[2 * h]);
+      }
+    }
+  }
+#pragma unroll
+  for (int i = 0; i < D; ++i) xp[i] = x[i] + xp[i];
+  return u;
+}
+
+// the acceptance uniform of step t alone
+template <int D>
+__device__ __forceinline__ float mh_uniform(uint64_t c, uint32_t t, uint64_t seed) {
+  constexpr int kWord = 2 * ((D + 1) / 2);
+  return u01_open(philox4x32(c, t, seed, (uint32_t)(kWord / 4)).c[kWord % 4]);
+}
+
+// the acceptance rule: a chain at zero density takes every finite proposal, a chain at positive density never takes a
+// zero-density one, a NaN or inf proposal is never taken
+__device__ __forceinline__ bool mh_accept(float rho_prop, float u, float rho) {
+  return isfinite(rho_prop) && rho_prop >= u * rho;
+}
+
+struct MhChains {
+  uint64_t chain0;          // global index of the first chain
+  int64_t n;                // chains
+  const float* start;       // [D] or NULL
+  float start_scale;
+  const float* chol;        // [D][D] lower Cholesky factor of the proposal covariance
+  int64_t burnin, steps, thin;
+  uint64_t seed;
+};
+
+// one thread per chain: x and rho(x) stay in registers, rho is ment_prob_kernel's arithmetic; only the recorded
+// states x_{burnin + r thin}, r < steps, are written, chain i's at rows i * steps + r of out
+// Minimum resident CTAs of the chain kernel: 3 (<= 80 registers) up to D = 7, 2 at D = 8, with and without kicks.  The
+// chain state x, the proposal and the Philox words sit beside the density's registers: at the density kernels'
+// minimum (5 with kicks) ptxas spills from D = 1 on, and with no minimum it picks 64 - 80 registers and spills in
+// some dimensions.
+template <int D>
+constexpr int mh_min_ctas() { return D < 8 ? 3 : 2; }
+template <int D, bool kMP>
+__global__ void __launch_bounds__(kMentThreads, mh_min_ctas<D>())
+ment_mh_kernel(const float* __restrict__ proj, const float* __restrict__ coords, const float* __restrict__ tables,
+               int K, int B, MentPrior prior, const Tables2D t2, const float* __restrict__ mp,
+               const float* __restrict__ mp2, const MhChains ch, float* __restrict__ out,
+               unsigned long long* __restrict__ accepted) {
+  extern __shared__ __align__(16) float sm[];
+  __shared__ float s_chol[D * D];
+  float* s_proj = sm;
+  float* s_c = s_proj + (((size_t)K * D + 3) & ~(size_t)3);
+  float* s_h = s_c + (size_t)K * B;
+  float* s_inv = s_h + (size_t)K * B;
+  double* s_dinv = reinterpret_cast<double*>(s_inv + ((K + 1) & ~1));
+  load_tables(s_proj, s_c, s_h, s_inv, s_dinv, proj, coords, tables, K, B, D);
+  float* s_mp = nullptr;
+  if constexpr (kMP) {
+    s_mp = mp_smem(s_dinv, K, B);
+    for (int i = threadIdx.x; i < K * MFB_MP_STRIDE(D); i += blockDim.x) s_mp[i] = mp[i];
+  }
+  for (int i = threadIdx.x; i < D * D; i += blockDim.x) s_chol[i] = ch.chol[i];
+  __syncthreads();
+  const int64_t total = ch.burnin + (ch.steps - 1) * ch.thin;
+  unsigned long long acc = 0;
+  for (int64_t i = (int64_t)blockIdx.x * kMentThreads + threadIdx.x; i < ch.n; i += (int64_t)gridDim.x * kMentThreads) {
+    const uint64_t c = ch.chain0 + (uint64_t)i;
+    float x[D];
+    mh_start<D>(c, ch.seed, ch.start, ch.start_scale, x);
+    float rho = ment_density<D, kMP>(x, s_proj, s_c, s_h, s_inv, s_dinv, K, B, prior, s_mp);
+    if (t2.k > 0) rho *= tables2d_product<D, kMP>(x, t2, mp2);
+    float* row = out + i * ch.steps * D;
+    int64_t next = ch.burnin;         // next step to record
+    for (int64_t t = 0;; ++t) {
+      if (t > 0) {
+        float xp[D];
+        const float u = mh_propose<D>(c, (uint32_t)t, ch.seed, s_chol, x, xp);
+        float rp = ment_density<D, kMP>(xp, s_proj, s_c, s_h, s_inv, s_dinv, K, B, prior, s_mp);
+        if (t2.k > 0) rp *= tables2d_product<D, kMP>(xp, t2, mp2);
+        if (mh_accept(rp, u, rho)) {
+#pragma unroll
+          for (int j = 0; j < D; ++j) x[j] = xp[j];
+          rho = rp;
+          ++acc;
+        }
+      }
+      if (t == next) {
+#pragma unroll
+        for (int j = 0; j < D; ++j) row[j] = x[j];
+        row += D;
+        next += ch.thin;
+      }
+      if (t == total) break;
+    }
+  }
+  acc = warp_sum_u64(acc);
+  if ((threadIdx.x & 31) == 0 && acc) atomicAdd(accepted, acc);
+}
+
+// the same steps one at a time around a density the library cannot see: t = 0 writes the start draws, t >= 1 the
+// proposals from the current states x
+template <int D>
+__global__ void __launch_bounds__(kMentThreads)
+mh_propose_kernel(const float* __restrict__ x, int64_t n, uint64_t chain0, const float* __restrict__ start,
+                  float start_scale, const float* __restrict__ chol, uint32_t t, uint64_t seed, float* __restrict__ xp) {
+  for (int64_t i = (int64_t)blockIdx.x * kMentThreads + threadIdx.x; i < n; i += (int64_t)gridDim.x * kMentThreads) {
+    const uint64_t c = chain0 + (uint64_t)i;
+    float y[D];
+    if (t == 0) {
+      mh_start<D>(c, seed, start, start_scale, y);
+    } else {
+      float xr[D];
+#pragma unroll
+      for (int j = 0; j < D; ++j) xr[j] = x[i * D + j];
+      mh_propose<D>(c, t, seed, chol, xr, y);
+    }
+#pragma unroll
+    for (int j = 0; j < D; ++j) xp[i * D + j] = y[j];
+  }
+}
+
+template <int D>
+__global__ void __launch_bounds__(kMentThreads)
+mh_accept_kernel(float* __restrict__ x, float* __restrict__ rho, const float* __restrict__ xp,
+                 const float* __restrict__ rho_prop, int64_t n, uint64_t chain0, uint32_t t, uint64_t seed,
+                 unsigned long long* __restrict__ accepted) {
+  unsigned long long acc = 0;
+  for (int64_t i = (int64_t)blockIdx.x * kMentThreads + threadIdx.x; i < n; i += (int64_t)gridDim.x * kMentThreads) {
+    const float u = mh_uniform<D>(chain0 + (uint64_t)i, t, seed);
+    const float rp = rho_prop[i];
+    if (mh_accept(rp, u, rho[i])) {
+#pragma unroll
+      for (int j = 0; j < D; ++j) x[i * D + j] = xp[i * D + j];
+      rho[i] = rp;
+      ++acc;
+    }
+  }
+  acc = warp_sum_u64(acc);
+  if ((threadIdx.x & 31) == 0 && acc) atomicAdd(accepted, acc);
+}
+
 // Gauss-Seidel update of one table (ment.py:360-367)
 __global__ void gs_update_kernel(float* __restrict__ table, const float* __restrict__ meas,
                                  const float* __restrict__ pred, int n, float lr, float thresh) {
@@ -657,6 +865,29 @@ static int launch_integrate(bool kick, const float* mc, int nb, int ax, const fl
   kernel<<<pixels, kMentThreads, smem, st>>>(mc, nb, ax, mc2, nb2, ax2, grid, minv, proj, coords, tables, k, b, pr, t2,
                                              pred, mp, mp2, imp);
   return launch_status();
+}
+
+// one CTA per 256 chains, no grid-stride cap: a chain is a whole run, and the block scheduler evens out chains of
+// different cost better than a thread walking several of them
+static int mh_grid(int64_t n) { return (int)((n + kMentThreads - 1) / kMentThreads); }
+
+template <int D>
+static int launch_mh(bool kick, const float* proj, const float* coords, const float* tables, int K, int B,
+                     const float* mp, const Tables2D& t2, const float* mp2, MentPrior prior, const MhChains& ch,
+                     float* out, int64_t* accepted, cudaStream_t st) {
+  const size_t smem = kick ? ment_smem_mp(K, B, D) : ment_smem(K, B, D);
+  if (smem > 200 * 1024) return MFB_E_UNSUPPORTED;
+  const auto kernel = kick ? ment_mh_kernel<D, true> : ment_mh_kernel<D, false>;
+  MFB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kernel<<<mh_grid(ch.n), kMentThreads, smem, st>>>(proj, coords, tables, K, B, prior, t2, mp, mp2, ch, out,
+                                                    reinterpret_cast<unsigned long long*>(accepted));
+  return launch_status();
+}
+
+// the last step of a run must fit the 32-bit stream word: burnin + (steps - 1) thin < 2^32
+static bool mh_steps_ok(int64_t burnin, int64_t steps, int64_t thin) {
+  if (burnin < 0 || steps < 1 || thin < 1 || burnin > (int64_t)UINT32_MAX) return false;
+  return steps - 1 <= ((int64_t)UINT32_MAX - burnin) / thin;
 }
 
 }  // namespace mfb
@@ -813,6 +1044,83 @@ int mfb_cdf_sample(const double* cdf, int64_t g, const void* workspace, int d, c
     default: MFB_SAMPLE(8); break;
   }
 #undef MFB_SAMPLE
+  return launch_status();
+}
+
+int mfb_ment_mh(int d, const float* proj, const float* coords, const float* tables, int k, int b, const float* mp,
+                const float* proj2, const float* cx2, const float* cy2, const float* tables2, int k2, int bx, int by,
+                const float* mp2, float prior_neg_half_inv_s2, float prior_log_norm, uint64_t chain0, int64_t nchains,
+                const float* start, float start_scale, const float* chol, int64_t burnin, int64_t steps, int64_t thin,
+                uint64_t seed, float* out, int64_t* accepted, void* stream) {
+  const bool kick = mp || mp2;
+  MFB_CHECK_ARG(out && chol && accepted && d >= 1 && d <= kMaxDim && nchains >= 0 && mh_steps_ok(burnin, steps, thin));
+  MFB_CHECK_ARG(start || isfinite(start_scale));
+  MFB_CHECK_ARG((uint64_t)nchains <= UINT64_MAX - chain0 && nchains <= INT64_MAX / (steps * d) &&
+                nchains <= (int64_t)INT32_MAX * kMentThreads);
+  const Tables2D t2{k2, bx, by, proj2, cx2, cy2, tables2};
+  MFB_CHECK_ARG(tables_ok(k, b, proj, coords, tables, mp, t2, mp2, kick));
+  if (nchains == 0) return 0;
+  if (k == 0) b = 2;
+  const MentPrior pr{prior_neg_half_inv_s2, prior_log_norm};
+  const MhChains ch{chain0, nchains, start, start_scale, chol, burnin, steps, thin, seed};
+  cudaStream_t st = (cudaStream_t)stream;
+#define MFB_CALL(DD) launch_mh<DD>(kick, proj, coords, tables, k, b, mp, t2, mp2, pr, ch, out, accepted, st)
+  switch (d) {
+    case 1: return MFB_CALL(1);
+    case 2: return MFB_CALL(2);
+    case 3: return MFB_CALL(3);
+    case 4: return MFB_CALL(4);
+    case 5: return MFB_CALL(5);
+    case 6: return MFB_CALL(6);
+    case 7: return MFB_CALL(7);
+    default: return MFB_CALL(8);
+  }
+#undef MFB_CALL
+}
+
+int mfb_mh_propose(const float* x, int64_t n, int d, uint64_t chain0, const float* start, float start_scale,
+                   const float* chol, int64_t t, uint64_t seed, float* xp, void* stream) {
+  MFB_CHECK_ARG(xp && n >= 0 && d >= 1 && d <= kMaxDim && t >= 0 && t <= (int64_t)UINT32_MAX);
+  MFB_CHECK_ARG(t == 0 ? (start || isfinite(start_scale)) : (x && chol));
+  MFB_CHECK_ARG((uint64_t)n <= UINT64_MAX - chain0);
+  if (n == 0) return 0;
+  cudaStream_t st = (cudaStream_t)stream;
+#define MFB_CALL(DD) \
+  mh_propose_kernel<DD><<<mh_grid(n), kMentThreads, 0, st>>>(x, n, chain0, start, start_scale, chol, (uint32_t)t, seed, xp)
+  switch (d) {
+    case 1: MFB_CALL(1); break;
+    case 2: MFB_CALL(2); break;
+    case 3: MFB_CALL(3); break;
+    case 4: MFB_CALL(4); break;
+    case 5: MFB_CALL(5); break;
+    case 6: MFB_CALL(6); break;
+    case 7: MFB_CALL(7); break;
+    default: MFB_CALL(8); break;
+  }
+#undef MFB_CALL
+  return launch_status();
+}
+
+int mfb_mh_accept(float* x, float* rho, const float* xp, const float* rho_prop, int64_t n, int d, uint64_t chain0,
+                  int64_t t, uint64_t seed, int64_t* accepted, void* stream) {
+  MFB_CHECK_ARG(x && rho && xp && rho_prop && accepted && n >= 0 && d >= 1 && d <= kMaxDim);
+  MFB_CHECK_ARG(t >= 1 && t <= (int64_t)UINT32_MAX && (uint64_t)n <= UINT64_MAX - chain0);
+  if (n == 0) return 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  unsigned long long* acc = reinterpret_cast<unsigned long long*>(accepted);
+#define MFB_CALL(DD) \
+  mh_accept_kernel<DD><<<mh_grid(n), kMentThreads, 0, st>>>(x, rho, xp, rho_prop, n, chain0, (uint32_t)t, seed, acc)
+  switch (d) {
+    case 1: MFB_CALL(1); break;
+    case 2: MFB_CALL(2); break;
+    case 3: MFB_CALL(3); break;
+    case 4: MFB_CALL(4); break;
+    case 5: MFB_CALL(5); break;
+    case 6: MFB_CALL(6); break;
+    case 7: MFB_CALL(7); break;
+    default: MFB_CALL(8); break;
+  }
+#undef MFB_CALL
   return launch_status();
 }
 

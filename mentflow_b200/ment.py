@@ -254,6 +254,16 @@ class MENT:
         return ops.ment_prob_grid(list(sampler.shape), sampler.first_centres(), sampler.cell_sizes(), g1, g2, a, b,
                                   device)
 
+    def mh_chains(self, sampler, chain0: int, nchains: int, seed: int):
+        """Metropolis-Hastings chains chain0 .. chain0 + nchains - 1 of a MetropolisHastingsSampler over rho, in one
+        fused kernel: (recorded states (nchains * steps, D), proposals taken (1,) int64)."""
+        device = torch.device(self.device if self.device is not None else "cuda")
+        g1, g2 = self._groups(device)
+        a, b = self._prior_args()
+        chol, start = sampler.chain_args(device)
+        return ops.ment_mh(g1, g2, a, b, self.ndim, chain0, nchains, chol, sampler.burnin, sampler.steps, sampler.thin,
+                           seed, start=start, start_scale=sampler.start_scale)
+
     def log_prob(self, x: torch.Tensor, pad: float = 1.0e-12) -> torch.Tensor:
         return torch.log(self.prob(x) + pad)
 

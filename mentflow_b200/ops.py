@@ -1167,6 +1167,82 @@ def cdf_sample(rho: torch.Tensor, shape, first_edge, cell, size: int, seed: int,
     return out
 
 
+def _cuda_device(device, what: str) -> torch.device:
+    device = torch.device(device)
+    if device.type != "cuda":
+        raise RuntimeError(f"{what}: mentflow_b200 kernels need a CUDA device (got {device}); there is no CPU fallback")
+    return device
+
+
+def _mh_start(start, d: int):
+    if start is None:
+        return None
+    start = _check_f32("start", start)
+    if tuple(start.shape) != (d,):
+        raise ValueError(f"start must have shape ({d},), got {tuple(start.shape)}")
+    return start
+
+
+def ment_mh(g1, g2, neg_half_inv_s2: float, log_norm: float, d: int, chain0: int, nchains: int, chol: torch.Tensor,
+            burnin: int, steps: int, thin: int, seed: int, start: Optional[torch.Tensor] = None,
+            start_scale: float = 1.0):
+    """Metropolis-Hastings chains chain0 .. chain0 + nchains - 1 over the MENT density of ``ment_prob`` in one fused
+    kernel (the sampling rule and the Philox layout: ``mfb_ment_mh`` in the header).  ``chol`` (D, D): lower Cholesky
+    factor of the proposal covariance.  Returns the recorded states (nchains * steps, D), chain-major, and the number
+    of proposals taken as a (1,) int64 device tensor."""
+    chol = _check_f32("chol", chol)
+    device = _cuda_device(chol.device, "ment_mh")
+    if tuple(chol.shape) != (d, d):
+        raise ValueError(f"chol must have shape ({d}, {d}), got {tuple(chol.shape)}")
+    start = _mh_start(start, d)
+    lib = _lib.load()
+    args, keep, _ = _ment_tables(g1, g2, d, device)
+    out = torch.empty((int(nchains) * int(steps), d), dtype=torch.float32, device=device)
+    accepted = torch.zeros(1, dtype=torch.int64, device=device)
+    with torch.cuda.device(device):
+        _lib.check(lib.mfb_ment_mh(d, *args, float(neg_half_inv_s2), float(log_norm), int(chain0), int(nchains),
+                                   _ptr(start), float(start_scale), _ptr(chol), int(burnin), int(steps), int(thin),
+                                   int(seed) & (2 ** 64 - 1), _ptr(out), _ptr(accepted), _stream()), "ment_mh")
+    return out, accepted
+
+
+def mh_propose(x: Optional[torch.Tensor], n: int, d: int, chain0: int, chol: Optional[torch.Tensor], t: int, seed: int,
+               device, start: Optional[torch.Tensor] = None, start_scale: float = 1.0) -> torch.Tensor:
+    """Step t of n chains: t = 0 the start draws (x and chol unused), t >= 1 the proposals from the states x (n, D)."""
+    device = _cuda_device(device, "mh_propose")
+    if t > 0:
+        x, chol = _check_f32("x", x), _check_f32("chol", chol)
+        if tuple(x.shape) != (n, d) or tuple(chol.shape) != (d, d):
+            raise ValueError(f"mh_propose: x ({n}, {d}) and chol ({d}, {d}) expected")
+    start = _mh_start(start, d)
+    lib = _lib.load()
+    xp = torch.empty((n, d), dtype=torch.float32, device=device)
+    with torch.cuda.device(device):
+        _lib.check(lib.mfb_mh_propose(_ptr(x) if t > 0 else None, n, d, int(chain0), _ptr(start), float(start_scale),
+                                      _ptr(chol) if t > 0 else None, int(t), int(seed) & (2 ** 64 - 1), _ptr(xp),
+                                      _stream()), "mh_propose")
+    return xp
+
+
+def mh_accept(x: torch.Tensor, rho: torch.Tensor, xp: torch.Tensor, rho_prop: torch.Tensor, chain0: int, t: int,
+              seed: int, accepted: torch.Tensor) -> None:
+    """In place: where the rule takes the proposal of step t, x <- xp and rho <- rho_prop; accepted (1,) int64 += the
+    count.  x and rho must be contiguous CUDA float32 tensors (they are written)."""
+    n, d = x.shape
+    for name, t_ in (("x", x), ("rho", rho)):
+        if not (t_.is_cuda and t_.is_contiguous() and t_.dtype == torch.float32):
+            raise RuntimeError(f"mh_accept: {name} must be a contiguous CUDA float32 tensor (no CPU fallback)")
+    xp, rho_prop = _check_f32("xp", xp), _check_f32("rho_prop", rho_prop.reshape(-1))
+    if tuple(xp.shape) != (n, d) or rho.numel() != n or rho_prop.numel() != n:
+        raise ValueError(f"mh_accept: x, xp ({n}, {d}) and rho, rho_prop ({n},) expected")
+    if not (accepted.is_cuda and accepted.dtype == torch.int64):
+        raise RuntimeError("mh_accept: accepted must be a CUDA int64 tensor (no CPU fallback)")
+    lib = _lib.load()
+    with torch.cuda.device(x.device):
+        _lib.check(lib.mfb_mh_accept(_ptr(x), _ptr(rho), _ptr(xp), _ptr(rho_prop), n, d, int(chain0), int(t),
+                                     int(seed) & (2 ** 64 - 1), _ptr(accepted), _stream()), "mh_accept")
+
+
 def gs_update(table: torch.Tensor, meas: torch.Tensor, pred: torch.Tensor, lr: float, thresh: float) -> None:
     """In-place Gauss-Seidel update of one Lagrange table."""
     lib = _lib.load()
