@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define MFB_ABI_VERSION 5
+#define MFB_ABI_VERSION 6
 
 #define MFB_E_BADARG (-1)      /* null pointer / non-positive size / unsupported shape   */
 #define MFB_E_UNSUPPORTED (-2) /* combination not compiled (e.g. D > 8, hidden != 64)    */
@@ -255,42 +255,35 @@ int mfb_f64_split(const double* in, int n, float* out_hi_lo, void* stream);
 int mfb_f64_join(const float* in_hi_lo, int n, double* out, void* stream);
 
 /* ---- k-nearest-neighbour entropy (KNNEntropyEstimator) ----------------------------------------
- * x[n][d], 1 <= d <= 8, 1 <= k <= 16, k < n < 2^31.  r[i] = distance from x_i to its k-th nearest OTHER particle
- * (self excluded by index, so a duplicate is a neighbour at distance 0), idx[i] = that particle's index, neighbours
- * ordered by (r^2, j): ties go to the smaller index.  A particle without k others at a finite distance (NaN or inf
- * coordinates, r^2 overflowing) gets r[i] = inf, idx[i] = i.  logsum[0] = sum_i log(r_i + pad) in double.  All
- * pairs in fp32 direct differences; deterministic (no floating-point atomics).  d > 8 or k > 16: MFB_E_UNSUPPORTED. */
-int64_t mfb_knn_workspace_bytes(int64_t n, int d, int k);
-int mfb_knn_kth(const float* x, int64_t n, int d, int k, double pad, float* r, int32_t* idx, double* logsum,
-                void* workspace, int64_t workspace_bytes, void* stream);
-/* gx[n][d] = glogsum[0] * d logsum / dx with the neighbours held fixed:
- *   w_i (x_i - x_idx[i]) + sum over j with idx[j] = i, ascending j, of w_j (x_i - x_j),  w_j = 1 / (r_j (r_j + pad)),
- * 0 where r_j = 0.  sorted_idx[n] = idx stably sorted, perm[n] (int64) the positions it came from.            */
-int mfb_knn_kth_bwd(const float* x, int64_t n, int d, const float* r, const int32_t* idx,
-                    const int32_t* sorted_idx, const int64_t* perm, double pad, const double* glogsum,
-                    float* gx, void* stream);
-/* Row ranges, for particles sharded over ranks.  x[n][d] is the whole batch (every rank's particles in rank order);
- * a rank searches and differentiates only its rows [row0, row0 + nrows), 0 <= row0 <= row0 + nrows <= n.  The
- * results are bit for bit the rows of mfb_knn_kth / mfb_knn_kth_bwd on the whole batch, whatever the range.
- * Arguments are checked before any launch: a range outside [0, n], k >= n, n >= 2^31 or a NULL pointer return
- * MFB_E_BADARG, d > 8 or k > 16 MFB_E_UNSUPPORTED.  nrows = 0 launches nothing and returns 0 (the outputs r, idx
- * of mfb_knn_kth_rows, gx of mfb_knn_kth_bwd_rows and the workspace may then be NULL).
- *   mfb_knn_kth_rows: r[nrows], idx[nrows] of the queries row0 + q (idx indexes the whole batch; a query without k
- *     others at a finite distance gets r = inf and its own index row0 + q).  No log sum: it needs every rank's r.
- *     Workspace: mfb_knn_rows_workspace_bytes(n, nrows, d, k) (0 for nrows = 0 or bad arguments).
+ * x[n][d] is the whole batch (for particles sharded over ranks, every rank's particles in rank order), 1 <= d <= 8,
+ * 1 <= k <= 16, k < n < 2^31.  The search and the backward run for the queries [row0, row0 + nrows),
+ * 0 <= row0 <= row0 + nrows <= n, against all n particles; their results are bit for bit the rows of the whole batch
+ * (row0 = 0, nrows = n), whatever the range.
+ *   mfb_knn_kth: r[nrows] = distance from x_(row0+q) to its k-th nearest OTHER particle (self excluded by index, so a
+ *     duplicate is a neighbour at distance 0), idx[nrows] = that particle's index in the whole batch, neighbours
+ *     ordered by (r^2, j): ties go to the smaller index.  A query without k others at a finite distance (NaN or inf
+ *     coordinates, r^2 overflowing) gets r = inf and its own index row0 + q.  logsum (may be NULL; non-NULL only for
+ *     the whole batch): logsum[0] = sum_i log(r_i + pad) in double.  All pairs in fp32 direct differences;
+ *     deterministic (no floating-point atomics).  Workspace: mfb_knn_workspace_bytes(n, nrows, d, k) (0 for
+ *     nrows = 0 or bad arguments).
  *   mfb_knn_logsum: logsum[0] = sum_i log(r_i + pad) over r[n] of the whole batch (the concatenated r of the ranges),
  *     added in the same order as mfb_knn_kth adds it, so it equals mfb_knn_kth's logsum bit for bit.  Workspace:
  *     8 * ceil(n / 256) bytes.
- *   mfb_knn_kth_bwd_rows: gx[nrows][d] = rows row0 .. row0 + nrows - 1 of mfb_knn_kth_bwd's gx; r, idx, sorted_idx
- *     and perm are those of the whole batch.                                                                       */
-int64_t mfb_knn_rows_workspace_bytes(int64_t n, int64_t nrows, int d, int k);
-int mfb_knn_kth_rows(const float* x, int64_t n, int d, int k, int64_t row0, int64_t nrows, float* r, int32_t* idx,
-                     void* workspace, int64_t workspace_bytes, void* stream);
+ *   mfb_knn_kth_bwd: gx[nrows][d] = rows row0 .. row0 + nrows - 1 of glogsum[0] * d logsum / dx with the neighbours
+ *     held fixed:  w_i (x_i - x_idx[i]) + sum over j with idx[j] = i, ascending j, of w_j (x_i - x_j),
+ *     w_j = 1 / (r_j (r_j + pad)), 0 where r_j = 0.  r[n] and idx[n] are the whole batch's, sorted_idx[n] = idx
+ *     stably sorted, perm[n] (int64) the positions it came from.
+ * Arguments are checked before any launch: a range outside [0, n], k >= n, n >= 2^31, a NULL pointer or a non-NULL
+ * logsum with a range other than the whole batch return MFB_E_BADARG, d > 8 or k > 16 MFB_E_UNSUPPORTED.
+ * nrows = 0 launches nothing and returns 0 (r, idx, gx and the workspace may then be NULL).                     */
+int64_t mfb_knn_workspace_bytes(int64_t n, int64_t nrows, int d, int k);
+int mfb_knn_kth(const float* x, int64_t n, int d, int k, int64_t row0, int64_t nrows, double pad, float* r,
+                int32_t* idx, double* logsum, void* workspace, int64_t workspace_bytes, void* stream);
 int mfb_knn_logsum(const float* r, int64_t n, double pad, double* logsum, void* workspace, int64_t workspace_bytes,
                    void* stream);
-int mfb_knn_kth_bwd_rows(const float* x, int64_t n, int d, const float* r, const int32_t* idx,
-                         const int32_t* sorted_idx, const int64_t* perm, int64_t row0, int64_t nrows, double pad,
-                         const double* glogsum, float* gx, void* stream);
+int mfb_knn_kth_bwd(const float* x, int64_t n, int d, const float* r, const int32_t* idx,
+                    const int32_t* sorted_idx, const int64_t* perm, int64_t row0, int64_t nrows, double pad,
+                    const double* glogsum, float* gx, void* stream);
 
 /* ---- sliced Wasserstein distance (loss.py sliced_wasserstein_distance; POT's ot.sliced_wasserstein_distance) ------
  * x[n][d], 1 <= d <= 8, 1 <= n < 2^31; theta[nproj][d] the directions.  u_k = x theta_k, each an fp32 fused

@@ -13,7 +13,7 @@ LIB_PATH = os.environ.get("MENTFLOW_B200_LIB") or os.path.join(PKG_DIR, "libment
 
 P = c_void_p  # every device pointer crosses the ABI as a plain address
 
-ABI_VERSION = 5  # MFB_ABI_VERSION of the header SIGNATURES mirrors
+ABI_VERSION = 6  # MFB_ABI_VERSION of the header SIGNATURES mirrors
 
 # name -> (restype, argtypes); mirrors include/mentflow_b200.h line by line
 SIGNATURES = {
@@ -77,13 +77,10 @@ SIGNATURES = {
     "mfb_f64_join": (c_int, [P, c_int, P, P]),
     "mfb_mc_entropy": (c_int, [P, c_double, c_double, c_double, P, P]),
     "mfb_loss_tail": (c_int, [P, c_int, P, c_float, P, P]),
-    "mfb_knn_workspace_bytes": (c_int64, [c_int64, c_int, c_int]),
-    "mfb_knn_kth": (c_int, [P, c_int64, c_int, c_int, c_double, P, P, P, P, c_int64, P]),
-    "mfb_knn_kth_bwd": (c_int, [P, c_int64, c_int, P, P, P, P, c_double, P, P, P]),
-    "mfb_knn_rows_workspace_bytes": (c_int64, [c_int64, c_int64, c_int, c_int]),
-    "mfb_knn_kth_rows": (c_int, [P, c_int64, c_int, c_int, c_int64, c_int64, P, P, P, c_int64, P]),
+    "mfb_knn_workspace_bytes": (c_int64, [c_int64, c_int64, c_int, c_int]),
+    "mfb_knn_kth": (c_int, [P, c_int64, c_int, c_int, c_int64, c_int64, c_double, P, P, P, P, c_int64, P]),
     "mfb_knn_logsum": (c_int, [P, c_int64, c_double, P, P, c_int64, P]),
-    "mfb_knn_kth_bwd_rows": (c_int, [P, c_int64, c_int, P, P, P, P, c_int64, c_int64, c_double, P, P, P]),
+    "mfb_knn_kth_bwd": (c_int, [P, c_int64, c_int, P, P, P, P, c_int64, c_int64, c_double, P, P, P]),
     "mfb_swd_workspace_bytes": (c_int64, [c_int64, c_int]),
     "mfb_swd_sort": (c_int, [P, c_int64, c_int, P, c_int, P, P, P, c_int64, P]),
     "mfb_swd_wpp": (c_int, [P, c_int64, c_int, P, c_int, P, c_int64, c_double, P, P, P, c_int64, P]),

@@ -381,8 +381,8 @@ static int64_t knn_logparts(int64_t n) { return (n + kKnnThreads - 1) / kKnnThre
 // choice follow nrows.  Splits of the candidate axis: with few queries (25,000 fill 49 CTAs of 512) the grid would
 // leave most SMs idle, so the candidate tiles are cut into `splits` ranges.  The choice rounds the CTA count up to
 // whole waves of resident CTAs (preferring fewer splits unless more are 2 % better), at least kKnnMinTilesPerSplit
-// tiles each.  with_logsum: room for the merge's log partials (the whole-batch call).
-static int knn_plan(int64_t n, int64_t nrows, int d, int k, bool with_logsum, KnnPlan& p) {
+// tiles each.
+static int knn_plan(int64_t n, int64_t nrows, int d, int k, KnnPlan& p) {
   p.ntiles = (int)((n + kKnnTile - 1) / kKnnTile);
   p.npad = (int64_t)p.ntiles * kKnnTile;
   p.qblocks = (int)((nrows + kKnnRows - 1) / kKnnRows);
@@ -407,7 +407,7 @@ static int knn_plan(int64_t n, int64_t nrows, int d, int k, bool with_logsum, Kn
   p.off_pd2 = (size_t)d * p.npad * 4;
   p.off_pidx = p.off_pd2 + list;
   p.off_logpart = p.off_pidx + list;
-  p.bytes = p.off_logpart + (with_logsum ? (size_t)p.mblocks * 8 : 0);
+  p.bytes = p.off_logpart + (size_t)p.mblocks * 8;
   return 0;
 }
 
@@ -422,13 +422,34 @@ static bool knn_range_ok(int64_t n, int64_t row0, int64_t nrows) {
   return row0 >= 0 && nrows >= 0 && row0 <= n && nrows <= n - row0;
 }
 
-// transpose, pair search and merge for the queries [row0, row0 + nrows); logsum NULL: no log sum
-static int knn_search(const float* x, int64_t n, int d, int k, int64_t row0, int64_t nrows, double pad, float* r,
-                      int32_t* idx, double* logsum, void* workspace, int64_t workspace_bytes, cudaStream_t st) {
+}  // namespace mfb
+
+using namespace mfb;
+
+extern "C" {
+
+int64_t mfb_knn_workspace_bytes(int64_t n, int64_t nrows, int d, int k) {
+  if (knn_check((const float*)1, n, d, k) || !knn_range_ok(n, 0, nrows) || nrows == 0) return 0;
   KnnPlan p;
-  int rc = knn_plan(n, nrows, d, k, logsum != nullptr, p);
+  if (knn_plan(n, nrows, d, k, p)) return 0;
+  return (int64_t)p.bytes;
+}
+
+// transpose, pair search and merge for the queries [row0, row0 + nrows); with logsum (whole batch only) the merge's
+// log partials and their fixed-order sum
+int mfb_knn_kth(const float* x, int64_t n, int d, int k, int64_t row0, int64_t nrows, double pad, float* r,
+                int32_t* idx, double* logsum, void* workspace, int64_t workspace_bytes, void* stream) {
+  int rc = knn_check(x, n, d, k);
+  if (rc) return rc;
+  MFB_CHECK_ARG(knn_range_ok(n, row0, nrows));
+  MFB_CHECK_ARG(!logsum || (row0 == 0 && nrows == n));
+  if (nrows == 0) return 0;
+  MFB_CHECK_ARG(r && idx && workspace);
+  KnnPlan p;
+  rc = knn_plan(n, nrows, d, k, p);
   if (rc) return rc;
   if (workspace_bytes < (int64_t)p.bytes) return MFB_E_WORKSPACE;
+  cudaStream_t st = (cudaStream_t)stream;
   char* ws = (char*)workspace;
   float* xt = (float*)ws;
   float* pd2 = (float*)(ws + p.off_pd2);
@@ -447,59 +468,6 @@ static int knn_search(const float* x, int64_t n, int d, int k, int64_t row0, int
   return launch_status();
 }
 
-static int knn_backward(const float* x, int64_t n, int d, const float* r, const int32_t* idx,
-                        const int32_t* sorted_idx, const int64_t* perm, int64_t row0, int64_t nrows, double pad,
-                        const double* glogsum, float* gx, cudaStream_t st) {
-  MFB_CUDA(launch_pdl(knn_bwd_for(d), dim3((unsigned)((nrows + kKnnThreads - 1) / kKnnThreads)), dim3(kKnnThreads), 0,
-                      st, x, n, r, idx, sorted_idx, perm, row0, nrows, pad, glogsum, gx));
-  return launch_status();
-}
-
-}  // namespace mfb
-
-using namespace mfb;
-
-extern "C" {
-
-int64_t mfb_knn_workspace_bytes(int64_t n, int d, int k) {
-  if (knn_check((const float*)1, n, d, k)) return 0;
-  KnnPlan p;
-  if (knn_plan(n, n, d, k, true, p)) return 0;
-  return (int64_t)p.bytes;
-}
-
-int mfb_knn_kth(const float* x, int64_t n, int d, int k, double pad, float* r, int32_t* idx, double* logsum,
-                void* workspace, int64_t workspace_bytes, void* stream) {
-  int rc = knn_check(x, n, d, k);
-  if (rc) return rc;
-  MFB_CHECK_ARG(r && idx && logsum && workspace);
-  return knn_search(x, n, d, k, 0, n, pad, r, idx, logsum, workspace, workspace_bytes, (cudaStream_t)stream);
-}
-
-int mfb_knn_kth_bwd(const float* x, int64_t n, int d, const float* r, const int32_t* idx, const int32_t* sorted_idx,
-                    const int64_t* perm, double pad, const double* glogsum, float* gx, void* stream) {
-  MFB_CHECK_ARG(x && r && idx && sorted_idx && perm && glogsum && gx && n >= 2 && n <= INT32_MAX && d >= 1);
-  if (d > kMaxDim) return MFB_E_UNSUPPORTED;
-  return knn_backward(x, n, d, r, idx, sorted_idx, perm, 0, n, pad, glogsum, gx, (cudaStream_t)stream);
-}
-
-int64_t mfb_knn_rows_workspace_bytes(int64_t n, int64_t nrows, int d, int k) {
-  if (knn_check((const float*)1, n, d, k) || !knn_range_ok(n, 0, nrows) || nrows == 0) return 0;
-  KnnPlan p;
-  if (knn_plan(n, nrows, d, k, false, p)) return 0;
-  return (int64_t)p.bytes;
-}
-
-int mfb_knn_kth_rows(const float* x, int64_t n, int d, int k, int64_t row0, int64_t nrows, float* r, int32_t* idx,
-                     void* workspace, int64_t workspace_bytes, void* stream) {
-  int rc = knn_check(x, n, d, k);
-  if (rc) return rc;
-  MFB_CHECK_ARG(knn_range_ok(n, row0, nrows));
-  if (nrows == 0) return 0;
-  MFB_CHECK_ARG(r && idx && workspace);
-  return knn_search(x, n, d, k, row0, nrows, 0.0, r, idx, nullptr, workspace, workspace_bytes, (cudaStream_t)stream);
-}
-
 int mfb_knn_logsum(const float* r, int64_t n, double pad, double* logsum, void* workspace, int64_t workspace_bytes,
                    void* stream) {
   MFB_CHECK_ARG(r && logsum && workspace && n >= 1 && n <= INT32_MAX);
@@ -513,15 +481,17 @@ int mfb_knn_logsum(const float* r, int64_t n, double pad, double* logsum, void* 
   return launch_status();
 }
 
-int mfb_knn_kth_bwd_rows(const float* x, int64_t n, int d, const float* r, const int32_t* idx,
-                         const int32_t* sorted_idx, const int64_t* perm, int64_t row0, int64_t nrows, double pad,
-                         const double* glogsum, float* gx, void* stream) {
+int mfb_knn_kth_bwd(const float* x, int64_t n, int d, const float* r, const int32_t* idx, const int32_t* sorted_idx,
+                    const int64_t* perm, int64_t row0, int64_t nrows, double pad, const double* glogsum, float* gx,
+                    void* stream) {
   MFB_CHECK_ARG(x && r && idx && sorted_idx && perm && glogsum && n >= 2 && n <= INT32_MAX && d >= 1);
   if (d > kMaxDim) return MFB_E_UNSUPPORTED;
   MFB_CHECK_ARG(knn_range_ok(n, row0, nrows));
   if (nrows == 0) return 0;
   MFB_CHECK_ARG(gx);
-  return knn_backward(x, n, d, r, idx, sorted_idx, perm, row0, nrows, pad, glogsum, gx, (cudaStream_t)stream);
+  MFB_CUDA(launch_pdl(knn_bwd_for(d), dim3((unsigned)((nrows + kKnnThreads - 1) / kKnnThreads)), dim3(kKnnThreads), 0,
+                      (cudaStream_t)stream, x, n, r, idx, sorted_idx, perm, row0, nrows, pad, glogsum, gx));
+  return launch_status();
 }
 
 }  // extern "C"

@@ -546,22 +546,29 @@ KNN_MAX_K = 16
 KNN_MAX_DIM = 8
 
 
+def _knn_search(x: torch.Tensor, k: int, pad: float, row0: int, nrows: int, with_logsum: bool):
+    """(r, idx, logsum) of the queries [row0, row0 + nrows) of the checked float32 CUDA tensor ``x``, searched against
+    every row of ``x``; logsum is None unless ``with_logsum`` (the whole batch only)."""
+    lib = _lib.load()
+    n, d = x.shape
+    r = torch.empty(nrows, dtype=torch.float32, device=x.device)
+    idx = torch.empty(nrows, dtype=torch.int32, device=x.device)
+    logsum = torch.empty((), dtype=torch.float64, device=x.device) if with_logsum else None
+    with torch.cuda.device(x.device):
+        wbytes = lib.mfb_knn_workspace_bytes(n, nrows, d, k)
+        work = torch.empty(max(wbytes, 16), dtype=torch.uint8, device=x.device)
+        _lib.check(lib.mfb_knn_kth(_ptr(x), n, d, k, row0, nrows, float(pad), _ptr(r), _ptr(idx), _ptr(logsum),
+                                   _ptr(work), wbytes, _stream()), "knn_kth")
+    return r, idx, logsum
+
+
 class KNNKth(torch.autograd.Function):
     """(r, idx, logsum) of ``knn_kth``; only ``logsum`` carries a gradient, with the neighbours held fixed."""
 
     @staticmethod
     def forward(ctx, x, k, pad):
-        lib = _lib.load()
         x = _check_f32("x", x.detach())
-        n, d = x.shape
-        r = torch.empty(n, dtype=torch.float32, device=x.device)
-        idx = torch.empty(n, dtype=torch.int32, device=x.device)
-        logsum = torch.empty((), dtype=torch.float64, device=x.device)
-        with torch.cuda.device(x.device):
-            wbytes = lib.mfb_knn_workspace_bytes(n, d, k)
-            work = torch.empty(max(wbytes, 16), dtype=torch.uint8, device=x.device)
-            _lib.check(lib.mfb_knn_kth(_ptr(x), n, d, k, float(pad), _ptr(r), _ptr(idx), _ptr(logsum), _ptr(work),
-                                       wbytes, _stream()), "knn_kth")
+        r, idx, logsum = _knn_search(x, k, pad, 0, x.shape[0], with_logsum=True)
         ctx.save_for_backward(x, r, idx)
         ctx.pad = float(pad)
         ctx.mark_non_differentiable(r, idx)
@@ -618,16 +625,7 @@ def knn_kth(x: torch.Tensor, k: int, pad: float = 1.0e-12, rows: Optional[slice]
         _check_f32("x", x)
         return KNNKth.apply(x, k, float(pad))
     row0, nrows = knn_rows(rows, n)
-    x = _check_f32("x", x.detach())
-    r = torch.empty(nrows, dtype=torch.float32, device=x.device)
-    idx = torch.empty(nrows, dtype=torch.int32, device=x.device)
-    lib = _lib.load()
-    with torch.cuda.device(x.device):
-        wbytes = lib.mfb_knn_rows_workspace_bytes(n, nrows, d, k)
-        work = torch.empty(max(wbytes, 16), dtype=torch.uint8, device=x.device)
-        _lib.check(lib.mfb_knn_kth_rows(_ptr(x), n, d, k, row0, nrows, _ptr(r), _ptr(idx), _ptr(work), wbytes,
-                                        _stream()), "knn_kth_rows")
-    return r, idx, None
+    return _knn_search(_check_f32("x", x.detach()), k, pad, row0, nrows, with_logsum=False)
 
 
 def knn_logsum(r: torch.Tensor, pad: float = 1.0e-12) -> torch.Tensor:
@@ -676,8 +674,8 @@ def knn_kth_bwd(x: torch.Tensor, r: torch.Tensor, idx: torch.Tensor, glogsum: to
     g = glogsum.detach().to(device=x.device, dtype=torch.float64).reshape(()).contiguous()
     lib = _lib.load()
     with torch.cuda.device(x.device):
-        _lib.check(lib.mfb_knn_kth_bwd_rows(_ptr(x), n, d, _ptr(r), _ptr(idx), _ptr(sorted_idx), _ptr(perm), row0,
-                                            nrows, float(pad), _ptr(g), _ptr(gx), _stream()), "knn_kth_bwd_rows")
+        _lib.check(lib.mfb_knn_kth_bwd(_ptr(x), n, d, _ptr(r), _ptr(idx), _ptr(sorted_idx), _ptr(perm), row0, nrows,
+                                       float(pad), _ptr(g), _ptr(gx), _stream()), "knn_kth_bwd")
     return gx
 
 

@@ -17,12 +17,12 @@ def candidate_splits(n, d, k):
     """Number of candidate-axis splits the library plans, read back from the workspace size:
     d Npad floats + two lists of splits * k * n 4-byte entries (each rounded to 16 bytes) + one double per 256 rows."""
     npad = -(-n // 256) * 256
-    lists = (int(_lib.load().mfb_knn_workspace_bytes(n, d, k)) - d * npad * 4 - (-(-n // 256)) * 8) // 2
+    lists = (int(_lib.load().mfb_knn_workspace_bytes(n, n, d, k)) - d * npad * 4 - (-(-n // 256)) * 8) // 2
     return lists // (k * n * 4)
 
 
 @pytest.mark.parametrize("d,side", [(1, 2400), (2, 110), (3, 23)])
-def test_lattice_ties_across_candidate_splits(d, side):
+def test_lattice_ties_across_the_planned_candidate_splits(d, side):
     """12,000 integer points at about one per cell: equal distances are exact and the tied candidates of a query lie
     in every split of the candidate axis, so the merge of the splits decides them."""
     rng = np.random.default_rng(7 + d)

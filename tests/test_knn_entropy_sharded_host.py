@@ -17,16 +17,16 @@ from mentflow_b200.entropy import KNNEntropyEstimator
 MFB_E_BADARG, MFB_E_UNSUPPORTED, MFB_E_WORKSPACE = -1, -2, -3
 
 
-def test_c_entry_points_refuse_bad_arguments_before_any_launch():
+def test_knn_c_entry_points_refuse_bad_arguments_before_any_launch():
     lib = _lib.load()
     buf = (ctypes.c_float * 64)()
     p = ctypes.cast(buf, ctypes.c_void_p)
 
-    def kth(n=100, d=3, k=5, row0=0, nrows=10, r=p, idx=p, ws=p):
-        return lib.mfb_knn_kth_rows(p, n, d, k, row0, nrows, r, idx, ws, 0, None)
+    def kth(n=100, d=3, k=5, row0=0, nrows=10, r=p, idx=p, logsum=None, ws=p):
+        return lib.mfb_knn_kth(p, n, d, k, row0, nrows, 1e-12, r, idx, logsum, ws, 0, None)
 
     def bwd(n=100, d=3, row0=0, nrows=10, gx=p):
-        return lib.mfb_knn_kth_bwd_rows(p, n, d, p, p, p, p, row0, nrows, 1e-12, p, gx, None)
+        return lib.mfb_knn_kth_bwd(p, n, d, p, p, p, p, row0, nrows, 1e-12, p, gx, None)
 
     for row0, nrows in [(-1, 10), (95, 10), (101, 0), (0, -1), (0, 101), (100, 1)]:
         assert kth(row0=row0, nrows=nrows) == MFB_E_BADARG, (row0, nrows)
@@ -42,14 +42,17 @@ def test_c_entry_points_refuse_bad_arguments_before_any_launch():
     assert bwd(n=2 ** 31, nrows=0) == MFB_E_BADARG
     assert kth(r=None) == MFB_E_BADARG and kth(idx=None) == MFB_E_BADARG and kth(ws=None) == MFB_E_BADARG
     assert bwd(gx=None) == MFB_E_BADARG
-    assert lib.mfb_knn_kth_rows(None, 100, 3, 5, 0, 10, p, p, p, 0, None) == MFB_E_BADARG
+    assert lib.mfb_knn_kth(None, 100, 3, 5, 0, 10, 1e-12, p, p, None, p, 0, None) == MFB_E_BADARG
+    # a sub-range has no log sum of its own (it comes from mfb_knn_logsum over the gathered r)
+    for row0, nrows in [(0, 10), (1, 99), (0, 99), (37, 0)]:
+        assert kth(row0=row0, nrows=nrows, logsum=p) == MFB_E_BADARG, (row0, nrows)
     # an empty range (a rank without particles) launches nothing and succeeds, without outputs or a workspace
     for row0 in (0, 37, 100):
         assert kth(row0=row0, nrows=0, r=None, idx=None, ws=None) == 0
         assert bwd(row0=row0, nrows=0, gx=None) == 0
-    assert lib.mfb_knn_rows_workspace_bytes(100, 0, 3, 5) == 0
+    assert lib.mfb_knn_workspace_bytes(100, 0, 3, 5) == 0
     for bad in [(100, 10, 9, 5), (100, 10, 3, 17), (100, 10, 3, 100), (100, 101, 3, 5), (100, -1, 3, 5)]:
-        assert lib.mfb_knn_rows_workspace_bytes(*bad) == 0, bad
+        assert lib.mfb_knn_workspace_bytes(*bad) == 0, bad
     # the log sum: pointers, n and the workspace size are checked before the launch
     assert lib.mfb_knn_logsum(None, 100, 1e-12, p, p, 64, None) == MFB_E_BADARG
     assert lib.mfb_knn_logsum(p, 100, 1e-12, None, p, 64, None) == MFB_E_BADARG
