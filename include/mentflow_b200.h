@@ -25,6 +25,8 @@
 extern "C" {
 #endif
 
+/* The version changes when an existing entry point changes its arguments.  Entry points that are only added (the
+ * ragged MENT ones) keep it: the ctypes layer refuses a library that lacks any symbol it binds. */
 #define MFB_ABI_VERSION 6
 
 #define MFB_E_BADARG (-1)      /* null pointer / non-positive size / unsupported shape   */
@@ -373,6 +375,39 @@ int mfb_ment_integrate(int d, const float* meas_coords, int nb_meas, int meas_ax
                        int b, const float* mp, const float* proj2, const float* cx2, const float* cy2,
                        const float* tables2, int k2, int bx, int by, const float* mp2,
                        float prior_neg_half_inv_s2, float prior_log_norm, float* pred, void* stream);
+/* Screens of different sizes: the ragged layout.  The _ragged entry points take their uniform sibling's arguments
+ * with `int b` replaced by `const int32_t* offsets, int total` and `int bx, int by` by `const int32_t* offsets2`:
+ *   1-D screens: table k holds coords[offsets[k] .. offsets[k+1]) and tables[offsets[k] .. offsets[k+1]), at least 2
+ *     bins each; offsets[k + 1] (DEVICE, offsets[0] = 0, non-decreasing) and total = offsets[k] (HOST) sizes the
+ *     shared memory.
+ *   2-D screens: offsets2[3][k2 + 1] (DEVICE) gives the start of table k in cx2, cy2 and tables2: bx_k =
+ *     offsets2[0][k+1] - offsets2[0][k], by_k = offsets2[1][k+1] - offsets2[1][k] (both >= 2), and table k is
+ *     tables2[offsets2[2][k] ..][bx_k][by_k].
+ * The interpolation, clamp, product order and prior are the uniform kernels' own, so a model of equal sizes gives
+ * the uniform entry points' results bit for bit.  A family may be empty (k = 0: offsets may be NULL and total 0;
+ * k2 = 0: offsets2 may be NULL).  The offsets are not read on the host: the caller guarantees them.  MFB_E_BADARG
+ * for a NULL required pointer or total < 2 k; MFB_E_UNSUPPORTED, before any launch, when the 1-D family does not fit
+ * the shared memory (200 KB: 4 (4 ceil(k d / 4) + 2 ceil((k + 1) / 2) + 2 total + 2 ceil(k / 2)) + 8 total + 16
+ * bytes, plus 4 (k (2 d + 4) + 4 d + 2) with kicks).                                     */
+int mfb_ment_prob_ragged(const float* x, int64_t g, int d, const float* proj, const float* coords,
+                         const float* tables, int k, const int32_t* offsets, int total, const float* mp,
+                         const float* proj2, const float* cx2, const float* cy2, const float* tables2, int k2,
+                         const int32_t* offsets2, const float* mp2, float prior_neg_half_inv_s2,
+                         float prior_log_norm, float* out, void* stream);
+int mfb_ment_prob_grid_ragged(int d, const int32_t* shape_host, const float* first_centre_host,
+                              const float* step_host, const float* proj, const float* coords, const float* tables,
+                              int k, const int32_t* offsets, int total, const float* mp, const float* proj2,
+                              const float* cx2, const float* cy2, const float* tables2, int k2,
+                              const int32_t* offsets2, const float* mp2, float prior_neg_half_inv_s2,
+                              float prior_log_norm, float* out, void* stream);
+int mfb_ment_integrate_ragged(int d, const float* meas_coords, int nb_meas, int meas_axis,
+                              const float* meas_coords2, int nb_meas2, int meas_axis2, int n_int_axes,
+                              const int32_t* int_shape_host, const float* int_first_host,
+                              const float* int_step_host, const float* linv, const float* inv_mp, const float* proj,
+                              const float* coords, const float* tables, int k, const int32_t* offsets, int total,
+                              const float* mp, const float* proj2, const float* cx2, const float* cy2,
+                              const float* tables2, int k2, const int32_t* offsets2, const float* mp2,
+                              float prior_neg_half_inv_s2, float prior_log_norm, float* pred, void* stream);
 /* sample.py:27-57: cdf of (rho + pad) over the cells in double, then `size` draws: cell by
  * inverse-CDF search with a Philox4x32-10 stream (seed, offset), uniform position inside the
  * cell (+ 0.5*U(-delta,delta) when jitter != 0).  workspace[0] (device double) = total mass. */
@@ -409,6 +444,13 @@ int mfb_ment_mh(int d, const float* proj, const float* coords, const float* tabl
                 const float* mp2, float prior_neg_half_inv_s2, float prior_log_norm, uint64_t chain0,
                 int64_t nchains, const float* start, float start_scale, const float* chol, int64_t burnin,
                 int64_t steps, int64_t thin, uint64_t seed, float* out, int64_t* accepted, void* stream);
+/* the same chains over ragged tables (layout: mfb_ment_prob_ragged) */
+int mfb_ment_mh_ragged(int d, const float* proj, const float* coords, const float* tables, int k,
+                       const int32_t* offsets, int total, const float* mp, const float* proj2, const float* cx2,
+                       const float* cy2, const float* tables2, int k2, const int32_t* offsets2, const float* mp2,
+                       float prior_neg_half_inv_s2, float prior_log_norm, uint64_t chain0, int64_t nchains,
+                       const float* start, float start_scale, const float* chol, int64_t burnin, int64_t steps,
+                       int64_t thin, uint64_t seed, float* out, int64_t* accepted, void* stream);
 /* The same chains one step at a time around a density the library cannot see (same words, arithmetic and rule).
  * mfb_mh_propose: t = 0 writes the start draws x_0 of chains chain0 .. chain0 + n - 1 to xp[n][d] (x and chol may be
  * NULL); t >= 1 writes the proposals from the current states x[n][d].  mfb_mh_accept (t >= 1): where the rule takes

@@ -54,6 +54,12 @@ SIGNATURES = {
                                    c_float, P, P]),
     "mfb_ment_integrate": (c_int, [c_int, P, c_int, c_int, P, c_int, c_int, c_int, P, P, P, P, P, P, P, P, c_int, c_int,
                                    P, P, P, P, P, c_int, c_int, c_int, P, c_float, c_float, P, P]),
+    "mfb_ment_prob_ragged": (c_int, [P, c_int64, c_int, P, P, P, c_int, P, c_int, P, P, P, P, P, c_int, P, P, c_float,
+                                     c_float, P, P]),
+    "mfb_ment_prob_grid_ragged": (c_int, [c_int, P, P, P, P, P, P, c_int, P, c_int, P, P, P, P, P, c_int, P, P,
+                                          c_float, c_float, P, P]),
+    "mfb_ment_integrate_ragged": (c_int, [c_int, P, c_int, c_int, P, c_int, c_int, c_int, P, P, P, P, P, P, P, P,
+                                          c_int, P, c_int, P, P, P, P, P, c_int, P, P, c_float, c_float, P, P]),
     "mfb_randn_offset_increment": (c_int64, [c_int64]),
     "mfb_randn_philox": (c_int, [P, c_int64, c_uint64, c_uint64, P]),
     "mfb_randn_philox_state": (c_int, [P, c_int64, P, c_int, P]),
@@ -62,6 +68,8 @@ SIGNATURES = {
     "mfb_cdf_sample": (c_int, [P, c_int64, P, c_int, P, P, P, c_int, c_uint64, c_uint64, c_int64, P, P]),
     "mfb_ment_mh": (c_int, [c_int, P, P, P, c_int, c_int, P, P, P, P, P, c_int, c_int, c_int, P, c_float, c_float,
                             c_uint64, c_int64, P, c_float, P, c_int64, c_int64, c_int64, c_uint64, P, P, P]),
+    "mfb_ment_mh_ragged": (c_int, [c_int, P, P, P, c_int, P, c_int, P, P, P, P, P, c_int, P, P, c_float, c_float,
+                                   c_uint64, c_int64, P, c_float, P, c_int64, c_int64, c_int64, c_uint64, P, P, P]),
     "mfb_mh_propose": (c_int, [P, c_int64, c_int, c_uint64, P, c_float, P, c_int64, c_uint64, P, P]),
     "mfb_mh_accept": (c_int, [P, P, P, P, c_int64, c_int, c_uint64, c_int64, c_uint64, P, P]),
     "mfb_gs_update": (c_int, [P, P, P, c_int, c_float, c_float, P]),

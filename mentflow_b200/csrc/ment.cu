@@ -27,6 +27,11 @@ constexpr int kMentThreads = 256;
 // The linear kernels keep no minimum (0).
 template <bool kMP>
 constexpr int ment_min_ctas() { return kMP ? 5 : 0; }
+// The ragged kernels (screens of different sizes) are kernels of their own, so that the uniform kernels keep their
+// code: they carry the table offsets beside the uniform kernels' state, and at the uniform minimum the integrate kernel
+// spills (with kicks, D = 6 ... 8; without, D = 8).  Minimum 4 with kicks (<= 64 registers), 3 without (<= 80).
+template <bool kMP>
+constexpr int ment_ragged_min_ctas() { return kMP ? 4 : 3; }
 
 struct MentGrid {            // regular grid of cell centres (GridSampler) or an integration grid
   int ndim;
@@ -108,9 +113,19 @@ __device__ __forceinline__ bool axis_locate(const float* __restrict__ c, int B, 
   return true;
 }
 
-template <int D, bool kMP = false>
+// the four corners tb[0], tb[1], tb[by], tb[by + 1] of the cell at normalised distances (wx, wy)
+__device__ __forceinline__ float bilinear(const float* __restrict__ tb, int by, double wx, double wy) {
+  const double v00 = (double)__ldg(tb), v01 = (double)__ldg(tb + 1);
+  const double v10 = (double)__ldg(tb + by), v11 = (double)__ldg(tb + by + 1);
+  return (float)(v00 * (1.0 - wx) * (1.0 - wy) + v01 * (1.0 - wx) * wy + v10 * wx * (1.0 - wy) + v11 * wx * wy);
+}
+
+// kRagged (screens of different sizes): off2[3][t2.k + 1] holds the start of table k in t2.cx, t2.cy and t2.tab, so
+// bx_k = off2[k + 1] - off2[k] and by_k = off2[t2.k + 2 + k] - off2[t2.k + 1 + k]; t2.bx and t2.by are unused
+template <int D, bool kMP = false, bool kRagged = false>
 __device__ __forceinline__ float tables2d_product(const float (&x)[D], const Tables2D& t2,
-                                                  const float* __restrict__ mp2 = nullptr) {
+                                                  const float* __restrict__ mp2 = nullptr,
+                                                  const int32_t* __restrict__ off2 = nullptr) {
   float prob = 1.0f;
   for (int k = 0; k < t2.k; ++k) {
     const float* pr = t2.proj + (size_t)k * 2 * D;
@@ -131,12 +146,16 @@ __device__ __forceinline__ float tables2d_product(const float (&x)[D], const Tab
     int ix, iy;
     double wx, wy;
     float h = 0.f;
-    if (axis_locate(t2.cx + (size_t)k * t2.bx, t2.bx, ux, ix, wx) &&
-        axis_locate(t2.cy + (size_t)k * t2.by, t2.by, uy, iy, wy)) {
-      const float* tb = t2.tab + ((size_t)k * t2.bx + ix) * t2.by + iy;
-      const double v00 = (double)__ldg(tb), v01 = (double)__ldg(tb + 1);
-      const double v10 = (double)__ldg(tb + t2.by), v11 = (double)__ldg(tb + t2.by + 1);
-      h = (float)(v00 * (1.0 - wx) * (1.0 - wy) + v01 * (1.0 - wx) * wy + v10 * wx * (1.0 - wy) + v11 * wx * wy);
+    if constexpr (kRagged) {
+      const int32_t* ox = off2 + k;
+      const int32_t* oy = ox + t2.k + 1;
+      const int x0 = __ldg(ox), y0 = __ldg(oy);
+      const int bx = __ldg(ox + 1) - x0, by = __ldg(oy + 1) - y0;
+      if (axis_locate(t2.cx + x0, bx, ux, ix, wx) && axis_locate(t2.cy + y0, by, uy, iy, wy))
+        h = bilinear(t2.tab + __ldg(oy + t2.k + 1) + (size_t)ix * by + iy, by, wx, wy);
+    } else if (axis_locate(t2.cx + (size_t)k * t2.bx, t2.bx, ux, ix, wx) &&
+               axis_locate(t2.cy + (size_t)k * t2.by, t2.by, uy, iy, wy)) {
+      h = bilinear(t2.tab + ((size_t)k * t2.bx + ix) * t2.by + iy, t2.by, wx, wy);
     }
     h = fminf(fmaxf(h, 0.0f), 1.0e10f);   // ment.py:246
     prob *= h;
@@ -145,12 +164,17 @@ __device__ __forceinline__ float tables2d_product(const float (&x)[D], const Tab
   return prob;
 }
 
-template <int D, bool kMP = false>
+// kRagged: table k holds s_off[k] .. s_off[k + 1] - 1 of s_c, s_h and s_dinv (B unused); the end of one table is
+// the start of the next, so each table loads one offset
+template <int D, bool kMP = false, bool kRagged = false>
 __device__ __forceinline__ float ment_density(const float (&x)[D], const float* __restrict__ s_proj,
                                               const float* __restrict__ s_c, const float* __restrict__ s_h,
                                               const float* __restrict__ s_inv, const double* __restrict__ s_dinv, int K,
-                                              int B, MentPrior prior, const float* __restrict__ s_mp = nullptr) {
+                                              int B, MentPrior prior, const float* __restrict__ s_mp = nullptr,
+                                              const int32_t* __restrict__ s_off = nullptr) {
   float prob = 1.0f;
+  int end = 0;
+  if constexpr (kRagged) end = s_off[0];
   for (int k = 0; k < K; ++k) {
     float u = 0.f;
 #pragma unroll
@@ -160,7 +184,14 @@ __device__ __forceinline__ float ment_density(const float (&x)[D], const float* 
       float zr, zi;
       if (mp_z<D, false>(row, x, zr, zi)) u = mp_add<D, false>(row, zr, zi, u);
     }
-    float h = lagrange_eval(s_c + (size_t)k * B, s_h + (size_t)k * B, s_dinv + (size_t)k * B, B, s_inv[k], u);
+    float h;
+    if constexpr (kRagged) {
+      const int o = end;
+      end = s_off[k + 1];
+      h = lagrange_eval(s_c + o, s_h + o, s_dinv + o, end - o, s_inv[k], u);
+    } else {
+      h = lagrange_eval(s_c + (size_t)k * B, s_h + (size_t)k * B, s_dinv + (size_t)k * B, B, s_inv[k], u);
+    }
     h = fminf(fmaxf(h, 0.0f), 1.0e10f);   // ment.py:246
     prob *= h;
     if (prob == 0.f) break;               // every remaining factor is finite (clamped): the product stays 0 -- on a 6-D
@@ -172,24 +203,63 @@ __device__ __forceinline__ float ment_density(const float (&x)[D], const float* 
   return prob * expf(fmaf(prior.neg_half_inv_s2, ss, prior.log_norm));
 }
 
+// kRagged: B is the total T of the K tables, table k is coords[off[k] .. off[k + 1]); the offsets go to s_off[K + 1]
+// (0 for an empty family, whose off may be NULL) and dinv of a table's last centre is never read
+template <bool kRagged = false>
 __device__ __forceinline__ void load_tables(float* s_proj, float* s_c, float* s_h, float* s_inv, double* s_dinv,
                                             const float* __restrict__ proj, const float* __restrict__ coords,
-                                            const float* __restrict__ tables, int K, int B, int D) {
+                                            const float* __restrict__ tables, int K, int B, int D,
+                                            int32_t* s_off = nullptr, const int32_t* __restrict__ off = nullptr) {
   for (int i = threadIdx.x; i < K * D; i += blockDim.x) s_proj[i] = proj[i];
-  for (int i = threadIdx.x; i < K * B; i += blockDim.x) {
-    s_c[i] = coords[i];
-    s_h[i] = tables[i];
-    s_dinv[i] = (i % B < B - 1) ? 1.0 / ((double)coords[i + 1] - (double)coords[i]) : 0.0;
+  if constexpr (kRagged) {
+    for (int i = threadIdx.x; i <= K; i += blockDim.x) s_off[i] = K > 0 ? off[i] : 0;
+    for (int i = threadIdx.x; i < B; i += blockDim.x) {
+      s_c[i] = coords[i];
+      s_h[i] = tables[i];
+      s_dinv[i] = i + 1 < B ? 1.0 / ((double)coords[i + 1] - (double)coords[i]) : 0.0;
+    }
+    for (int k = threadIdx.x; k < K; k += blockDim.x) {
+      const int o = off[k], n = off[k + 1] - o;
+      s_inv[k] = (float)(n - 1) / (coords[o + n - 1] - coords[o]);
+    }
+  } else {
+    for (int i = threadIdx.x; i < K * B; i += blockDim.x) {
+      s_c[i] = coords[i];
+      s_h[i] = tables[i];
+      s_dinv[i] = (i % B < B - 1) ? 1.0 / ((double)coords[i + 1] - (double)coords[i]) : 0.0;
+    }
+    for (int k = threadIdx.x; k < K; k += blockDim.x)
+      s_inv[k] = (float)(B - 1) / (coords[(size_t)k * B + B - 1] - coords[(size_t)k * B]);
   }
-  for (int k = threadIdx.x; k < K; k += blockDim.x)
-    s_inv[k] = (float)(B - 1) / (coords[(size_t)k * B + B - 1] - coords[(size_t)k * B]);
 }
 
 // (kMP) the multipole rows of the 1-D screens, [K][2D+4], follow the tables in shared memory
 __device__ __forceinline__ float* mp_smem(double* s_dinv, int K, int B) {
   return reinterpret_cast<float*>(s_dinv + (size_t)K * B);
 }
+// the same after the T entries of ragged tables
+__device__ __forceinline__ float* mp_smem(double* s_dinv, size_t T) {
+  return reinterpret_cast<float*>(s_dinv + T);
+}
 
+// Shared-memory image of the 1-D family: proj[K][D] (padded to 4 floats) | (kRagged) off[K + 1] (padded to 2) | c[T]
+// | h[T] | inv[K] (padded to 2) | dinv[T] (double) | (kMP) mp.  Declares s_proj .. s_dinv, s_off and T in the body.
+#define MFB_MENT_SMEM(kRagged)                                                                                         \
+  extern __shared__ __align__(16) float sm[];                                                                          \
+  float* s_proj = sm;                                                                                                  \
+  float* s_c = s_proj + (((size_t)K * D + 3) & ~(size_t)3);                                                            \
+  int32_t* s_off = nullptr;                                                                                            \
+  if constexpr (kRagged) {                                                                                             \
+    s_off = reinterpret_cast<int32_t*>(s_c);                                                                           \
+    s_c += (K + 2) & ~1;                                                                                               \
+  }                                                                                                                    \
+  const size_t T = kRagged ? (size_t)B : (size_t)K * B;                                                                \
+  float* s_h = s_c + T;                                                                                                \
+  float* s_inv = s_h + T;                                                                                              \
+  double* s_dinv = reinterpret_cast<double*>(s_inv + ((K + 1) & ~1))
+
+// MODE 0: explicit points x[G][D];  MODE 1: points of a regular grid generated from the index
+// kMP: mp[K][2D+4] and mp2[K2][2][2D+4] add the multipole terms to the projections
 // MODE 0: explicit points x[G][D];  MODE 1: points of a regular grid generated from the index
 // kMP: mp[K][2D+4] and mp2[K2][2][2D+4] add the multipole terms to the projections
 template <int D, int MODE, bool kMP = false>
@@ -227,6 +297,43 @@ ment_prob_kernel(const float* __restrict__ x, int64_t G, MentGrid grid, const fl
     }
     float rho = ment_density<D, kMP>(xr, s_proj, s_c, s_h, s_inv, s_dinv, K, B, prior, s_mp);
     if (t2.k > 0) rho *= tables2d_product<D, kMP>(xr, t2, mp2);
+    out[g] = rho;
+  }
+}
+
+// The same over tables in the ragged layout: off[K + 1] and off2[3][t2.k + 1] (nt: the 1-D entries in all)
+template <int D, int MODE, bool kMP>
+__global__ void __launch_bounds__(kMentThreads, ment_ragged_min_ctas<kMP>())
+ment_prob_ragged_kernel(const float* __restrict__ x, int64_t G, MentGrid grid, const float* __restrict__ proj,
+                        const float* __restrict__ coords, const float* __restrict__ tables, int K, int nt,
+                        MentPrior prior, const Tables2D t2, float* __restrict__ out, const float* __restrict__ mp,
+                        const float* __restrict__ mp2, const int32_t* __restrict__ off,
+                        const int32_t* __restrict__ off2) {
+  const int B = nt;
+  MFB_MENT_SMEM(true);
+  load_tables<true>(s_proj, s_c, s_h, s_inv, s_dinv, proj, coords, tables, K, B, D, s_off, off);
+  float* s_mp = nullptr;
+  if constexpr (kMP) {
+    s_mp = mp_smem(s_dinv, T);
+    for (int i = threadIdx.x; i < K * MFB_MP_STRIDE(D); i += blockDim.x) s_mp[i] = mp[i];
+  }
+  __syncthreads();
+  for (int64_t g = (int64_t)blockIdx.x * kMentThreads + threadIdx.x; g < G; g += (int64_t)gridDim.x * kMentThreads) {
+    float xr[D];
+    if (MODE == 0) {
+#pragma unroll
+      for (int i = 0; i < D; ++i) xr[i] = x[g * D + i];
+    } else {
+      int64_t rem = g;
+#pragma unroll
+      for (int i = D - 1; i >= 0; --i) {
+        const int idx = (int)(rem % grid.shape[i]);
+        rem /= grid.shape[i];
+        xr[i] = fmaf((float)idx, grid.step[i], grid.lo[i]);
+      }
+    }
+    float rho = ment_density<D, kMP, true>(xr, s_proj, s_c, s_h, s_inv, s_dinv, K, B, prior, s_mp, s_off);
+    if (t2.k > 0) rho *= tables2d_product<D, kMP, true>(xr, t2, mp2, off2);
     out[g] = rho;
   }
 }
@@ -314,6 +421,97 @@ ment_integrate_kernel(const float* __restrict__ meas_coords, int nb_meas, int me
     }
     float rho = ment_density<D, kMP>(xr, s_proj, s_c, s_h, s_inv, s_dinv, K, B, prior, s_mp);
     if (t2.k > 0) rho *= tables2d_product<D, kMP>(xr, t2, mp2);
+    dacc += (double)rho;
+  }
+  (void)acc;
+  dacc = warp_sum(dacc);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = dacc;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double t = 0.0;
+    for (int i = 0; i < kMentThreads / 32; ++i) t += red[i];
+    pred[b] = (float)t;
+  }
+}
+
+// The same over tables in the ragged layout (as ment_prob_ragged_kernel)
+template <int D, bool kMP>
+__global__ void __launch_bounds__(kMentThreads, ment_ragged_min_ctas<kMP>())
+ment_integrate_ragged_kernel(const float* __restrict__ meas_coords, int nb_meas, int meas_axis,
+                             const float* __restrict__ meas_coords2, int nb_meas2, int meas_axis2, MentGrid igrid,
+                             const float* __restrict__ minv, const float* __restrict__ proj,
+                             const float* __restrict__ coords, const float* __restrict__ tables, int K, int nt,
+                             MentPrior prior, const Tables2D t2, float* __restrict__ pred,
+                             const float* __restrict__ mp, const float* __restrict__ mp2,
+                             const float* __restrict__ imp, const int32_t* __restrict__ off,
+                             const int32_t* __restrict__ off2) {
+  constexpr bool kRagged = true;
+  const int B = nt;
+  MFB_MENT_SMEM(kRagged);
+  __shared__ float s_minv[D * D];
+  __shared__ double red[kMentThreads / 32];
+  load_tables<kRagged>(s_proj, s_c, s_h, s_inv, s_dinv, proj, coords, tables, K, B, D, s_off, off);
+  for (int i = threadIdx.x; i < D * D; i += blockDim.x) s_minv[i] = minv[i];
+  float* s_mp = nullptr;
+  float* s_imp = nullptr;
+  if constexpr (kMP) {
+    s_mp = mp_smem(s_dinv, T);
+    s_imp = s_mp + (size_t)K * MFB_MP_STRIDE(D);
+    for (int i = threadIdx.x; i < K * MFB_MP_STRIDE(D); i += blockDim.x) s_mp[i] = mp[i];
+    for (int i = threadIdx.x; i < 4 * D + 2; i += blockDim.x) s_imp[i] = imp[i];
+  }
+  __syncthreads();
+  int64_t Q = 1;
+  for (int i = 0; i < igrid.ndim; ++i) Q *= igrid.shape[i];
+  // pixel of the screen: b (1-D) or (b / nb_meas2, b % nb_meas2) (2-D, meas_axis2 >= 0)
+  const int b = blockIdx.x;
+  const float cm = meas_coords[meas_axis2 >= 0 ? b / nb_meas2 : b];
+  const float cm2 = meas_axis2 >= 0 ? meas_coords2[b % nb_meas2] : 0.f;
+  float acc = 0.f;  // the reference sums fp32 densities with torch.sum
+  double dacc = 0.0;
+  for (int64_t q = threadIdx.x; q < Q; q += kMentThreads) {
+    float u[D];
+    int64_t rem = q;
+    int ia = igrid.ndim - 1;
+#pragma unroll
+    for (int i = D - 1; i >= 0; --i) {
+      if (i == meas_axis) {
+        u[i] = cm;
+      } else if (i == meas_axis2) {
+        u[i] = cm2;
+      } else {
+        const int idx = (int)(rem % igrid.shape[ia]);
+        rem /= igrid.shape[ia];
+        u[i] = fmaf((float)idx, igrid.step[ia], igrid.lo[ia]);
+        --ia;
+      }
+    }
+    float xr[D];
+#pragma unroll
+    for (int i = 0; i < D; ++i) {
+      float s = 0.f;
+#pragma unroll
+      for (int j = 0; j < D; ++j) s = fmaf(u[j], s_minv[i * D + j], s);
+      xr[i] = s;
+    }
+    if constexpr (kMP) {
+      // kick of the inverse map: zi = r0 . u + i r2 . u, x += p Re(zi^m) + q Im(zi^m)
+      const int m = (int)s_imp[4 * D] - 1;
+      if (m >= 1) {
+        float xm = 0.f, ym = 0.f;
+#pragma unroll
+        for (int j = 0; j < D; ++j) {
+          xm = fmaf(s_imp[j], u[j], xm);
+          ym = fmaf(s_imp[D + j], u[j], ym);
+        }
+        float zr, zi, pr, pi;
+        zpow(xm, ym, m, zr, zi, pr, pi);
+#pragma unroll
+        for (int i = 0; i < D; ++i) xr[i] = fmaf(s_imp[3 * D + i], zi, fmaf(s_imp[2 * D + i], zr, xr[i]));
+      }
+    }
+    float rho = ment_density<D, kMP, kRagged>(xr, s_proj, s_c, s_h, s_inv, s_dinv, K, B, prior, s_mp, s_off);
+    if (t2.k > 0) rho *= tables2d_product<D, kMP, kRagged>(xr, t2, mp2, off2);
     dacc += (double)rho;
   }
   (void)acc;
@@ -699,6 +897,9 @@ struct MhChains {
 // some dimensions.
 template <int D>
 constexpr int mh_min_ctas() { return D < 8 ? 3 : 2; }
+// the ragged chain kernel: at 3 CTAs it spills a word at D = 1 and 2, so those take 2
+template <int D>
+constexpr int mh_ragged_min_ctas() { return D > 2 && D < 8 ? 3 : 2; }
 template <int D, bool kMP>
 __global__ void __launch_bounds__(kMentThreads, mh_min_ctas<D>())
 ment_mh_kernel(const float* __restrict__ proj, const float* __restrict__ coords, const float* __restrict__ tables,
@@ -736,6 +937,62 @@ ment_mh_kernel(const float* __restrict__ proj, const float* __restrict__ coords,
         const float u = mh_propose<D>(c, (uint32_t)t, ch.seed, s_chol, x, xp);
         float rp = ment_density<D, kMP>(xp, s_proj, s_c, s_h, s_inv, s_dinv, K, B, prior, s_mp);
         if (t2.k > 0) rp *= tables2d_product<D, kMP>(xp, t2, mp2);
+        if (mh_accept(rp, u, rho)) {
+#pragma unroll
+          for (int j = 0; j < D; ++j) x[j] = xp[j];
+          rho = rp;
+          ++acc;
+        }
+      }
+      if (t == next) {
+#pragma unroll
+        for (int j = 0; j < D; ++j) row[j] = x[j];
+        row += D;
+        next += ch.thin;
+      }
+      if (t == total) break;
+    }
+  }
+  acc = warp_sum_u64(acc);
+  if ((threadIdx.x & 31) == 0 && acc) atomicAdd(accepted, acc);
+}
+
+// The same chains over tables in the ragged layout (as ment_prob_ragged_kernel)
+template <int D, bool kMP>
+__global__ void __launch_bounds__(kMentThreads, mh_ragged_min_ctas<D>())
+ment_mh_ragged_kernel(const float* __restrict__ proj, const float* __restrict__ coords,
+                      const float* __restrict__ tables, int K, int nt, MentPrior prior, const Tables2D t2,
+                      const float* __restrict__ mp, const float* __restrict__ mp2, const MhChains ch,
+                      float* __restrict__ out, unsigned long long* __restrict__ accepted,
+                      const int32_t* __restrict__ off, const int32_t* __restrict__ off2) {
+  constexpr bool kRagged = true;
+  const int B = nt;
+  MFB_MENT_SMEM(kRagged);
+  __shared__ float s_chol[D * D];
+  load_tables<kRagged>(s_proj, s_c, s_h, s_inv, s_dinv, proj, coords, tables, K, B, D, s_off, off);
+  float* s_mp = nullptr;
+  if constexpr (kMP) {
+    s_mp = mp_smem(s_dinv, T);
+    for (int i = threadIdx.x; i < K * MFB_MP_STRIDE(D); i += blockDim.x) s_mp[i] = mp[i];
+  }
+  for (int i = threadIdx.x; i < D * D; i += blockDim.x) s_chol[i] = ch.chol[i];
+  __syncthreads();
+  const int64_t total = ch.burnin + (ch.steps - 1) * ch.thin;
+  unsigned long long acc = 0;
+  for (int64_t i = (int64_t)blockIdx.x * kMentThreads + threadIdx.x; i < ch.n; i += (int64_t)gridDim.x * kMentThreads) {
+    const uint64_t c = ch.chain0 + (uint64_t)i;
+    float x[D];
+    mh_start<D>(c, ch.seed, ch.start, ch.start_scale, x);
+    float rho = ment_density<D, kMP, kRagged>(x, s_proj, s_c, s_h, s_inv, s_dinv, K, B, prior, s_mp, s_off);
+    if (t2.k > 0) rho *= tables2d_product<D, kMP, kRagged>(x, t2, mp2, off2);
+    float* row = out + i * ch.steps * D;
+    int64_t next = ch.burnin;         // next step to record
+    for (int64_t t = 0;; ++t) {
+      if (t > 0) {
+        float xp[D];
+        const float u = mh_propose<D>(c, (uint32_t)t, ch.seed, s_chol, x, xp);
+        float rp = ment_density<D, kMP, kRagged>(xp, s_proj, s_c, s_h, s_inv, s_dinv, K, B, prior, s_mp, s_off);
+        if (t2.k > 0) rp *= tables2d_product<D, kMP, kRagged>(xp, t2, mp2, off2);
         if (mh_accept(rp, u, rho)) {
 #pragma unroll
           for (int j = 0; j < D; ++j) x[j] = xp[j];
@@ -812,10 +1069,24 @@ __global__ void gs_update_kernel(float* __restrict__ table, const float* __restr
 static size_t ment_smem(int K, int B, int d) {
   return ((((size_t)K * d + 3) & ~(size_t)3) + 2 * (size_t)K * B + ((K + 1) & ~1)) * 4 + (size_t)K * B * 8 + 16;
 }
-// kMP: the 1-D screens' multipole rows and the inverse kick of integrate mode follow (mp_smem)
+// kMP: the 1-D screens' multipole rows and the inverse kick of integrate mode follow (MentSmem::end)
 static size_t ment_smem_mp(int K, int B, int d) {
   return ment_smem(K, B, d) + ((size_t)K * MFB_MP_STRIDE(d) + 4 * (size_t)d + 2) * 4;
 }
+// the ragged layout of K tables of T bins in all: ment_smem's image plus the offsets off[K + 1]
+static size_t ment_smem_ragged(int K, int T, int d) {
+  return ((((size_t)K * d + 3) & ~(size_t)3) + ((K + 2) & ~1) + 2 * (size_t)T + ((K + 1) & ~1)) * 4 +
+         (size_t)T * 8 + 16;
+}
+static size_t ment_smem_ragged_mp(int K, int T, int d) {
+  return ment_smem_ragged(K, T, d) + ((size_t)K * MFB_MP_STRIDE(d) + 4 * (size_t)d + 2) * 4;
+}
+// b: the bins of every table (uniform) or the total (ragged)
+static size_t ment_smem_of(bool ragged, bool kick, int K, int b, int d) {
+  if (ragged) return kick ? ment_smem_ragged_mp(K, b, d) : ment_smem_ragged(K, b, d);
+  return kick ? ment_smem_mp(K, b, d) : ment_smem(K, b, d);
+}
+constexpr size_t kMentSmemCap = 200 * 1024;
 
 static MentGrid make_grid(int ndim, const int32_t* shape, const float* lo, const float* step) {
   MentGrid g;
@@ -828,43 +1099,65 @@ static MentGrid make_grid(int ndim, const int32_t* shape, const float* lo, const
   return g;
 }
 
-// The 1-D family (k tables of b bins) and the 2-D family t2; behind kicks a non-empty family needs its multipole rows
-static bool tables_ok(int k, int b, const float* proj, const float* coords, const float* tables, const float* mp,
-                      const Tables2D& t2, const float* mp2, bool kick) {
-  if (k < 0 || (k > 0 && !(proj && coords && tables && b >= 2))) return false;
-  if (t2.k < 0 || (t2.k > 0 && !(t2.proj && t2.cx && t2.cy && t2.tab && t2.bx >= 2 && t2.by >= 2))) return false;
+// The 1-D family (k tables of b bins, or ragged: offsets off and b bins in all, at least 2 per table) and the 2-D
+// family t2 (ragged: offsets off2); behind kicks a non-empty family needs its multipole rows
+static bool tables_ok(bool ragged, int k, int b, const int32_t* off, const float* proj, const float* coords,
+                      const float* tables, const float* mp, const Tables2D& t2, const int32_t* off2, const float* mp2,
+                      bool kick) {
+  const bool sizes1 = ragged ? off && (int64_t)b >= 2 * (int64_t)k : b >= 2;
+  const bool sizes2 = ragged ? off2 != nullptr : t2.bx >= 2 && t2.by >= 2;
+  if (k < 0 || (k > 0 && !(proj && coords && tables && sizes1))) return false;
+  if (t2.k < 0 || (t2.k > 0 && !(t2.proj && t2.cx && t2.cy && t2.tab && sizes2))) return false;
   return !kick || ((k == 0 || mp) && (t2.k == 0 || mp2));
 }
 
-template <int D>
-static int launch_prob(int mode, bool kick, const float* x, int64_t G, const MentGrid& grid, const float* proj,
-                       const float* coords, const float* tables, int K, int B, const float* mp, const Tables2D& t2,
-                       const float* mp2, MentPrior prior, float* out, cudaStream_t st) {
-  const size_t smem = kick ? ment_smem_mp(K, B, D) : ment_smem(K, B, D);
-  if (smem > 200 * 1024) return MFB_E_UNSUPPORTED;
-  int64_t blocks = (G + kMentThreads - 1) / kMentThreads;
-  int64_t cap = (int64_t)sm_count() * 8;
-  const int gridx = (int)(blocks < cap ? blocks : cap);
-  const auto kernel = mode == 0 ? (kick ? ment_prob_kernel<D, 0, true> : ment_prob_kernel<D, 0, false>)
-                                : (kick ? ment_prob_kernel<D, 1, true> : ment_prob_kernel<D, 1, false>);
+// set the kernel's dynamic shared memory and launch it with kMentThreads threads per CTA
+template <typename... P, typename... A>
+static int launch_ment(void (*kernel)(P...), int64_t blocks, size_t smem, cudaStream_t st, A... args) {
   MFB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  kernel<<<gridx, kMentThreads, smem, st>>>(x, G, grid, proj, coords, tables, K, B, prior, t2, out, mp, mp2);
+  kernel<<<(int)blocks, kMentThreads, smem, st>>>(args...);
   return launch_status();
 }
 
+// ragged: the tables in the ragged layout (off, off2; B is the 1-D total), through the _ragged_ kernels
 template <int D>
-static int launch_integrate(bool kick, const float* mc, int nb, int ax, const float* mc2, int nb2, int ax2,
-                            const MentGrid& grid, const float* minv, const float* imp, const float* proj,
-                            const float* coords, const float* tables, int k, int b, const float* mp,
-                            const Tables2D& t2, const float* mp2, MentPrior pr, float* pred, cudaStream_t st) {
-  const size_t smem = kick ? ment_smem_mp(k, b, D) : ment_smem(k, b, D);
-  if (smem > 200 * 1024) return MFB_E_UNSUPPORTED;
-  const auto kernel = kick ? ment_integrate_kernel<D, true> : ment_integrate_kernel<D, false>;
-  MFB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+static int launch_prob(int mode, bool kick, bool ragged, const float* x, int64_t G, const MentGrid& grid,
+                       const float* proj, const float* coords, const float* tables, int K, int B, const int32_t* off,
+                       const int32_t* off2, const float* mp, const Tables2D& t2, const float* mp2, MentPrior prior,
+                       float* out, cudaStream_t st) {
+  const size_t smem = ment_smem_of(ragged, kick, K, B, D);
+  if (smem > kMentSmemCap) return MFB_E_UNSUPPORTED;
+  int64_t blocks = (G + kMentThreads - 1) / kMentThreads;
+  int64_t cap = (int64_t)sm_count() * 8;
+  blocks = blocks < cap ? blocks : cap;
+  if (ragged) {
+    const auto kernel = mode == 0 ? (kick ? ment_prob_ragged_kernel<D, 0, true> : ment_prob_ragged_kernel<D, 0, false>)
+                                  : (kick ? ment_prob_ragged_kernel<D, 1, true> : ment_prob_ragged_kernel<D, 1, false>);
+    return launch_ment(kernel, blocks, smem, st, x, G, grid, proj, coords, tables, K, B, prior, t2, out, mp, mp2, off,
+                       off2);
+  }
+  const auto kernel = mode == 0 ? (kick ? ment_prob_kernel<D, 0, true> : ment_prob_kernel<D, 0, false>)
+                                : (kick ? ment_prob_kernel<D, 1, true> : ment_prob_kernel<D, 1, false>);
+  return launch_ment(kernel, blocks, smem, st, x, G, grid, proj, coords, tables, K, B, prior, t2, out, mp, mp2);
+}
+
+template <int D>
+static int launch_integrate(bool kick, bool ragged, const float* mc, int nb, int ax, const float* mc2, int nb2,
+                            int ax2, const MentGrid& grid, const float* minv, const float* imp, const float* proj,
+                            const float* coords, const float* tables, int k, int b, const int32_t* off,
+                            const int32_t* off2, const float* mp, const Tables2D& t2, const float* mp2, MentPrior pr,
+                            float* pred, cudaStream_t st) {
+  const size_t smem = ment_smem_of(ragged, kick, k, b, D);
+  if (smem > kMentSmemCap) return MFB_E_UNSUPPORTED;
   const int pixels = ax2 >= 0 ? nb * nb2 : nb;
-  kernel<<<pixels, kMentThreads, smem, st>>>(mc, nb, ax, mc2, nb2, ax2, grid, minv, proj, coords, tables, k, b, pr, t2,
-                                             pred, mp, mp2, imp);
-  return launch_status();
+  if (ragged) {
+    const auto kernel = kick ? ment_integrate_ragged_kernel<D, true> : ment_integrate_ragged_kernel<D, false>;
+    return launch_ment(kernel, pixels, smem, st, mc, nb, ax, mc2, nb2, ax2, grid, minv, proj, coords, tables, k, b, pr,
+                       t2, pred, mp, mp2, imp, off, off2);
+  }
+  const auto kernel = kick ? ment_integrate_kernel<D, true> : ment_integrate_kernel<D, false>;
+  return launch_ment(kernel, pixels, smem, st, mc, nb, ax, mc2, nb2, ax2, grid, minv, proj, coords, tables, k, b, pr,
+                     t2, pred, mp, mp2, imp);
 }
 
 // one CTA per 256 chains, no grid-stride cap: a chain is a whole run, and the block scheduler evens out chains of
@@ -872,16 +1165,19 @@ static int launch_integrate(bool kick, const float* mc, int nb, int ax, const fl
 static int mh_grid(int64_t n) { return (int)((n + kMentThreads - 1) / kMentThreads); }
 
 template <int D>
-static int launch_mh(bool kick, const float* proj, const float* coords, const float* tables, int K, int B,
-                     const float* mp, const Tables2D& t2, const float* mp2, MentPrior prior, const MhChains& ch,
-                     float* out, int64_t* accepted, cudaStream_t st) {
-  const size_t smem = kick ? ment_smem_mp(K, B, D) : ment_smem(K, B, D);
-  if (smem > 200 * 1024) return MFB_E_UNSUPPORTED;
+static int launch_mh(bool kick, bool ragged, const float* proj, const float* coords, const float* tables, int K, int B,
+                     const int32_t* off, const int32_t* off2, const float* mp, const Tables2D& t2, const float* mp2,
+                     MentPrior prior, const MhChains& ch, float* out, int64_t* accepted, cudaStream_t st) {
+  const size_t smem = ment_smem_of(ragged, kick, K, B, D);
+  if (smem > kMentSmemCap) return MFB_E_UNSUPPORTED;
+  unsigned long long* acc = reinterpret_cast<unsigned long long*>(accepted);
+  if (ragged) {
+    const auto kernel = kick ? ment_mh_ragged_kernel<D, true> : ment_mh_ragged_kernel<D, false>;
+    return launch_ment(kernel, mh_grid(ch.n), smem, st, proj, coords, tables, K, B, prior, t2, mp, mp2, ch, out, acc,
+                       off, off2);
+  }
   const auto kernel = kick ? ment_mh_kernel<D, true> : ment_mh_kernel<D, false>;
-  MFB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  kernel<<<mh_grid(ch.n), kMentThreads, smem, st>>>(proj, coords, tables, K, B, prior, t2, mp, mp2, ch, out,
-                                                    reinterpret_cast<unsigned long long*>(accepted));
-  return launch_status();
+  return launch_ment(kernel, mh_grid(ch.n), smem, st, proj, coords, tables, K, B, prior, t2, mp, mp2, ch, out, acc);
 }
 
 // the last step of a run must fit the 32-bit stream word: burnin + (steps - 1) thin < 2^32
@@ -896,23 +1192,100 @@ using namespace mfb;
 
 extern "C" {
 
-// rho at the g points x (mode 0) or on the g cells of `grid` (mode 1): the body of mfb_ment_prob and mfb_ment_prob_grid
-static int ment_prob_impl(int mode, const float* x, int64_t g, const MentGrid& grid, int d, const float* proj,
-                          const float* coords, const float* tables, int k, int b, const float* mp, const float* proj2,
-                          const float* cx2, const float* cy2, const float* tables2, int k2, int bx, int by,
-                          const float* mp2, float prior_neg_half_inv_s2, float prior_log_norm, float* out,
-                          void* stream) {
-  const bool kick = mp || mp2;
+// The tables of a call: the 1-D family with b bins per table (uniform) or off[k + 1] and b bins in all (ragged), and
+// the 2-D family t2 (ragged: off2[3][t2.k + 1]).  An empty 1-D family takes b = 2 (uniform) or 0 (ragged).
+struct MentTables {
+  bool ragged;
+  int k, b;
+  const int32_t* off;
+  const float *proj, *coords, *tables, *mp;
+  Tables2D t2;
+  const int32_t* off2;
+  const float* mp2;
+  bool ok(bool kick) const { return tables_ok(ragged, k, b, off, proj, coords, tables, mp, t2, off2, mp2, kick); }
+  int bins() const { return k > 0 ? b : (ragged ? 0 : 2); }
+};
+
+static MentTables uniform_tables(const float* proj, const float* coords, const float* tables, int k, int b,
+                                 const float* mp, const float* proj2, const float* cx2, const float* cy2,
+                                 const float* tables2, int k2, int bx, int by, const float* mp2) {
+  return MentTables{false, k, b, nullptr, proj, coords, tables, mp, Tables2D{k2, bx, by, proj2, cx2, cy2, tables2},
+                    nullptr, mp2};
+}
+
+static MentTables ragged_tables(const float* proj, const float* coords, const float* tables, int k,
+                                const int32_t* offsets, int total, const float* mp, const float* proj2,
+                                const float* cx2, const float* cy2, const float* tables2, int k2,
+                                const int32_t* offsets2, const float* mp2) {
+  return MentTables{true, k, total, offsets, proj, coords, tables, mp,
+                    Tables2D{k2, 0, 0, proj2, cx2, cy2, tables2}, offsets2, mp2};
+}
+
+// rho at the g points x (mode 0) or on the g cells of `grid` (mode 1): the body of the mfb_ment_prob* entry points
+static int ment_prob_impl(int mode, const float* x, int64_t g, const MentGrid& grid, int d, const MentTables& t,
+                          float prior_neg_half_inv_s2, float prior_log_norm, float* out, void* stream) {
+  const bool kick = t.mp || t.mp2;
   MFB_CHECK_ARG(out && d >= 1 && d <= kMaxDim);
-  const Tables2D t2{k2, bx, by, proj2, cx2, cy2, tables2};
-  MFB_CHECK_ARG(tables_ok(k, b, proj, coords, tables, mp, t2, mp2, kick));
+  MFB_CHECK_ARG(t.ok(kick));
   if (g == 0) return 0;
-  if (k == 0) b = 2;
   const MentPrior pr{prior_neg_half_inv_s2, prior_log_norm};
   cudaStream_t st = (cudaStream_t)stream;
-#define MFB_CALL(DD) launch_prob<DD>(mode, kick, x, g, grid, proj, coords, tables, k, b, mp, t2, mp2, pr, out, st)
+#define MFB_CALL(DD)                                                                                                   \
+  launch_prob<DD>(mode, kick, t.ragged, x, g, grid, t.proj, t.coords, t.tables, t.k, t.bins(), t.off, t.off2, t.mp,   \
+                  t.t2, t.mp2, pr, out, st)
   switch (d) {
     case 1: return MFB_CALL(1);
+    case 2: return MFB_CALL(2);
+    case 3: return MFB_CALL(3);
+    case 4: return MFB_CALL(4);
+    case 5: return MFB_CALL(5);
+    case 6: return MFB_CALL(6);
+    case 7: return MFB_CALL(7);
+    default: return MFB_CALL(8);
+  }
+#undef MFB_CALL
+}
+
+static int ment_prob_points(const float* x, int64_t g, int d, const MentTables& t, float prior_neg_half_inv_s2,
+                            float prior_log_norm, float* out, void* stream) {
+  MFB_CHECK_ARG(x && g >= 0);
+  return ment_prob_impl(0, x, g, make_grid(0, nullptr, nullptr, nullptr), d, t, prior_neg_half_inv_s2, prior_log_norm,
+                        out, stream);
+}
+
+static int ment_prob_grid(int d, const int32_t* shape_host, const float* first_centre_host, const float* step_host,
+                          const MentTables& t, float prior_neg_half_inv_s2, float prior_log_norm, float* out,
+                          void* stream) {
+  MFB_CHECK_ARG(shape_host && first_centre_host && step_host && d >= 1 && d <= kMaxDim);
+  int64_t g = 1;
+  for (int i = 0; i < d; ++i) {
+    MFB_CHECK_ARG(shape_host[i] >= 1);
+    g *= shape_host[i];
+  }
+  return ment_prob_impl(1, nullptr, g, make_grid(d, shape_host, first_centre_host, step_host), d, t,
+                        prior_neg_half_inv_s2, prior_log_norm, out, stream);
+}
+
+static int ment_integrate(int d, const float* meas_coords, int nb_meas, int meas_axis, const float* meas_coords2,
+                          int nb_meas2, int meas_axis2, int n_int_axes, const int32_t* int_shape_host,
+                          const float* int_first_host, const float* int_step_host, const float* linv,
+                          const float* inv_mp, const MentTables& t, float prior_neg_half_inv_s2,
+                          float prior_log_norm, float* pred, void* stream) {
+  const bool kick = t.mp || t.mp2 || inv_mp;
+  MFB_CHECK_ARG(meas_coords && linv && (inv_mp || !kick) && pred && int_shape_host && int_first_host && int_step_host);
+  const int n_meas = meas_axis2 >= 0 ? 2 : 1;
+  MFB_CHECK_ARG(d >= 2 && d <= kMaxDim && n_int_axes == d - n_meas && n_int_axes >= 1);
+  MFB_CHECK_ARG(meas_axis >= 0 && meas_axis < d && nb_meas >= 1 && meas_axis2 < d && meas_axis2 != meas_axis);
+  MFB_CHECK_ARG(meas_axis2 < 0 || (meas_coords2 && nb_meas2 >= 1));
+  MFB_CHECK_ARG(t.ok(kick));
+  const MentPrior pr{prior_neg_half_inv_s2, prior_log_norm};
+  const MentGrid grid = make_grid(n_int_axes, int_shape_host, int_first_host, int_step_host);
+  cudaStream_t st = (cudaStream_t)stream;
+#define MFB_CALL(DD)                                                                                                   \
+  launch_integrate<DD>(kick, t.ragged, meas_coords, nb_meas, meas_axis, meas_coords2, nb_meas2, meas_axis2, grid,     \
+                       linv, inv_mp, t.proj, t.coords, t.tables, t.k, t.bins(), t.off, t.off2, t.mp, t.t2, t.mp2, pr, \
+                       pred, st)
+  switch (d) {
     case 2: return MFB_CALL(2);
     case 3: return MFB_CALL(3);
     case 4: return MFB_CALL(4);
@@ -928,9 +1301,19 @@ int mfb_ment_prob(const float* x, int64_t g, int d, const float* proj, const flo
                   int b, const float* mp, const float* proj2, const float* cx2, const float* cy2, const float* tables2,
                   int k2, int bx, int by, const float* mp2, float prior_neg_half_inv_s2, float prior_log_norm,
                   float* out, void* stream) {
-  MFB_CHECK_ARG(x && g >= 0);
-  return ment_prob_impl(0, x, g, make_grid(0, nullptr, nullptr, nullptr), d, proj, coords, tables, k, b, mp, proj2,
-                        cx2, cy2, tables2, k2, bx, by, mp2, prior_neg_half_inv_s2, prior_log_norm, out, stream);
+  return ment_prob_points(x, g, d,
+                          uniform_tables(proj, coords, tables, k, b, mp, proj2, cx2, cy2, tables2, k2, bx, by, mp2),
+                          prior_neg_half_inv_s2, prior_log_norm, out, stream);
+}
+
+int mfb_ment_prob_ragged(const float* x, int64_t g, int d, const float* proj, const float* coords,
+                         const float* tables, int k, const int32_t* offsets, int total, const float* mp,
+                         const float* proj2, const float* cx2, const float* cy2, const float* tables2, int k2,
+                         const int32_t* offsets2, const float* mp2, float prior_neg_half_inv_s2, float prior_log_norm,
+                         float* out, void* stream) {
+  return ment_prob_points(
+      x, g, d, ragged_tables(proj, coords, tables, k, offsets, total, mp, proj2, cx2, cy2, tables2, k2, offsets2, mp2),
+      prior_neg_half_inv_s2, prior_log_norm, out, stream);
 }
 
 int mfb_ment_prob_grid(int d, const int32_t* shape_host, const float* first_centre_host, const float* step_host,
@@ -938,15 +1321,21 @@ int mfb_ment_prob_grid(int d, const int32_t* shape_host, const float* first_cent
                        const float* proj2, const float* cx2, const float* cy2, const float* tables2, int k2, int bx,
                        int by, const float* mp2, float prior_neg_half_inv_s2, float prior_log_norm, float* out,
                        void* stream) {
-  MFB_CHECK_ARG(shape_host && first_centre_host && step_host && d >= 1 && d <= kMaxDim);
-  int64_t g = 1;
-  for (int i = 0; i < d; ++i) {
-    MFB_CHECK_ARG(shape_host[i] >= 1);
-    g *= shape_host[i];
-  }
-  return ment_prob_impl(1, nullptr, g, make_grid(d, shape_host, first_centre_host, step_host), d, proj, coords, tables,
-                        k, b, mp, proj2, cx2, cy2, tables2, k2, bx, by, mp2, prior_neg_half_inv_s2, prior_log_norm,
-                        out, stream);
+  return ment_prob_grid(d, shape_host, first_centre_host, step_host,
+                        uniform_tables(proj, coords, tables, k, b, mp, proj2, cx2, cy2, tables2, k2, bx, by, mp2),
+                        prior_neg_half_inv_s2, prior_log_norm, out, stream);
+}
+
+int mfb_ment_prob_grid_ragged(int d, const int32_t* shape_host, const float* first_centre_host,
+                              const float* step_host, const float* proj, const float* coords, const float* tables,
+                              int k, const int32_t* offsets, int total, const float* mp, const float* proj2,
+                              const float* cx2, const float* cy2, const float* tables2, int k2,
+                              const int32_t* offsets2, const float* mp2, float prior_neg_half_inv_s2,
+                              float prior_log_norm, float* out, void* stream) {
+  return ment_prob_grid(
+      d, shape_host, first_centre_host, step_host,
+      ragged_tables(proj, coords, tables, k, offsets, total, mp, proj2, cx2, cy2, tables2, k2, offsets2, mp2),
+      prior_neg_half_inv_s2, prior_log_norm, out, stream);
 }
 
 int mfb_ment_integrate(int d, const float* meas_coords, int nb_meas, int meas_axis, const float* meas_coords2,
@@ -956,31 +1345,25 @@ int mfb_ment_integrate(int d, const float* meas_coords, int nb_meas, int meas_ax
                        const float* proj2, const float* cx2, const float* cy2, const float* tables2, int k2, int bx,
                        int by, const float* mp2, float prior_neg_half_inv_s2, float prior_log_norm, float* pred,
                        void* stream) {
-  const bool kick = mp || mp2 || inv_mp;
-  MFB_CHECK_ARG(meas_coords && linv && (inv_mp || !kick) && pred && int_shape_host && int_first_host && int_step_host);
-  const int n_meas = meas_axis2 >= 0 ? 2 : 1;
-  MFB_CHECK_ARG(d >= 2 && d <= kMaxDim && n_int_axes == d - n_meas && n_int_axes >= 1);
-  MFB_CHECK_ARG(meas_axis >= 0 && meas_axis < d && nb_meas >= 1 && meas_axis2 < d && meas_axis2 != meas_axis);
-  MFB_CHECK_ARG(meas_axis2 < 0 || (meas_coords2 && nb_meas2 >= 1));
-  const Tables2D t2{k2, bx, by, proj2, cx2, cy2, tables2};
-  MFB_CHECK_ARG(tables_ok(k, b, proj, coords, tables, mp, t2, mp2, kick));
-  if (k == 0) b = 2;
-  const MentPrior pr{prior_neg_half_inv_s2, prior_log_norm};
-  const MentGrid grid = make_grid(n_int_axes, int_shape_host, int_first_host, int_step_host);
-  cudaStream_t st = (cudaStream_t)stream;
-#define MFB_CALL(DD)                                                                                                   \
-  launch_integrate<DD>(kick, meas_coords, nb_meas, meas_axis, meas_coords2, nb_meas2, meas_axis2, grid, linv, inv_mp, \
-                       proj, coords, tables, k, b, mp, t2, mp2, pr, pred, st)
-  switch (d) {
-    case 2: return MFB_CALL(2);
-    case 3: return MFB_CALL(3);
-    case 4: return MFB_CALL(4);
-    case 5: return MFB_CALL(5);
-    case 6: return MFB_CALL(6);
-    case 7: return MFB_CALL(7);
-    default: return MFB_CALL(8);
-  }
-#undef MFB_CALL
+  return ment_integrate(d, meas_coords, nb_meas, meas_axis, meas_coords2, nb_meas2, meas_axis2, n_int_axes,
+                        int_shape_host, int_first_host, int_step_host, linv, inv_mp,
+                        uniform_tables(proj, coords, tables, k, b, mp, proj2, cx2, cy2, tables2, k2, bx, by, mp2),
+                        prior_neg_half_inv_s2, prior_log_norm, pred, stream);
+}
+
+int mfb_ment_integrate_ragged(int d, const float* meas_coords, int nb_meas, int meas_axis, const float* meas_coords2,
+                              int nb_meas2, int meas_axis2, int n_int_axes, const int32_t* int_shape_host,
+                              const float* int_first_host, const float* int_step_host, const float* linv,
+                              const float* inv_mp, const float* proj, const float* coords, const float* tables, int k,
+                              const int32_t* offsets, int total, const float* mp, const float* proj2,
+                              const float* cx2, const float* cy2, const float* tables2, int k2,
+                              const int32_t* offsets2, const float* mp2, float prior_neg_half_inv_s2,
+                              float prior_log_norm, float* pred, void* stream) {
+  return ment_integrate(
+      d, meas_coords, nb_meas, meas_axis, meas_coords2, nb_meas2, meas_axis2, n_int_axes, int_shape_host,
+      int_first_host, int_step_host, linv, inv_mp,
+      ragged_tables(proj, coords, tables, k, offsets, total, mp, proj2, cx2, cy2, tables2, k2, offsets2, mp2),
+      prior_neg_half_inv_s2, prior_log_norm, pred, stream);
 }
 
 int64_t mfb_cdf_workspace_bytes(int64_t g) {
@@ -1047,24 +1430,22 @@ int mfb_cdf_sample(const double* cdf, int64_t g, const void* workspace, int d, c
   return launch_status();
 }
 
-int mfb_ment_mh(int d, const float* proj, const float* coords, const float* tables, int k, int b, const float* mp,
-                const float* proj2, const float* cx2, const float* cy2, const float* tables2, int k2, int bx, int by,
-                const float* mp2, float prior_neg_half_inv_s2, float prior_log_norm, uint64_t chain0, int64_t nchains,
-                const float* start, float start_scale, const float* chol, int64_t burnin, int64_t steps, int64_t thin,
-                uint64_t seed, float* out, int64_t* accepted, void* stream) {
-  const bool kick = mp || mp2;
+static int ment_mh(int d, const MentTables& t, float prior_neg_half_inv_s2, float prior_log_norm, uint64_t chain0,
+                   int64_t nchains, const float* start, float start_scale, const float* chol, int64_t burnin,
+                   int64_t steps, int64_t thin, uint64_t seed, float* out, int64_t* accepted, void* stream) {
+  const bool kick = t.mp || t.mp2;
   MFB_CHECK_ARG(out && chol && accepted && d >= 1 && d <= kMaxDim && nchains >= 0 && mh_steps_ok(burnin, steps, thin));
   MFB_CHECK_ARG(start || isfinite(start_scale));
   MFB_CHECK_ARG((uint64_t)nchains <= UINT64_MAX - chain0 && nchains <= INT64_MAX / (steps * d) &&
                 nchains <= (int64_t)INT32_MAX * kMentThreads);
-  const Tables2D t2{k2, bx, by, proj2, cx2, cy2, tables2};
-  MFB_CHECK_ARG(tables_ok(k, b, proj, coords, tables, mp, t2, mp2, kick));
+  MFB_CHECK_ARG(t.ok(kick));
   if (nchains == 0) return 0;
-  if (k == 0) b = 2;
   const MentPrior pr{prior_neg_half_inv_s2, prior_log_norm};
   const MhChains ch{chain0, nchains, start, start_scale, chol, burnin, steps, thin, seed};
   cudaStream_t st = (cudaStream_t)stream;
-#define MFB_CALL(DD) launch_mh<DD>(kick, proj, coords, tables, k, b, mp, t2, mp2, pr, ch, out, accepted, st)
+#define MFB_CALL(DD)                                                                                                   \
+  launch_mh<DD>(kick, t.ragged, t.proj, t.coords, t.tables, t.k, t.bins(), t.off, t.off2, t.mp, t.t2, t.mp2, pr, ch,  \
+                out, accepted, st)
   switch (d) {
     case 1: return MFB_CALL(1);
     case 2: return MFB_CALL(2);
@@ -1076,6 +1457,28 @@ int mfb_ment_mh(int d, const float* proj, const float* coords, const float* tabl
     default: return MFB_CALL(8);
   }
 #undef MFB_CALL
+}
+
+int mfb_ment_mh(int d, const float* proj, const float* coords, const float* tables, int k, int b, const float* mp,
+                const float* proj2, const float* cx2, const float* cy2, const float* tables2, int k2, int bx, int by,
+                const float* mp2, float prior_neg_half_inv_s2, float prior_log_norm, uint64_t chain0, int64_t nchains,
+                const float* start, float start_scale, const float* chol, int64_t burnin, int64_t steps, int64_t thin,
+                uint64_t seed, float* out, int64_t* accepted, void* stream) {
+  return ment_mh(d, uniform_tables(proj, coords, tables, k, b, mp, proj2, cx2, cy2, tables2, k2, bx, by, mp2),
+                 prior_neg_half_inv_s2, prior_log_norm, chain0, nchains, start, start_scale, chol, burnin, steps, thin,
+                 seed, out, accepted, stream);
+}
+
+int mfb_ment_mh_ragged(int d, const float* proj, const float* coords, const float* tables, int k,
+                       const int32_t* offsets, int total, const float* mp, const float* proj2, const float* cx2,
+                       const float* cy2, const float* tables2, int k2, const int32_t* offsets2, const float* mp2,
+                       float prior_neg_half_inv_s2, float prior_log_norm, uint64_t chain0, int64_t nchains,
+                       const float* start, float start_scale, const float* chol, int64_t burnin, int64_t steps,
+                       int64_t thin, uint64_t seed, float* out, int64_t* accepted, void* stream) {
+  return ment_mh(d,
+                 ragged_tables(proj, coords, tables, k, offsets, total, mp, proj2, cx2, cy2, tables2, k2, offsets2, mp2),
+                 prior_neg_half_inv_s2, prior_log_norm, chain0, nchains, start, start_scale, chol, burnin, steps, thin,
+                 seed, out, accepted, stream);
 }
 
 int mfb_mh_propose(const float* x, int64_t n, int d, uint64_t chain0, const float* start, float start_scale,

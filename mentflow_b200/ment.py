@@ -6,8 +6,10 @@ library: ``prob`` is one fused kernel over all measurements (the reference does 
 ->scipy->device round trip per measurement), sampling is a scan + inverse-CDF kernel, the
 predicted profile of the sampled particles is the fused projection+KDE kernel, and the table
 update is one elementwise kernel.  One- and two-dimensional screens (Histogram1D / Histogram2D:
-experiments/config/rec_nd_1d_ment.yaml, rec_nd_2d_ment.yaml) may be mixed; within each family the
-screens must have the same number of bins.
+experiments/config/rec_nd_1d_ment.yaml, rec_nd_2d_ment.yaml) of any size may be mixed, as in the reference: a
+family whose screens all have the same bins is passed as stacked tables, one whose sizes differ as concatenated
+tables with offsets (``ops.RaggedTables1D`` / ``ops.RaggedTables2D``), which the same kernels read in their ragged
+layout.
 
 Transfer maps are linear (``LinearTransform``, or a ``CompositeTransform`` of them) or a chain
 linear* -> MultipoleTransform (order 3, 4 or 5, normal or skew) -> linear* (experiments/rec_2d/nonlinear), in
@@ -146,7 +148,8 @@ class MENT:
     def _pack(self, device):
         """Static part of the kernel arguments: projection rows and bin centres of every table, the 1-D and
         the 2-D screens as two families; with a multipole kick anywhere in the model, the multipole rows of every
-        screen as well (order 0 behind linear maps)."""
+        screen as well (order 0 behind linear maps).  A family of equal sizes stacks its centres; one whose sizes
+        differ concatenates them and keeps the offsets of the ragged layout ("offsets", "offsets2")."""
         if self._packed is not None and self._packed["device"] == device:
             return self._packed
         slots1, proj1, coords1, mp1 = [], [], [], []
@@ -175,10 +178,19 @@ class MENT:
                 proj1.append(d.projection_vector(matrix, nd, device) if chain is None else vec[0])
                 mp1.append(mp[0] if chain is not None else None)
                 coords1.append(coords_from_edges(d.edges.to(torch.float32)).to(device))
-        for family in (coords1, cx2, cy2):
-            if len({int(c.shape[0]) for c in family}) > 1:
-                raise NotImplementedError("all screens of one kind in a MENT model must have the same number of bins")
         kicked = any(m is not None for m in mp1 + mp2)
+
+        def starts(sizes):
+            out = [0]
+            for n in sizes:
+                out.append(out[-1] + n)
+            return out
+
+        bins1 = [int(c.shape[0]) for c in coords1]
+        bins2 = [(int(x.shape[0]), int(y.shape[0])) for x, y in zip(cx2, cy2)]
+        offsets = starts(bins1) if len(set(bins1)) > 1 else None
+        offsets2 = ([starts(bx for bx, _ in bins2), starts(by for _, by in bins2), starts(bx * by for bx, by in bins2)]
+                    if len(set(bins2)) > 1 else None)
 
         def stack_mp(rows, shape):
             if not kicked or not rows:
@@ -186,30 +198,44 @@ class MENT:
             return torch.stack([m if m is not None else torch.zeros(shape, dtype=torch.float32, device=device)
                                 for m in rows]).contiguous()
 
+        def pack(family, ragged):
+            if not family:
+                return None
+            return (torch.cat(family) if ragged else torch.stack(family)).contiguous()
+
         self._packed = {"device": device, "slots1": slots1, "slots2": slots2,
                         "proj": torch.stack(proj1).contiguous() if proj1 else None,
-                        "coords": torch.stack(coords1).contiguous() if coords1 else None,
+                        "coords": pack(coords1, offsets is not None), "offsets": offsets,
                         "proj2": torch.stack(proj2).contiguous() if proj2 else None,
-                        "cx2": torch.stack(cx2).contiguous() if cx2 else None,
-                        "cy2": torch.stack(cy2).contiguous() if cy2 else None,
+                        "cx2": pack(cx2, offsets2 is not None), "cy2": pack(cy2, offsets2 is not None),
+                        "offsets2": offsets2,
                         "mp": stack_mp(mp1, (2 * nd + 4,)), "mp2": stack_mp(mp2, (2, 2 * nd + 4)),
                         "kicked": kicked, "inverse": {}}
         return self._packed
 
     def _groups(self, device):
         """(g1, g2) for ``ops.ment_prob``: the current tables of the two screen families, followed by their
-        multipole rows when the model has a kick."""
+        multipole rows when the model has a kick; a family whose sizes differ as ``ops.RaggedTables1D`` /
+        ``ops.RaggedTables2D`` of the concatenated tables."""
         pk = self._pack(device)
 
-        def stack(slots):
-            return torch.stack([self.lagrange_functions[i][j].values.to(device=device, dtype=torch.float32)
-                                for i, j in slots]).contiguous()
+        def tables(slots, ragged):
+            values = [self.lagrange_functions[i][j].values.to(device=device, dtype=torch.float32) for i, j in slots]
+            return (torch.cat([v.reshape(-1) for v in values]) if ragged else torch.stack(values)).contiguous()
 
-        g1 = (pk["proj"], pk["coords"], stack(pk["slots1"])) if pk["slots1"] else None
-        g2 = (pk["proj2"], pk["cx2"], pk["cy2"], stack(pk["slots2"])) if pk["slots2"] else None
-        if pk["kicked"]:
-            g1 = g1 + (pk["mp"],) if g1 is not None else None
-            g2 = g2 + (pk["mp2"],) if g2 is not None else None
+        g1 = g2 = None
+        if pk["slots1"]:
+            h = tables(pk["slots1"], pk["offsets"] is not None)
+            if pk["offsets"] is not None:
+                g1 = ops.RaggedTables1D(pk["proj"], pk["coords"], h, pk["offsets"], pk["mp"])
+            else:
+                g1 = (pk["proj"], pk["coords"], h) + ((pk["mp"],) if pk["kicked"] else ())
+        if pk["slots2"]:
+            h = tables(pk["slots2"], pk["offsets2"] is not None)
+            if pk["offsets2"] is not None:
+                g2 = ops.RaggedTables2D(pk["proj2"], pk["cx2"], pk["cy2"], h, pk["offsets2"], pk["mp2"])
+            else:
+                g2 = (pk["proj2"], pk["cx2"], pk["cy2"], h) + ((pk["mp2"],) if pk["kicked"] else ())
         return g1, g2
 
     def _inverse(self, index: int, device):
@@ -404,5 +430,7 @@ class MENT:
         for row in self.lagrange_functions:
             for lf in row:
                 lf.values = self.send(lf.values)
-                lf.coords = self.send(lf.coords)
+                # a 2-D screen's centres are one tensor per axis
+                lf.coords = ([self.send(c) for c in lf.coords] if isinstance(lf.coords, (list, tuple))
+                             else self.send(lf.coords))
         return self

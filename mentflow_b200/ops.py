@@ -8,8 +8,9 @@ thread, so nothing here caches streams or keeps global state).  Differentiable o
 from __future__ import annotations
 
 import ctypes
+import functools
 import math
-from typing import Optional
+from typing import NamedTuple, Optional, Sequence
 
 import torch
 
@@ -1032,31 +1033,150 @@ def _host_f32(values):
     return arr, ctypes.cast(arr, ctypes.c_void_p)
 
 
+class RaggedTables1D(NamedTuple):
+    """The 1-D screens when their tables differ in size: table k holds ``coords[offsets[k]:offsets[k + 1]]`` and
+    ``values[offsets[k]:offsets[k + 1]]``, at least 2 bins each.  proj (K, D), coords and values (T,), offsets: K + 1
+    HOST integers from 0 to T (a sequence or a CPU tensor), mp (K, 2D+4) the optional multipole rows."""
+    proj: torch.Tensor
+    coords: torch.Tensor
+    values: torch.Tensor
+    offsets: Sequence[int]
+    mp: Optional[torch.Tensor] = None
+
+
+class RaggedTables2D(NamedTuple):
+    """The 2-D screens when their tables differ in size: offsets2 holds three rows of K2 + 1 HOST integers, the start
+    of every table in cx, cy and values.  Table k has bx_k = offsets2[0][k+1] - offsets2[0][k] and by_k (row 1) >= 2
+    centres per axis and is ``values[offsets2[2][k]:offsets2[2][k+1]].view(bx_k, by_k)``, the tables back to back.
+    proj2 (K2, 2, D), cx, cy and values flat, mp2 (K2, 2, 2D+4) the optional multipole rows."""
+    proj2: torch.Tensor
+    cx: torch.Tensor
+    cy: torch.Tensor
+    values: torch.Tensor
+    offsets2: Sequence[Sequence[int]]
+    mp2: Optional[torch.Tensor] = None
+
+
+_INT32_MAX = 2 ** 31 - 1
+
+
+def _host_offsets(name: str, offsets, k: int, total: int):
+    """The offsets as a list after the checks of the ragged layout: k + 1 entries from 0 to ``total``, at least 2 bins
+    per table, within int32.  Returns (offsets, bins per table)."""
+    off = [int(v) for v in (offsets.tolist() if isinstance(offsets, torch.Tensor) else offsets)]
+    if len(off) != k + 1 or off[0] != 0 or off[-1] != total:
+        raise ValueError(f"{name}: {k + 1} offsets from 0 to {total} expected, got {len(off)} ending at "
+                         f"{off[-1] if off else None}")
+    if total > _INT32_MAX:
+        raise ValueError(f"{name}: {total} entries do not fit int32 offsets")
+    bins = [b - a for a, b in zip(off, off[1:])]
+    short = [i for i, b in enumerate(bins) if b < 2]
+    if short:
+        raise ValueError(f"{name}: every table needs at least 2 bins, table {short[0]} has {bins[short[0]]}")
+    return off, bins
+
+
+def _as_ragged1(g) -> tuple:
+    """(RaggedTables1D, host offsets) of a 1-D family; a uniform one (proj, coords (K,B), tables (K,B)[, mp]) is
+    expressed with offsets k B."""
+    if not isinstance(g, RaggedTables1D):
+        k, b = g[2].shape
+        g = RaggedTables1D(g[0], g[1].reshape(-1), g[2].reshape(-1), [i * b for i in range(k + 1)],
+                           g[3] if len(g) > 3 else None)
+    if g.coords.ndim != 1 or g.values.shape != g.coords.shape:
+        raise ValueError("ragged 1-D Lagrange tables: coords and values (T,) expected")
+    off, _ = _host_offsets("offsets", g.offsets, int(g.proj.shape[0]), int(g.coords.numel()))
+    return g, off
+
+
+def _as_ragged2(g) -> tuple:
+    """(RaggedTables2D, host offsets2 flattened) of a 2-D family; a uniform one is expressed with offsets
+    (k Bx, k By, k Bx By)."""
+    if not isinstance(g, RaggedTables2D):
+        k, bx, by = g[3].shape
+        g = RaggedTables2D(g[0], g[1].reshape(-1), g[2].reshape(-1), g[3].reshape(-1),
+                           [[i * n for i in range(k + 1)] for n in (bx, by, bx * by)], g[4] if len(g) > 4 else None)
+    k = int(g.proj2.shape[0])
+    if g.proj2.ndim != 3 or g.proj2.shape[1] != 2 or not all(t.ndim == 1 for t in (g.cx, g.cy, g.values)):
+        raise ValueError("ragged 2-D Lagrange tables: proj2 (K,2,D) and flat cx, cy, values expected")
+    rows = g.offsets2.tolist() if isinstance(g.offsets2, torch.Tensor) else list(g.offsets2)
+    if len(rows) != 3:
+        raise ValueError(f"offsets2: 3 rows of {k + 1} offsets expected, got {len(rows)} rows")
+    ox, bx = _host_offsets("offsets2[0]", rows[0], k, int(g.cx.numel()))
+    oy, by = _host_offsets("offsets2[1]", rows[1], k, int(g.cy.numel()))
+    ot = [0]
+    for nx, ny in zip(bx, by):
+        ot.append(ot[-1] + nx * ny)
+    if [int(v) for v in rows[2]] != ot or ot[-1] != g.values.numel():
+        raise ValueError(f"offsets2[2]: the tables of bx_k x by_k values back to back, {ot}, over values of "
+                         f"{g.values.numel()} entries expected")
+    if ot[-1] > _INT32_MAX:
+        raise ValueError(f"offsets2[2]: {ot[-1]} entries do not fit int32 offsets")
+    return g, ox + oy + ot
+
+
+@functools.lru_cache(maxsize=64)
+def _offsets_on(offsets: tuple, index: int) -> torch.Tensor:
+    return torch.tensor(offsets, dtype=torch.int32).to(torch.device("cuda", index))
+
+
+def _device_offsets(offsets: tuple, device) -> torch.Tensor:
+    """int32 offsets on ``device``, uploaded once per layout and GPU (a model's layout does not change between calls).
+    An unindexed "cuda" means the current device, resolved here, so that the cache never hands out another GPU's
+    copy."""
+    device = torch.device(device)
+    if device.type != "cuda":
+        raise RuntimeError(f"ragged MENT tables need a CUDA device (got {device}); there is no CPU fallback")
+    return _offsets_on(offsets, torch.cuda.current_device() if device.index is None else device.index)
+
+
 def _ment_tables(g1, g2, d: int, device, kick: bool = False):
-    """C-ABI arguments of the two table families in ABI order (proj, coords, tables, k, b, mp, proj2, cx, cy, tables2,
-    k2, bx, by, mp2), the tensors they point into, and whether the model has kicks.
-    g1 = (proj (K,D), coords (K,B), tables (K,B)[, mp (K,2D+4)]) or None,
-    g2 = (proj2 (K2,2,D), cx (K2,Bx), cy (K2,By), tables2 (K2,Bx,By)[, mp2 (K2,2,2D+4)]) or None.
+    """C-ABI arguments of the two table families in ABI order, the tensors they point into, whether the model has
+    kicks, and whether the call goes to the ragged entry points.
+    g1 = (proj (K,D), coords (K,B), tables (K,B)[, mp (K,2D+4)]), a RaggedTables1D, or None,
+    g2 = (proj2 (K2,2,D), cx (K2,Bx), cy (K2,By), tables2 (K2,Bx,By)[, mp2 (K2,2,2D+4)]), a RaggedTables2D, or None.
+    Uniform families give (proj, coords, tables, k, b, mp, proj2, cx, cy, tables2, k2, bx, by, mp2).  If either family
+    is ragged, both are passed in the ragged layout (a uniform family with offsets k B), as (proj, coords, tables, k,
+    offsets, total, mp, proj2, cx, cy, tables2, k2, offsets2, mp2), after the host checks of the offsets.
     The optional multipole rows have the layout of ``simulate.multipole_terms``, order 0 for the rows of linear maps.
     The model has kicks when either family carries rows or ``kick`` is set; then a family without rows gets order-0
     rows.  A linear model passes NULL for both."""
     keep = []
-    if g1 is not None:
-        proj, coords, tables = (_check_f32(n, t) for n, t in zip(("proj", "coords", "tables"), g1))
-        keep += [proj, coords, tables]
-        a1 = [_ptr(proj), _ptr(coords), _ptr(tables), tables.shape[0], tables.shape[1]]
+    ragged = isinstance(g1, RaggedTables1D) or isinstance(g2, RaggedTables2D)
+    if ragged:
+        if g1 is not None:
+            g1, off = _as_ragged1(g1)
+            proj, coords, tables = (_check_f32(n, t) for n, t in zip(("proj", "coords", "tables"), g1[:3]))
+            offsets = _device_offsets(tuple(off), device)
+            keep += [proj, coords, tables, offsets]
+            a1 = [_ptr(proj), _ptr(coords), _ptr(tables), proj.shape[0], _ptr(offsets), off[-1]]
+        else:
+            a1 = [None, None, None, 0, None, 0]
+        if g2 is not None:
+            g2, off2 = _as_ragged2(g2)
+            proj2, cx, cy, tab2 = (_check_f32(n, t) for n, t in zip(("proj2", "cx", "cy", "tables2"), g2[:4]))
+            offsets2 = _device_offsets(tuple(off2), device)
+            keep += [proj2, cx, cy, tab2, offsets2]
+            a2 = [_ptr(proj2), _ptr(cx), _ptr(cy), _ptr(tab2), proj2.shape[0], _ptr(offsets2)]
+        else:
+            a2 = [None, None, None, None, 0, None]
     else:
-        a1 = [None, None, None, 0, 2]
-    if g2 is not None:
-        proj2, cx, cy, tab2 = (_check_f32(n, t) for n, t in zip(("proj2", "cx", "cy", "tables2"), g2))
-        if proj2.ndim != 3 or proj2.shape[1] != 2 or tab2.shape != (proj2.shape[0], cx.shape[1], cy.shape[1]):
-            raise ValueError("2-D Lagrange tables: proj2 (K,2,D), cx (K,Bx), cy (K,By), tables2 (K,Bx,By) expected")
-        keep += [proj2, cx, cy, tab2]
-        a2 = [_ptr(proj2), _ptr(cx), _ptr(cy), _ptr(tab2), tab2.shape[0], tab2.shape[1], tab2.shape[2]]
-    else:
-        a2 = [None, None, None, None, 0, 0, 0]
-    mp1 = g1[3] if g1 is not None and len(g1) > 3 else None
-    mp2 = g2[4] if g2 is not None and len(g2) > 4 else None
+        if g1 is not None:
+            proj, coords, tables = (_check_f32(n, t) for n, t in zip(("proj", "coords", "tables"), g1))
+            keep += [proj, coords, tables]
+            a1 = [_ptr(proj), _ptr(coords), _ptr(tables), tables.shape[0], tables.shape[1]]
+        else:
+            a1 = [None, None, None, 0, 2]
+        if g2 is not None:
+            proj2, cx, cy, tab2 = (_check_f32(n, t) for n, t in zip(("proj2", "cx", "cy", "tables2"), g2))
+            if proj2.ndim != 3 or proj2.shape[1] != 2 or tab2.shape != (proj2.shape[0], cx.shape[1], cy.shape[1]):
+                raise ValueError("2-D Lagrange tables: proj2 (K,2,D), cx (K,Bx), cy (K,By), tables2 (K,Bx,By) expected")
+            keep += [proj2, cx, cy, tab2]
+            a2 = [_ptr(proj2), _ptr(cx), _ptr(cy), _ptr(tab2), tab2.shape[0], tab2.shape[1], tab2.shape[2]]
+        else:
+            a2 = [None, None, None, None, 0, 0, 0]
+    mp1 = g1[-1] if ragged and g1 is not None else (g1[3] if g1 is not None and len(g1) > 3 else None)
+    mp2 = g2[-1] if ragged and g2 is not None else (g2[4] if g2 is not None and len(g2) > 4 else None)
     kick = kick or mp1 is not None or mp2 is not None
     rows = []
     stride = 2 * d + 4
@@ -1073,7 +1193,7 @@ def _ment_tables(g1, g2, d: int, device, kick: bool = False):
                              f"got {tuple(mp.shape)}")
         keep.append(mp)
         rows.append(_ptr(mp))
-    return a1 + [rows[0]] + a2 + [rows[1]], keep, kick
+    return a1 + [rows[0]] + a2 + [rows[1]], keep, kick, ragged
 
 
 def ment_prob(x, g1, g2, neg_half_inv_s2: float, log_norm: float) -> torch.Tensor:
@@ -1082,11 +1202,11 @@ def ment_prob(x, g1, g2, neg_half_inv_s2: float, log_norm: float) -> torch.Tenso
     lib = _lib.load()
     x = _check_f32("x", x)
     g, d = x.shape
-    args, keep, _ = _ment_tables(g1, g2, d, x.device)
+    args, keep, _, ragged = _ment_tables(g1, g2, d, x.device)
     out = torch.empty(g, dtype=torch.float32, device=x.device)
+    fn = lib.mfb_ment_prob_ragged if ragged else lib.mfb_ment_prob
     with torch.cuda.device(x.device):
-        _lib.check(lib.mfb_ment_prob(_ptr(x), g, d, *args, float(neg_half_inv_s2), float(log_norm), _ptr(out),
-                                     _stream()), "ment_prob")
+        _lib.check(fn(_ptr(x), g, d, *args, float(neg_half_inv_s2), float(log_norm), _ptr(out), _stream()), "ment_prob")
     return out
 
 
@@ -1097,14 +1217,15 @@ def ment_prob_grid(shape, first_centre, step, g1, g2, neg_half_inv_s2, log_norm,
     g = 1
     for s_ in shape:
         g *= int(s_)
-    args, keep, _ = _ment_tables(g1, g2, d, device)
+    args, keep, _, ragged = _ment_tables(g1, g2, d, device)
     out = torch.empty(g, dtype=torch.float32, device=device)
     h1, p1 = _host_i32(shape)
     h2, p2 = _host_f32(first_centre)
     h3, p3 = _host_f32(step)
+    fn = lib.mfb_ment_prob_grid_ragged if ragged else lib.mfb_ment_prob_grid
     with torch.cuda.device(device):
-        _lib.check(lib.mfb_ment_prob_grid(d, p1, p2, p3, *args, float(neg_half_inv_s2), float(log_norm), _ptr(out),
-                                          _stream()), "ment_prob_grid")
+        _lib.check(fn(d, p1, p2, p3, *args, float(neg_half_inv_s2), float(log_norm), _ptr(out), _stream()),
+                   "ment_prob_grid")
     return out
 
 
@@ -1123,7 +1244,7 @@ def ment_integrate(d, meas_coords, meas_axis, meas_coords2, meas_axis2, int_shap
     if meas_axis2 >= 0:
         meas_coords2 = _check_f32("meas_coords2", meas_coords2)
         nb2 = meas_coords2.shape[0]
-    args, keep, kick = _ment_tables(g1, g2, d, minv.device, kick=inv_mp is not None)
+    args, keep, kick, ragged = _ment_tables(g1, g2, d, minv.device, kick=inv_mp is not None)
     if kick:
         if inv_mp is None:
             inv_mp = torch.zeros(4 * d + 2, dtype=torch.float32, device=minv.device)
@@ -1135,11 +1256,11 @@ def ment_integrate(d, meas_coords, meas_axis, meas_coords2, meas_axis2, int_shap
     h2, p2 = _host_f32(int_first)
     h3, p3 = _host_f32(int_step)
     mc2 = _ptr(meas_coords2) if meas_axis2 >= 0 else None
+    fn = lib.mfb_ment_integrate_ragged if ragged else lib.mfb_ment_integrate
     with torch.cuda.device(minv.device):
-        _lib.check(lib.mfb_ment_integrate(d, _ptr(meas_coords), nb, int(meas_axis), mc2, nb2, int(meas_axis2),
-                                          len(int_shape), p1, p2, p3, _ptr(minv), _ptr(inv_mp), *args,
-                                          float(neg_half_inv_s2), float(log_norm), _ptr(pred), _stream()),
-                   "ment_integrate")
+        _lib.check(fn(d, _ptr(meas_coords), nb, int(meas_axis), mc2, nb2, int(meas_axis2), len(int_shape), p1, p2, p3,
+                      _ptr(minv), _ptr(inv_mp), *args, float(neg_half_inv_s2), float(log_norm), _ptr(pred),
+                      _stream()), "ment_integrate")
     return pred
 
 
@@ -1194,13 +1315,14 @@ def ment_mh(g1, g2, neg_half_inv_s2: float, log_norm: float, d: int, chain0: int
         raise ValueError(f"chol must have shape ({d}, {d}), got {tuple(chol.shape)}")
     start = _mh_start(start, d)
     lib = _lib.load()
-    args, keep, _ = _ment_tables(g1, g2, d, device)
+    args, keep, _, ragged = _ment_tables(g1, g2, d, device)
     out = torch.empty((int(nchains) * int(steps), d), dtype=torch.float32, device=device)
     accepted = torch.zeros(1, dtype=torch.int64, device=device)
+    fn = lib.mfb_ment_mh_ragged if ragged else lib.mfb_ment_mh
     with torch.cuda.device(device):
-        _lib.check(lib.mfb_ment_mh(d, *args, float(neg_half_inv_s2), float(log_norm), int(chain0), int(nchains),
-                                   _ptr(start), float(start_scale), _ptr(chol), int(burnin), int(steps), int(thin),
-                                   int(seed) & (2 ** 64 - 1), _ptr(out), _ptr(accepted), _stream()), "ment_mh")
+        _lib.check(fn(d, *args, float(neg_half_inv_s2), float(log_norm), int(chain0), int(nchains), _ptr(start),
+                      float(start_scale), _ptr(chol), int(burnin), int(steps), int(thin), int(seed) & (2 ** 64 - 1),
+                      _ptr(out), _ptr(accepted), _stream()), "ment_mh")
     return out, accepted
 
 
